@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the CPU oracle port, same model / data / optimizer
+    python bench.py ... --dump-outputs DIR                   # + the outputs of the last timed step as DIR/*.npy
 
 Workloads
   rr      (default, BASELINE.json configs[1]) graph_transformer_optimized (D=256, L=2, H=2, k_pe=16), BPR loss,
@@ -60,6 +61,7 @@ WORKLOADS = {
     "scaled": {"items": 1_000_000, "label": "graph_transformer_optimized training step (fwd+BPR+bwd+AdamW), 1M items / "
                                             "20M edges, Yoochoose-shaped sessions"},
 }
+DUMP_ROWS, DUMP_MAX_BYTES = 8192, 64 << 20     # --dump-outputs: rows kept of a larger array, bytes in all
 
 
 def parse_args():
@@ -82,6 +84,11 @@ def parse_args():
     ap.add_argument("--sweep-batches", type=str, default="32,1024,16384,65536,120436",
                     help="extra device-resident measurements at these batch sizes (rank 0, 1 GPU; '' = off)")
     ap.add_argument("--scaled-sessions", type=int, default=8_000_000, help="sessions of the scaled workload")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps of `value`, write what the last of them computed as DIR/<name>.npy: "
+                         "the loss, the session embeddings, every parameter after the optimizer step, the dense "
+                         f"gradients and the BatchNorm running statistics; an array of more than {DUMP_ROWS} rows as "
+                         "a fixed, seeded sample of its rows (rank 0, b200 arm)")
     return ap.parse_args()
 
 
@@ -217,6 +224,29 @@ def make_host_batches(data, edge_keys, first_session, batch, count, seed, pin):
         arrays["negatives"] = sample_negatives_host(rng, arrays["members"], data.num_items, NUM_NEG)
         out.append(HostBatch(arrays, pin))
     return out
+
+
+def dump_outputs(path, model, last):
+    """--dump-outputs: the step's outputs as float32 / float64 .npy files; inputs are seeded, so two builds given the
+    same arguments can be compared file by file."""
+    arrays = {"loss": last["loss"], "session_embeddings": last["session_embeddings"]}
+    for name, p in model.named_parameters():
+        arrays[f"param.{name}"] = p
+        if p.grad is not None:
+            arrays[f"grad.{name}"] = p.grad
+    arrays.update({f"buffer.{name}": b for name, b in model.named_buffers() if "running" in name})
+    out = {}
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy() if t.dtype != torch.float64 else t.detach().cpu().numpy()
+        if a.ndim and a.shape[0] > DUMP_ROWS:
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], DUMP_ROWS, replace=False))]
+        out[name] = a
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes (limit {DUMP_MAX_BYTES})")
+    Path(path).mkdir(parents=True, exist_ok=True)
+    for name, a in out.items():
+        np.save(Path(path) / f"{name}.npy", a)
 
 
 def cached_pe(num_items):
@@ -388,11 +418,13 @@ def run_b200(args, rank, world_size, local_rank):
     # forward + BPR loss + backward through the C++ step driver (etpgt_gt_step_run: the same kernels as the
     # per-operator autograd path, bit-identical results, one host call); ETPGT_BENCH_AUTOGRAD=1 times that path
     fused = None if os.environ.get("ETPGT_BENCH_AUTOGRAD") else FusedTrainStep(model, "bpr")
+    last = {}       # what the latest step handed its caller besides the updated model (for --dump-outputs)
 
     def step(batch):
         opt.zero_grad()
         if fused is not None:
             loss = fused(batch, total_sessions=total_sessions)[0]
+            sess = fused.session_embeddings
             if distributed and peer is None:
                 fused.allreduce_gradients()      # NCCL variant; the peer exchange is part of opt.step()
         else:
@@ -403,6 +435,7 @@ def run_b200(args, rank, world_size, local_rank):
             if distributed and peer is None:
                 parallel.allreduce_gradients(params)
         opt.step()
+        last["loss"], last["session_embeddings"] = loss, sess
         return loss
 
     def sync():
@@ -559,6 +592,8 @@ def run_b200(args, rank, world_size, local_rank):
         _lib.reset_launch_count()
         ms_total = timed(value_step, args.steps)
         launches = _lib.launch_count()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, model, last)
         drop_pending()
         value = total_sessions * args.steps / (ms_total / 1e3)
         # ---- end to end (e2e): host batches (rr) / host session ids + device batch build (scaled)
@@ -1028,6 +1063,8 @@ def main():
     world_size = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("bench.py: --dump-outputs writes the outputs of the b200 arm only")
         run_reference(args, rank)
         return
     if world_size == 1 and args.gpus > 1:

@@ -26,6 +26,9 @@ sys.path.insert(0, "/root/reference")
 
 from torch_geometric.data import Batch, Data  # noqa: E402
 
+sys.path.insert(0, str(ROOT / "tests"))
+from golden_util import compact  # noqa: E402
+
 from etpgt.model import (  # noqa: E402
     create_gat,
     create_graph_transformer,
@@ -61,7 +64,9 @@ def random_sessions_batch(rng, num_sessions, num_items, min_nodes=2, max_nodes=7
     return Batch.from_data_list(graphs)
 
 
-def run_model_case(name, factory, kwargs, batch, targets, negatives, loss_type, seed, pe=None):
+def run_model_case(name, factory, kwargs, batch, targets, negatives, loss_type, seed, pe=None, compact_pe_seed=None):
+    """compact_pe_seed: `pe` is randn(num_items, k, seed compact_pe_seed).abs(); the fixture is written compact
+    (tests/golden_util.py: the state as seeds + digest, large gradients sampled) to stay under 1 MB."""
     torch.manual_seed(seed)
     model = factory(**kwargs)
     if pe is not None:
@@ -106,6 +111,8 @@ def run_model_case(name, factory, kwargs, batch, targets, negatives, loss_type, 
                 if "running" in bname:
                     out["after/" + bname] = npy(b).astype(np.float32)
     torch.set_default_dtype(torch.float32)
+    if compact_pe_seed is not None:
+        out = compact(out, seed, compact_pe_seed)
     np.savez_compressed(OUT / f"{name}.npz", **out)
     print(f"wrote {name}.npz: N={batch.x.numel()} E={batch.edge_index.size(1)} loss={float(out['loss_f64']):.6f}")
 
@@ -136,7 +143,8 @@ def model_cases():
     neg = torch.tensor(rng.integers(1, items, size=(32, 5)))
     prod = dict(num_items=items, embedding_dim=256, hidden_dim=256, num_layers=2, num_heads=2, dropout=0.0)
     pe = torch.randn(items, 16, generator=torch.Generator().manual_seed(7)).abs()
-    run_model_case("gt_opt_b32", create_graph_transformer_optimized, prod, b32, tgt, neg, "bpr", 11, pe)
+    run_model_case("gt_opt_b32", create_graph_transformer_optimized, prod, b32, tgt, neg, "bpr", 11, pe,
+                   compact_pe_seed=7)
     mid_pe = dict(num_items=items, embedding_dim=64, hidden_dim=64, num_layers=2, num_heads=2, dropout=0.0)
     run_model_case("gt_opt_b32_dual", create_graph_transformer_optimized, mid_pe, b32, tgt, neg, "dual", 12, pe)
 

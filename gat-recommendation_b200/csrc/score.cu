@@ -24,11 +24,15 @@ struct Cand { float val; int32_t idx; };
 // ascending id order.  Each session keeps a sorted (desc) k-list in shared memory; a candidate
 // enters only if it is strictly greater than the current k-th value, so equal scores keep the
 // earlier (lower) id.
-template <int DIM>
+// EXCL: `excl` [batch, excl_width] lists ids each row must not receive (ascending; ids outside the
+// scored range are ignored).  Every register-blocked row keeps a cursor into its list, started at the
+// lower bound of the chunk's first id and advanced as the scan passes the listed ids.
+template <int DIM, bool EXCL>
 __global__ void __launch_bounds__(kThreads)
 score_topk_f32_kernel(const float* __restrict__ sess, const float* __restrict__ table, int64_t batch,
                       int64_t num_items, int k, int64_t chunk, int64_t id_base, int parts,
-                      float* __restrict__ cand_val, int64_t* __restrict__ cand_idx) {
+                      float* __restrict__ cand_val, int64_t* __restrict__ cand_idx,
+                      const int64_t* __restrict__ excl, int64_t excl_width) {
   using G = RowGeom<DIM>;
   constexpr int V = G::V, LPN = G::LPN;
   constexpr int GROUPS_PER_CTA = (kThreads / 32) * G::GROUPS;
@@ -55,6 +59,23 @@ score_topk_f32_kernel(const float* __restrict__ sess, const float* __restrict__ 
   }
   __syncwarp();
   int filled[kRowsPerGroup] = {0, 0, 0, 0};
+  const int64_t* ex_next[kRowsPerGroup];   // EXCL: the row's next listed id >= the scan position
+  const int64_t* ex_end[kRowsPerGroup];
+  if (EXCL) {
+#pragma unroll
+    for (int r = 0; r < kRowsPerGroup; ++r) {
+      const int64_t row = row0 + r < batch ? row0 + r : batch - 1;
+      const int64_t* ids = excl + row * excl_width;
+      int64_t lo = 0, hi = excl_width;
+      while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (ids[mid] < id_base + begin) lo = mid + 1;
+        else hi = mid;
+      }
+      ex_next[r] = ids + lo;
+      ex_end[r] = ids + excl_width;
+    }
+  }
 
   for (int64_t item = begin; item < end; ++item) {
     float4 e[V];
@@ -66,8 +87,15 @@ score_topk_f32_kernel(const float* __restrict__ sess, const float* __restrict__ 
 #pragma unroll
       for (int v = 0; v < V; ++v) part += dot4(s[r][v], e[v]);
       const float sc = group_sum<LPN>(part);
+      bool listed = false;   // uniform within the lane group (one row, one item)
+      if (EXCL) {
+        while (ex_next[r] < ex_end[r] && *ex_next[r] <= id_base + item) {
+          listed = listed || *ex_next[r] == id_base + item;
+          ++ex_next[r];
+        }
+      }
       // enters while the list is not full, or when strictly better than the k-th entry
-      if (filled[r] < k || sc > thr[r]) {
+      if (!listed && (filled[r] < k || sc > thr[r])) {
         if (lig == 0) {
           int t = filled[r] < k ? filled[r] : k - 1;
           while (t > 0 && mine[r][t - 1].val < sc) { mine[r][t] = mine[r][t - 1]; --t; }
@@ -279,13 +307,22 @@ extern "C" int etpgt_topk_merge(const float* cand_val, const int64_t* cand_idx, 
   return ETPGT_OK;
 }
 
-extern "C" int etpgt_score_topk_f32(const float* sess, const float* table, int64_t batch, int64_t num_items, int dim,
-                                    int k, int64_t id_base, float* top_val, int64_t* top_idx, void* ws,
-                                    size_t ws_bytes, etpgt_stream_t stream_) {
+namespace {
+
+// The scorer behind etpgt_score_topk_f32 (excl == nullptr) and etpgt_score_topk_f32_exclude (k_any: k may exceed the
+// eligible items, whose missing slots become (-inf, INT64_MAX) sentinels).
+int score_topk_f32_run(const float* sess, const float* table, int64_t batch, int64_t num_items, int dim, int k,
+                       int64_t id_base, float* top_val, int64_t* top_idx, const int64_t* excl, int64_t excl_width,
+                       bool k_any, void* ws, size_t ws_bytes, etpgt_stream_t stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   ETPGT_REQUIRE(supported_dim(dim), "score_topk: unsupported dim %d", dim);
   ETPGT_REQUIRE(batch >= 0 && num_items >= 1, "score_topk: bad sizes");
-  ETPGT_REQUIRE(k >= 1 && k <= kMaxK && k <= num_items, "score_topk: k=%d must be in [1, min(%d, num_items)]", k, kMaxK);
+  if (k_any) {
+    ETPGT_REQUIRE(k >= 1 && k <= kMaxK, "score_topk: k=%d must be in [1, %d]", k, kMaxK);
+  } else {
+    ETPGT_REQUIRE(k >= 1 && k <= kMaxK && k <= num_items, "score_topk: k=%d must be in [1, min(%d, num_items)]", k,
+                  kMaxK);
+  }
   if (ws_bytes < etpgt_score_topk_workspace_bytes(batch, num_items, dim, k)) {
     set_error("score_topk: workspace too small");
     return ETPGT_EWORKSPACE;
@@ -296,18 +333,43 @@ extern "C" int etpgt_score_topk_f32(const float* sess, const float* table, int64
   const size_t m = (size_t)batch * p.parts * k;
   float* cand_val = w.take<float>(m);
   int64_t* cand_idx = w.take<int64_t>(m);
-#define CALL(D)                                                                                          \
-  {                                                                                                      \
-    const size_t smem = (size_t)(kThreads / 32) * RowGeom<D>::GROUPS * kRowsPerGroup * k * sizeof(Cand); \
-    if (smem > 48 * 1024)                                                                                \
-      cudaFuncSetAttribute(score_topk_f32_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-    score_topk_f32_kernel<D><<<dim3(p.parts, p.row_blocks), kThreads, smem, stream>>>(                    \
-        sess, table, batch, num_items, k, p.chunk, id_base, p.parts, cand_val, cand_idx);                \
+#define CALL2(D, EX)                                                                                         \
+  {                                                                                                          \
+    const size_t smem = (size_t)(kThreads / 32) * RowGeom<D>::GROUPS * kRowsPerGroup * k * sizeof(Cand);     \
+    if (smem > 48 * 1024)                                                                                    \
+      cudaFuncSetAttribute(score_topk_f32_kernel<D, EX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+    score_topk_f32_kernel<D, EX><<<dim3(p.parts, p.row_blocks), kThreads, smem, stream>>>(                    \
+        sess, table, batch, num_items, k, p.chunk, id_base, p.parts, cand_val, cand_idx, excl, excl_width);  \
+  }
+#define CALL(D)                             \
+  {                                         \
+    if (excl != nullptr) CALL2(D, true)     \
+    else CALL2(D, false)                    \
   }
   ETPGT_DISPATCH_DIM(dim, CALL)
 #undef CALL
+#undef CALL2
   ETPGT_CHECK_LAUNCH("score_topk_f32");
   return etpgt_topk_merge(cand_val, cand_idx, batch, p.parts, k, top_val, top_idx, stream_);
+}
+
+}  // namespace
+
+extern "C" int etpgt_score_topk_f32(const float* sess, const float* table, int64_t batch, int64_t num_items, int dim,
+                                    int k, int64_t id_base, float* top_val, int64_t* top_idx, void* ws,
+                                    size_t ws_bytes, etpgt_stream_t stream) {
+  return score_topk_f32_run(sess, table, batch, num_items, dim, k, id_base, top_val, top_idx, nullptr, 0, false, ws,
+                            ws_bytes, stream);
+}
+
+extern "C" int etpgt_score_topk_f32_exclude(const float* sess, const float* table, int64_t batch, int64_t num_items,
+                                            int dim, int k, int64_t id_base, float* top_val, int64_t* top_idx,
+                                            const int64_t* exclude, int64_t exclude_width, void* ws, size_t ws_bytes,
+                                            etpgt_stream_t stream) {
+  ETPGT_REQUIRE(exclude_width >= 0, "score_topk_exclude: negative exclude_width");
+  ETPGT_REQUIRE(exclude_width == 0 || batch == 0 || exclude != nullptr, "score_topk_exclude: null exclude list");
+  return score_topk_f32_run(sess, table, batch, num_items, dim, k, id_base, top_val, top_idx,
+                            exclude_width > 0 ? exclude : nullptr, exclude_width, true, ws, ws_bytes, stream);
 }
 
 extern "C" int etpgt_topk_metrics(const int64_t* top_idx, const int64_t* targets, int64_t batch, int k_stride, int k,

@@ -50,6 +50,15 @@
 // ~215), reads only those (two pieces per warp step, one score per lane) and picks the exact top-k by (score desc,
 // id asc) with a bitonic sort of 64-bit keys in registers.  Rows whose slot buffer overflowed (adversarial score
 // orders) are recomputed exactly by a CUDA-core fallback kernel, so the result is always exact.
+//
+// Exclusion (etpgt_score_topk_bf16_exclude, the EXCL variant): every row may name item ids it must not receive (the
+// session's own items, the padding id).  The epilogue sets those columns to -inf BEFORE the piece maxima are taken:
+// an excluded item holding one of the K best piece maxima would otherwise raise the threshold above the K-th best
+// ELIGIBLE score, and the pieces that hold the eligible top-k would never be dumped.  Each epilogue thread walks its
+// row's ascending list with one cursor; per 32-column chunk that costs one compare, and only the few chunks that
+// contain an excluded id (about 6 per row at 82k items) take the masking branch.  Dumped pieces carry the -inf, the
+// select kernel never keeps a -inf score and the fallback kernel skips the listed ids, so a row with fewer than k
+// eligible items ends in (-inf, INT64_MAX) sentinels.
 #include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -130,6 +139,29 @@ struct Schedule {
   }
 };
 
+// Exclusion lists: ids [batch, width], each row ascending (duplicates allowed); ids outside [id_base, id_base +
+// num_items) are ignored, so an item shard takes the global list unchanged and -1 pads a row.
+struct Exclusion {
+  const int64_t* ids;
+  int64_t width;
+  int64_t id_base;
+};
+constexpr int64_t kMaxExcludeWidth = 16384;   // the fallback kernel stages a row's list in shared memory
+
+// One epilogue thread's cursor into its row's list.  Only the next entry's column (relative to the thread's range;
+// INT_MAX once the list is used up) stays in a register: the hot loop compares against it once per chunk.  The rest
+// is read on the rare masking path only, so it lives in shared memory (in registers it made ptxas spill).
+struct ExclCursor {
+  const int64_t* next;
+  int64_t base;   // id of the range's column 0
+  int left;       // entries from `next` on
+};
+
+__device__ __forceinline__ int excl_col(int64_t id, int64_t base) {
+  const int64_t c = id - base;   // >= 0: ids below the range were skipped by a lower bound
+  return c < (int64_t)INT_MAX ? (int)c : INT_MAX;
+}
+
 // Per-row state of the piece-dump epilogue (one thread = one session row = one TMEM lane, one column half).
 template <int KCAP>
 struct RowState {
@@ -143,18 +175,34 @@ struct RowState {
 //   slot_first / slot_step: this warp fills the slot buffer upwards from 0 or downwards from cap - 1
 // (The hot loop has to stay inside the instruction cache: with four inlined copies of chunk + merge ncu showed 1.8
 // "no instruction" stall cycles per issued instruction; the merge exists once per kernel now.)
-template <int KCAP>
+template <int KCAP, bool EXCL>
 __device__ __forceinline__ void chunk_hits(const uint32_t (&raw)[CHUNK], RowState<KCAP>& st, int col,
                                            int limit_rel /* real columns left from this chunk on */,
                                            float* my_scores, int2* my_meta, int cap, int slot_first, int slot_step,
                                            uint32_t my_pending,
-                                           float thr_other /* a little stale at worst: still a valid bound */) {
+                                           float thr_other /* a little stale at worst: still a valid bound */,
+                                           int& ex_col, ExclCursor* ex) {
   float v[CHUNK];
 #pragma unroll
   for (int j = 0; j < CHUNK; ++j) v[j] = __uint_as_float(raw[j]);
   if (limit_rel < CHUNK) {  // only the table's last tile: columns past the end never qualify
 #pragma unroll
     for (int j = 0; j < CHUNK; ++j) v[j] = j < limit_rel ? v[j] : -INFINITY;
+  }
+  if (EXCL && ex_col < col + CHUNK) {   // rare: the row's next excluded id lies in (or before) this chunk
+    const int64_t* next = ex->next;
+    const int64_t base = ex->base;
+    int left = ex->left;
+    do {
+      const int e = ex_col - col;         // < 0: an id among another column part's columns, nothing to mask here
+#pragma unroll
+      for (int j = 0; j < CHUNK; ++j) v[j] = j == e ? -INFINITY : v[j];   // a select, no dynamic register index
+      ++next;
+      --left;
+      ex_col = left > 0 ? excl_col(*next, base) : INT_MAX;
+    } while (ex_col < col + CHUNK);
+    ex->next = next;
+    ex->left = left;
   }
   float g[8];
 #pragma unroll
@@ -216,12 +264,13 @@ __device__ __forceinline__ void merge_pending(RowState<KCAP>& st, uint32_t my_pe
   st_shared_f32(thr_own_addr, st.thr);
 }
 
-// NUM_KB = DIM / 64; KCAP = piece maxima tracked per row and column part (>= k); PAIR = CTA pairs; CP = column parts
-template <int NUM_KB, int KCAP, bool PAIR, int CP>
+// NUM_KB = DIM / 64; KCAP = piece maxima tracked per row and column part (>= k); PAIR = CTA pairs; CP = column parts;
+// EXCL = the rows' exclusion lists are applied (`excl` is ignored otherwise)
+template <int NUM_KB, int KCAP, bool PAIR, int CP, bool EXCL>
 __global__ void __launch_bounds__(threads_for(CP), 1)
 score_dump_tc_kernel(const __grid_constant__ CUtensorMap map_sess, const __grid_constant__ CUtensorMap map_items,
                      int64_t batch, int64_t num_items, int stages, Schedule sch, DumpBuffers dump,
-                     int pending_merge /* <= kPendingMerge */) {
+                     int pending_merge /* <= kPendingMerge */, Exclusion excl) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
   constexpr int LOAD_N = PAIR ? BLOCK_N / 2 : BLOCK_N;          // item rows this CTA loads per k-block
@@ -366,6 +415,21 @@ score_dump_tc_kernel(const __grid_constant__ CUtensorMap map_sess, const __grid_
     int cap = dump.cap_sub, merge_at = pending_merge;
     int slot_first = (cpart & 1) ? dump.cap_sub - 1 : 0, slot_step = (cpart & 1) ? -1 : 1;
     asm volatile("" : "+r"(cap), "+r"(merge_at), "+r"(slot_first), "+r"(slot_step));
+    // exclusion cursor: starts at the lower bound of the range's first id in the row's list
+    ExclCursor* ex = reinterpret_cast<ExclCursor*>(bars + 1) + (threadIdx.x - 64);
+    int ex_col = INT_MAX;
+    if (EXCL && live) {
+      const int64_t base = excl.id_base + tile_begin * BLOCK_N;
+      const int64_t* ids = excl.ids + grow * excl.width;
+      int lo = 0, hi = (int)excl.width;
+      while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (ids[mid] < base) lo = mid + 1;
+        else hi = mid;
+      }
+      *ex = ExclCursor{ids + lo, base, (int)excl.width - lo};
+      ex_col = lo < excl.width ? excl_col(ids[lo], base) : INT_MAX;
+    }
     for (int t = 0; t < num_tiles; ++t) {
       const int acc = t & 1;
       const uint32_t acc_phase = (uint32_t)(t >> 1) & 1;
@@ -393,7 +457,8 @@ score_dump_tc_kernel(const __grid_constant__ CUtensorMap map_sess, const __grid_
 #pragma unroll
       for (int c = 0; c < NBUF; ++c) tmem_ld_wait(raw[c]);
       if (NCH > NBUF) {
-        chunk_hits<KCAP>(raw[0], st, col0, limit, my_scores, my_meta, cap, slot_first, slot_step, my_pending, thr_other);
+        chunk_hits<KCAP, EXCL>(raw[0], st, col0, limit, my_scores, my_meta, cap, slot_first, slot_step, my_pending,
+                               thr_other, ex_col, ex);
         tmem_ld_32x32(taddr + (uint32_t)(NBUF * CHUNK), raw[0]);
       }
       tc_fence_before();
@@ -407,8 +472,8 @@ score_dump_tc_kernel(const __grid_constant__ CUtensorMap map_sess, const __grid_
       merge_pending<KCAP>(st, my_pending, thr_own_addr, merge_at);
 #pragma unroll
       for (int c = NCH > NBUF ? 1 : 0; c < NCH; ++c)
-        chunk_hits<KCAP>(raw[c % NBUF], st, col0 + c * CHUNK, limit - c * CHUNK, my_scores, my_meta, cap, slot_first,
-                         slot_step, my_pending, thr_other);
+        chunk_hits<KCAP, EXCL>(raw[c % NBUF], st, col0 + c * CHUNK, limit - c * CHUNK, my_scores, my_meta, cap,
+                               slot_first, slot_step, my_pending, thr_other, ex_col, ex);
     }
     merge_pending<KCAP>(st, my_pending, thr_own_addr, 1);   // what is still waiting: the final threshold
     if (live) {
@@ -520,7 +585,7 @@ score_select_kernel(DumpBuffers dump, int64_t batch, Schedule sch, int k, int64_
         }
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
-          const bool keep = v[u] >= tau && v[u] > -INFINITY;   // -inf marks columns past the end of the table
+          const bool keep = v[u] >= tau && v[u] > -INFINITY;   // -inf: past the table's end, or an excluded id
           const unsigned mask = __ballot_sync(0xffffffffu, keep);
           if (keep) {
             const int pos = n_surv + __popc(mask & ((1u << lane) - 1));
@@ -614,14 +679,27 @@ score_select_kernel(DumpBuffers dump, int64_t batch, Schedule sch, int k, int64_
 // Exact CUDA-core recomputation of the rows flagged in `redo` (slot-buffer or tie overflow): one CTA
 // per row, every thread scores a strided share of the items (fp32 accumulation of the same bf16
 // operands) and keeps a private sorted k-list; lists are merged through shared memory.
+// EXCL: the row's exclusion list is staged in shared memory and an item that would enter a list is
+// looked up there first (a binary search; rare once the lists have filled).
 constexpr int kRedoThreads = 256;
 
+__device__ __forceinline__ bool listed(const int64_t* ids, int n, int64_t id) {
+  int lo = 0, hi = n;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (ids[mid] < id) lo = mid + 1;
+    else hi = mid;
+  }
+  return lo < n && ids[lo] == id;
+}
+
+template <bool EXCL>
 __global__ void __launch_bounds__(kRedoThreads)
 score_redo_kernel(const __nv_bfloat16* __restrict__ sess, const __nv_bfloat16* __restrict__ table, int64_t batch,
                   int64_t num_items, int dim, int k, int64_t id_base, const int32_t* __restrict__ redo,
                   float* __restrict__ top_val, int64_t* __restrict__ top_idx, const int64_t* __restrict__ targets,
-                  int32_t* __restrict__ hit_pos) {
-  extern __shared__ float redo_smem[];       // session row [dim], then lists
+                  int32_t* __restrict__ hit_pos, Exclusion excl) {
+  extern __shared__ float redo_smem[];       // session row [dim], then lists, then (EXCL) the row's exclusion list
   // a small persistent grid; the flags of kRedoThreads rows are read at once, so rows that need no
   // recomputation (normally all of them) cost one coalesced load per 256 rows
   __shared__ int32_t s_flag[kRedoThreads];
@@ -641,6 +719,9 @@ score_redo_kernel(const __nv_bfloat16* __restrict__ sess, const __nv_bfloat16* _
   float* mv = l_val + threadIdx.x * k;
   int32_t* mi = l_idx + threadIdx.x * k;
   for (int t = 0; t < k; ++t) { mv[t] = -INFINITY; mi[t] = INT32_MAX; }
+  int64_t* s_excl = reinterpret_cast<int64_t*>(l_idx + kRedoThreads * k);   // 8-byte aligned: dim % 64 == 0
+  if (EXCL)
+    for (int64_t i = threadIdx.x; i < excl.width; i += kRedoThreads) s_excl[i] = excl.ids[row * excl.width + i];
   __syncthreads();
   for (int64_t item = threadIdx.x; item < num_items; item += kRedoThreads) {
     const __nv_bfloat16* e = table + item * dim;
@@ -650,7 +731,8 @@ score_redo_kernel(const __nv_bfloat16* __restrict__ sess, const __nv_bfloat16* _
       acc = fmaf(s_row[d], p.x, acc);
       acc = fmaf(s_row[d + 1], p.y, acc);
     }
-    if (acc > mv[k - 1]) {  // ascending ids per thread: strict '>' keeps the lower id
+    if (acc > mv[k - 1] && !(EXCL && listed(s_excl, (int)excl.width, id_base + item))) {
+      // ascending ids per thread: strict '>' keeps the lower id
       int t = k - 1;
       while (t > 0 && mv[t - 1] < acc) { mv[t] = mv[t - 1]; mi[t] = mi[t - 1]; --t; }
       mv[t] = acc;
@@ -819,17 +901,26 @@ extern "C" size_t etpgt_score_topk_bf16_workspace_bytes(int64_t batch, int64_t n
          2 * align_up(kMaxColParts * units * sizeof(float)) + 2 * align_up((size_t)batch * sizeof(int32_t)) + 256;
 }
 
-extern "C" int etpgt_score_topk_bf16_eval(const void* sess_bf16, const void* table_bf16, int64_t batch,
-                                          int64_t num_items, int dim, int k, int64_t id_base, float* top_val,
-                                          int64_t* top_idx, const int64_t* targets, int32_t* hit_pos, void* ws,
-                                          size_t ws_bytes, etpgt_stream_t stream_) {
+namespace {
+
+// The scorer behind etpgt_score_topk_bf16_eval (excl.ids == nullptr) and etpgt_score_topk_bf16_exclude (k_any: k may
+// exceed the eligible items, whose missing slots become (-inf, INT64_MAX) sentinels).
+int score_topk_bf16_run(const void* sess_bf16, const void* table_bf16, int64_t batch, int64_t num_items, int dim,
+                        int k, int64_t id_base, float* top_val, int64_t* top_idx, const int64_t* targets,
+                        int32_t* hit_pos, Exclusion excl, bool k_any, void* ws, size_t ws_bytes,
+                        etpgt_stream_t stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  const bool use_excl = excl.ids != nullptr;
   ETPGT_REQUIRE((targets == nullptr) == (hit_pos == nullptr), "score_topk_bf16: targets and hit_pos come together");
   ETPGT_REQUIRE(dim == 64 || dim == 128 || dim == 192 || dim == 256,
                 "score_topk_bf16: dim %d must be a multiple of 64 up to 256", dim);
   ETPGT_REQUIRE(batch >= 0 && num_items >= 1 && num_items < (int64_t(1) << 31), "score_topk_bf16: bad sizes");
-  ETPGT_REQUIRE(k >= 1 && k <= kMaxKTc && k <= num_items, "score_topk_bf16: k=%d must be in [1, min(%d, num_items)]",
-                k, kMaxKTc);
+  if (k_any) {
+    ETPGT_REQUIRE(k >= 1 && k <= kMaxKTc, "score_topk_bf16: k=%d must be in [1, %d]", k, kMaxKTc);
+  } else {
+    ETPGT_REQUIRE(k >= 1 && k <= kMaxKTc && k <= num_items, "score_topk_bf16: k=%d must be in [1, min(%d, num_items)]",
+                  k, kMaxKTc);
+  }
   ETPGT_REQUIRE(((uintptr_t)sess_bf16 & 15) == 0 && ((uintptr_t)table_bf16 & 15) == 0,
                 "score_topk_bf16: operands must be 16-byte aligned");
   if (ws_bytes < etpgt_score_topk_bf16_workspace_bytes(batch, num_items, k)) {
@@ -838,6 +929,10 @@ extern "C" int etpgt_score_topk_bf16_eval(const void* sess_bf16, const void* tab
   }
   if (batch == 0) return ETPGT_OK;
   const TcPlan p = tc_plan(batch, num_items, k);
+  // the exclusion variant exists for the default kernel shape only (CTA pairs, two column parts)
+  ETPGT_REQUIRE(!use_excl || (p.pairs && p.col_parts == 2),
+                "score_topk_bf16_exclude: exclusion needs the default scorer configuration (unset ETPGT_SCORE_2CTA and "
+                "ETPGT_SCORE_EPI)");
   Workspace w(ws, ws_bytes);
   const size_t units = (size_t)p.sch.num_parts(batch);
   DumpBuffers dump;
@@ -863,7 +958,8 @@ extern "C" int etpgt_score_topk_bf16_eval(const void* sess_bf16, const void* tab
     const int f = atoi(forced);
     if (f >= 1 && f <= kPendingMerge + 1 - BLOCK_N / 2 / DUMPW) pending_merge = f;
   }
-  const size_t smem = tc_smem_bytes(num_kb, stages, p.pairs);
+  // the exclusion variant keeps its epilogue threads' cursors behind the barriers
+  const size_t smem = tc_smem_bytes(num_kb, stages, p.pairs) + (use_excl ? 4 * 2 * 32 * sizeof(ExclCursor) : 0);
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(p.grid);
   cfg.blockDim = dim3(threads_for(p.col_parts));
@@ -876,22 +972,23 @@ extern "C" int etpgt_score_topk_bf16_eval(const void* sess_bf16, const void* tab
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-#define LAUNCH4(NKB, KC, PR, CP_)                                                                                  \
+#define LAUNCH4(NKB, KC, PR, CP_, EX)                                                                              \
   {                                                                                                                \
-    cudaFuncSetAttribute(score_dump_tc_kernel<NKB, KC, PR, CP_>, cudaFuncAttributeMaxDynamicSharedMemorySize,      \
+    cudaFuncSetAttribute(score_dump_tc_kernel<NKB, KC, PR, CP_, EX>, cudaFuncAttributeMaxDynamicSharedMemorySize,  \
                          (int)smem);                                                                               \
-    cudaLaunchKernelEx(&cfg, score_dump_tc_kernel<NKB, KC, PR, CP_>, map_sess, map_items, batch, num_items, stages, \
-                       p.sch, dump, pending_merge);                                                                \
+    cudaLaunchKernelEx(&cfg, score_dump_tc_kernel<NKB, KC, PR, CP_, EX>, map_sess, map_items, batch, num_items,    \
+                       stages, p.sch, dump, pending_merge, excl);                                                  \
   }
-#define LAUNCH3(NKB, KC, PR)                    \
-  {                                             \
-    if (p.col_parts == 4) LAUNCH4(NKB, KC, PR, 4) \
-    else LAUNCH4(NKB, KC, PR, 2)                \
+#define LAUNCH3(NKB, KC, PR)                           \
+  {                                                    \
+    if (p.col_parts == 4) LAUNCH4(NKB, KC, PR, 4, false) \
+    else LAUNCH4(NKB, KC, PR, 2, false)                \
   }
-#define LAUNCH2(NKB, KC)                  \
-  {                                       \
-    if (p.pairs) LAUNCH3(NKB, KC, true)   \
-    else LAUNCH3(NKB, KC, false)          \
+#define LAUNCH2(NKB, KC)                            \
+  {                                                 \
+    if (use_excl) LAUNCH4(NKB, KC, true, 2, true)   \
+    else if (p.pairs) LAUNCH3(NKB, KC, true)        \
+    else LAUNCH3(NKB, KC, false)                    \
   }
 #define LAUNCH(NKB)                    \
   {                                    \
@@ -921,14 +1018,23 @@ extern "C" int etpgt_score_topk_bf16_eval(const void* sess_bf16, const void* tab
       dump, batch, p.sch, k, id_base, top_val, top_idx, redo, targets, hit_pos);
   ETPGT_CHECK_LAUNCH("score_select");
   if (stats) cudaEventRecord(ev[2], stream);
-  const size_t redo_smem = ((size_t)dim + (size_t)kRedoThreads * k * 2) * sizeof(float);
-  if (redo_smem > 48 * 1024)
-    cudaFuncSetAttribute(score_redo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)redo_smem);
+  const size_t redo_smem = ((size_t)dim + (size_t)kRedoThreads * k * 2) * sizeof(float) +
+                           (use_excl ? (size_t)excl.width * sizeof(int64_t) : 0);
   const int64_t redo_blocks = (batch + kRedoThreads - 1) / kRedoThreads;
   const unsigned redo_grid = (unsigned)(redo_blocks < 2 * kNumSMs ? redo_blocks : 2 * kNumSMs);
-  score_redo_kernel<<<redo_grid, kRedoThreads, redo_smem, stream>>>(
-      static_cast<const __nv_bfloat16*>(sess_bf16), static_cast<const __nv_bfloat16*>(table_bf16), batch, num_items,
-      dim, k, id_base, redo, top_val, top_idx, targets, hit_pos);
+  if (use_excl) {
+    if (redo_smem > 48 * 1024)
+      cudaFuncSetAttribute(score_redo_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)redo_smem);
+    score_redo_kernel<true><<<redo_grid, kRedoThreads, redo_smem, stream>>>(
+        static_cast<const __nv_bfloat16*>(sess_bf16), static_cast<const __nv_bfloat16*>(table_bf16), batch,
+        num_items, dim, k, id_base, redo, top_val, top_idx, targets, hit_pos, excl);
+  } else {
+    if (redo_smem > 48 * 1024)
+      cudaFuncSetAttribute(score_redo_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)redo_smem);
+    score_redo_kernel<false><<<redo_grid, kRedoThreads, redo_smem, stream>>>(
+        static_cast<const __nv_bfloat16*>(sess_bf16), static_cast<const __nv_bfloat16*>(table_bf16), batch,
+        num_items, dim, k, id_base, redo, top_val, top_idx, targets, hit_pos, excl);
+  }
   ETPGT_CHECK_LAUNCH("score_redo");
   if (stats) {   // dump volume, fallback rows, kernel times
     std::vector<int32_t> h_redo(batch), h_count(kMaxColParts * units);
@@ -952,6 +1058,31 @@ extern "C" int etpgt_score_topk_bf16_eval(const void* sess_bf16, const void* tab
             p.grid, units, p.cap, (double)pieces / (double)units, (long long)worst, (long long)redo_rows);
   }
   return ETPGT_OK;
+}
+
+}  // namespace
+
+extern "C" int etpgt_score_topk_bf16_eval(const void* sess_bf16, const void* table_bf16, int64_t batch,
+                                          int64_t num_items, int dim, int k, int64_t id_base, float* top_val,
+                                          int64_t* top_idx, const int64_t* targets, int32_t* hit_pos, void* ws,
+                                          size_t ws_bytes, etpgt_stream_t stream) {
+  return score_topk_bf16_run(sess_bf16, table_bf16, batch, num_items, dim, k, id_base, top_val, top_idx, targets,
+                             hit_pos, Exclusion{nullptr, 0, 0}, false, ws, ws_bytes, stream);
+}
+
+extern "C" int etpgt_score_topk_bf16_exclude(const void* sess_bf16, const void* table_bf16, int64_t batch,
+                                             int64_t num_items, int dim, int k, int64_t id_base, float* top_val,
+                                             int64_t* top_idx, const int64_t* targets, int32_t* hit_pos,
+                                             const int64_t* exclude, int64_t exclude_width, void* ws, size_t ws_bytes,
+                                             etpgt_stream_t stream) {
+  ETPGT_REQUIRE(exclude_width >= 0 && exclude_width <= kMaxExcludeWidth,
+                "score_topk_bf16_exclude: exclude_width %lld must be in [0, %lld]", (long long)exclude_width,
+                (long long)kMaxExcludeWidth);
+  ETPGT_REQUIRE(exclude_width == 0 || batch == 0 || exclude != nullptr, "score_topk_bf16_exclude: null exclude list");
+  // width 0: nothing to exclude, the unfiltered kernels run (k > num_items still yields sentinels)
+  const Exclusion excl{exclude_width > 0 ? exclude : nullptr, exclude_width, id_base};
+  return score_topk_bf16_run(sess_bf16, table_bf16, batch, num_items, dim, k, id_base, top_val, top_idx, targets,
+                             hit_pos, excl, true, ws, ws_bytes, stream);
 }
 
 extern "C" int etpgt_score_topk_bf16(const void* sess_bf16, const void* table_bf16, int64_t batch,

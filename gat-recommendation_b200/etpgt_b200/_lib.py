@@ -96,6 +96,8 @@ _PROTOTYPES = {
     "etpgt_score_topk_bf16_workspace_bytes": (Z, [L, L, I]),
     "etpgt_score_topk_bf16": (I, [P, P, L, L, I, I, L, P, P, P, Z, P]),
     "etpgt_score_topk_bf16_eval": (I, [P, P, L, L, I, I, L, P, P, P, P, P, Z, P]),
+    "etpgt_score_topk_bf16_exclude": (I, [P, P, L, L, I, I, L, P, P, P, P, P, L, P, Z, P]),
+    "etpgt_score_topk_f32_exclude": (I, [P, P, L, L, I, I, L, P, P, P, L, P, Z, P]),
     "etpgt_topk_merge": (I, [P, P, L, I, I, P, P, P]),
     "etpgt_topk_metrics": (I, [P, P, L, I, I, P, P]),
     "etpgt_scatter_rows_workspace_bytes": (Z, [L]),

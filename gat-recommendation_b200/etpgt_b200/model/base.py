@@ -31,17 +31,32 @@ class BaseRecommendationModel(nn.Module, ABC):
     def get_item_embeddings(self) -> torch.Tensor:
         return self.item_embedding.weight
 
-    def predict(self, session_embeddings: torch.Tensor, k: int = 20) -> torch.Tensor:
+    def predict(self, session_embeddings: torch.Tensor, k: int = 20, exclude_items: torch.Tensor | None = None,
+                exclude_sorted: bool = False) -> torch.Tensor:
         """Top-k item ids per session by dot product against the whole table; the [B, I] score
-        matrix is never materialised (fused scoring + top-k kernel)."""
+        matrix is never materialised (fused scoring + top-k kernel).
+
+        exclude_items [B, L] int64 (e.g. `ops.seen_items(batch)`): ids each session must not receive, filtered inside
+        the scorer; slots a session has no eligible item for hold INT64_MAX.  None ranks every id, like the
+        reference's offline predict (base.py:73-76).  exclude_sorted: rows already ascending (skips a sort)."""
         precision = self.score_precision
         if precision == "auto":
             # small batches: fp32 CUDA-core scorer (the reference's arithmetic); evaluation-sized batches:
             # tcgen05 bf16 scorer (BASELINE.json: bf16 GEMM within 1e-2, ties to the lower id)
             big = session_embeddings.size(0) >= 64
             precision = "bf16" if big and ops.tensor_core_scoring_supported(session_embeddings.size(1), k) else "fp32"
-        _, top = ops.score_topk(session_embeddings, self.get_item_embeddings(), k, precision=precision)
+        _, top = ops.score_topk(session_embeddings, self.get_item_embeddings(), k, precision=precision,
+                                exclude=exclude_items, exclude_sorted=exclude_sorted)
         return top
+
+    @torch.no_grad()
+    def recommend(self, batch, k: int = 20, exclude_seen: bool = True) -> torch.Tensor:
+        """What each session of `batch` should see next: forward pass, then the top-k items leaving out the session's
+        own items and the padding id 0 (exclude_seen) — the batched form of the reference's serving path
+        (recommender.py:133-134).  Like the reference it leaves train / eval mode to the caller."""
+        sess = self(batch)
+        exclude = ops.seen_items(batch, num_sessions=sess.size(0)) if exclude_seen else None
+        return self.predict(sess, k, exclude_items=exclude, exclude_sorted=True)
 
     def compute_loss(self, session_embeddings, target_items, negative_items) -> torch.Tensor:
         """The model's default (BPR) loss — base.py:80-113."""

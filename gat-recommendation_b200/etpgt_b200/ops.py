@@ -1391,9 +1391,22 @@ def tensor_core_scoring_supported(dim: int, k: int) -> bool:
     return dim in (64, 128, 192, 256) and 1 <= k <= 32
 
 
+def _exclusion_rows(exclude: torch.Tensor, b: int, dev, rows_sorted: bool) -> torch.Tensor:
+    """Checks an exclusion list ([B, L] int64 on the scoring device) and returns it with every row sorted."""
+    if not torch.is_tensor(exclude) or not exclude.is_cuda or exclude.device != dev:
+        raise RuntimeError("score_topk: `exclude` must be a CUDA tensor on the device of the session embeddings")
+    if exclude.dtype != torch.int64 or exclude.dim() != 2 or exclude.size(0) != b:
+        raise RuntimeError(f"score_topk: `exclude` must be int64 [B={b}, L], got {exclude.dtype} "
+                           f"{tuple(exclude.shape)}")
+    if exclude.size(1) == 0 or rows_sorted:
+        return exclude.contiguous()
+    return torch.sort(exclude, dim=1).values.contiguous()
+
+
 @torch.no_grad()
 def score_topk(sess: torch.Tensor, table: torch.Tensor, k: int, id_base: int = 0, precision: str = "fp32",
-               out: tuple | None = None, targets: torch.Tensor | None = None):
+               out: tuple | None = None, targets: torch.Tensor | None = None, exclude: torch.Tensor | None = None,
+               exclude_sorted: bool = False):
     """Top-k item ids by dot product, ties to the lower id — etpgt/model/base.py:59-78.
 
     precision "fp32": CUDA-core scorer with the reference's fp32 arithmetic.
@@ -1401,11 +1414,19 @@ def score_topk(sess: torch.Tensor, table: torch.Tensor, k: int, id_base: int = 0
     may already be a bf16 copy (an evaluation loop converts it once).
     out: (top_val [B, k] f32, top_idx [B, k] i64) to write into (contiguous), else fresh tensors.
     targets [B] (bf16 scorer): also returns hit_pos [B] int32 — the position of each target in its row's results or
-    -1, taken inside the scorer's select epilogue (the input of `hit_metrics`): (top_val, top_idx, hit_pos)."""
+    -1, taken inside the scorer's select epilogue (the input of `hit_metrics`): (top_val, top_idx, hit_pos).
+    exclude [B, L] int64: ids each row must not receive (e.g. `seen_items(batch)`), ranked as if they were absent
+    from the table.  Rows need not be sorted (they are sorted here); duplicates, -1 padding and ids outside
+    [id_base, id_base + rows of `table`) are ignored, so an item shard takes the global list.  k may then exceed a
+    row's eligible items: the missing slots are (-inf, INT64_MAX), and an excluded target has hit_pos -1.
+    exclude_sorted: the rows are already ascending (`seen_items` returns them so): skips the sort, which at
+    evaluation size costs about a third of the scoring time."""
     _require_cuda(sess, "session embeddings")
     b, dim = sess.shape
     items = table.size(0)
     dev = sess.device
+    if exclude is not None:
+        exclude = _exclusion_rows(exclude, b, dev, exclude_sorted)
     if out is not None:
         top_val, top_idx = out
         if tuple(top_val.shape) != (b, k) or tuple(top_idx.shape) != (b, k) or top_val.dtype != torch.float32 \
@@ -1421,21 +1442,68 @@ def score_topk(sess: torch.Tensor, table: torch.Tensor, k: int, id_base: int = 0
         if targets is not None:
             targets = _i64(targets)
             hit_pos = torch.empty(b, dtype=torch.int32, device=dev)
-        call("etpgt_score_topk_bf16_eval", ptr(sess_h), ptr(table_h), b, items, dim, k, id_base, ptr(top_val),
-             ptr(top_idx), ptr(targets), ptr(hit_pos), ptr(ws), ws.numel(), stream())
+        if exclude is None:
+            call("etpgt_score_topk_bf16_eval", ptr(sess_h), ptr(table_h), b, items, dim, k, id_base, ptr(top_val),
+                 ptr(top_idx), ptr(targets), ptr(hit_pos), ptr(ws), ws.numel(), stream())
+        else:
+            call("etpgt_score_topk_bf16_exclude", ptr(sess_h), ptr(table_h), b, items, dim, k, id_base, ptr(top_val),
+                 ptr(top_idx), ptr(targets), ptr(hit_pos), ptr(exclude), exclude.size(1), ptr(ws), ws.numel(),
+                 stream())
         return (top_val, top_idx) if targets is None else (top_val, top_idx, hit_pos)
     if precision != "fp32":
         raise ValueError(f"Unknown scoring precision: {precision}")
     sess_c, table_c = _f32(sess.detach()), _f32(table.detach())
     ws = workspace(size("etpgt_score_topk_workspace_bytes", b, items, dim, k), dev)
-    call("etpgt_score_topk_f32", ptr(sess_c), ptr(table_c), b, items, dim, k, id_base, ptr(top_val), ptr(top_idx),
-         ptr(ws), ws.numel(), stream())
+    if exclude is None:
+        call("etpgt_score_topk_f32", ptr(sess_c), ptr(table_c), b, items, dim, k, id_base, ptr(top_val),
+             ptr(top_idx), ptr(ws), ws.numel(), stream())
+    else:
+        call("etpgt_score_topk_f32_exclude", ptr(sess_c), ptr(table_c), b, items, dim, k, id_base, ptr(top_val),
+             ptr(top_idx), ptr(exclude), exclude.size(1), ptr(ws), ws.numel(), stream())
     if targets is None:
         return top_val, top_idx
     # the fp32 CUDA-core scorer (small batches) has no fused epilogue: positions from its id matrix
     match = top_idx == _i64(targets).view(-1, 1)
     hit_pos = torch.where(match.any(dim=1), match.float().argmax(dim=1), torch.full((b,), -1, device=dev)).int()
     return top_val, top_idx, hit_pos
+
+
+@torch.no_grad()
+def seen_items(batch, num_sessions: int | None = None, width: int | None = None,
+               exclude_padding: bool = True) -> torch.Tensor:
+    """Exclusion rows for `score_topk(exclude=...)`: [B, L] int64, row b = the item ids of session b's graph
+    (`batch.x` grouped by `batch.ptr`, or by `batch.batch` when the batch has no ptr), plus the padding id 0 when
+    `exclude_padding`, sorted, padded with -1.
+
+    width: L.  A loader that cuts sessions to `max_session_length` items gives width = max_session_length + 1 (the +1
+    for id 0), and then no value is read back to the host; a session with more than L (L - 1 with id 0) items keeps
+    only its first ones in the list.  None: L is the longest session (+1), which costs one host read."""
+    x, bvec = batch.x, batch.batch
+    dev = x.device
+    if num_sessions is None:
+        n = getattr(batch, "num_graphs", None)
+        num_sessions = int(n) if isinstance(n, int) else None
+    node_ptr = getattr(batch, "ptr", None)
+    if num_sessions is None:
+        num_sessions = node_ptr.numel() - 1 if node_ptr is not None else (int(bvec.max().item()) + 1 if x.numel() else 0)
+    if node_ptr is None:
+        counts = torch.bincount(bvec, minlength=num_sessions)
+        node_ptr = torch.zeros(num_sessions + 1, dtype=torch.int64, device=dev)
+        torch.cumsum(counts, 0, out=node_ptr[1:])
+    node_ptr = node_ptr.to(torch.int64)
+    pad = 1 if exclude_padding else 0
+    if width is None:
+        longest = int((node_ptr[1:] - node_ptr[:-1]).max().item()) if num_sessions > 0 else 0
+        width = longest + pad
+    out = torch.full((num_sessions, max(int(width), pad)), -1, dtype=torch.int64, device=dev)
+    if exclude_padding:
+        out[:, 0] = 0
+    if x.numel() and out.size(1) > pad:
+        bvec = bvec.to(torch.int64)
+        col = torch.arange(x.numel(), device=dev) - node_ptr[bvec] + pad
+        keep = col < out.size(1)
+        out.view(-1).index_put_(((bvec * out.size(1) + col)[keep],), x.to(torch.int64)[keep])
+    return torch.sort(out, dim=1).values
 
 
 @torch.no_grad()

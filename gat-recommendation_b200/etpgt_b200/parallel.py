@@ -99,7 +99,7 @@ def _compact_index(counts: tuple, device) -> torch.Tensor:
 
 @torch.no_grad()
 def sharded_predict(model, session_embeddings: torch.Tensor, k: int = 20, group=None, counts=None, targets=None,
-                    precision: str = "auto"):
+                    precision: str = "auto", exclude=None, exclude_sorted: bool = False):
     """Item-sharded full-catalogue top-k (SURVEY.md section 8e): one all-gather of the session vectors, ONE scoring
     call of this rank's contiguous id range for all sessions (fused top-k), one all-gather of the packed
     (value, id) candidates, one exact merge kernel that reads the gathered layout directly.  Returns the top-k ids
@@ -109,7 +109,12 @@ def sharded_predict(model, session_embeddings: torch.Tensor, k: int = 20, group=
     counts: every rank's session count (host ints), when the caller knows them (a sharding loader does);
     otherwise they are exchanged, which costs one host read.
     group=False: score on this process alone even when a process group is initialised (a single-process replica
-    inside a data-parallel job: no collective is entered)."""
+    inside a data-parallel job: no collective is entered).
+
+    exclude [B, L] int64 (ops.score_topk's format, e.g. ops.seen_items(batch)): ids each of this rank's sessions must
+    not receive.  The rows travel with the session vectors (same padding and compaction) and every shard filters
+    against the global ids.  With `counts` given every rank passes the same L (a loader's max_session_length + 1);
+    without, the widths are exchanged together with the counts.  exclude_sorted: the rows are already ascending."""
     from . import ops
 
     rank, size = (0, 1) if group is False else world()
@@ -122,14 +127,18 @@ def sharded_predict(model, session_embeddings: torch.Tensor, k: int = 20, group=
         if precision == "auto":
             precision = "bf16" if b_local >= 64 and ops.tensor_core_scoring_supported(width, k) else "fp32"
         if targets is None:
-            return ops.score_topk(session_embeddings, table, k, precision=precision)[1]
-        _, top, hit = ops.score_topk(session_embeddings, table, k, precision=precision, targets=targets)
+            return ops.score_topk(session_embeddings, table, k, precision=precision, exclude=exclude,
+                                  exclude_sorted=exclude_sorted)[1]
+        _, top, hit = ops.score_topk(session_embeddings, table, k, precision=precision, targets=targets,
+                                     exclude=exclude, exclude_sorted=exclude_sorted)
         return top, hit
+    ex_width = int(exclude.size(1)) if exclude is not None else 0
     if counts is None:
-        mine = torch.tensor([b_local], dtype=torch.int64, device=dev)
-        everyone_counts = torch.empty(size, dtype=torch.int64, device=dev)
+        mine = torch.tensor([b_local, ex_width], dtype=torch.int64, device=dev)
+        everyone_counts = torch.empty(2 * size, dtype=torch.int64, device=dev)
         dist.all_gather_into_tensor(everyone_counts, mine, group=group)
-        counts = everyone_counts.tolist()
+        exchanged = everyone_counts.tolist()
+        counts, ex_width = exchanged[0::2], max(exchanged[1::2])
     counts = tuple(int(c) for c in counts)
     total, widest = sum(counts), max(counts)
     send = ops._f32(session_embeddings)
@@ -140,6 +149,16 @@ def sharded_predict(model, session_embeddings: torch.Tensor, k: int = 20, group=
     gathered = torch.empty(size * widest, width, dtype=torch.float32, device=dev)
     dist.all_gather_into_tensor(gathered, send, group=group)
     everyone = gathered if total == size * widest else gathered.index_select(0, _compact_index(counts, dev))
+    everyone_ex = None
+    if exclude is not None:   # the exclusion rows of all sessions, gathered like the session vectors (-1: no id)
+        send_ex = torch.full((widest, ex_width), -1, dtype=torch.int64, device=dev)
+        send_ex[:b_local, :exclude.size(1)] = exclude
+        gathered_ex = torch.empty(size * widest, ex_width, dtype=torch.int64, device=dev)
+        dist.all_gather_into_tensor(gathered_ex, send_ex, group=group)
+        everyone_ex = gathered_ex if total == size * widest else \
+            gathered_ex.index_select(0, _compact_index(counts, dev))
+        if not exclude_sorted:   # sorted once here rather than by every scoring call below
+            everyone_ex = torch.sort(everyone_ex, dim=1).values
     if precision == "auto":
         precision = "bf16" if total >= 64 and ops.tensor_core_scoring_supported(width, k) else "fp32"
     # this rank's candidates for ALL sessions, packed as one block: val [total, k] f32 | idx [total, k] i64
@@ -150,12 +169,14 @@ def sharded_predict(model, session_embeddings: torch.Tensor, k: int = 20, group=
     val = block[: total * k * 4].view(torch.float32).view(total, k)
     idx = block[val_bytes:].view(torch.int64).view(total, k)
     if kk == k:
-        ops.score_topk(everyone, table[lo:hi], k, id_base=lo, precision=precision, out=(val, idx))
+        ops.score_topk(everyone, table[lo:hi], k, id_base=lo, precision=precision, out=(val, idx), exclude=everyone_ex,
+                       exclude_sorted=True)
     else:   # a shard with fewer than k items: pad with sentinels that lose every comparison
         val.fill_(float("-inf"))
         idx.fill_(torch.iinfo(torch.int64).max)
         if kk > 0:
-            v, i = ops.score_topk(everyone, table[lo:hi], kk, id_base=lo, precision=precision)
+            v, i = ops.score_topk(everyone, table[lo:hi], kk, id_base=lo, precision=precision, exclude=everyone_ex,
+                                  exclude_sorted=True)
             val[:, :kk], idx[:, :kk] = v, i
     parts = torch.empty(size * block.numel(), dtype=torch.uint8, device=dev)
     dist.all_gather_into_tensor(parts, block, group=group)

@@ -50,7 +50,8 @@ def _driver_for(model, loss_fn):
 class Trainer:
     def __init__(self, model, train_loader, val_loader, optimizer, device: str = "cuda",
                  output_dir: Path | str = "outputs", max_epochs: int = 100, patience: int = 10, eval_every: int = 1,
-                 k_values: list[int] | None = None, loss_fn=None, process_group=None, exchange: str = "peer"):
+                 k_values: list[int] | None = None, loss_fn=None, process_group=None, exchange: str = "peer",
+                 exclude_seen: bool = False):
         self.model = model.to(device)
         self.train_loader, self.val_loader, self.optimizer = train_loader, val_loader, optimizer
         self.device = device
@@ -58,6 +59,9 @@ class Trainer:
         self.max_epochs, self.patience, self.eval_every = max_epochs, patience, eval_every
         self.k_values = k_values if k_values is not None else [10, 20]
         self.loss_fn = loss_fn
+        # evaluate() ranks without each session's own items and the padding id 0: the Recall / NDCG of what a
+        # deployed recommender returns (the reference's serving filter, recommender.py:133-134)
+        self.exclude_seen = exclude_seen
         self.output_dir.mkdir(parents=True, exist_ok=True)
         self.current_epoch = 0
         self.best_val_metric = 0.0
@@ -145,14 +149,21 @@ class Trainer:
         # [hits, ndcg] per k, then the session count: ONE tensor, so that data parallelism sums it in one collective
         acc = torch.zeros(2 * len(self.k_values) + 1, dtype=torch.float64, device=self.device)
         sessions = 0
+        # exclusion rows of a fixed width when the loader says how long a session can be (no host read per batch,
+        # and every rank of a data-parallel job agrees on it)
+        max_len = getattr(self.val_loader, "max_session_length", None)
+        width = max_len + 1 if max_len is not None else None
         for batch in self.val_loader:
             batch = batch.to(self.device)
             sess = self.model(batch)
+            exclude = ops.seen_items(batch, num_sessions=sess.size(0), width=width) if self.exclude_seen else None
             if self._world > 1:
                 # item-sharded scoring: every rank scores all sessions of the global batch against its id range
-                _, hit = parallel.sharded_predict(self.model, sess, k=k_max, group=self._group,
-                                                  counts=getattr(batch, "rank_sessions", None),
-                                                  targets=batch.target_item)
+                counts = getattr(batch, "rank_sessions", None)
+                if exclude is not None and width is None:
+                    counts = None              # the ranks' list widths differ: exchanged with the counts
+                _, hit = parallel.sharded_predict(self.model, sess, k=k_max, group=self._group, counts=counts,
+                                                  targets=batch.target_item, exclude=exclude, exclude_sorted=True)
                 if getattr(batch, "replicated", False) and self._rank != 0:
                     continue                   # every rank holds the same sessions: counted once
                 for j, k in enumerate(self.k_values):
@@ -160,7 +171,8 @@ class Trainer:
             else:
                 # fused scoring + top-k; the target's position comes out of the scorer's select epilogue
                 # (group=False: this Trainer is not data parallel, even if the process has a group initialised)
-                _, hit = parallel.sharded_predict(self.model, sess, k=k_max, group=False, targets=batch.target_item)
+                _, hit = parallel.sharded_predict(self.model, sess, k=k_max, group=False, targets=batch.target_item,
+                                                  exclude=exclude, exclude_sorted=True)
                 for j, k in enumerate(self.k_values):
                     ops.hit_metrics(hit, k, acc[2 * j:2 * j + 2])
             sessions += int(batch.target_item.shape[0])

@@ -462,6 +462,21 @@ int etpgt_score_topk_bf16_eval(const void* sess_bf16, const void* table_bf16, in
                                int dim, int k, int64_t id_base, float* top_val, int64_t* top_idx,
                                const int64_t* targets, int32_t* hit_pos, void* ws, size_t ws_bytes,
                                etpgt_stream_t stream);
+/* Filtered scoring: the same results with each row's listed ids left out (a session's own items, the padding id).
+ * exclude: int64 [batch, exclude_width], row-major, one row per session; each row sorted ascending, duplicates
+ * allowed, ids outside [id_base, id_base + num_items) ignored (so an item shard takes the global list unchanged and
+ * rows may be padded with -1).  exclude_width == 0 excludes nothing.  Unlike the unfiltered entry points k may exceed
+ * the eligible items of a row: the missing slots are (-inf, INT64_MAX).  An excluded target gets hit_pos -1.
+ * bf16: same workspace as etpgt_score_topk_bf16_workspace_bytes, exclude_width <= 16384, default kernel shape only
+ * (an error while the ETPGT_SCORE_2CTA=0 / ETPGT_SCORE_EPI=4 comparison knobs are set); targets / hit_pos nullable. */
+int etpgt_score_topk_bf16_exclude(const void* sess_bf16, const void* table_bf16, int64_t batch, int64_t num_items,
+                                  int dim, int k, int64_t id_base, float* top_val, int64_t* top_idx,
+                                  const int64_t* targets, int32_t* hit_pos, const int64_t* exclude,
+                                  int64_t exclude_width, void* ws, size_t ws_bytes, etpgt_stream_t stream);
+/* fp32: same workspace as etpgt_score_topk_workspace_bytes. */
+int etpgt_score_topk_f32_exclude(const float* sess, const float* table, int64_t batch, int64_t num_items, int dim,
+                                 int k, int64_t id_base, float* top_val, int64_t* top_idx, const int64_t* exclude,
+                                 int64_t exclude_width, void* ws, size_t ws_bytes, etpgt_stream_t stream);
 /* exact merge of `parts` candidate lists per row ([B, parts*k] values + ids). */
 int etpgt_topk_merge(const float* cand_val, const int64_t* cand_idx, int64_t batch, int parts, int k,
                      float* top_val, int64_t* top_idx, etpgt_stream_t stream);

@@ -1,0 +1,634 @@
+// Full-catalogue softmax cross-entropy on the tensor cores (sm_100a: tcgen05 + TMA), forward and backward.
+//
+// For session rows S [B, D], the item table E [I, D] (row padding_idx left out), targets t and temperature T:
+//   z = S E^T / T,  lse = logsumexp_j z[:, j],  loss = sum_b (lse[b] - z[b, t[b]]) / B_total
+//   G = (softmax(z) - onehot(t)) / (T B_total),  dS = G E,  dE += G^T S
+// The [B, I] logits never exist in memory, not even in chunks.  One warp-specialised kernel serves all three
+// passes.  A CTA keeps 128 "rows" of one operand on the TMEM lanes and streams 128-row tiles of the other operand
+// (the "columns") through a TMA ring, one 64-wide k-block of hi / lo bf16 parts at a time:
+//   FWD  rows = sessions, columns = items.  The epilogue folds each logits tile into a per-row online
+//        (max, sum exp) and picks up the target's logit; a combine kernel merges the column ranges in order.
+//   DS   rows = sessions, columns = items.  The epilogue turns the recomputed logits tile into G (fp32), splits it
+//        into a bf16 pair in swizzled shared memory (K-major A operand), and the MMA warp adds G . E_tile into a
+//        [128, D] TMEM accumulator.  The item tile is streamed a second time for that product: the same 128-row x
+//        64-column TMA box that is the K-major B operand of the logits is the MN-major B operand of G . E_tile.
+//   DE   the same with the roles swapped: rows = items, columns = sessions, lse and targets are per column.
+// Every product is split-bf16 ("bf16x3": hi.hi + hi.lo + lo.hi, fp32 accumulation in TMEM), the convention of
+// gemm_tc.cu.  TMEM: two 128-column logits buffers (the epilogue drains one while the next is computed) and, for
+// the gradients, D accumulator columns.  Column ranges split across CTAs are combined in a fixed order: no
+// atomics, bit-reproducible.
+// The backward recomputes the forward's logits bit for bit (same MMA sequence, operands swapped in DE) and keeps
+// them, lse and the running maxima in natural units (exp(x) = 2^(x log2 e) on the MUFU unit): where the softmax
+// is exact — one eligible column, P = 1 — the gradient is exactly zero, not rounding noise.
+#include <math.h>
+
+#include "tc_common.cuh"
+
+namespace etpgt {
+namespace {
+
+using namespace tc;
+
+constexpr int TILE = 128;                              // TMEM lanes = rows of a CTA = columns of a logits tile
+constexpr int kThreads = 192;                          // warp 0 TMA, warp 1 MMA, warps 2-5 epilogue
+constexpr uint32_t KB_BYTES = TILE * BLOCK_K * 2;      // one 128-row x 64-k bf16 box: 16 KB
+constexpr uint32_t STAGE_BYTES = 4 * KB_BYTES;         // row hi, row lo, column hi, column lo
+constexpr uint32_t G_BYTES = 4 * KB_BYTES;             // G tile: hi then lo, two 64-column k-blocks each
+constexpr uint32_t ACC_COL = 2 * TILE;                 // first TMEM column of the gradient accumulator
+// The tensor cores add each MMA's products into the fp32 accumulator with truncation, not round-to-nearest: over a
+// whole column range (thousands of MMAs) that bias reached 3e-4 relative in dS at 32,768 x 82,174.  The accumulator
+// is therefore drained every kDrainTiles column tiles (192 MMAs) and summed in fp32 by the epilogue threads.
+constexpr int kDrainTiles = 8;
+constexpr float kLog2e = 1.4426950408889634f;
+
+enum Mode { FWD = 0, DS = 1, DE = 2 };
+
+// 2^x on the MUFU unit (relative error ~2^-22, far inside the 1e-4 bound; -inf -> 0)
+__device__ __forceinline__ float fast_exp2(float x) {
+  float y;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+  return y;
+}
+// position of `id` inside the 32 columns from `base` on, or -1: the per-element tests of a chunk become
+// compares against a compile-time column index
+__device__ __forceinline__ int chunk_pos(int64_t id, int64_t base) {
+  const int64_t d = id - base;
+  return d >= 0 && d < 32 ? (int)d : -1;
+}
+template <int MODE> struct Cfg {
+  static constexpr int stages = MODE == FWD ? 3 : 2;
+  static constexpr uint32_t tmem_cols = MODE == FWD ? 256 : 512;
+  static constexpr size_t smem = 1024 + (size_t)stages * STAGE_BYTES + (MODE == FWD ? 0 : G_BYTES) + 256;
+};
+
+struct __align__(8) Bars {
+  uint64_t full[3], empty[3];
+  uint64_t lfull[2], lempty[2];   // logits buffers
+  uint64_t gfull, gempty;         // G tile in shared memory
+  uint64_t accfull, accempty;    // gradient accumulator: one phase per drain group
+  uint32_t tmem_base;
+};
+
+struct Params {
+  int64_t rows, cols;           // the logits of a CTA are rows x (its range of) cols
+  int dim;
+  int tiles_per_range, ranges;
+  float inv_t;                  // 1 / T
+  float gscale;                 // 1 / (T * B_total)
+  const int64_t* targets;       // per row (FWD, DS) or per column (DE)
+  const float* lse;             // natural log; per row (DS) or per column (DE)
+  const float* d_loss;
+  int64_t padding_idx;          // item id left out (-1: none)
+  float* part;                  // FWD: [3][ranges][rows]; DS / DE with ranges > 1: [ranges][rows][dim]
+  float* out;                   // DS: d_sess (written), DE: d_table (added), when ranges == 1
+};
+
+template <int MODE>
+__global__ void __launch_bounds__(kThreads, 1)
+full_softmax_tc_kernel(const __grid_constant__ CUtensorMap map_r_hi, const __grid_constant__ CUtensorMap map_r_lo,
+                       const __grid_constant__ CUtensorMap map_c_hi, const __grid_constant__ CUtensorMap map_c_lo,
+                       const Params p) {
+  extern __shared__ __align__(1024) uint8_t smem_raw[];
+  uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
+  constexpr int kStages = Cfg<MODE>::stages;
+  uint8_t* smem_g = smem + kStages * STAGE_BYTES;
+  Bars* bars = reinterpret_cast<Bars*>(smem_g + (MODE == FWD ? 0 : G_BYTES));
+
+  const int warp = threadIdx.x >> 5;
+  const int lane = threadIdx.x & 31;
+  const int row_tiles = (int)((p.rows + TILE - 1) / TILE);
+  const int col_tiles = (int)((p.cols + TILE - 1) / TILE);
+  // consecutive CTAs take different row tiles of the same column range: they stream the same column tiles
+  const int rt = blockIdx.x % row_tiles, range = blockIdx.x / row_tiles;
+  const int ct0 = range * p.tiles_per_range;
+  const int ct1 = min(ct0 + p.tiles_per_range, col_tiles);
+  const int n = ct1 - ct0;
+  const int nkb = p.dim / BLOCK_K;
+
+  if (threadIdx.x == 0) {
+    for (int s = 0; s < kStages; ++s) { mbar_init(&bars->full[s], 1); mbar_init(&bars->empty[s], 1); }
+    for (int b = 0; b < 2; ++b) { mbar_init(&bars->lfull[b], 1); mbar_init(&bars->lempty[b], 4); }
+    mbar_init(&bars->gfull, 4);
+    mbar_init(&bars->gempty, 1);
+    mbar_init(&bars->accfull, 1);
+    mbar_init(&bars->accempty, 4);
+    fence_barrier_init();
+    tma_prefetch_desc(&map_r_hi);
+    tma_prefetch_desc(&map_r_lo);
+    tma_prefetch_desc(&map_c_hi);
+    tma_prefetch_desc(&map_c_lo);
+  }
+  if (warp == 1) tmem_alloc(&bars->tmem_base, Cfg<MODE>::tmem_cols);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = bars->tmem_base;
+
+  if (warp == 0) {
+    if (lane == 0) {
+      int stage = 0;
+      uint32_t phase = 0;
+      // the k-blocks of column tile ct, with the row tile's (logits) or alone (second pass of the gradients)
+      auto load = [&](int ct, bool with_rows) {
+        for (int kb = 0; kb < nkb; ++kb) {
+          mbar_wait(&bars->empty[stage], phase ^ 1);
+          uint8_t* st = smem + stage * STAGE_BYTES;
+          mbar_expect_tx(&bars->full[stage], with_rows ? STAGE_BYTES : 2 * KB_BYTES);
+          if (with_rows) {
+            tma_load_2d(&map_r_hi, &bars->full[stage], st, kb * BLOCK_K, rt * TILE);
+            tma_load_2d(&map_r_lo, &bars->full[stage], st + KB_BYTES, kb * BLOCK_K, rt * TILE);
+          }
+          tma_load_2d(&map_c_hi, &bars->full[stage], st + 2 * KB_BYTES, kb * BLOCK_K, ct * TILE);
+          tma_load_2d(&map_c_lo, &bars->full[stage], st + 3 * KB_BYTES, kb * BLOCK_K, ct * TILE);
+          if (++stage == kStages) { stage = 0; phase ^= 1; }
+        }
+      };
+      // the order the MMA warp consumes: logits of tile j, then the gradient product of tile j - 1
+      for (int j = 0; j < n; ++j) {
+        load(ct0 + j, true);
+        if (MODE != FWD && j > 0) load(ct0 + j - 1, false);
+      }
+      if (MODE != FWD) load(ct1 - 1, false);
+    }
+  } else if (warp == 1) {
+    if (lane == 0) {
+      int stage = 0;
+      uint32_t phase = 0;
+      constexpr uint32_t idesc_l = instr_desc_bf16(TILE, TILE);
+      // G [rows, 128 columns] (K-major) x column tile [128 columns, 64 of D] (MN-major): one 64-wide slice of D
+      constexpr uint32_t idesc_g = instr_desc_bf16_major(TILE, BLOCK_K, false, true);
+      const uint32_t g_hi = smem_u32(smem_g), g_lo = g_hi + 2 * KB_BYTES;
+      auto grad = [&](int j) {
+        const int group = j / kDrainTiles;
+        const bool group_start = j % kDrainTiles == 0, group_end = (j + 1) % kDrainTiles == 0 || j == n - 1;
+        if (group_start && group > 0) mbar_wait(&bars->accempty, (uint32_t)(group - 1) & 1);  // drained
+        mbar_wait(&bars->gfull, (uint32_t)j & 1);
+        tc_fence_after();
+        for (int kb = 0; kb < nkb; ++kb) {
+          mbar_wait(&bars->full[stage], phase);
+          tc_fence_after();
+          const uint32_t c_hi = smem_u32(smem + stage * STAGE_BYTES) + 2 * KB_BYTES, c_lo = c_hi + KB_BYTES;
+          const uint32_t tmem_d = tmem_base + ACC_COL + (uint32_t)(kb * BLOCK_K);
+#pragma unroll
+          for (int kk = 0; kk < TILE / UMMA_K; ++kk) {
+            // A: 32 bytes along a swizzle row of G's k-block kk / 4; B: 16 rows (2 KB) of the column tile
+            const uint32_t off_a = (uint32_t)(kk >> 2) * KB_BYTES + (uint32_t)(kk & 3) * UMMA_K * 2;
+            const uint32_t off_b = (uint32_t)kk * UMMA_K * 128;
+            const uint32_t accumulate = (group_start && kk == 0) ? 0u : 1u;
+            const uint64_t da_hi = make_desc_sw128(g_hi + off_a), da_lo = make_desc_sw128(g_lo + off_a);
+            const uint64_t db_hi = make_desc_mn_sw128(c_hi + off_b, KB_BYTES);
+            const uint64_t db_lo = make_desc_mn_sw128(c_lo + off_b, KB_BYTES);
+            umma_bf16(tmem_d, da_hi, db_hi, idesc_g, accumulate);
+            umma_bf16(tmem_d, da_hi, db_lo, idesc_g, 1u);
+            umma_bf16(tmem_d, da_lo, db_hi, idesc_g, 1u);
+          }
+          umma_commit(&bars->empty[stage]);
+          if (++stage == kStages) { stage = 0; phase ^= 1; }
+        }
+        umma_commit(&bars->gempty);
+        if (group_end) umma_commit(&bars->accfull);
+      };
+      for (int j = 0; j < n; ++j) {
+        const int b = j & 1;
+        mbar_wait(&bars->lempty[b], ((uint32_t)(j >> 1) & 1) ^ 1);
+        tc_fence_after();
+        const uint32_t tmem_d = tmem_base + (uint32_t)(b * TILE);
+        for (int kb = 0; kb < nkb; ++kb) {
+          mbar_wait(&bars->full[stage], phase);
+          tc_fence_after();
+          const uint32_t r_hi = smem_u32(smem + stage * STAGE_BYTES), r_lo = r_hi + KB_BYTES;
+          const uint32_t c_hi = r_hi + 2 * KB_BYTES, c_lo = r_hi + 3 * KB_BYTES;
+#pragma unroll
+          for (int kk = 0; kk < BLOCK_K / UMMA_K; ++kk) {
+            const uint32_t off = (uint32_t)kk * UMMA_K * 2;
+            const uint32_t accumulate = (kb == 0 && kk == 0) ? 0u : 1u;
+            const uint64_t da_hi = make_desc_sw128(r_hi + off), db_hi = make_desc_sw128(c_hi + off);
+            umma_bf16(tmem_d, da_hi, db_hi, idesc_l, accumulate);
+            // the same three products in the same order in every pass (DE has the operands swapped), so the
+            // recomputed logits are the forward's bit for bit
+            if constexpr (MODE == DE) {
+              umma_bf16(tmem_d, make_desc_sw128(r_lo + off), db_hi, idesc_l, 1u);
+              umma_bf16(tmem_d, da_hi, make_desc_sw128(c_lo + off), idesc_l, 1u);
+            } else {
+              umma_bf16(tmem_d, da_hi, make_desc_sw128(c_lo + off), idesc_l, 1u);
+              umma_bf16(tmem_d, make_desc_sw128(r_lo + off), db_hi, idesc_l, 1u);
+            }
+          }
+          umma_commit(&bars->empty[stage]);
+          if (++stage == kStages) { stage = 0; phase ^= 1; }
+        }
+        umma_commit(&bars->lfull[b]);
+        if (MODE != FWD && j > 0) grad(j - 1);
+      }
+      if (MODE != FWD) grad(n - 1);
+    }
+  } else {
+    // TMEM lane quarter = warp % 4; thread = one row of the CTA
+    const int q = warp & 3;
+    const int r_local = q * 32 + lane;
+    const int64_t row = (int64_t)rt * TILE + r_local;
+    const bool row_ok = row < p.rows;
+    const uint32_t lane_addr = tmem_base + ((uint32_t)(q * 32) << 16);
+    if constexpr (MODE == FWD) {
+      const int64_t tgt = row_ok ? p.targets[row] : -1;
+      float m = -INFINITY, s = 0.f, zt = 0.f;
+      for (int j = 0; j < n; ++j) {
+        const int b = j & 1;
+        mbar_wait(&bars->lfull[b], (uint32_t)(j >> 1) & 1);
+        tc_fence_after();
+        const int64_t col0 = (int64_t)(ct0 + j) * TILE;
+#pragma unroll 1
+        for (int c = 0; c < TILE; c += 32) {
+          uint32_t v[32];
+          tmem_ld_32x32(lane_addr + (uint32_t)(b * TILE + c), v);
+          if (c + 32 == TILE) {  // logits buffer fully read: the MMA warp may overwrite it
+            tc_fence_before();
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&bars->lempty[b]);
+          }
+          const int64_t base = col0 + c;
+          const int lim = p.cols - base < 32 ? (int)(p.cols - base) : 32;
+          const int pad_e = chunk_pos(p.padding_idx, base), tgt_e = chunk_pos(tgt, base);
+          float y[32];
+          float mc = -INFINITY;
+#pragma unroll
+          for (int e = 0; e < 32; ++e) {
+            y[e] = __uint_as_float(v[e]) * p.inv_t;
+            if (e >= lim || e == pad_e) y[e] = -INFINITY;
+            if (e == tgt_e) zt = y[e];
+            mc = fmaxf(mc, y[e]);
+          }
+          if (mc == -INFINITY) continue;  // nothing of this chunk takes part
+          if (mc > m) {
+            s *= fast_exp2((m - mc) * kLog2e);
+            m = mc;
+          }
+#pragma unroll
+          for (int e = 0; e < 32; ++e) s += fast_exp2((y[e] - m) * kLog2e);
+        }
+      }
+      if (row_ok) {
+        p.part[(int64_t)range * p.rows + row] = m;
+        p.part[((int64_t)p.ranges + range) * p.rows + row] = s;
+        p.part[((int64_t)2 * p.ranges + range) * p.rows + row] = zt;
+      }
+    } else {
+      const float gscale = __ldg(p.d_loss) * p.gscale;
+      float lse_row = 0.f;
+      int64_t tgt_row = -1;
+      if (MODE == DS && row_ok) {
+        lse_row = p.lse[row];
+        tgt_row = p.targets[row];
+      }
+      uint8_t* g_row = smem_g + r_local * 128;
+      const bool direct = p.ranges == 1;
+      const bool store = row_ok && !(MODE == DE && row == p.padding_idx);
+      float* dst = direct ? p.out + row * p.dim : p.part + ((int64_t)range * p.rows + row) * p.dim;
+      // group `group` of column tiles is complete in the accumulator: add it to this thread's row in fp32 (the first
+      // group overwrites, except that d_table is always accumulated into), then hand the accumulator back
+      auto drain = [&](int group) {
+        mbar_wait(&bars->accfull, (uint32_t)group & 1);
+        tc_fence_after();
+        const bool add = group > 0 || (MODE == DE && direct);
+#pragma unroll 1
+        for (int c = 0; c < p.dim; c += 32) {
+          uint32_t v[32];
+          tmem_ld_32x32(lane_addr + ACC_COL + (uint32_t)c, v);
+          if (c + 32 == p.dim) {
+            tc_fence_before();
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&bars->accempty);
+          }
+          if (!store) continue;
+#pragma unroll
+          for (int e = 0; e < 32; e += 4) {
+            float4 o = make_float4(__uint_as_float(v[e]), __uint_as_float(v[e + 1]), __uint_as_float(v[e + 2]),
+                                   __uint_as_float(v[e + 3]));
+            if (add) o = add4(ld4(dst + c + e), o);
+            st4(dst + c + e, o);
+          }
+        }
+      };
+      for (int j = 0; j < n; ++j) {
+        const int b = j & 1;
+        mbar_wait(&bars->lfull[b], (uint32_t)(j >> 1) & 1);
+        mbar_wait(&bars->gempty, ((uint32_t)j & 1) ^ 1);  // the product of the previous G has completed
+        tc_fence_after();
+        const int64_t col0 = (int64_t)(ct0 + j) * TILE;
+#pragma unroll 1
+        for (int c = 0; c < TILE; c += 32) {
+          uint32_t v[32];
+          tmem_ld_32x32(lane_addr + (uint32_t)(b * TILE + c), v);
+          if (c + 32 == TILE) {
+            tc_fence_before();
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&bars->lempty[b]);
+          }
+          const int64_t base = col0 + c;
+          const int lim = !row_ok ? 0 : p.cols - base < 32 ? (int)(p.cols - base) : 32;
+          // DS: the padding column and the row's target as positions in the chunk.  DE: the chunk's 32 columns are
+          // sessions; lane e fetches column e's lse and its target as a row of this CTA (-1: none), shared by shuffles
+          int pad_e = -1, tgt_e = -1, tgt_lane = -1;
+          float lse_lane = 0.f;
+          if constexpr (MODE == DS) {
+            pad_e = chunk_pos(p.padding_idx, base);
+            tgt_e = chunk_pos(tgt_row, base);
+          } else if (base + lane < p.cols) {
+            lse_lane = p.lse[base + lane];
+            const int64_t t = p.targets[base + lane] - (int64_t)rt * TILE;
+            tgt_lane = t >= 0 && t < TILE ? (int)t : -1;
+          }
+          float g[32];
+#pragma unroll
+          for (int e = 0; e < 32; ++e) {
+            const float y = __uint_as_float(v[e]) * p.inv_t;
+            float pr;
+            if constexpr (MODE == DS) {
+              pr = fast_exp2((y - lse_row) * kLog2e) - (e == tgt_e ? 1.f : 0.f);
+              if (e >= lim || e == pad_e) pr = 0.f;
+            } else {
+              const float l = __shfl_sync(0xffffffffu, lse_lane, e);
+              const int t = __shfl_sync(0xffffffffu, tgt_lane, e);
+              pr = fast_exp2((y - l) * kLog2e) - (t == r_local ? 1.f : 0.f);
+              if (e >= lim) pr = 0.f;
+            }
+            g[e] = pr * gscale;
+          }
+          // split into the bf16 pair; 128-byte swizzle of the K-major A operand (16-byte unit ^ row % 8)
+          uint8_t* g_kb = g_row + (c >> 6) * KB_BYTES;
+#pragma unroll
+          for (int u = 0; u < 4; ++u) {
+            uint32_t h[4], l[4];
+#pragma unroll
+            for (int t = 0; t < 4; ++t) {
+              const float x0 = g[8 * u + 2 * t], x1 = g[8 * u + 2 * t + 1];
+              const __nv_bfloat16 h0 = __float2bfloat16_rn(x0), h1 = __float2bfloat16_rn(x1);
+              const __nv_bfloat16 l0 = __float2bfloat16_rn(x0 - __bfloat162float(h0));
+              const __nv_bfloat16 l1 = __float2bfloat16_rn(x1 - __bfloat162float(h1));
+              h[t] = (uint32_t)__bfloat16_as_ushort(h0) | ((uint32_t)__bfloat16_as_ushort(h1) << 16);
+              l[t] = (uint32_t)__bfloat16_as_ushort(l0) | ((uint32_t)__bfloat16_as_ushort(l1) << 16);
+            }
+            const uint32_t off = (uint32_t)(((((c & 63) >> 3) + u) ^ (lane & 7)) << 4);
+            *reinterpret_cast<uint4*>(g_kb + off) = make_uint4(h[0], h[1], h[2], h[3]);
+            *reinterpret_cast<uint4*>(g_kb + 2 * KB_BYTES + off) = make_uint4(l[0], l[1], l[2], l[3]);
+          }
+        }
+        fence_proxy_async_smem();  // generic-proxy writes -> visible to the tensor cores
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&bars->gfull);
+        if ((j + 1) % kDrainTiles == 0 || j == n - 1) drain(j / kDrainTiles);
+      }
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 1) {
+    tc_fence_after();
+    tmem_dealloc(tmem_base, Cfg<MODE>::tmem_cols);
+  }
+}
+
+// lse[b] and the loss from the per-range (max, sum) partials, ranges merged in ascending order, rows summed by a
+// fixed tree: one block, deterministic.
+constexpr int kCombineThreads = 1024;
+__global__ void __launch_bounds__(kCombineThreads)
+fwd_combine_kernel(const float* __restrict__ part, int ranges, int tiles_per_range, int64_t rows, int64_t cols,
+                   const int64_t* __restrict__ targets, double total, float* __restrict__ lse, float* __restrict__ loss) {
+  __shared__ double red[kCombineThreads];
+  double acc = 0.0;
+  for (int64_t b = threadIdx.x; b < rows; b += kCombineThreads) {
+    float m = -INFINITY;
+    for (int r = 0; r < ranges; ++r) m = fmaxf(m, part[(int64_t)r * rows + b]);
+    float s = 0.f;
+    for (int r = 0; r < ranges; ++r) {
+      const float mr = part[(int64_t)r * rows + b];
+      if (mr != -INFINITY) s += part[((int64_t)ranges + r) * rows + b] * exp2f((mr - m) * kLog2e);
+    }
+    const float l = m + logf(s);
+    const int64_t t = targets[b];
+    const float zt = (t >= 0 && t < cols) ? part[((int64_t)2 * ranges + (t / TILE) / tiles_per_range) * rows + b] : 0.f;
+    lse[b] = l;
+    acc += (double)(l - zt);
+  }
+  red[threadIdx.x] = acc;
+  __syncthreads();
+  for (int w = kCombineThreads / 2; w > 0; w >>= 1) {
+    if (threadIdx.x < w) red[threadIdx.x] += red[threadIdx.x + w];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) loss[0] = (float)(red[0] / total);
+}
+
+// out[row] (=|+=) sum_r part[r][row], r ascending; DE leaves row padding_idx untouched
+__global__ void __launch_bounds__(256)
+grad_combine_kernel(const float* __restrict__ part, int ranges, int64_t rows, int dim, int accumulate,
+                    int64_t skip_row, float* __restrict__ out) {
+  const int64_t total4 = rows * dim / 4;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total4; i += (int64_t)gridDim.x * blockDim.x) {
+    if ((4 * i) / dim == skip_row) continue;
+    float4 acc = accumulate ? ld4(out + 4 * i) : zero4();
+    for (int r = 0; r < ranges; ++r) acc = add4(acc, ldg4(part + (int64_t)r * rows * dim + 4 * i));
+    st4(out + 4 * i, acc);
+  }
+}
+
+struct Plan {
+  int tiles_per_range, ranges, grid;
+};
+
+// Column ranges per row tile: the count that minimises (waves of CTAs) x (column tiles per CTA), the fewest on a
+// tie, at most max_ranges.
+Plan plan_ranges(int64_t rows, int64_t cols, int max_ranges) {
+  const int64_t row_tiles = (rows + TILE - 1) / TILE, col_tiles = (cols + TILE - 1) / TILE;
+  int64_t best_cost = -1;
+  Plan best = {};
+  const int64_t top = col_tiles < max_ranges ? col_tiles : max_ranges;
+  for (int64_t want = 1; want <= top; ++want) {
+    const int64_t tpr = (col_tiles + want - 1) / want, r = (col_tiles + tpr - 1) / tpr;
+    const int64_t cost = ((row_tiles * r + kNumSMs - 1) / kNumSMs) * tpr;
+    if (best_cost < 0 || cost < best_cost) {
+      best_cost = cost;
+      best.tiles_per_range = (int)tpr;
+      best.ranges = (int)r;
+      best.grid = (int)(row_tiles * r);
+    }
+  }
+  return best;
+}
+// forward partials are 3 floats per (row, range): ranges are limited by the column tiles only
+Plan plan_fwd(int64_t batch, int64_t items) { return plan_ranges(batch, items, 1 << 20); }
+// gradient partials are [ranges][rows][D]: at most about four waves' worth of CTAs, so the workspace stays
+// within a few row-tile multiples of B x D (I x D)
+Plan plan_grad(int64_t rows, int64_t cols) {
+  const int64_t row_tiles = (rows + TILE - 1) / TILE;
+  const int64_t cap = (4 * kNumSMs + row_tiles - 1) / row_tiles;
+  return plan_ranges(rows, cols, (int)(cap < 1 ? 1 : cap));
+}
+
+bool softmax_dim_ok(int dim) { return dim == 64 || dim == 128 || dim == 192 || dim == 256; }
+
+struct Layout {
+  size_t s_pair, e_pair, fwd_part, grad_part, total;
+};
+Layout layout(int64_t batch, int64_t items, int dim) {
+  Layout l;
+  l.s_pair = align_up((size_t)batch * dim * 2);
+  l.e_pair = align_up((size_t)items * dim * 2);
+  const Plan pf = plan_fwd(batch, items), ps = plan_grad(batch, items), pe = plan_grad(items, batch);
+  l.fwd_part = align_up((size_t)3 * pf.ranges * batch * sizeof(float));
+  const size_t gs = ps.ranges > 1 ? (size_t)ps.ranges * batch * dim * sizeof(float) : 0;
+  const size_t ge = pe.ranges > 1 ? (size_t)pe.ranges * items * dim * sizeof(float) : 0;
+  l.grad_part = align_up(gs > ge ? gs : ge);
+  l.total = 2 * l.s_pair + 2 * l.e_pair + (l.fwd_part > l.grad_part ? l.fwd_part : l.grad_part) + 256;
+  return l;
+}
+
+struct Operands {
+  CUtensorMap s_hi, s_lo, e_hi, e_lo;
+  float* part;
+};
+
+// splits sess and table into their bf16 pairs inside the workspace and encodes the four tensor maps
+int prepare(const float* sess, const float* table, int64_t batch, int64_t items, int dim, void* ws, size_t ws_bytes,
+            cudaStream_t stream, Operands* o) {
+  const Layout l = layout(batch, items, dim);
+  if (ws == nullptr || ws_bytes < l.total) {
+    set_error("full_softmax: workspace too small (%zu < %zu bytes)", ws_bytes, l.total);
+    return ETPGT_EWORKSPACE;
+  }
+  Workspace w(ws, ws_bytes);
+  void* s_hi = w.take<char>(l.s_pair);
+  void* s_lo = w.take<char>(l.s_pair);
+  void* e_hi = w.take<char>(l.e_pair);
+  void* e_lo = w.take<char>(l.e_pair);
+  o->part = w.take<float>((l.fwd_part > l.grad_part ? l.fwd_part : l.grad_part) / sizeof(float));
+  int rc = etpgt_split_bf16(sess, batch, dim, dim, s_hi, s_lo, dim, nullptr, nullptr, 0, nullptr, nullptr, 0, stream);
+  if (rc != ETPGT_OK) return rc;
+  rc = etpgt_split_bf16(table, items, dim, dim, e_hi, e_lo, dim, nullptr, nullptr, 0, nullptr, nullptr, 0, stream);
+  if (rc != ETPGT_OK) return rc;
+  if (!(make_map_bf16(&o->s_hi, s_hi, batch, dim, dim, TILE) && make_map_bf16(&o->s_lo, s_lo, batch, dim, dim, TILE) &&
+        make_map_bf16(&o->e_hi, e_hi, items, dim, dim, TILE) && make_map_bf16(&o->e_lo, e_lo, items, dim, dim, TILE))) {
+    set_error("full_softmax: cuTensorMapEncodeTiled failed");
+    return ETPGT_ECUDA;
+  }
+  return ETPGT_OK;
+}
+
+int check_args(const float* sess, const float* table, const int64_t* targets, int64_t batch, int64_t items, int dim,
+               float temperature, int64_t padding_idx) {
+  ETPGT_REQUIRE(softmax_dim_ok(dim), "full_softmax: dim %d is not supported (dim must be one of 64, 128, 192, 256)",
+                dim);
+  ETPGT_REQUIRE(batch >= 1 && items >= 2 && batch < (int64_t(1) << 31) && items < (int64_t(1) << 31),
+                "full_softmax: need batch >= 1 and num_items >= 2 (got %lld, %lld)", (long long)batch,
+                (long long)items);
+  ETPGT_REQUIRE(sess != nullptr && table != nullptr && targets != nullptr, "full_softmax: null argument");
+  ETPGT_REQUIRE(temperature > 0.f, "full_softmax: temperature must be positive");
+  ETPGT_REQUIRE(padding_idx >= -1 && padding_idx < items, "full_softmax: padding_idx must be -1 or an item id");
+  return ETPGT_OK;
+}
+
+template <int MODE>
+int launch(const CUtensorMap& r_hi, const CUtensorMap& r_lo, const CUtensorMap& c_hi, const CUtensorMap& c_lo,
+           const Params& p, int grid, cudaStream_t stream) {
+  const size_t smem = Cfg<MODE>::smem + sizeof(Bars);
+  cudaFuncSetAttribute(full_softmax_tc_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  full_softmax_tc_kernel<MODE><<<grid, kThreads, smem, stream>>>(r_hi, r_lo, c_hi, c_lo, p);
+  ETPGT_CHECK_LAUNCH(MODE == FWD ? "full_softmax_fwd" : MODE == DS ? "full_softmax_bwd_sess" : "full_softmax_bwd_table");
+  return ETPGT_OK;
+}
+
+}  // namespace
+}  // namespace etpgt
+
+using namespace etpgt;
+
+extern "C" size_t etpgt_full_softmax_workspace_bytes(int64_t batch, int64_t num_items, int dim) {
+  if (batch < 1 || num_items < 1 || dim < 1) return 256;
+  return layout(batch, num_items, dim).total;
+}
+
+extern "C" int etpgt_full_softmax_fwd(const float* sess, const float* table, const int64_t* targets, int64_t batch,
+                                      int64_t num_items, int dim, float temperature, double total_sessions,
+                                      int64_t padding_idx, float* lse, float* loss, void* ws, size_t ws_bytes,
+                                      etpgt_stream_t stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  int rc = check_args(sess, table, targets, batch, num_items, dim, temperature, padding_idx);
+  if (rc != ETPGT_OK) return rc;
+  ETPGT_REQUIRE(lse != nullptr && loss != nullptr, "full_softmax_fwd: lse and loss are required");
+  Operands o;
+  rc = prepare(sess, table, batch, num_items, dim, ws, ws_bytes, stream, &o);
+  if (rc != ETPGT_OK) return rc;
+  const Plan pl = plan_fwd(batch, num_items);
+  Params p = {};
+  p.rows = batch;
+  p.cols = num_items;
+  p.dim = dim;
+  p.tiles_per_range = pl.tiles_per_range;
+  p.ranges = pl.ranges;
+  p.inv_t = 1.f / temperature;
+  p.targets = targets;
+  p.padding_idx = padding_idx;
+  p.part = o.part;
+  rc = launch<FWD>(o.s_hi, o.s_lo, o.e_hi, o.e_lo, p, pl.grid, stream);
+  if (rc != ETPGT_OK) return rc;
+  const double total = total_sessions > 0 ? total_sessions : (double)batch;
+  fwd_combine_kernel<<<1, kCombineThreads, 0, stream>>>(o.part, pl.ranges, pl.tiles_per_range, batch, num_items,
+                                                        targets, total, lse, loss);
+  ETPGT_CHECK_LAUNCH("full_softmax_fwd_combine");
+  return ETPGT_OK;
+}
+
+extern "C" int etpgt_full_softmax_bwd(const float* sess, const float* table, const int64_t* targets, const float* lse,
+                                      const float* d_loss, int64_t batch, int64_t num_items, int dim, float temperature,
+                                      double total_sessions, int64_t padding_idx, float* d_sess,
+                                      float* d_table_accumulate, void* ws, size_t ws_bytes, etpgt_stream_t stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  int rc = check_args(sess, table, targets, batch, num_items, dim, temperature, padding_idx);
+  if (rc != ETPGT_OK) return rc;
+  ETPGT_REQUIRE(lse != nullptr && d_loss != nullptr, "full_softmax_bwd: lse and d_loss are required");
+  if (d_sess == nullptr && d_table_accumulate == nullptr) return ETPGT_OK;
+  Operands o;
+  rc = prepare(sess, table, batch, num_items, dim, ws, ws_bytes, stream, &o);
+  if (rc != ETPGT_OK) return rc;
+  const double total = total_sessions > 0 ? total_sessions : (double)batch;
+  Params p = {};
+  p.dim = dim;
+  p.inv_t = 1.f / temperature;
+  p.gscale = (float)(1.0 / ((double)temperature * total));
+  p.targets = targets;
+  p.lse = lse;
+  p.d_loss = d_loss;
+  p.padding_idx = padding_idx;
+  p.part = o.part;
+  if (d_sess != nullptr) {
+    const Plan pl = plan_grad(batch, num_items);
+    p.rows = batch;
+    p.cols = num_items;
+    p.tiles_per_range = pl.tiles_per_range;
+    p.ranges = pl.ranges;
+    p.out = d_sess;
+    rc = launch<DS>(o.s_hi, o.s_lo, o.e_hi, o.e_lo, p, pl.grid, stream);
+    if (rc != ETPGT_OK) return rc;
+    if (pl.ranges > 1) {
+      grad_combine_kernel<<<grid_for(batch * dim / 4, 256, 8), 256, 0, stream>>>(o.part, pl.ranges, batch, dim, 0, -1,
+                                                                                 d_sess);
+      ETPGT_CHECK_LAUNCH("full_softmax_bwd_sess_combine");
+    }
+  }
+  if (d_table_accumulate != nullptr) {
+    const Plan pl = plan_grad(num_items, batch);
+    p.rows = num_items;
+    p.cols = batch;
+    p.tiles_per_range = pl.tiles_per_range;
+    p.ranges = pl.ranges;
+    p.out = d_table_accumulate;
+    rc = launch<DE>(o.e_hi, o.e_lo, o.s_hi, o.s_lo, p, pl.grid, stream);
+    if (rc != ETPGT_OK) return rc;
+    if (pl.ranges > 1) {
+      grad_combine_kernel<<<grid_for(num_items * dim / 4, 256, 8), 256, 0, stream>>>(
+          o.part, pl.ranges, num_items, dim, 1, padding_idx, d_table_accumulate);
+      ETPGT_CHECK_LAUNCH("full_softmax_bwd_table_combine");
+    }
+  }
+  return ETPGT_OK;
+}

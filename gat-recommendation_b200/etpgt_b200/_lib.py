@@ -90,6 +90,9 @@ _PROTOTYPES = {
     "etpgt_sampled_loss_workspace_bytes": (Z, [L, I, I]),
     "etpgt_sampled_loss_fwd": (I, [P, P, P, P, L, I, I, I, F, F, D, P, P, P, Z, P]),
     "etpgt_sampled_loss_bwd": (I, [P, P, P, P, L, I, I, I, F, F, D, P, P, L, L, P, P, P, Z, P]),
+    "etpgt_full_softmax_workspace_bytes": (Z, [L, L, I]),
+    "etpgt_full_softmax_fwd": (I, [P, P, P, L, L, I, F, D, L, P, P, P, Z, P]),
+    "etpgt_full_softmax_bwd": (I, [P, P, P, P, P, L, L, I, F, D, L, P, P, P, Z, P]),
     "etpgt_score_topk_workspace_bytes": (Z, [L, L, I, I]),
     "etpgt_score_topk_f32": (I, [P, P, L, L, I, I, L, P, P, P, Z, P]),
     "etpgt_f32_to_bf16": (I, [P, P, L, P]),

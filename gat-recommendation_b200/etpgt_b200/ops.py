@@ -1374,6 +1374,67 @@ def sampled_loss(sess, item_embeddings, targets, negatives, kind: str, alpha=0.7
                              total_sessions, padding_idx)
 
 
+# ------------------------------------------------------------------------------ full-catalogue softmax
+
+
+class FullSoftmaxLoss(torch.autograd.Function):
+    """Cross-entropy over every item of the table (the padding row left out), etpgt_full_softmax_fwd / _bwd:
+    tcgen05 split-bf16 GEMMs with the softmax in the epilogue, so the [B, I] logits never exist.  Returns the
+    scalar mean over `total_sessions` (default: the batch)."""
+
+    @staticmethod
+    def forward(ctx, sess, table, targets, temperature, total_sessions, padding_idx):
+        _require_cuda(sess, "session embeddings")
+        _require_cuda(table, "item embeddings")
+        _require_cuda(targets, "targets")
+        sess_c, table_c, targets = _f32(sess), _f32(table), _i64(targets)
+        if sess_c.dim() != 2 or table_c.dim() != 2 or sess_c.size(1) != table_c.size(1):
+            raise RuntimeError(f"full_softmax_loss: sess [B, D] and table [I, D] expected; got "
+                               f"{tuple(sess_c.shape)} and {tuple(table_c.shape)}")
+        b, dim = sess_c.shape
+        if targets.dim() != 1 or targets.size(0) != b:
+            raise RuntimeError(f"target_items must be [batch={b}]; got {tuple(targets.shape)}")
+        dev = sess_c.device
+        total = float(total_sessions if total_sessions else b)
+        pad = -1 if padding_idx is None else int(padding_idx)
+        lse = torch.empty(b, dtype=torch.float32, device=dev)
+        loss = torch.empty(1, dtype=torch.float32, device=dev)
+        ws = workspace(size("etpgt_full_softmax_workspace_bytes", b, table_c.size(0), dim), dev)
+        call("etpgt_full_softmax_fwd", ptr(sess_c), ptr(table_c), ptr(targets), b, table_c.size(0), dim,
+             float(temperature), total, pad, ptr(lse), ptr(loss), ptr(ws), ws.numel(), stream())
+        ctx.save_for_backward(sess_c, table_c, targets, lse)
+        ctx.table_ref = table
+        ctx.meta = (float(temperature), total, pad)
+        ctx.mark_non_differentiable(lse)
+        return loss[0], lse
+
+    @staticmethod
+    def backward(ctx, d_loss, _d_lse):
+        sess, table, targets, lse = ctx.saved_tensors
+        temperature, total, pad = ctx.meta
+        b, dim = sess.shape
+        dev = sess.device
+        d_loss = _f32(d_loss).reshape(1).contiguous()
+        d_sess = torch.empty_like(sess) if ctx.needs_input_grad[0] else None
+        d_table = sink = None
+        if ctx.needs_input_grad[1]:
+            sink = _grad_sink(ctx.table_ref)
+            d_table = sink if sink is not None else torch.zeros_like(table)
+        ws = workspace(size("etpgt_full_softmax_workspace_bytes", b, table.size(0), dim), dev)
+        call("etpgt_full_softmax_bwd", ptr(sess), ptr(table), ptr(targets), ptr(lse), ptr(d_loss), b, table.size(0),
+             dim, temperature, total, pad, ptr(d_sess), ptr(d_table), ptr(ws), ws.numel(), stream())
+        return d_sess, (None if sink is not None else d_table), None, None, None, None
+
+
+def full_softmax_loss(sess, item_embeddings, targets, temperature=1.0, total_sessions=None) -> torch.Tensor:
+    """Softmax cross-entropy of `targets` over the whole catalogue.  `item_embeddings` is the nn.Embedding (its
+    padding_idx column is left out of the softmax and its row gets no gradient) or a bare weight tensor.  The table
+    gradient goes into the etpgt_b200.optim gradient sink when one is registered, else it is returned densely."""
+    weight = item_embeddings.weight if hasattr(item_embeddings, "weight") else item_embeddings
+    padding_idx = getattr(item_embeddings, "padding_idx", None)
+    return FullSoftmaxLoss.apply(sess, weight, targets, temperature, total_sessions, padding_idx)[0]
+
+
 # ------------------------------------------------------------------------------ scoring / top-k
 
 

@@ -1,3 +1,3 @@
-from .losses import BPRLoss, DualLoss, ListwiseLoss, SampledSoftmaxLoss, create_loss_function
+from .losses import BPRLoss, DualLoss, FullSoftmaxLoss, ListwiseLoss, SampledSoftmaxLoss, create_loss_function
 
-__all__ = ["BPRLoss", "DualLoss", "ListwiseLoss", "SampledSoftmaxLoss", "create_loss_function"]
+__all__ = ["BPRLoss", "DualLoss", "FullSoftmaxLoss", "ListwiseLoss", "SampledSoftmaxLoss", "create_loss_function"]

@@ -1,6 +1,6 @@
-"""BPR / listwise / dual / sampled-softmax losses with the reference's call signature
+"""BPR / listwise / dual / sampled-softmax / full-catalogue softmax losses with the reference's call signature
 `loss(session_embeddings, target_items, negative_items, item_embeddings: nn.Embedding)`
-(etpgt/train/losses.py), computed by the fused sampled-loss kernel."""
+(etpgt/train/losses.py), computed by the fused sampled-loss kernel (full_softmax: the tensor-core full-catalogue kernels)."""
 
 from __future__ import annotations
 
@@ -46,6 +46,19 @@ class SampledSoftmaxLoss(ListwiseLoss):
     """Softmax over target + sampled negatives: identical to the listwise loss (losses.py:198-201)."""
 
 
+class FullSoftmaxLoss(nn.Module):
+    """Softmax cross-entropy over the whole catalogue (SR-GNN / GCE-GNN style) instead of the sampled negatives;
+    `negative_items` is accepted for the common signature and not used.  Deliberately not a ListwiseLoss: the fused
+    step driver has no full-catalogue mode, so the trainer takes the per-operator path for it."""
+
+    def __init__(self, temperature: float = 1.0):
+        super().__init__()
+        self.temperature = temperature
+
+    def forward(self, session_embeddings, target_items, negative_items, item_embeddings) -> torch.Tensor:
+        return ops.full_softmax_loss(session_embeddings, item_embeddings, target_items, temperature=self.temperature)
+
+
 def create_loss_function(loss_type: str = "dual", alpha: float = 0.7, temperature: float = 1.0) -> nn.Module:
     if loss_type == "bpr":
         return BPRLoss()
@@ -55,4 +68,6 @@ def create_loss_function(loss_type: str = "dual", alpha: float = 0.7, temperatur
         return DualLoss(alpha=alpha, temperature=temperature)
     if loss_type == "sampled_softmax":
         return SampledSoftmaxLoss(temperature=temperature)
+    if loss_type == "full_softmax":
+        return FullSoftmaxLoss(temperature=temperature)
     raise ValueError(f"Unknown loss type: {loss_type}")

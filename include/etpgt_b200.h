@@ -438,6 +438,26 @@ int etpgt_sampled_loss_bwd(const float* sess, const float* table, const int64_t*
                            int64_t padding_idx, float* d_sess, float* d_table, void* ws, size_t ws_bytes,
                            etpgt_stream_t stream);
 
+/* ---- a8: full-catalogue softmax cross-entropy (tensor cores) ----------------------------
+ * Replaces the listwise loss of etpgt/train/losses.py and the scoring of etpgt/model/base.py:80-113 with the
+ * objective over the whole catalogue: z = sess . table^T / temperature over every item except padding_idx (-1: none),
+ * lse[b] = logsumexp_j z[b, j], loss = sum_b (lse[b] - z[b, targets[b]]) / total_sessions (<= 0: batch; the GLOBAL
+ * batch under data parallelism).  tcgen05 split-bf16 GEMMs with the softmax in the epilogue: the [batch, num_items]
+ * logits are never materialised.  dim in {64, 128, 192, 256}; any batch >= 1, num_items >= 2.  Deterministic.
+ * fwd: lse [batch] (saved for backward) and loss [1] are written.
+ * bwd: d_loss is a device scalar.  d_sess [batch, dim] is overwritten; d_table_accumulate [num_items, dim] has
+ * the table gradient ADDED (row padding_idx untouched).  Either may be NULL to skip it.  Both calls take the same
+ * workspace size. */
+size_t etpgt_full_softmax_workspace_bytes(int64_t batch, int64_t num_items, int dim);
+int etpgt_full_softmax_fwd(const float* sess, const float* table, const int64_t* targets, int64_t batch,
+                           int64_t num_items, int dim, float temperature, double total_sessions,
+                           int64_t padding_idx, float* lse, float* loss, void* ws, size_t ws_bytes,
+                           etpgt_stream_t stream);
+int etpgt_full_softmax_bwd(const float* sess, const float* table, const int64_t* targets, const float* lse,
+                           const float* d_loss, int64_t batch, int64_t num_items, int dim, float temperature,
+                           double total_sessions, int64_t padding_idx, float* d_sess,
+                           float* d_table_accumulate, void* ws, size_t ws_bytes, etpgt_stream_t stream);
+
 /* ---- a9/a10: full-catalogue scoring with fused top-k and metrics ------------------------
  * etpgt/model/base.py:59-78, etpgt/utils/metrics.py:6-66.  Scores are never materialised.
  * Ties go to the lower item id.  id_base offsets the ids of an item-table shard. */

@@ -543,7 +543,8 @@ extern "C" int etpgt_sage_mean_fwd_split(const float* x, int64_t num_nodes, int 
                                          const int32_t* col, float* mean, void* mean_hi, void* mean_lo, int64_t ld,
                                          etpgt_stream_t stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  ETPGT_REQUIRE(supported_dim(dim), "sage_mean_fwd: unsupported dim %d", dim);
+  ETPGT_REQUIRE(supported_dim(dim), "sage_mean_fwd: dim %d is not supported (dim must be one of 32, 64, 128, 256)",
+                dim);
   ETPGT_REQUIRE(num_nodes >= 0 && x && rowptr && (mean || mean_hi) && (mean_hi == nullptr) == (mean_lo == nullptr),
                 "sage_mean_fwd: bad arguments");
   ETPGT_REQUIRE(mean_hi == nullptr || (ld >= dim && ld % 4 == 0 && (((uintptr_t)mean_hi | (uintptr_t)mean_lo) & 7) == 0),
@@ -571,7 +572,8 @@ extern "C" int etpgt_sage_mean_bwd_ld(const float* d_mean, int64_t ld, const flo
                                       const int32_t* rowptr, const int32_t* colptr, const int32_t* row, float* d_x,
                                       etpgt_stream_t stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  ETPGT_REQUIRE(supported_dim(dim), "sage_mean_bwd: unsupported dim %d", dim);
+  ETPGT_REQUIRE(supported_dim(dim), "sage_mean_bwd: dim %d is not supported (dim must be one of 32, 64, 128, 256)",
+                dim);
   ETPGT_REQUIRE(num_nodes >= 0 && d_mean && rowptr && colptr && d_x && ld >= dim && ld % 4 == 0,
                 "sage_mean_bwd: bad arguments");
   if (num_nodes == 0) return ETPGT_OK;

@@ -178,6 +178,177 @@ bool fill_scalars(AdamScalars& s, double lr, double beta1, double beta2, double 
   return true;
 }
 
+// ---------------------------------------------------------------------------- row-sparse ("lazy") updates
+// The item table's gradient touches only the rows of the batch (its items + negatives): at B = 1,024 and 82k
+// items ~10 % of them.  These kernels read the whole gradient (4 B per element) but load, update and store
+// p / m / v (and clear g) only for touched rows: rows * dim * 4 + touched * dim * 28 bytes instead of 32 per
+// element.  A row is touched iff an element of its gradient row compares != 0 (+0 and -0 do not, NaN does).
+// Listed mode (torch sparse gradients) instead updates every listed row, all-zero ones included.
+
+// torch/optim/_functional.py::sparse_adam, one rounding per torch op (no FMA contraction):
+//   mu = (g - m) * (1-b1);  m += mu;  vu = (g*g - v) * (1-b2);  v += vu
+//   p += (-step_size) * ((mu + m_old) / (sqrt(vu + v_old) + eps))
+struct SparseScalars {
+  float one_minus_b1, one_minus_b2, neg_step_size, eps;
+  int maximize;
+};
+
+__device__ __forceinline__ void sparse_adam_one(float& p, float g, float& m, float& v, const SparseScalars& s) {
+  if (s.maximize) g = -g;
+  const float mu = __fmul_rn(__fsub_rn(g, m), s.one_minus_b1);
+  const float vu = __fmul_rn(__fsub_rn(__fmul_rn(g, g), v), s.one_minus_b2);
+  const float numer = __fadd_rn(mu, m);
+  const float denom = __fadd_rn(__fsqrt_rn(__fadd_rn(vu, v)), s.eps);
+  m = __fadd_rn(m, mu);
+  v = __fadd_rn(v, vu);
+  p = __fadd_rn(p, __fmul_rn(__fdiv_rn(numer, denom), s.neg_step_size));
+}
+
+// adam_one outside the caller's data flow: inlined into a kernel, nvcc picks which of the two products of
+// `v * b2 + (1-b2) * g * g` it contracts into an FMA from the surrounding code, and the row kernels for
+// DIM <= 128 got the other one than adam_step_kernel (results 1 ulp apart).  Compiled once as its own function it
+// takes adam_step_kernel's choice, so a touched row is bit-identical to the dense step.
+struct AdamPMV {
+  float p, m, v;
+};
+__device__ __noinline__ AdamPMV adam_one_isolated(float p, float g, float m, float v, const AdamScalars s) {
+  adam_one(p, g, m, v, s);
+  return {p, m, v};
+}
+struct AdamRowOp {
+  AdamScalars s;
+  __device__ __forceinline__ void operator()(float& p, float& g, float& m, float& v) const {
+    const AdamPMV r = adam_one_isolated(p, g, m, v, s);
+    p = r.p;
+    m = r.m;
+    v = r.v;
+  }
+};
+struct SparseAdamRowOp {
+  SparseScalars s;
+  __device__ __forceinline__ void operator()(float& p, float& g, float& m, float& v) const {
+    sparse_adam_one(p, g, m, v, s);
+  }
+};
+
+constexpr int kRowThreads = 256;
+constexpr int kRowCtasPerSM = 8;
+
+struct RowArgs {
+  float *param, *grad, *exp_avg, *exp_avg_sq;   // [rows, dim]; grad: [rows, dim] (scan) or [count, dim] (listed)
+  const int64_t* index;                         // listed mode: table row of gradient row i
+  int64_t rows, count;                          // count: gradient rows (scan: == rows)
+  int dim, zero_grad;                           // zero_grad: clear touched gradient rows (scan mode)
+  unsigned long long* touched;                  // optional: += rows updated
+};
+
+__device__ __forceinline__ bool nonzero4(float4 a) { return a.x != 0.f || a.y != 0.f || a.z != 0.f || a.w != 0.f; }
+
+__device__ __forceinline__ void count_touched(unsigned n, unsigned long long* touched) {
+  if (touched == nullptr) return;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
+  if ((threadIdx.x & 31) == 0 && n) atomicAdd(touched, (unsigned long long)n);
+}
+
+// DIM in {32, 64, 128, 256}: one lane group (RowGeom) per gradient row, grid-stride; float4 accesses (the caller
+// checks 16-byte alignment).  The loop bound is warp-uniform, so every lane reaches the ballot.
+template <int DIM, bool LISTED, class Op>
+__global__ void __launch_bounds__(kRowThreads) adam_rows_kernel(const RowArgs a, const Op op) {
+  using G = RowGeom<DIM>;
+  const int lane = threadIdx.x & 31;
+  const int grp = lane / G::LPN, lig = lane % G::LPN;
+  const unsigned grp_mask = (G::LPN == 32 ? 0xffffffffu : ((1u << G::LPN) - 1u)) << (grp * G::LPN);
+  const int64_t warp = ((int64_t)blockIdx.x * kRowThreads + threadIdx.x) >> 5;
+  const int64_t nwarps = ((int64_t)gridDim.x * kRowThreads) >> 5;
+  unsigned updated = 0;
+  for (int64_t first = warp * G::GROUPS; first < a.count; first += nwarps * G::GROUPS) {
+    const int64_t i = first + grp;
+    int64_t row = i;
+    bool live = i < a.count;
+    if (LISTED && live) {
+      row = a.index[i];
+      live = row >= 0 && row < a.rows;
+    }
+    float4 g[G::V];
+    bool nz = false;
+    if (live) {
+      const float* gr = a.grad + i * DIM;
+#pragma unroll
+      for (int v = 0; v < G::V; ++v) {
+        g[v] = ld4(gr + 4 * (v * G::LPN + lig));
+        nz |= nonzero4(g[v]);
+      }
+    }
+    if ((__ballot_sync(0xffffffffu, LISTED ? live : nz) & grp_mask) == 0) continue;
+    const int64_t off = row * DIM;
+#pragma unroll
+    for (int v = 0; v < G::V; ++v) {
+      const int64_t e = off + 4 * (v * G::LPN + lig);
+      float4 P = ld4(a.param + e), M = ld4(a.exp_avg + e), V = ld4(a.exp_avg_sq + e);
+      op(P.x, g[v].x, M.x, V.x);
+      op(P.y, g[v].y, M.y, V.y);
+      op(P.z, g[v].z, M.z, V.z);
+      op(P.w, g[v].w, M.w, V.w);
+      st4(a.param + e, P);
+      st4(a.exp_avg + e, M);
+      st4(a.exp_avg_sq + e, V);
+      if (!LISTED && a.zero_grad) st4(a.grad + i * DIM + 4 * (v * G::LPN + lig), zero4());
+    }
+    if (lig == 0) ++updated;
+  }
+  count_touched(updated, a.touched);
+}
+
+// any other dim: one warp per gradient row, scalar accesses
+template <bool LISTED, class Op>
+__global__ void __launch_bounds__(kRowThreads) adam_rows_scalar_kernel(const RowArgs a, const Op op) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp = ((int64_t)blockIdx.x * kRowThreads + threadIdx.x) >> 5;
+  const int64_t nwarps = ((int64_t)gridDim.x * kRowThreads) >> 5;
+  const int64_t dim = a.dim;
+  unsigned updated = 0;
+  for (int64_t i = warp; i < a.count; i += nwarps) {
+    int64_t row = i;
+    if (LISTED) {
+      row = a.index[i];
+      if (row < 0 || row >= a.rows) continue;   // warp-uniform
+    }
+    float* gr = a.grad + i * dim;
+    if (!LISTED) {
+      bool nz = false;
+      for (int64_t c = lane; c < dim; c += 32) nz |= gr[c] != 0.f;
+      if (!__any_sync(0xffffffffu, nz)) continue;
+    }
+    const int64_t off = row * dim;
+    for (int64_t c = lane; c < dim; c += 32) {
+      float P = a.param[off + c], Gv = gr[c], M = a.exp_avg[off + c], V = a.exp_avg_sq[off + c];
+      op(P, Gv, M, V);
+      a.param[off + c] = P;
+      a.exp_avg[off + c] = M;
+      a.exp_avg_sq[off + c] = V;
+      if (!LISTED && a.zero_grad) gr[c] = 0.f;
+    }
+    if (lane == 0) ++updated;
+  }
+  count_touched(updated, a.touched);
+}
+
+template <bool LISTED, class Op>
+void launch_rows(const RowArgs& a, const Op& op, cudaStream_t stream) {
+  const int rows_per_cta = (kRowThreads / 32) * (a.dim == 32 ? 4 : a.dim == 64 ? 2 : 1);
+  const int grid = grid_for(a.count, rows_per_cta, kRowCtasPerSM);
+  switch (a.dim) {
+    case 32: adam_rows_kernel<32, LISTED><<<grid, kRowThreads, 0, stream>>>(a, op); break;
+    case 64: adam_rows_kernel<64, LISTED><<<grid, kRowThreads, 0, stream>>>(a, op); break;
+    case 128: adam_rows_kernel<128, LISTED><<<grid, kRowThreads, 0, stream>>>(a, op); break;
+    case 256: adam_rows_kernel<256, LISTED><<<grid, kRowThreads, 0, stream>>>(a, op); break;
+    default: adam_rows_scalar_kernel<LISTED><<<grid, kRowThreads, 0, stream>>>(a, op); break;
+  }
+}
+
+bool aligned16(const void* p) { return ((uintptr_t)p & 15) == 0; }
+
 }  // namespace
 }  // namespace etpgt
 
@@ -272,5 +443,79 @@ extern "C" int etpgt_dp_adam_table(const etpgt_comm_t* comm, size_t param_offset
     dp_adam_table_kernel<2, 8><<<grid_of(2), kThreads, 0, stream>>>(c, a, s);
   }
   ETPGT_CHECK_LAUNCH("dp_adam_table");
+  return ETPGT_OK;
+}
+
+namespace {
+
+int check_rows(const char* name, const float* param, const float* grad, const float* exp_avg,
+               const float* exp_avg_sq, int64_t rows, int dim, int64_t step) {
+  ETPGT_REQUIRE(rows >= 0 && dim >= 1 && rows < (int64_t(1) << 40) / dim, "%s: bad shape (rows %lld, dim %d)", name,
+                (long long)rows, dim);
+  ETPGT_REQUIRE(param && grad && exp_avg && exp_avg_sq, "%s: NULL pointer", name);
+  ETPGT_REQUIRE(step >= 1, "%s: step must be >= 1 (1-based, as torch counts it)", name);
+  ETPGT_REQUIRE(!supported_dim(dim) ||
+                    (aligned16(param) && aligned16(grad) && aligned16(exp_avg) && aligned16(exp_avg_sq)),
+                "%s: buffers must be 16-byte aligned for dim %d", name, dim);
+  return ETPGT_OK;
+}
+
+}  // namespace
+
+extern "C" int etpgt_adam_rows(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int64_t rows, int dim,
+                               double lr, double beta1, double beta2, double eps, double weight_decay, int decoupled,
+                               int64_t step, int zero_grad, int64_t* touched, etpgt_stream_t stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  const int rc = check_rows("adam_rows", param, grad, exp_avg, exp_avg_sq, rows, dim, step);
+  if (rc != ETPGT_OK) return rc;
+  ETPGT_REQUIRE(beta1 >= 0.0 && beta1 < 1.0 && beta2 >= 0.0 && beta2 < 1.0 && eps >= 0.0 && lr >= 0.0 &&
+                    weight_decay >= 0.0,
+                "adam_rows: hyper-parameters out of range");
+  if (touched && cudaMemsetAsync(touched, 0, sizeof(int64_t), stream) != cudaSuccess) {
+    set_error("adam_rows: clearing the touched-row counter failed");
+    return ETPGT_ECUDA;
+  }
+  if (rows == 0) return ETPGT_OK;
+  AdamRowOp op;
+  fill_scalars(op.s, lr, beta1, beta2, eps, weight_decay, decoupled, step, zero_grad);
+  const RowArgs a{param, grad, exp_avg, exp_avg_sq, nullptr, rows, rows, dim, zero_grad != 0,
+                  reinterpret_cast<unsigned long long*>(touched)};
+  launch_rows<false>(a, op, stream);
+  ETPGT_CHECK_LAUNCH("adam_rows");
+  return ETPGT_OK;
+}
+
+extern "C" int etpgt_sparse_adam(float* param, float* exp_avg, float* exp_avg_sq, int64_t rows, int dim, float* grad,
+                                 const int64_t* indices, int64_t nnz, double lr, double beta1, double beta2, double eps,
+                                 int maximize, int64_t step, int zero_grad, int64_t* touched, etpgt_stream_t stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  const bool listed = indices != nullptr;
+  const int rc = check_rows("sparse_adam", param, grad, exp_avg, exp_avg_sq, rows, dim, step);
+  if (rc != ETPGT_OK) return rc;
+  ETPGT_REQUIRE(!listed || (nnz >= 0 && nnz < (int64_t(1) << 40) / dim),
+                "sparse_adam: bad number of listed rows (%lld)", (long long)nnz);
+  ETPGT_REQUIRE(!listed || zero_grad == 0, "sparse_adam: zero_grad applies to the dense (scan) mode only");
+  ETPGT_REQUIRE(beta1 >= 0.0 && beta1 < 1.0 && beta2 >= 0.0 && beta2 < 1.0 && eps >= 0.0 && lr >= 0.0,
+                "sparse_adam: hyper-parameters out of range");
+  if (touched && cudaMemsetAsync(touched, 0, sizeof(int64_t), stream) != cudaSuccess) {
+    set_error("sparse_adam: clearing the touched-row counter failed");
+    return ETPGT_ECUDA;
+  }
+  const int64_t count = listed ? nnz : rows;
+  if (count == 0 || rows == 0) return ETPGT_OK;
+  // constants as torch forms them: Python floats (double), rounded to fp32 where they meet the fp32 tensors
+  const double bc1 = 1.0 - pow(beta1, (double)step);
+  const double bc2 = 1.0 - pow(beta2, (double)step);
+  SparseAdamRowOp op;
+  op.s.one_minus_b1 = (float)(1.0 - beta1);
+  op.s.one_minus_b2 = (float)(1.0 - beta2);
+  op.s.neg_step_size = (float)(-(lr * sqrt(bc2) / bc1));
+  op.s.eps = (float)eps;
+  op.s.maximize = maximize != 0;
+  const RowArgs a{param, grad, exp_avg, exp_avg_sq, indices, rows, count, dim, zero_grad != 0,
+                  reinterpret_cast<unsigned long long*>(touched)};
+  if (listed) launch_rows<true>(a, op, stream);
+  else launch_rows<false>(a, op, stream);
+  ETPGT_CHECK_LAUNCH("sparse_adam");
   return ETPGT_OK;
 }

@@ -123,6 +123,8 @@ _PROTOTYPES = {
     "etpgt_graph_rebuilds": (L, [P]),
     "etpgt_gt_step_run_graph": (I, [P, I, I, P, P]),
     "etpgt_adam_step": (I, [P, I, D, D, D, D, D, I, L, I, P]),
+    "etpgt_adam_rows": (I, [P, P, P, P, L, I, D, D, D, D, D, I, L, I, P, P]),
+    "etpgt_sparse_adam": (I, [P, P, P, L, I, P, P, L, D, D, D, D, I, L, I, P, P]),
     "etpgt_topk_merge_parts": (I, [P, I, Z, Z, L, I, L, L, P, P, P, P, P]),
     "etpgt_hit_metrics": (I, [P, L, I, P, P]),
     "etpgt_ids_check": (I, [P, L, P, L, P, L, L, P, P]),

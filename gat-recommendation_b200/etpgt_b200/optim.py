@@ -17,6 +17,14 @@ Data parallelism over peer memory (`parallel.PeerDataParallel`, created BEFORE t
 gradient buffer inside this rank's peer region, and `step()` runs the whole gradient exchange itself —
 barrier, dense-gradient sum over the peers, the table's reduce-scatter + AdamW + all-gather as one kernel
 (`etpgt_dp_adam_table`), barrier — so no `allreduce_gradients` call and no NCCL collective is on the step.
+
+Row-sparse ("lazy") updates of the sink tables, for large catalogues and small batches where a step touches a few
+percent of the item rows: `AdamW(..., lazy_rows=True)` / `Adam(..., lazy_rows=True)` step each sink table with
+`etpgt_adam_rows` (rows whose gradient row is all zero keep their value and moments: no weight decay, no moment
+decay — NOT the reference's dense semantics), and `SparseAdam` is torch.optim.SparseAdam on `etpgt_sparse_adam`.
+Both read the whole gradient but move p / m / v only for touched rows.  Under data parallelism they need the NCCL
+exchange (every rank sees the same summed sink, so all make the same row decisions); a row-sparse table inside a
+peer region raises NotImplementedError.
 """
 
 from __future__ import annotations
@@ -65,17 +73,13 @@ def grad_sink_for(table: torch.Tensor):
     return buf
 
 
-class _DeviceAdam(torch.optim.Optimizer):
-    _decoupled = True
+class _SinkOptimizer(torch.optim.Optimizer):
+    """Gradient-sink bookkeeping shared by the device optimizers (see the module docstring)."""
 
-    def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, amsgrad=False,
-                 grad_sinks=True, sink_bytes=4 << 20):
-        if amsgrad:
-            raise NotImplementedError("etpgt_b200 optimizers implement amsgrad=False (the reference's setting)")
-        if lr < 0.0 or eps < 0.0 or weight_decay < 0.0 or not 0.0 <= betas[0] < 1.0 or not 0.0 <= betas[1] < 1.0:
-            raise ValueError("Invalid optimizer hyper-parameter")
-        defaults = dict(lr=lr, betas=tuple(betas), eps=eps, weight_decay=weight_decay, amsgrad=False)
-        super().__init__(params, defaults)
+    # row-sparse update of the sink tables (lazy AdamW / Adam, SparseAdam): they keep no exchange over peer memory
+    row_sparse = False
+
+    def _install_sinks(self, grad_sinks: bool, sink_bytes: int) -> None:
         self._dirty = False
         self._sinks: list[torch.nn.Parameter] = []
         self._plan_key = None
@@ -96,6 +100,8 @@ class _DeviceAdam(torch.optim.Optimizer):
         from .parallel import peer_for
 
         peer = peer_for(p)
+        if peer is not None and self.row_sparse:
+            self._refuse_peer()
         if peer is not None:       # the gradient buffer inside the peer region: the other ranks read it
             buf, self._peer = peer.table_grad, peer
         else:
@@ -108,6 +114,8 @@ class _DeviceAdam(torch.optim.Optimizer):
         """Moves the item table's gradient sink into the peer region of `peer` (parallel.PeerDataParallel created
         AFTER this optimizer, e.g. by Trainer(process_group=...)): the table's storage address changed when it was
         re-homed, so the old registration is dropped and the region's gradient buffer takes over."""
+        if self.row_sparse:
+            self._refuse_peer()
         for group in self.param_groups:
             for p in group["params"]:
                 if p.data_ptr() != peer.table.data_ptr():
@@ -118,6 +126,12 @@ class _DeviceAdam(torch.optim.Optimizer):
                 self._sinks = [q for q in self._sinks if q is not p]
                 self._install_sink(p)
         self._plan_key = None
+
+    def _refuse_peer(self):
+        raise NotImplementedError(
+            f"{type(self).__name__}: a row-sparse table update over peer memory is not implemented; "
+            'use data parallelism with exchange="nccl" (Trainer(..., exchange="nccl") or '
+            'parallel.enable_data_parallel(model, group, exchange="nccl"))')
 
     def _is_sink(self, p) -> bool:
         entry = _GRAD_SINKS.get(p.data_ptr())
@@ -138,6 +152,23 @@ class _DeviceAdam(torch.optim.Optimizer):
                         p.grad.detach_()
                         p.grad.zero_()
         self._dirty = False
+
+
+class _DeviceAdam(_SinkOptimizer):
+    _decoupled = True
+
+    def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, amsgrad=False,
+                 grad_sinks=True, sink_bytes=4 << 20, lazy_rows=False):
+        if amsgrad:
+            raise NotImplementedError("etpgt_b200 optimizers implement amsgrad=False (the reference's setting)")
+        if lr < 0.0 or eps < 0.0 or weight_decay < 0.0 or not 0.0 <= betas[0] < 1.0 or not 0.0 <= betas[1] < 1.0:
+            raise ValueError("Invalid optimizer hyper-parameter")
+        if lazy_rows and not grad_sinks:
+            raise ValueError("lazy_rows=True updates the tables that have a gradient sink: it needs grad_sinks=True")
+        defaults = dict(lr=lr, betas=tuple(betas), eps=eps, weight_decay=weight_decay, amsgrad=False)
+        super().__init__(params, defaults)
+        self.lazy_rows = self.row_sparse = bool(lazy_rows)
+        self._install_sinks(grad_sinks, sink_bytes)
 
     # ------------------------------------------------------------------ the step
     @torch.no_grad()
@@ -230,18 +261,23 @@ class _DeviceAdam(torch.optim.Optimizer):
         key = tuple((p.data_ptr(), g.data_ptr(), self.state[p]["exp_avg"].data_ptr(),
                      self.state[p]["exp_avg_sq"].data_ptr()) for p, g in zip(plist, grads))
         if key != self._plan_key:
-            plain, sinks = [], []
+            plain, sinks, lazy = [], [], []
             for p, g in zip(plist, grads):
                 if not p.is_contiguous():
                     raise RuntimeError("etpgt_b200 optimizers need contiguous parameters")
                 st = self.state[p]
                 entry = _AdamTensor(p.data_ptr(), g.data_ptr(), st["exp_avg"].data_ptr(),
                                     st["exp_avg_sq"].data_ptr(), p.numel())
-                (sinks if self._is_sink(p) else plain).append(entry)
+                if not self._is_sink(p):
+                    plain.append(entry)
+                elif self.lazy_rows:      # one row-sparse launch per table
+                    lazy.append((entry.param, entry.grad, entry.exp_avg, entry.exp_avg_sq, p.size(0), p.size(1)))
+                else:
+                    sinks.append(entry)
             self._plan_key = key
             self._plan = ((_AdamTensor * max(len(plain), 1))(*plain), len(plain),
-                          (_AdamTensor * max(len(sinks), 1))(*sinks), len(sinks))
-        arr_plain, n_plain, arr_sink, n_sink = self._plan
+                          (_AdamTensor * max(len(sinks), 1))(*sinks), len(sinks), lazy)
+        arr_plain, n_plain, arr_sink, n_sink, lazy = self._plan
         common = (float(group["lr"]), float(beta1), float(beta2), float(group["eps"]), float(group["weight_decay"]),
                   int(self._decoupled), int(step_no))
         # the sink gradients are cleared by the kernel (zero_grad flag); the others are released by
@@ -250,6 +286,8 @@ class _DeviceAdam(torch.optim.Optimizer):
             _lib.call("etpgt_adam_step", arr_plain, n_plain, *common, 0, stream())
         if n_sink:
             _lib.call("etpgt_adam_step", arr_sink, n_sink, *common, 1, stream())
+        for table in lazy:
+            _lib.call("etpgt_adam_rows", *table, *common, 1, None, stream())
 
 
 class AdamW(_DeviceAdam):
@@ -268,3 +306,86 @@ class Adam(_DeviceAdam):
 
     def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, amsgrad=False, **kw):
         super().__init__(params, lr, betas, eps, weight_decay, amsgrad, **kw)
+
+
+class SparseAdam(_SinkOptimizer):
+    """torch.optim.SparseAdam on `etpgt_sparse_adam`: the same constructor checks, the same state (integer `step`,
+    `exp_avg`, `exp_avg_sq`; state dicts load both ways with torch's class) and the same fp32 arithmetic, one
+    rounding per torch operation.  Only the rows present in a step's gradient move: their moments and values are
+    updated, every other row keeps its bits.
+
+    * A sparse COO gradient (`nn.Embedding(sparse=True)`) is coalesced and every listed row is updated, all-zero
+      rows included, as in torch.
+    * Unlike torch, a dense gradient is accepted too: its rows with a nonzero element (or a NaN) are updated.  This
+      is how the item table is trained here: 2-D fp32 CUDA parameters of at least `sink_bytes` get a persistent
+      gradient buffer (a sink, as for `AdamW`) that the backward kernels accumulate rows into and the step clears.
+    """
+
+    row_sparse = True
+
+    def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, maximize=False, *, grad_sinks=True,
+                 sink_bytes=4 << 20):
+        if isinstance(lr, torch.Tensor) and lr.numel() != 1:
+            raise ValueError("Tensor lr must be 1-element")
+        if not 0.0 < lr:
+            raise ValueError(f"Invalid learning rate: {lr}")
+        if not 0.0 < eps:
+            raise ValueError(f"Invalid epsilon value: {eps}")
+        if not 0.0 <= betas[0] < 1.0:
+            raise ValueError(f"Invalid beta parameter at index 0: {betas[0]}")
+        if not 0.0 <= betas[1] < 1.0:
+            raise ValueError(f"Invalid beta parameter at index 1: {betas[1]}")
+        super().__init__(params, dict(lr=lr, betas=betas, eps=eps, maximize=maximize))
+        for index, group in enumerate(self.param_groups):
+            for d_index, p in enumerate(group["params"]):
+                if p.is_sparse:
+                    raise ValueError(f"Sparse params at indices {[[index, d_index]]}: SparseAdam requires dense "
+                                     "parameter tensors")
+                if p.is_complex():
+                    raise ValueError(f"Complex params at indices {[[index, d_index]]}: SparseAdam does not support "
+                                     "complex parameters")
+        self._install_sinks(grad_sinks, sink_bytes)
+
+    @torch.no_grad()
+    def step(self, closure=None):
+        loss = None
+        if closure is not None:
+            with torch.enable_grad():
+                loss = closure()
+        for group in self.param_groups:
+            beta1, beta2 = group["betas"]
+            lr = float(group["lr"])
+            for p in group["params"]:
+                if p.grad is None:
+                    continue
+                if not (p.is_cuda and p.dtype == torch.float32 and p.is_contiguous()):
+                    raise RuntimeError("etpgt_b200 SparseAdam needs contiguous fp32 CUDA parameters (no CPU fallback)")
+                state = self.state[p]
+                if len(state) == 0:
+                    state["step"] = 0
+                    state["exp_avg"] = torch.zeros_like(p, memory_format=torch.preserve_format)
+                    state["exp_avg_sq"] = torch.zeros_like(p, memory_format=torch.preserve_format)
+                state["step"] += 1
+                rows = p.size(0) if p.dim() else 1
+                dim = p.numel() // rows if rows else 1
+                grad = p.grad
+                if grad.is_sparse:
+                    grad = grad.coalesce()
+                    if grad.sparse_dim() != 1 or grad.dtype != torch.float32:
+                        raise RuntimeError("SparseAdam: sparse gradients must be fp32 with one sparse dimension "
+                                           "(rows, as nn.Embedding(sparse=True) produces)")
+                    index = grad._indices()[0].contiguous()
+                    values = grad._values().contiguous()
+                    if values.numel() == 0:      # torch skips an empty gradient (the step still counts)
+                        continue
+                    g_ptr, i_ptr, nnz, zero = _lib.ptr(values), _lib.ptr(index), index.numel(), 0
+                else:
+                    if grad.dtype != torch.float32 or not grad.is_contiguous():
+                        raise RuntimeError("SparseAdam: dense gradients must be contiguous fp32")
+                    g_ptr, i_ptr, nnz, zero = _lib.ptr(grad), None, 0, int(self._is_sink(p))
+                _lib.call("etpgt_sparse_adam", _lib.ptr(p), _lib.ptr(state["exp_avg"]),
+                          _lib.ptr(state["exp_avg_sq"]), rows, dim, g_ptr, i_ptr, nnz, lr, float(beta1),
+                          float(beta2), float(group["eps"]), int(bool(group["maximize"])), int(state["step"]), zero,
+                          None, stream())
+        self._dirty = False
+        return loss

@@ -79,6 +79,10 @@ class Trainer:
             if exchange == "peer" and not ours:
                 logger.warning("exchange='peer' needs an etpgt_b200.optim optimizer; using NCCL all-reduces")
                 exchange = "nccl"
+            elif exchange == "peer" and getattr(optimizer, "row_sparse", False):
+                logger.warning("exchange='peer' has no row-sparse table update (lazy_rows=True / SparseAdam); "
+                               "using NCCL all-reduces")
+                exchange = "nccl"
             self._peer = parallel.enable_data_parallel(self.model, self._group, exchange)
             if self._peer is not None:
                 optimizer.attach_peer(self._peer)      # the table moved into the peer region after the optimizer was built

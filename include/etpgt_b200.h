@@ -541,6 +541,29 @@ typedef struct etpgt_adam_tensor {
 int etpgt_adam_step(const etpgt_adam_tensor* tensors, int count, double lr, double beta1, double beta2,
                     double eps, double weight_decay, int decoupled, int64_t step, int zero_grad,
                     etpgt_stream_t stream);
+/* Row-sparse ("lazy") AdamW / Adam over ONE [rows, dim] fp32 table with a dense gradient buffer.  A row is
+ * touched iff an element of its gradient row compares != 0 (+0 / -0 do not, NaN does).  Every element of a
+ * touched row gets exactly the etpgt_adam_step update (decoupled / L2 decay of touched rows only, bias
+ * corrections from the global `step`) and, with zero_grad != 0, its gradient row is cleared; an untouched
+ * row's parameter and moments are neither read nor written.  NOT equivalent to the dense step (which decays
+ * and moves every row).  Bytes: rows*dim*4 + touched*dim*28.  dim in {32, 64, 128, 256} needs 16-byte aligned
+ * buffers; any other dim >= 1 takes a scalar path.  `touched` (optional, device int64) receives the number of
+ * rows updated.  No allocation, no synchronisation. */
+int etpgt_adam_rows(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int64_t rows, int dim,
+                    double lr, double beta1, double beta2, double eps, double weight_decay, int decoupled,
+                    int64_t step, int zero_grad, int64_t* touched, etpgt_stream_t stream);
+/* torch.optim.SparseAdam's arithmetic (torch/optim/_functional.py::sparse_adam, one fp32 rounding per torch
+ * op, no contraction; step_size = lr*sqrt(1-b2^step)/(1-b1^step) formed in double; maximize negates g) over
+ * one [rows, dim] table.  Two modes:
+ *   indices == NULL (scan): `grad` is a dense [rows, dim] buffer; touched rows as etpgt_adam_rows, cleared
+ *     with zero_grad != 0.
+ *   indices != NULL (listed): a coalesced sparse gradient, `indices` [nnz] strictly ascending rows and `grad`
+ *     its values [nnz, dim]; every listed row is updated (all-zero ones too: torch's index-set semantics),
+ *     listed rows outside [0, rows) are skipped; zero_grad must be 0.
+ * Alignment, `touched`, allocation and synchronisation as etpgt_adam_rows. */
+int etpgt_sparse_adam(float* param, float* exp_avg, float* exp_avg_sq, int64_t rows, int dim, float* grad,
+                      const int64_t* indices, int64_t nnz, double lr, double beta1, double beta2, double eps,
+                      int maximize, int64_t step, int zero_grad, int64_t* touched, etpgt_stream_t stream);
 
 /* ---- §8(f3): co-occurrence graph construction ----------------------------------------------
  * scripts/data/04_build_graph.py:25-127 (`build_co_event_graph`): sessions are

@@ -72,7 +72,7 @@ inline int grid_for(int64_t work_units, int units_per_cta, int ctas_per_sm) {
 template <int DIM>
 struct RowGeom {
   static constexpr int F4 = DIM / 4;                 // float4 per row
-  static constexpr int LPN = F4 < 32 ? F4 : 32;      // lanes per node
+  static constexpr int LPN = F4 < 32 ? F4 : F4 % 32 == 0 ? 32 : 16;  // lanes per node (16 for DIM = 192)
   static constexpr int V = F4 / LPN;                 // float4 per lane
   static constexpr int GROUPS = 32 / LPN;            // nodes per warp
 };

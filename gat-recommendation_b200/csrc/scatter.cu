@@ -168,7 +168,8 @@ extern "C" int etpgt_scatter_rows(const int64_t* keys, const float* coef, const 
                                   int src_div, int dim, int64_t num_rows, int64_t skip_key, float* d_table,
                                   void* ws, size_t ws_bytes, etpgt_stream_t stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  ETPGT_REQUIRE(supported_dim(dim), "scatter_rows: unsupported dim %d", dim);
+  // 192 as well: the table gradient of the shared-pool softmax, whose dims are those of the tensor-core losses
+  ETPGT_REQUIRE(supported_dim(dim) || dim == 192, "scatter_rows: unsupported dim %d", dim);
   ETPGT_REQUIRE(m >= 0 && m < (int64_t(1) << 31) && num_rows < (int64_t(1) << 31) && src_div >= 1,
                 "scatter_rows: bad size");
   if (m == 0) return ETPGT_OK;
@@ -195,7 +196,11 @@ extern "C" int etpgt_scatter_rows(const int64_t* keys, const float* coef, const 
     segment_rows_add_kernel<D><<<grid_for(m, (int)gpc, 8), kThreads, 0, stream>>>(key_s, perm, coef, src, m, \
                                                                                  src_div, (int)skip_key, d_table); \
   }
-  ETPGT_DISPATCH_DIM(dim, CALL)
+  if (dim == 192) {
+    CALL(192);
+  } else {
+    ETPGT_DISPATCH_DIM(dim, CALL)
+  }
 #undef CALL
   ETPGT_CHECK_LAUNCH("segment_rows_add");
   return ETPGT_OK;

@@ -20,6 +20,19 @@
 // The backward recomputes the forward's logits bit for bit (same MMA sequence, operands swapped in DE) and keeps
 // them, lse and the running maxima in natural units (exp(x) = 2^(x log2 e) on the MUFU unit): where the softmax
 // is exact — one eligible column, P = 1 — the gradient is exactly zero, not rounding noise.
+//
+// The same kernel, instantiated with POOL, computes the sampled softmax over one pool of M negatives shared by the
+// batch, with the log-Q correction (Bengio & Senecal 2008; Jean et al. 2015; Yi et al. 2019).  For pool ids p [M]
+// (ascending) and log_q[j] = log(M q(p_j)):
+//   z_pos[b]  = s_b . e_{t_b} / T                  (the positive: no correction)
+//   z[b, j]   = s_b . e_{p_j} / T - log_q[j]       (-inf where p_j == t_b or p_j == padding_idx)
+//   lse[b]    = logsumexp(z_pos[b], z[b, :]),   loss = sum_b (lse[b] - z_pos[b]) / B_total
+// exp(z_pos) + sum_j exp(z_j) is an unbiased estimate of the full partition function, and a pool holding every
+// non-padding item once with log_q = 0 gives the full-catalogue loss.  The columns are the gathered pool rows; the
+// accidental hits of a session are one range of positions of the sorted pool ([hit_lo, hit_hi), masked by a
+// position compare) and the padding entries get log_q = +inf.  The positive is an fp32 gather-dot outside the
+// kernel, folded into lse by the combine; DE writes d_pool [M, D] and two row scatters add it, and the
+// positive's c_b s_b, into the table.
 #include <math.h>
 
 #include "tc_common.cuh"
@@ -81,9 +94,11 @@ struct Params {
   int64_t padding_idx;          // item id left out (-1: none)
   float* part;                  // FWD: [3][ranges][rows]; DS / DE with ranges > 1: [ranges][rows][dim]
   float* out;                   // DS: d_sess (written), DE: d_table (added), when ranges == 1
+  const float* bias;            // POOL: per column (FWD, DS) or row (DE): log_q, +inf for a padding entry
+  const int2* hits;             // POOL: per session, the pool positions [x, y) equal to its target
 };
 
-template <int MODE>
+template <int MODE, bool POOL = false>
 __global__ void __launch_bounds__(kThreads, 1)
 full_softmax_tc_kernel(const __grid_constant__ CUtensorMap map_r_hi, const __grid_constant__ CUtensorMap map_r_lo,
                        const __grid_constant__ CUtensorMap map_c_hi, const __grid_constant__ CUtensorMap map_c_lo,
@@ -230,7 +245,8 @@ full_softmax_tc_kernel(const __grid_constant__ CUtensorMap map_r_hi, const __gri
     const bool row_ok = row < p.rows;
     const uint32_t lane_addr = tmem_base + ((uint32_t)(q * 32) << 16);
     if constexpr (MODE == FWD) {
-      const int64_t tgt = row_ok ? p.targets[row] : -1;
+      const int64_t tgt = !POOL && row_ok ? p.targets[row] : -1;
+      const int2 hit = POOL && row_ok ? p.hits[row] : make_int2(0, 0);
       float m = -INFINITY, s = 0.f, zt = 0.f;
       for (int j = 0; j < n; ++j) {
         const int b = j & 1;
@@ -248,15 +264,28 @@ full_softmax_tc_kernel(const __grid_constant__ CUtensorMap map_r_hi, const __gri
           }
           const int64_t base = col0 + c;
           const int lim = p.cols - base < 32 ? (int)(p.cols - base) : 32;
-          const int pad_e = chunk_pos(p.padding_idx, base), tgt_e = chunk_pos(tgt, base);
           float y[32];
           float mc = -INFINITY;
+          if constexpr (POOL) {
+            // lane e holds column e's log_q; the row's accidental hits as positions in the chunk
+            const float bias_lane = lane < lim ? p.bias[base + lane] : 0.f;
+            const int hit_lo = (int)max((int64_t)0, min((int64_t)32, hit.x - base));
+            const int hit_hi = (int)max((int64_t)0, min((int64_t)32, hit.y - base));
 #pragma unroll
-          for (int e = 0; e < 32; ++e) {
-            y[e] = __uint_as_float(v[e]) * p.inv_t;
-            if (e >= lim || e == pad_e) y[e] = -INFINITY;
-            if (e == tgt_e) zt = y[e];
-            mc = fmaxf(mc, y[e]);
+            for (int e = 0; e < 32; ++e) {
+              y[e] = __fmaf_rn(__uint_as_float(v[e]), p.inv_t, -__shfl_sync(0xffffffffu, bias_lane, e));
+              if (e >= lim || (e >= hit_lo && e < hit_hi)) y[e] = -INFINITY;
+              mc = fmaxf(mc, y[e]);
+            }
+          } else {
+            const int pad_e = chunk_pos(p.padding_idx, base), tgt_e = chunk_pos(tgt, base);
+#pragma unroll
+            for (int e = 0; e < 32; ++e) {
+              y[e] = __uint_as_float(v[e]) * p.inv_t;
+              if (e >= lim || e == pad_e) y[e] = -INFINITY;
+              if (e == tgt_e) zt = y[e];
+              mc = fmaxf(mc, y[e]);
+            }
           }
           if (mc == -INFINITY) continue;  // nothing of this chunk takes part
           if (mc > m) {
@@ -276,20 +305,24 @@ full_softmax_tc_kernel(const __grid_constant__ CUtensorMap map_r_hi, const __gri
       const float gscale = __ldg(p.d_loss) * p.gscale;
       float lse_row = 0.f;
       int64_t tgt_row = -1;
+      int2 hit = make_int2(0, 0);
       if (MODE == DS && row_ok) {
         lse_row = p.lse[row];
-        tgt_row = p.targets[row];
+        if constexpr (POOL) hit = p.hits[row];
+        else tgt_row = p.targets[row];
       }
+      const float bias_row = POOL && MODE == DE && row_ok ? p.bias[row] : 0.f;
       uint8_t* g_row = smem_g + r_local * 128;
       const bool direct = p.ranges == 1;
-      const bool store = row_ok && !(MODE == DE && row == p.padding_idx);
+      // POOL: rows of DE are pool positions, and d_pool is written whole
+      const bool store = row_ok && !(!POOL && MODE == DE && row == p.padding_idx);
       float* dst = direct ? p.out + row * p.dim : p.part + ((int64_t)range * p.rows + row) * p.dim;
       // group `group` of column tiles is complete in the accumulator: add it to this thread's row in fp32 (the first
       // group overwrites, except that d_table is always accumulated into), then hand the accumulator back
       auto drain = [&](int group) {
         mbar_wait(&bars->accfull, (uint32_t)group & 1);
         tc_fence_after();
-        const bool add = group > 0 || (MODE == DE && direct);
+        const bool add = group > 0 || (!POOL && MODE == DE && direct);
 #pragma unroll 1
         for (int c = 0; c < p.dim; c += 32) {
           uint32_t v[32];
@@ -328,22 +361,48 @@ full_softmax_tc_kernel(const __grid_constant__ CUtensorMap map_r_hi, const __gri
           const int lim = !row_ok ? 0 : p.cols - base < 32 ? (int)(p.cols - base) : 32;
           // DS: the padding column and the row's target as positions in the chunk.  DE: the chunk's 32 columns are
           // sessions; lane e fetches column e's lse and its target as a row of this CTA (-1: none), shared by shuffles
-          int pad_e = -1, tgt_e = -1, tgt_lane = -1;
-          float lse_lane = 0.f;
+          // POOL, DS: lane e holds column e's log_q, and the row's hits are positions in the chunk.  POOL, DE: lane e
+          // packs session e's hits as rows of this CTA, [tgt_lane & 0xffff, tgt_lane >> 16)
+          int pad_e = -1, tgt_e = -1, tgt_lane = POOL ? 0 : -1, hit_lo = 0, hit_hi = 0;
+          float lse_lane = 0.f, bias_lane = 0.f;
           if constexpr (MODE == DS) {
-            pad_e = chunk_pos(p.padding_idx, base);
-            tgt_e = chunk_pos(tgt_row, base);
+            if constexpr (POOL) {
+              if (base + lane < p.cols) bias_lane = p.bias[base + lane];
+              hit_lo = (int)max((int64_t)0, min((int64_t)32, hit.x - base));
+              hit_hi = (int)max((int64_t)0, min((int64_t)32, hit.y - base));
+            } else {
+              pad_e = chunk_pos(p.padding_idx, base);
+              tgt_e = chunk_pos(tgt_row, base);
+            }
           } else if (base + lane < p.cols) {
             lse_lane = p.lse[base + lane];
-            const int64_t t = p.targets[base + lane] - (int64_t)rt * TILE;
-            tgt_lane = t >= 0 && t < TILE ? (int)t : -1;
+            if constexpr (POOL) {
+              const int2 h = p.hits[base + lane];
+              const int64_t r0 = (int64_t)rt * TILE;
+              const int lo = (int)max((int64_t)0, min((int64_t)TILE, h.x - r0));
+              const int hi = (int)max((int64_t)0, min((int64_t)TILE, h.y - r0));
+              tgt_lane = lo | (hi << 16);
+            } else {
+              const int64_t t = p.targets[base + lane] - (int64_t)rt * TILE;
+              tgt_lane = t >= 0 && t < TILE ? (int)t : -1;
+            }
           }
           float g[32];
 #pragma unroll
           for (int e = 0; e < 32; ++e) {
             const float y = __uint_as_float(v[e]) * p.inv_t;
             float pr;
-            if constexpr (MODE == DS) {
+            if constexpr (POOL && MODE == DS) {
+              const float z = __fmaf_rn(__uint_as_float(v[e]), p.inv_t, -__shfl_sync(0xffffffffu, bias_lane, e));
+              pr = fast_exp2((z - lse_row) * kLog2e);
+              if (e >= lim || (e >= hit_lo && e < hit_hi)) pr = 0.f;
+            } else if constexpr (POOL) {
+              const float l = __shfl_sync(0xffffffffu, lse_lane, e);
+              const int t = __shfl_sync(0xffffffffu, tgt_lane, e);
+              const float z = __fmaf_rn(__uint_as_float(v[e]), p.inv_t, -bias_row);
+              pr = fast_exp2((z - l) * kLog2e);
+              if (e >= lim || (r_local >= (t & 0xffff) && r_local < (t >> 16))) pr = 0.f;
+            } else if constexpr (MODE == DS) {
               pr = fast_exp2((y - lse_row) * kLog2e) - (e == tgt_e ? 1.f : 0.f);
               if (e >= lim || e == pad_e) pr = 0.f;
             } else {
@@ -527,13 +586,205 @@ int check_args(const float* sess, const float* table, const int64_t* targets, in
   return ETPGT_OK;
 }
 
-template <int MODE>
+template <int MODE, bool POOL = false>
 int launch(const CUtensorMap& r_hi, const CUtensorMap& r_lo, const CUtensorMap& c_hi, const CUtensorMap& c_lo,
            const Params& p, int grid, cudaStream_t stream) {
   const size_t smem = Cfg<MODE>::smem + sizeof(Bars);
-  cudaFuncSetAttribute(full_softmax_tc_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  full_softmax_tc_kernel<MODE><<<grid, kThreads, smem, stream>>>(r_hi, r_lo, c_hi, c_lo, p);
-  ETPGT_CHECK_LAUNCH(MODE == FWD ? "full_softmax_fwd" : MODE == DS ? "full_softmax_bwd_sess" : "full_softmax_bwd_table");
+  cudaFuncSetAttribute(full_softmax_tc_kernel<MODE, POOL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  full_softmax_tc_kernel<MODE, POOL><<<grid, kThreads, smem, stream>>>(r_hi, r_lo, c_hi, c_lo, p);
+  if (POOL) {
+    ETPGT_CHECK_LAUNCH(MODE == FWD ? "pool_softmax_fwd" : MODE == DS ? "pool_softmax_bwd_sess" : "pool_softmax_bwd_pool");
+  } else {
+    ETPGT_CHECK_LAUNCH(MODE == FWD ? "full_softmax_fwd" : MODE == DS ? "full_softmax_bwd_sess" : "full_softmax_bwd_table");
+  }
+  return ETPGT_OK;
+}
+
+// ---------------------------------------------------------------------------- shared-pool softmax: small kernels
+
+// pool rows gathered from the table and split into the bf16 pair (hi = bf16(x), lo = bf16(x - hi), as
+// etpgt_split_bf16), and bias[j] = log_q[j], or +inf for a padding entry (its logit is then -inf in every pass)
+__global__ void __launch_bounds__(256)
+pool_gather_split_kernel(const int64_t* __restrict__ pool, const float* __restrict__ log_q,
+                         const float* __restrict__ table, int64_t m, int dim, int64_t padding_idx,
+                         __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo, float* __restrict__ bias) {
+  const int q = dim / 4;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < m * q; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t j = i / q;
+    const int64_t id = pool[j];
+    const int k = (int)(i - j * q) * 4;
+    if (k == 0) bias[j] = id == padding_idx ? INFINITY : log_q[j];
+    const float4 x = ldg4(table + id * dim + k);
+    const float xs[4] = {x.x, x.y, x.z, x.w};
+#pragma unroll
+    for (int t = 0; t < 4; ++t) {
+      const __nv_bfloat16 h = __float2bfloat16_rn(xs[t]);
+      hi[j * dim + k + t] = h;
+      lo[j * dim + k + t] = __float2bfloat16_rn(xs[t] - __bfloat162float(h));
+    }
+  }
+}
+
+// one warp per session: its hit range [lower_bound, upper_bound) of the target in the sorted pool and, with
+// z_pos != NULL, z_pos = (s_b . e_{t_b}) / T in fp32 (lane-strided products, then a fixed butterfly)
+__global__ void __launch_bounds__(256)
+pool_rows_kernel(const float* __restrict__ sess, const float* __restrict__ table, const int64_t* __restrict__ targets,
+                 const int64_t* __restrict__ pool, int64_t batch, int64_t m, int dim, float inv_t,
+                 int2* __restrict__ hits, float* __restrict__ z_pos) {
+  const int lane = threadIdx.x & 31;
+  const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+  for (int64_t b = blockIdx.x * (int64_t)(blockDim.x >> 5) + (threadIdx.x >> 5); b < batch; b += nwarps) {
+    const int64_t t = targets[b];
+    if (lane == 0) {
+      int64_t lo = 0, hi = m;
+      while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (pool[mid] < t) lo = mid + 1; else hi = mid;
+      }
+      int64_t lo2 = lo, hi2 = m;
+      while (lo2 < hi2) {
+        const int64_t mid = (lo2 + hi2) >> 1;
+        if (pool[mid] <= t) lo2 = mid + 1; else hi2 = mid;
+      }
+      hits[b] = make_int2((int)lo, (int)lo2);
+    }
+    if (z_pos == nullptr) continue;
+    float acc = 0.f;
+    for (int k = lane; k < dim; k += 32) acc = fmaf(sess[b * dim + k], table[t * dim + k], acc);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    if (lane == 0) z_pos[b] = acc * inv_t;
+  }
+}
+
+// lse[b] = logsumexp of the per-range (max, sum) partials and z_pos[b], ranges merged in ascending order; the loss
+// sum_b (lse[b] - z_pos[b]) / total by a fixed tree: one block, deterministic
+__global__ void __launch_bounds__(kCombineThreads)
+pool_combine_kernel(const float* __restrict__ part, int ranges, int64_t rows, const float* __restrict__ z_pos,
+                    double total, float* __restrict__ lse, float* __restrict__ loss) {
+  __shared__ double red[kCombineThreads];
+  double acc = 0.0;
+  for (int64_t b = threadIdx.x; b < rows; b += kCombineThreads) {
+    const float zp = z_pos[b];
+    float m = zp;
+    for (int r = 0; r < ranges; ++r) m = fmaxf(m, part[(int64_t)r * rows + b]);
+    float s = exp2f((zp - m) * kLog2e);
+    for (int r = 0; r < ranges; ++r) {
+      const float mr = part[(int64_t)r * rows + b];
+      if (mr != -INFINITY) s += part[((int64_t)ranges + r) * rows + b] * exp2f((mr - m) * kLog2e);
+    }
+    const float l = m + logf(s);
+    lse[b] = l;
+    acc += (double)(l - zp);
+  }
+  red[threadIdx.x] = acc;
+  __syncthreads();
+  for (int w = kCombineThreads / 2; w > 0; w >>= 1) {
+    if (threadIdx.x < w) red[threadIdx.x] += red[threadIdx.x + w];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) loss[0] = (float)(red[0] / total);
+}
+
+// the positive's gradient: coef[b] = d_loss (exp(z_pos - lse) - 1) / (T B_total) and, with d_sess != NULL,
+// d_sess[b] += coef[b] e_{t_b}; one warp per session
+__global__ void __launch_bounds__(256)
+pool_positive_bwd_kernel(const float* __restrict__ table, const int64_t* __restrict__ targets,
+                         const float* __restrict__ z_pos, const float* __restrict__ lse, const float* __restrict__ d_loss,
+                         int64_t batch, int dim, float gscale, float* __restrict__ coef, float* __restrict__ d_sess) {
+  const int lane = threadIdx.x & 31;
+  const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+  const float dl = __ldg(d_loss) * gscale;
+  for (int64_t b = blockIdx.x * (int64_t)(blockDim.x >> 5) + (threadIdx.x >> 5); b < batch; b += nwarps) {
+    const float c = dl * (expf(z_pos[b] - lse[b]) - 1.f);
+    if (lane == 0) coef[b] = c;
+    if (d_sess == nullptr) continue;
+    const float* e = table + targets[b] * dim;
+    for (int k = lane; k < dim; k += 32) d_sess[b * dim + k] = fmaf(c, e[k], d_sess[b * dim + k]);
+  }
+}
+
+struct PoolLayout {
+  size_t s_pair, c_pair, part, d_pool, bias, hits, coef, scatter, total;
+};
+PoolLayout pool_layout(int64_t batch, int64_t m, int dim) {
+  PoolLayout l;
+  l.s_pair = align_up((size_t)batch * dim * 2);
+  l.c_pair = align_up((size_t)m * dim * 2);
+  const Plan pf = plan_fwd(batch, m), ps = plan_grad(batch, m), pe = plan_grad(m, batch);
+  const size_t fp = (size_t)3 * pf.ranges * batch * sizeof(float);
+  const size_t gs = ps.ranges > 1 ? (size_t)ps.ranges * batch * dim * sizeof(float) : 0;
+  const size_t ge = pe.ranges > 1 ? (size_t)pe.ranges * m * dim * sizeof(float) : 0;
+  l.part = align_up(fp > gs ? (fp > ge ? fp : ge) : (gs > ge ? gs : ge));
+  l.d_pool = align_up((size_t)m * dim * sizeof(float));
+  l.bias = align_up((size_t)m * sizeof(float));
+  l.hits = align_up((size_t)batch * sizeof(int2));
+  l.coef = align_up((size_t)batch * sizeof(float));
+  l.scatter = align_up(etpgt_scatter_rows_workspace_bytes(batch > m ? batch : m));
+  l.total = 2 * l.s_pair + 2 * l.c_pair + l.part + l.d_pool + l.bias + l.hits + l.coef + l.scatter + 256;
+  return l;
+}
+
+struct PoolOperands {
+  CUtensorMap s_hi, s_lo, c_hi, c_lo;
+  float *part, *d_pool, *bias, *coef;
+  int2* hits;
+  void* scatter_ws;
+  size_t scatter_bytes;
+};
+
+int pool_check_args(const float* sess, const float* table, const int64_t* targets, const int64_t* pool_ids,
+                    const float* log_q, int64_t batch, int64_t items, int64_t m, int dim, float temperature,
+                    int64_t padding_idx) {
+  ETPGT_REQUIRE(softmax_dim_ok(dim), "pool_softmax: dim %d is not supported (dim must be one of 64, 128, 192, 256)",
+                dim);
+  ETPGT_REQUIRE(batch >= 1 && batch < (int64_t(1) << 31), "pool_softmax: batch must be in [1, 2^31) (got %lld)",
+                (long long)batch);
+  ETPGT_REQUIRE(m >= 1 && m < (int64_t(1) << 31), "pool_softmax: num_sampled must be in [1, 2^31) (got %lld)",
+                (long long)m);
+  ETPGT_REQUIRE(items >= 1 && items < (int64_t(1) << 31), "pool_softmax: num_items must be in [1, 2^31) (got %lld)",
+                (long long)items);
+  ETPGT_REQUIRE(sess != nullptr && table != nullptr && targets != nullptr && pool_ids != nullptr && log_q != nullptr,
+                "pool_softmax: null argument");
+  ETPGT_REQUIRE(temperature > 0.f, "pool_softmax: temperature must be positive");
+  ETPGT_REQUIRE(padding_idx >= -1 && padding_idx < items, "pool_softmax: padding_idx must be -1 or an item id");
+  return ETPGT_OK;
+}
+
+// splits sess, gathers and splits the pool rows, finds the hit ranges (and z_pos when given) and encodes the maps
+int pool_prepare(const float* sess, const float* table, const int64_t* targets, const int64_t* pool_ids,
+                 const float* log_q, int64_t batch, int64_t m, int dim, float inv_t, int64_t padding_idx,
+                 float* z_pos, void* ws, size_t ws_bytes, cudaStream_t stream, PoolOperands* o) {
+  const PoolLayout l = pool_layout(batch, m, dim);
+  if (ws == nullptr || ws_bytes < l.total) {
+    set_error("pool_softmax: workspace too small (%zu < %zu bytes)", ws_bytes, l.total);
+    return ETPGT_EWORKSPACE;
+  }
+  Workspace w(ws, ws_bytes);
+  void* s_hi = w.take<char>(l.s_pair);
+  void* s_lo = w.take<char>(l.s_pair);
+  auto* c_hi = w.take<__nv_bfloat16>(l.c_pair / 2);
+  auto* c_lo = w.take<__nv_bfloat16>(l.c_pair / 2);
+  o->part = w.take<float>(l.part / sizeof(float));
+  o->d_pool = w.take<float>(l.d_pool / sizeof(float));
+  o->bias = w.take<float>(l.bias / sizeof(float));
+  o->hits = w.take<int2>(l.hits / sizeof(int2));
+  o->coef = w.take<float>(l.coef / sizeof(float));
+  o->scatter_bytes = l.scatter;
+  o->scatter_ws = w.take<char>(l.scatter);
+  int rc = etpgt_split_bf16(sess, batch, dim, dim, s_hi, s_lo, dim, nullptr, nullptr, 0, nullptr, nullptr, 0, stream);
+  if (rc != ETPGT_OK) return rc;
+  pool_gather_split_kernel<<<grid_for(m * dim / 4, 256, 8), 256, 0, stream>>>(pool_ids, log_q, table, m, dim,
+                                                                             padding_idx, c_hi, c_lo, o->bias);
+  ETPGT_CHECK_LAUNCH("pool_softmax_gather");
+  pool_rows_kernel<<<grid_for(batch, 8, 8), 256, 0, stream>>>(sess, table, targets, pool_ids, batch, m, dim, inv_t,
+                                                              o->hits, z_pos);
+  ETPGT_CHECK_LAUNCH("pool_softmax_rows");
+  if (!(make_map_bf16(&o->s_hi, s_hi, batch, dim, dim, TILE) && make_map_bf16(&o->s_lo, s_lo, batch, dim, dim, TILE) &&
+        make_map_bf16(&o->c_hi, c_hi, m, dim, dim, TILE) && make_map_bf16(&o->c_lo, c_lo, m, dim, dim, TILE))) {
+    set_error("pool_softmax: cuTensorMapEncodeTiled failed");
+    return ETPGT_ECUDA;
+  }
   return ETPGT_OK;
 }
 
@@ -629,6 +880,117 @@ extern "C" int etpgt_full_softmax_bwd(const float* sess, const float* table, con
           o.part, pl.ranges, num_items, dim, 1, padding_idx, d_table_accumulate);
       ETPGT_CHECK_LAUNCH("full_softmax_bwd_table_combine");
     }
+  }
+  return ETPGT_OK;
+}
+
+extern "C" size_t etpgt_pool_softmax_workspace_bytes(int64_t batch, int64_t num_sampled, int dim) {
+  if (batch < 1 || num_sampled < 1 || dim < 1) return 256;
+  return pool_layout(batch, num_sampled, dim).total;
+}
+
+extern "C" int etpgt_pool_softmax_fwd(const float* sess, const float* table, const int64_t* targets,
+                                      const int64_t* pool_ids, const float* log_q, int64_t batch, int64_t num_items,
+                                      int64_t num_sampled, int dim, float temperature, double total_sessions,
+                                      int64_t padding_idx, float* lse, float* z_pos, float* loss, void* ws,
+                                      size_t ws_bytes, etpgt_stream_t stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  int rc = pool_check_args(sess, table, targets, pool_ids, log_q, batch, num_items, num_sampled, dim, temperature,
+                           padding_idx);
+  if (rc != ETPGT_OK) return rc;
+  ETPGT_REQUIRE(lse != nullptr && z_pos != nullptr && loss != nullptr,
+                "pool_softmax_fwd: lse, z_pos and loss are required");
+  PoolOperands o;
+  rc = pool_prepare(sess, table, targets, pool_ids, log_q, batch, num_sampled, dim, 1.f / temperature, padding_idx,
+                    z_pos, ws, ws_bytes, stream, &o);
+  if (rc != ETPGT_OK) return rc;
+  const Plan pl = plan_fwd(batch, num_sampled);
+  Params p = {};
+  p.rows = batch;
+  p.cols = num_sampled;
+  p.dim = dim;
+  p.tiles_per_range = pl.tiles_per_range;
+  p.ranges = pl.ranges;
+  p.inv_t = 1.f / temperature;
+  p.padding_idx = -1;
+  p.part = o.part;
+  p.bias = o.bias;
+  p.hits = o.hits;
+  rc = launch<FWD, true>(o.s_hi, o.s_lo, o.c_hi, o.c_lo, p, pl.grid, stream);
+  if (rc != ETPGT_OK) return rc;
+  const double total = total_sessions > 0 ? total_sessions : (double)batch;
+  pool_combine_kernel<<<1, kCombineThreads, 0, stream>>>(o.part, pl.ranges, batch, z_pos, total, lse, loss);
+  ETPGT_CHECK_LAUNCH("pool_softmax_fwd_combine");
+  return ETPGT_OK;
+}
+
+extern "C" int etpgt_pool_softmax_bwd(const float* sess, const float* table, const int64_t* targets,
+                                      const int64_t* pool_ids, const float* log_q, const float* lse,
+                                      const float* z_pos, const float* d_loss, int64_t batch, int64_t num_items,
+                                      int64_t num_sampled, int dim, float temperature, double total_sessions,
+                                      int64_t padding_idx, float* d_sess, float* d_table_accumulate, void* ws,
+                                      size_t ws_bytes, etpgt_stream_t stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  int rc = pool_check_args(sess, table, targets, pool_ids, log_q, batch, num_items, num_sampled, dim, temperature,
+                           padding_idx);
+  if (rc != ETPGT_OK) return rc;
+  ETPGT_REQUIRE(lse != nullptr && z_pos != nullptr && d_loss != nullptr,
+                "pool_softmax_bwd: lse, z_pos and d_loss are required");
+  if (d_sess == nullptr && d_table_accumulate == nullptr) return ETPGT_OK;
+  PoolOperands o;
+  rc = pool_prepare(sess, table, targets, pool_ids, log_q, batch, num_sampled, dim, 1.f / temperature, padding_idx,
+                    nullptr, ws, ws_bytes, stream, &o);
+  if (rc != ETPGT_OK) return rc;
+  const double total = total_sessions > 0 ? total_sessions : (double)batch;
+  Params p = {};
+  p.dim = dim;
+  p.inv_t = 1.f / temperature;
+  p.gscale = (float)(1.0 / ((double)temperature * total));
+  p.lse = lse;
+  p.d_loss = d_loss;
+  p.padding_idx = -1;
+  p.part = o.part;
+  p.bias = o.bias;
+  p.hits = o.hits;
+  if (d_sess != nullptr) {
+    const Plan pl = plan_grad(batch, num_sampled);
+    p.rows = batch;
+    p.cols = num_sampled;
+    p.tiles_per_range = pl.tiles_per_range;
+    p.ranges = pl.ranges;
+    p.out = d_sess;
+    rc = launch<DS, true>(o.s_hi, o.s_lo, o.c_hi, o.c_lo, p, pl.grid, stream);
+    if (rc != ETPGT_OK) return rc;
+    if (pl.ranges > 1) {
+      grad_combine_kernel<<<grid_for(batch * dim / 4, 256, 8), 256, 0, stream>>>(o.part, pl.ranges, batch, dim, 0, -1,
+                                                                                 d_sess);
+      ETPGT_CHECK_LAUNCH("pool_softmax_bwd_sess_combine");
+    }
+  }
+  pool_positive_bwd_kernel<<<grid_for(batch, 8, 8), 256, 0, stream>>>(table, targets, z_pos, lse, d_loss, batch, dim,
+                                                                      p.gscale, o.coef, d_sess);
+  ETPGT_CHECK_LAUNCH("pool_softmax_bwd_positive");
+  if (d_table_accumulate != nullptr) {
+    const Plan pl = plan_grad(num_sampled, batch);
+    p.rows = num_sampled;
+    p.cols = batch;
+    p.tiles_per_range = pl.tiles_per_range;
+    p.ranges = pl.ranges;
+    p.out = o.d_pool;
+    rc = launch<DE, true>(o.c_hi, o.c_lo, o.s_hi, o.s_lo, p, pl.grid, stream);
+    if (rc != ETPGT_OK) return rc;
+    if (pl.ranges > 1) {
+      grad_combine_kernel<<<grid_for(num_sampled * dim / 4, 256, 8), 256, 0, stream>>>(
+          o.part, pl.ranges, num_sampled, dim, 0, -1, o.d_pool);
+      ETPGT_CHECK_LAUNCH("pool_softmax_bwd_pool_combine");
+    }
+    // d_table[p_j] += d_pool[j], then d_table[t_b] += coef[b] s_b: each in ascending position, padding skipped
+    rc = etpgt_scatter_rows(pool_ids, nullptr, o.d_pool, num_sampled, 1, dim, num_items, padding_idx,
+                            d_table_accumulate, o.scatter_ws, o.scatter_bytes, stream);
+    if (rc != ETPGT_OK) return rc;
+    rc = etpgt_scatter_rows(targets, o.coef, sess, batch, 1, dim, num_items, padding_idx, d_table_accumulate,
+                            o.scatter_ws, o.scatter_bytes, stream);
+    if (rc != ETPGT_OK) return rc;
   }
   return ETPGT_OK;
 }

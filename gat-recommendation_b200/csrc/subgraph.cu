@@ -213,10 +213,94 @@ sample_negatives_kernel(uint64_t seed, uint32_t step, int64_t session_base, cons
   }
 }
 
+// Shared negative pool: draw j uses Philox4x32-10 with key (seed lo, seed hi) and counter (j >> 1, "POOL", 0,
+// step), 64-bit word c[2 (j & 1)] | c[2 (j & 1) + 1] << 32.  The second counter word keeps the stream apart from
+// sample_negatives (whose second word is a slot < 64).  r = floor(u W / 2^64) picks the item i with
+// cum[i] <= r < cum[i + 1]: zero-weight items are never drawn.  Stream definition: sample_item_pool in
+// tests/shared_pool_ref.py.
+__device__ __forceinline__ int64_t upper_bound_i64(const int64_t* __restrict__ a, int64_t n, int64_t x) {
+  int64_t lo = 0, hi = n;
+  while (lo < hi) {
+    const int64_t mid = (lo + hi) >> 1;
+    if (a[mid] <= x) lo = mid + 1; else hi = mid;
+  }
+  return lo;
+}
+
+__global__ void __launch_bounds__(kThreads)
+sample_item_pool_kernel(const int64_t* __restrict__ cum, int64_t num_items, int64_t m, uint64_t seed, uint32_t step,
+                        uint64_t* __restrict__ out) {
+  const int64_t j = blockIdx.x * (int64_t)kThreads + threadIdx.x;
+  if (j >= m) return;
+  uint32_t c[4] = {(uint32_t)(j >> 1), 0x504F4F4Cu /* "POOL" */, 0u, step};
+  philox4x32_10(c, (uint32_t)seed, (uint32_t)(seed >> 32));
+  const int h = 2 * (int)(j & 1);
+  const uint64_t u = (uint64_t)c[h] | ((uint64_t)c[h + 1] << 32);
+  const uint64_t r = __umul64hi(u, (uint64_t)cum[num_items]);
+  int64_t i = upper_bound_i64(cum, num_items + 1, (int64_t)r) - 1;
+  if (i > num_items - 1) i = num_items - 1;  // only when W = 0, which the caller rules out
+  out[j] = (uint64_t)i;
+}
+
+// log_q[j] = log(M w / W) of the sorted pool, in fp64
+__global__ void __launch_bounds__(kThreads)
+pool_log_q_kernel(const int64_t* __restrict__ cum, int64_t num_items, const int64_t* __restrict__ pool, int64_t m,
+                  float* __restrict__ log_q) {
+  const int64_t j = blockIdx.x * (int64_t)kThreads + threadIdx.x;
+  if (j >= m) return;
+  const int64_t i = pool[j];
+  const double w = (double)(cum[i + 1] - cum[i]);
+  log_q[j] = (float)log((double)m * w / (double)cum[num_items]);
+}
+
+size_t sort_keys64_temp_bytes(int64_t n) {
+  size_t bytes = 0;
+  cub::DeviceRadixSort::SortKeys(nullptr, bytes, (const uint64_t*)nullptr, (uint64_t*)nullptr, (int)n, 0, 64);
+  return bytes;
+}
+
 }  // namespace
 }  // namespace etpgt
 
 using namespace etpgt;
+
+extern "C" size_t etpgt_sample_item_pool_workspace_bytes(int64_t num_sampled) {
+  const int64_t m = num_sampled > 0 ? num_sampled : 1;
+  return align_up(m * sizeof(uint64_t)) + align_up(sort_keys64_temp_bytes(m)) + 256;
+}
+
+extern "C" int etpgt_sample_item_pool(const int64_t* cum, int64_t num_items, int64_t num_sampled, uint64_t seed,
+                                      uint32_t step, int64_t* pool_ids, float* log_q, void* ws, size_t ws_bytes,
+                                      etpgt_stream_t stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  ETPGT_REQUIRE(num_items >= 1 && num_items < (int64_t(1) << 62), "sample_item_pool: num_items must be >= 1 (got %lld)",
+                (long long)num_items);
+  ETPGT_REQUIRE(num_sampled >= 1 && num_sampled < (int64_t(1) << 31),
+                "sample_item_pool: num_sampled must be in [1, 2^31) (got %lld)", (long long)num_sampled);
+  ETPGT_REQUIRE(cum != nullptr, "sample_item_pool: cum is required");
+  ETPGT_REQUIRE(pool_ids != nullptr && log_q != nullptr, "sample_item_pool: pool_ids and log_q are required");
+  const size_t need = etpgt_sample_item_pool_workspace_bytes(num_sampled);
+  if (ws == nullptr || ws_bytes < need) {
+    set_error("sample_item_pool: workspace too small (%zu < %zu bytes)", ws_bytes, need);
+    return ETPGT_EWORKSPACE;
+  }
+  Workspace w(ws, ws_bytes);
+  uint64_t* drawn = w.take<uint64_t>(num_sampled);
+  size_t temp_bytes = sort_keys64_temp_bytes(num_sampled);
+  void* temp = w.take<char>(temp_bytes);
+  const unsigned grid = (unsigned)((num_sampled + kThreads - 1) / kThreads);
+  sample_item_pool_kernel<<<grid, kThreads, 0, stream>>>(cum, num_items, num_sampled, seed, step, drawn);
+  ETPGT_CHECK_LAUNCH("sample_item_pool");
+  int bits = 1;
+  while (bits < 63 && (int64_t(1) << bits) < num_items) ++bits;
+  cudaError_t err = cub::DeviceRadixSort::SortKeys(temp, temp_bytes, drawn, reinterpret_cast<uint64_t*>(pool_ids),
+                                                   (int)num_sampled, 0, bits, stream);
+  if (err != cudaSuccess) { set_error("sample_item_pool sort: %s", cudaGetErrorString(err)); return ETPGT_ECUDA; }
+  count_launch(4);
+  pool_log_q_kernel<<<grid, kThreads, 0, stream>>>(cum, num_items, pool_ids, num_sampled, log_q);
+  ETPGT_CHECK_LAUNCH("sample_item_pool_log_q");
+  return ETPGT_OK;
+}
 
 extern "C" size_t etpgt_item_graph_workspace_bytes(int64_t num_edges) {
   const int64_t e = num_edges > 0 ? num_edges : 1;

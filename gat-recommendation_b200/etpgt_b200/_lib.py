@@ -31,6 +31,8 @@ _PROTOTYPES = {
     "etpgt_session_subgraphs_count": (I, [P, P, P, P, P, L, I, I, I, P, P, P, Z, P]),
     "etpgt_session_subgraphs_fill": (I, [P, P, P, P, P, P, L, I, I, I, P, P, L, P, P, P, P, P, P, Z, P]),
     "etpgt_sample_negatives": (I, [ctypes.c_uint64, ctypes.c_uint32, L, P, P, P, L, I, L, I, P, P]),
+    "etpgt_sample_item_pool_workspace_bytes": (Z, [L]),
+    "etpgt_sample_item_pool": (I, [P, L, L, ctypes.c_uint64, ctypes.c_uint32, P, P, P, Z, P]),
     "etpgt_embed_pe_fwd": (I, [P, L, P, L, P, I, P, P, I, I, P, P]),
     "etpgt_embed_pe_fwd_split": (I, [P, L, P, L, P, I, P, P, I, I, P, P, P, P]),
     "etpgt_embed_pe_bwd_workspace_bytes": (Z, [L, I, I]),
@@ -93,6 +95,9 @@ _PROTOTYPES = {
     "etpgt_full_softmax_workspace_bytes": (Z, [L, L, I]),
     "etpgt_full_softmax_fwd": (I, [P, P, P, L, L, I, F, D, L, P, P, P, Z, P]),
     "etpgt_full_softmax_bwd": (I, [P, P, P, P, P, L, L, I, F, D, L, P, P, P, Z, P]),
+    "etpgt_pool_softmax_workspace_bytes": (Z, [L, L, I]),
+    "etpgt_pool_softmax_fwd": (I, [P, P, P, P, P, L, L, L, I, F, D, L, P, P, P, P, Z, P]),
+    "etpgt_pool_softmax_bwd": (I, [P, P, P, P, P, P, P, P, L, L, L, I, F, D, L, P, P, P, Z, P]),
     "etpgt_score_topk_workspace_bytes": (Z, [L, L, I, I]),
     "etpgt_score_topk_f32": (I, [P, P, L, L, I, I, L, P, P, P, Z, P]),
     "etpgt_f32_to_bf16": (I, [P, P, L, P]),

@@ -1435,6 +1435,145 @@ def full_softmax_loss(sess, item_embeddings, targets, temperature=1.0, total_ses
     return FullSoftmaxLoss.apply(sess, weight, targets, temperature, total_sessions, padding_idx)[0]
 
 
+# ------------------------------------------------------------------------------ shared-pool sampled softmax
+
+
+def item_sampling_table(counts=None, power=0.75, padding_idx=0, *, num_items=None, device=None) -> torch.Tensor:
+    """The proposal q(i) = w_i / W of `sample_item_pool` as int64 cumulative weights cum [I + 1] (cum[0] = 0,
+    cum[i + 1] = cum[i] + w_i).  w_i = floor(count_i ** power * 2^s) in fp64, with s chosen so that W = cum[I] < 2^62;
+    counts=None is uniform (w_i = 1 before the scaling; `num_items` then gives I).  The padding row and items with
+    count 0 get weight 0 and are never drawn.  On `device` (default: that of `counts`, else CUDA)."""
+    import math
+
+    import numpy as np
+
+    if counts is None:
+        if num_items is None:
+            raise ValueError("item_sampling_table: num_items is required when counts is None")
+        w = np.ones(int(num_items), dtype=np.float64)
+    else:
+        if device is None and isinstance(counts, torch.Tensor):
+            device = counts.device
+        c = (counts.detach().double().cpu().numpy() if isinstance(counts, torch.Tensor)
+             else np.asarray(counts, dtype=np.float64)).reshape(-1)
+        if num_items is not None and c.size != int(num_items):
+            raise ValueError(f"item_sampling_table: {c.size} counts for {num_items} items")
+        if (c < 0).any() or not np.isfinite(c).all():
+            raise ValueError("item_sampling_table: counts must be finite and >= 0")
+        w = np.where(c > 0, np.power(c, float(power)), 0.0)
+    if padding_idx is not None and 0 <= padding_idx < w.size:
+        w[padding_idx] = 0.0
+    total = float(w.sum())
+    if not total > 0.0:
+        raise ValueError("item_sampling_table: no item has a positive weight")
+    s = 61 - math.ceil(math.log2(total))          # every w_i 2^s <= 2^61, so W <= 2^61 < 2^62
+    wi = np.floor(np.ldexp(w, s)).astype(np.int64)
+    cum = np.zeros(w.size + 1, dtype=np.int64)
+    np.cumsum(wi, out=cum[1:])
+    if cum[-1] <= 0:
+        raise ValueError("item_sampling_table: no item has a positive weight")
+    return torch.from_numpy(cum).to(device if device is not None else "cuda")
+
+
+def sample_item_pool(cum: torch.Tensor, num_sampled: int, seed: int, step: int):
+    """`num_sampled` item ids drawn with replacement from the proposal `cum` (item_sampling_table, on the device),
+    sorted ascending, and log_q = log(num_sampled * q(id)) [num_sampled] fp32 (etpgt_sample_item_pool).  The pool
+    depends on (seed, step) only, so data-parallel ranks draw the same one without communicating."""
+    _require_cuda(cum, "cum")
+    cum = _i64(cum)
+    if cum.dim() != 1 or cum.numel() < 2:
+        raise RuntimeError(f"sample_item_pool: cum must be [num_items + 1]; got {tuple(cum.shape)}")
+    m = int(num_sampled)
+    pool = torch.empty(max(m, 0), dtype=torch.int64, device=cum.device)
+    log_q = torch.empty(max(m, 0), dtype=torch.float32, device=cum.device)
+    ws = workspace(size("etpgt_sample_item_pool_workspace_bytes", max(m, 1)), cum.device)
+    call("etpgt_sample_item_pool", ptr(cum), cum.numel() - 1, m, int(seed) & 0xFFFFFFFFFFFFFFFF,
+         int(step) & 0xFFFFFFFF, ptr(pool), ptr(log_q), ptr(ws), ws.numel(), stream())
+    return pool, log_q
+
+
+class PoolSoftmaxLoss(torch.autograd.Function):
+    """Sampled softmax over one pool of negatives shared by the batch, with the log-Q correction
+    (etpgt_pool_softmax_fwd / _bwd, the tensor-core kernels of the full-catalogue loss with the pool rows as columns):
+        z_pos[b] = s_b . e_{t_b} / T,   z[b, j] = s_b . e_{p_j} / T - log_q[j]  (-inf where p_j is t_b or padding)
+        loss = sum_b (logsumexp(z_pos[b], z[b, :]) - z_pos[b]) / total_sessions
+    `validate` checks the pool ids against the table and sorts an unsorted pool (one device-to-host copy); pools from
+    `sample_item_pool` are sorted and in range already.  Returns (loss, lse)."""
+
+    @staticmethod
+    def forward(ctx, sess, table, targets, pool_ids, log_q, temperature, total_sessions, padding_idx, validate):
+        for t, what in ((sess, "session embeddings"), (table, "item embeddings"), (targets, "targets"),
+                        (pool_ids, "pool_ids"), (log_q, "log_q")):
+            _require_cuda(t, what)
+        sess_c, table_c, targets, pool, lq = _f32(sess), _f32(table), _i64(targets), _i64(pool_ids), _f32(log_q)
+        if sess_c.dim() != 2 or table_c.dim() != 2 or sess_c.size(1) != table_c.size(1):
+            raise RuntimeError(f"pool_softmax_loss: sess [B, D] and table [I, D] expected; got "
+                               f"{tuple(sess_c.shape)} and {tuple(table_c.shape)}")
+        b, dim = sess_c.shape
+        items = table_c.size(0)
+        if targets.dim() != 1 or targets.size(0) != b:
+            raise RuntimeError(f"target_items must be [batch={b}]; got {tuple(targets.shape)}")
+        if pool.dim() != 1 or pool.numel() == 0:
+            raise RuntimeError(f"pool_softmax_loss: pool_ids must be a non-empty [M]; got {tuple(pool.shape)}")
+        if lq.shape != pool.shape:
+            raise RuntimeError(f"pool_softmax_loss: log_q {tuple(lq.shape)} must match pool_ids {tuple(pool.shape)}")
+        if validate:
+            lo, hi, unsorted = torch.stack([pool.min(), pool.max(), (pool[1:] < pool[:-1]).any().long()]).tolist()
+            if lo < 0 or hi >= items:
+                raise RuntimeError(f"pool_softmax_loss: pool id out of range [0, {items}) (min {lo}, max {hi})")
+            if unsorted:
+                pool, order = torch.sort(pool)
+                lq = lq[order].contiguous()
+        m = pool.numel()
+        dev = sess_c.device
+        total = float(total_sessions if total_sessions else b)
+        pad = -1 if padding_idx is None else int(padding_idx)
+        lse = torch.empty(b, dtype=torch.float32, device=dev)
+        z_pos = torch.empty(b, dtype=torch.float32, device=dev)
+        loss = torch.empty(1, dtype=torch.float32, device=dev)
+        ws = workspace(size("etpgt_pool_softmax_workspace_bytes", b, m, dim), dev)
+        call("etpgt_pool_softmax_fwd", ptr(sess_c), ptr(table_c), ptr(targets), ptr(pool), ptr(lq), b, items, m, dim,
+             float(temperature), total, pad, ptr(lse), ptr(z_pos), ptr(loss), ptr(ws), ws.numel(), stream())
+        ctx.save_for_backward(sess_c, table_c, targets, pool, lq, lse, z_pos)
+        ctx.table_ref = table
+        ctx.meta = (float(temperature), total, pad)
+        ctx.mark_non_differentiable(lse)
+        return loss[0], lse
+
+    @staticmethod
+    def backward(ctx, d_loss, _d_lse):
+        sess, table, targets, pool, lq, lse, z_pos = ctx.saved_tensors
+        temperature, total, pad = ctx.meta
+        b, dim = sess.shape
+        m = pool.numel()
+        dev = sess.device
+        d_loss = _f32(d_loss).reshape(1).contiguous()
+        d_sess = torch.empty_like(sess) if ctx.needs_input_grad[0] else None
+        d_table = sink = None
+        if ctx.needs_input_grad[1]:
+            sink = _grad_sink(ctx.table_ref)
+            d_table = sink if sink is not None else torch.zeros_like(table)
+        ws = workspace(size("etpgt_pool_softmax_workspace_bytes", b, m, dim), dev)
+        call("etpgt_pool_softmax_bwd", ptr(sess), ptr(table), ptr(targets), ptr(pool), ptr(lq), ptr(lse), ptr(z_pos),
+             ptr(d_loss), b, table.size(0), m, dim, temperature, total, pad, ptr(d_sess), ptr(d_table), ptr(ws),
+             ws.numel(), stream())
+        return d_sess, (None if sink is not None else d_table), None, None, None, None, None, None, None
+
+
+def pool_softmax_loss(sess, item_embeddings, targets, pool_ids, log_q, temperature=1.0,
+                      total_sessions=None) -> torch.Tensor:
+    """Sampled softmax cross-entropy of `targets` against the shared negative pool `pool_ids` [M] with its log-Q
+    correction `log_q` [M] = log(M q(pool_ids)) (see PoolSoftmaxLoss; `sample_item_pool` draws both).  The pool is
+    sorted (with its log_q) when it is not sorted already; ids outside the table raise.  `item_embeddings` is the
+    nn.Embedding (its padding_idx never counts as a negative and its row gets no gradient) or a bare weight tensor.
+    The table gradient goes into the etpgt_b200.optim gradient sink when one is registered, else it is returned
+    densely (non-zero on the pool and target rows only)."""
+    weight = item_embeddings.weight if hasattr(item_embeddings, "weight") else item_embeddings
+    padding_idx = getattr(item_embeddings, "padding_idx", None)
+    return PoolSoftmaxLoss.apply(sess, weight, targets, pool_ids, log_q, temperature, total_sessions, padding_idx,
+                                 True)[0]
+
+
 # ------------------------------------------------------------------------------ scoring / top-k
 
 

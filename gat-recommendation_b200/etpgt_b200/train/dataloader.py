@@ -61,6 +61,11 @@ class DeviceSessionLoader:
     def __len__(self) -> int:
         return (self.sessions.num_sessions + self.batch_size - 1) // self.batch_size
 
+    def item_counts(self) -> torch.Tensor:
+        """Occurrences of every item id over all stored sessions, int64 [num_items] on the device: the counts of
+        the popularity proposal of train.losses.SharedPoolSoftmaxLoss."""
+        return torch.bincount(self.sessions.items, minlength=self.num_items)
+
     def _share(self, ids: np.ndarray):
         """This rank's contiguous share of one global batch (balanced by session length), every rank's session
         count, and whether the batch is replicated: a global batch too small to give every rank two sessions is

@@ -1,6 +1,7 @@
-"""BPR / listwise / dual / sampled-softmax / full-catalogue softmax losses with the reference's call signature
+"""BPR / listwise / dual / sampled-softmax / full-catalogue / shared-pool softmax losses with the reference's call signature
 `loss(session_embeddings, target_items, negative_items, item_embeddings: nn.Embedding)`
-(etpgt/train/losses.py), computed by the fused sampled-loss kernel (full_softmax: the tensor-core full-catalogue kernels)."""
+(etpgt/train/losses.py), computed by the fused sampled-loss kernel (full_softmax: the tensor-core full-catalogue kernels;
+shared_pool_softmax: the same kernels over one log-Q-corrected negative pool shared by the batch)."""
 
 from __future__ import annotations
 
@@ -59,7 +60,45 @@ class FullSoftmaxLoss(nn.Module):
         return ops.full_softmax_loss(session_embeddings, item_embeddings, target_items, temperature=self.temperature)
 
 
-def create_loss_function(loss_type: str = "dual", alpha: float = 0.7, temperature: float = 1.0) -> nn.Module:
+class SharedPoolSoftmaxLoss(nn.Module):
+    """Sampled softmax over one pool of `num_sampled` negatives shared by the whole batch, with the log-Q correction
+    (ops.pool_softmax_loss).  The pool is drawn with replacement from item_counts ** sampling_power (uniform when
+    item_counts is None; the padding row and zero-count items are never drawn), afresh on every call from
+    (seed, this loss's own step counter), so every data-parallel rank draws the same pool.  `negative_items` is
+    accepted for the common signature and not used.  Not a ListwiseLoss: the trainer takes the per-operator path."""
+
+    def __init__(self, num_sampled: int = 8192, item_counts=None, sampling_power: float = 0.75,
+                 temperature: float = 1.0, seed: int = 0):
+        super().__init__()
+        if int(num_sampled) < 1:
+            raise ValueError(f"num_sampled must be >= 1; got {num_sampled}")
+        self.num_sampled = int(num_sampled)
+        self.item_counts = item_counts
+        self.sampling_power = sampling_power
+        self.temperature = temperature
+        self.seed = int(seed)
+        self.step = 0
+        self._cum = None
+
+    def forward(self, session_embeddings, target_items, negative_items, item_embeddings) -> torch.Tensor:
+        weight = item_embeddings.weight if hasattr(item_embeddings, "weight") else item_embeddings
+        padding_idx = getattr(item_embeddings, "padding_idx", None)
+        items = weight.size(0)
+        if self._cum is None or self._cum.device != weight.device or self._cum.numel() != items + 1:
+            self._cum = ops.item_sampling_table(self.item_counts, self.sampling_power,
+                                                padding_idx=-1 if padding_idx is None else padding_idx,
+                                                num_items=items, device=weight.device)
+        pool, log_q = ops.sample_item_pool(self._cum, self.num_sampled, self.seed, self.step)
+        self.step += 1
+        return ops.PoolSoftmaxLoss.apply(session_embeddings, weight, target_items, pool, log_q, self.temperature,
+                                         None, padding_idx, False)[0]
+
+
+def create_loss_function(loss_type: str = "dual", alpha: float = 0.7, temperature: float = 1.0, *,
+                         num_sampled: int = 8192, item_counts=None, sampling_power: float = 0.75,
+                         seed: int = 0) -> nn.Module:
+    """The loss named `loss_type`.  num_sampled / item_counts / sampling_power / seed configure "shared_pool_softmax"
+    and are ignored by the other types."""
     if loss_type == "bpr":
         return BPRLoss()
     if loss_type == "listwise":
@@ -70,4 +109,7 @@ def create_loss_function(loss_type: str = "dual", alpha: float = 0.7, temperatur
         return SampledSoftmaxLoss(temperature=temperature)
     if loss_type == "full_softmax":
         return FullSoftmaxLoss(temperature=temperature)
+    if loss_type == "shared_pool_softmax":
+        return SharedPoolSoftmaxLoss(num_sampled=num_sampled, item_counts=item_counts, sampling_power=sampling_power,
+                                     temperature=temperature, seed=seed)
     raise ValueError(f"Unknown loss type: {loss_type}")

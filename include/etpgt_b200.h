@@ -100,6 +100,15 @@ int etpgt_sample_negatives(uint64_t seed, uint32_t step, int64_t session_base,
                            const int64_t* session_ids, int64_t num_sessions,
                            int max_len, int64_t num_items, int num_neg, int64_t* out,
                            etpgt_stream_t stream);
+/* Shared negative pool for the sampled softmax (etpgt_pool_softmax_*): num_sampled item ids drawn with replacement
+ * from q(i) = w_i / W, cum [num_items + 1] = (0, w_0, w_0 + w_1, ..., W) on the device, 0 < W < 2^62.  Draw j:
+ * Philox4x32-10, key (seed lo, seed hi), counter (j >> 1, 0x504F4F4C, 0, step), u = c[2(j&1)] | c[2(j&1)+1] << 32,
+ * r = umulhi64(u, W), the id i with cum[i] <= r < cum[i+1] (zero-weight ids are never drawn).  pool_ids [num_sampled]
+ * is written sorted ascending, log_q [num_sampled] = (float) log(num_sampled * w_id / W) in fp64.  Depends on
+ * (seed, step) only: every data-parallel rank draws the same pool.  No allocation, no synchronisation. */
+size_t etpgt_sample_item_pool_workspace_bytes(int64_t num_sampled);
+int etpgt_sample_item_pool(const int64_t* cum, int64_t num_items, int64_t num_sampled, uint64_t seed, uint32_t step,
+                           int64_t* pool_ids, float* log_q, void* ws, size_t ws_bytes, etpgt_stream_t stream);
 
 /* ---- a4: item embedding + Laplacian-PE projection -------------------------------------
  * out[n] = table[ids[n]] (+ pe[pe_row(n)] @ w_pe^T + b_pe);  pe_row(n) = n when
@@ -457,6 +466,25 @@ int etpgt_full_softmax_bwd(const float* sess, const float* table, const int64_t*
                            const float* d_loss, int64_t batch, int64_t num_items, int dim, float temperature,
                            double total_sessions, int64_t padding_idx, float* d_sess,
                            float* d_table_accumulate, void* ws, size_t ws_bytes, etpgt_stream_t stream);
+/* Sampled softmax over ONE pool of num_sampled negatives shared by the batch, with the log-Q correction, on the same
+ * tensor-core kernels.  pool_ids [M] ascending, inside [0, num_items); log_q [M] = log(M q(pool_ids[j])):
+ *   z_pos[b] = sess_b . table[targets[b]] / T (fp32 gather-dot, no correction)
+ *   z[b, j]  = sess_b . table[pool_ids[j]] / T - log_q[j], -inf where pool_ids[j] == targets[b] or == padding_idx
+ *   lse[b]   = logsumexp(z_pos[b], z[b, :]),  loss = sum_b (lse[b] - z_pos[b]) / total_sessions (<= 0: batch)
+ * dim in {64, 128, 192, 256}.  fwd writes lse, z_pos [batch] (both saved for backward) and loss [1].  bwd: d_loss is
+ * a device scalar; d_sess [batch, dim] is overwritten and d_table_accumulate [num_items, dim] has the gradient of the
+ * pool rows and target rows ADDED (row padding_idx untouched); either may be NULL.  Deterministic, no atomics, no
+ * allocation, no synchronisation; both calls take the same workspace size. */
+size_t etpgt_pool_softmax_workspace_bytes(int64_t batch, int64_t num_sampled, int dim);
+int etpgt_pool_softmax_fwd(const float* sess, const float* table, const int64_t* targets, const int64_t* pool_ids,
+                           const float* log_q, int64_t batch, int64_t num_items, int64_t num_sampled, int dim,
+                           float temperature, double total_sessions, int64_t padding_idx, float* lse, float* z_pos,
+                           float* loss, void* ws, size_t ws_bytes, etpgt_stream_t stream);
+int etpgt_pool_softmax_bwd(const float* sess, const float* table, const int64_t* targets, const int64_t* pool_ids,
+                           const float* log_q, const float* lse, const float* z_pos, const float* d_loss,
+                           int64_t batch, int64_t num_items, int64_t num_sampled, int dim, float temperature,
+                           double total_sessions, int64_t padding_idx, float* d_sess, float* d_table_accumulate,
+                           void* ws, size_t ws_bytes, etpgt_stream_t stream);
 
 /* ---- a9/a10: full-catalogue scoring with fused top-k and metrics ------------------------
  * etpgt/model/base.py:59-78, etpgt/utils/metrics.py:6-66.  Scores are never materialised.
@@ -517,7 +545,8 @@ int etpgt_hit_metrics(const int32_t* hit_pos, int64_t batch, int k, double* out,
 
 /* ---- generic helper shared by embedding / loss backward ---------------------------------
  * d_table[key] += sum_{p: keys[p]==key} coef[p] * src[p / src_div]  in ascending p, one writer
- * per row (deterministic).  coef may be NULL (=1); row skip_key (-1 = none) is left untouched. */
+ * per row (deterministic).  coef may be NULL (=1); row skip_key (-1 = none) is left untouched.  dim in
+ * {32, 64, 128, 192, 256}. */
 size_t etpgt_scatter_rows_workspace_bytes(int64_t m);
 int etpgt_scatter_rows(const int64_t* keys, const float* coef, const float* src, int64_t m,
                        int src_div, int dim, int64_t num_rows, int64_t skip_key, float* d_table,

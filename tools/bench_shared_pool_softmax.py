@@ -1,0 +1,177 @@
+"""Cost of the shared-pool sampled softmax (ops.pool_softmax_loss: csrc/softmax_tc.cu with POOL) next to the
+full-catalogue loss at the same B x I, in the same process; with --quality, what the objectives give on synth data.
+
+    python tools/bench_shared_pool_softmax.py [--reps 5] [--calls 5] [--shapes 1024x8192x82174,...] [--quality]
+
+D = 256.  Forward + backward are timed through the C ABI with CUDA events around `calls` back-to-back pairs, median
+over `reps` windows after a warm-up.  The backward adds into a d_table of the whole catalogue, as training does.
+The pool is drawn once per shape by etpgt_sample_item_pool (popularity^0.75 of zipf counts); its own time is listed
+apart.  Rates: executed MMA flops 15 * 2 * B * C * D (C = M for the pool, I for the full loss: three split-bf16 MMAs
+for the forward logits, the two recomputed logits and the two gradient products) over the time.  Prints one JSON line.
+--quality trains a 2-layer GraphTransformer (D = 64) for a few epochs on synth data with bpr, full_softmax and the
+shared pool (uniform and popularity proposals) and reports Recall@20 / NDCG@20 on held-out sessions.
+"""
+
+from __future__ import annotations
+
+import argparse
+import json
+import subprocess
+import sys
+import tempfile
+from pathlib import Path
+
+import numpy as np
+import torch
+
+ROOT = Path(__file__).resolve().parents[1]
+sys.path.insert(0, str(ROOT / "gat-recommendation_b200"))
+
+DIM = 256
+
+
+def gpu_info() -> dict:
+    info = {"gpu": torch.cuda.get_device_name(0)}
+    try:
+        out = subprocess.run(["nvidia-smi", "--id=0", "--query-gpu=power.limit,clocks.max.sm",
+                              "--format=csv,noheader,nounits"], capture_output=True, text=True, timeout=30).stdout
+        power, clock = [v.strip() for v in out.strip().split(",")]
+        info.update(power_limit_w=float(power), max_sm_clock_mhz=float(clock))
+    except Exception as e:   # the numbers still stand, without the card's limits
+        info["power_limit_w"] = f"unavailable ({type(e).__name__})"
+    return info
+
+
+def timed(fn, reps: int, calls: int) -> float:
+    """Median ms per call over `reps` windows of `calls` calls, after one warm-up call."""
+    fn()
+    torch.cuda.synchronize()
+    times = []
+    for _ in range(reps):
+        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        a.record()
+        for _ in range(calls):
+            fn()
+        b.record()
+        b.synchronize()
+        times.append(a.elapsed_time(b) / calls)
+    return sorted(times)[len(times) // 2]
+
+
+def bench_shape(b: int, m: int, items: int, reps: int, calls: int) -> dict:
+    from etpgt_b200 import _lib, ops
+    from etpgt_b200._lib import ptr
+
+    g = torch.Generator(device="cuda").manual_seed(b + m + items)
+    sess = torch.randn(b, DIM, device="cuda", generator=g) * 0.3
+    table = torch.randn(items, DIM, device="cuda", generator=g) * 0.3
+    targets = torch.randint(1, items, (b,), device="cuda", generator=g)
+    rng = np.random.default_rng(items)
+    counts = torch.from_numpy(np.bincount(rng.zipf(1.5, 4 * items) % items, minlength=items) + 1)
+    cum = ops.item_sampling_table(counts, 0.75, 0, device="cuda")
+    pool, log_q = ops.sample_item_pool(cum, m, seed=1, step=0)
+    sample_ms = timed(lambda: ops.sample_item_pool(cum, m, seed=1, step=0), reps, calls)
+    lse = torch.empty(b, device="cuda")
+    z_pos = torch.empty(b, device="cuda")
+    loss = torch.empty(1, device="cuda")
+    d_loss = torch.ones(1, device="cuda")
+    d_sess = torch.empty_like(sess)
+    d_table = torch.zeros_like(table)
+    st = _lib.stream()
+    ws = _lib.workspace(max(_lib.size("etpgt_pool_softmax_workspace_bytes", b, m, DIM),
+                            _lib.size("etpgt_full_softmax_workspace_bytes", b, items, DIM)), "cuda")
+
+    def pool_step():
+        _lib.call("etpgt_pool_softmax_fwd", ptr(sess), ptr(table), ptr(targets), ptr(pool), ptr(log_q), b, items, m,
+                  DIM, 1.0, 0.0, 0, ptr(lse), ptr(z_pos), ptr(loss), ptr(ws), ws.numel(), st)
+        _lib.call("etpgt_pool_softmax_bwd", ptr(sess), ptr(table), ptr(targets), ptr(pool), ptr(log_q), ptr(lse),
+                  ptr(z_pos), ptr(d_loss), b, items, m, DIM, 1.0, 0.0, 0, ptr(d_sess), ptr(d_table), ptr(ws),
+                  ws.numel(), st)
+
+    def full_step():
+        _lib.call("etpgt_full_softmax_fwd", ptr(sess), ptr(table), ptr(targets), b, items, DIM, 1.0, 0.0, 0,
+                  ptr(lse), ptr(loss), ptr(ws), ws.numel(), st)
+        _lib.call("etpgt_full_softmax_bwd", ptr(sess), ptr(table), ptr(targets), ptr(lse), ptr(d_loss), b, items, DIM,
+                  1.0, 0.0, 0, ptr(d_sess), ptr(d_table), ptr(ws), ws.numel(), st)
+
+    pool_ms = timed(pool_step, reps, calls)
+    full_ms = timed(full_step, reps, calls)
+    pool_flops, full_flops = 15 * 2 * b * m * DIM, 15 * 2 * b * items * DIM
+    out = {
+        "batch": b, "num_sampled": m, "items": items, "dim": DIM,
+        "pool_fwd_bwd_ms": round(pool_ms, 3), "sample_pool_ms": round(sample_ms, 3),
+        "pool_executed_tflops": round(pool_flops / pool_ms / 1e9, 1),
+        "full_fwd_bwd_ms": round(full_ms, 3),
+        "full_executed_tflops": round(full_flops / full_ms / 1e9, 1),
+        "full_ms_scaled_by_m_over_i": round(full_ms * m / items, 3),
+        "pool_over_scaled_full": round(pool_ms / (full_ms * m / items), 2),
+    }
+    del ws, d_table
+    torch.cuda.empty_cache()
+    return out
+
+
+def quality(epochs: int) -> list[dict]:
+    from etpgt_b200 import data, optim, synth
+    from etpgt_b200.model import create_graph_transformer_optimized
+    from etpgt_b200.train.losses import create_loss_function
+    from etpgt_b200.train.trainer import Trainer
+
+    d = synth.generate(num_sessions=24_000, graph_sessions=18_000, num_items=5_000, clusters=64, seed=7)
+    graph = data.ItemGraph(d.item_i, d.item_j, d.num_items)
+    store = data.SessionStore(d.sess_ptr, d.sess_items)
+    counts = torch.bincount(store.items, minlength=d.num_items)
+
+    def batches(lo, hi, step0):
+        out = []
+        for i, s in enumerate(range(lo, hi, 512)):
+            ids = np.arange(s, min(hi, s + 512))
+            bt = data.build_batch(graph, store, ids, 50, False, False)
+            bt.negative_items = data.sample_negatives(store, ids, d.num_items, 5, seed=3, step=step0 + i).view(-1)
+            out.append(bt)
+        return out
+
+    train, val = batches(0, 18_000, 0), batches(18_000, 24_000, 10_000)
+    arms = [("bpr", dict()), ("full_softmax", dict()),
+            ("shared_pool_softmax_uniform", dict(num_sampled=1024)),
+            ("shared_pool_softmax_popularity", dict(num_sampled=1024, item_counts=counts))]
+    results = []
+    for name, kw in arms:
+        torch.manual_seed(1)
+        model = create_graph_transformer_optimized(d.num_items, 64, 64, num_layers=2, num_heads=2, dropout=0.0,
+                                                   use_laplacian_pe=False).cuda()
+        kind = "shared_pool_softmax" if name.startswith("shared_pool") else name
+        loss_fn = create_loss_function(kind, **kw)
+        with tempfile.TemporaryDirectory() as tmp:
+            trainer = Trainer(model, train, val, optim.AdamW(model.parameters(), lr=3e-3), device="cuda",
+                              output_dir=tmp, max_epochs=epochs, patience=epochs, k_values=[20], loss_fn=loss_fn)
+            trainer.train()
+            metrics = trainer.evaluate()
+        results.append({"loss": name, "recall@20": round(float(metrics["recall@20"]), 4),
+                        "ndcg@20": round(float(metrics["ndcg@20"]), 4)})
+    return results
+
+
+def main() -> None:
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--reps", type=int, default=5)
+    ap.add_argument("--calls", type=int, default=5)
+    ap.add_argument("--shapes", default="1024x8192x82174,32768x8192x82174,8192x8192x1000000,32768x16384x1000000")
+    ap.add_argument("--quality", action="store_true")
+    ap.add_argument("--epochs", type=int, default=5)
+    args = ap.parse_args()
+    if not torch.cuda.is_available():
+        raise SystemExit("bench_shared_pool_softmax needs a CUDA device")
+    info = gpu_info()
+    results = []
+    for shape in args.shapes.split(","):
+        b, m, items = (int(v) for v in shape.split("x"))
+        results.append(bench_shape(b, m, items, args.reps, args.calls))
+    line = {"bench": "shared_pool_softmax", **info, "reps": args.reps, "calls": args.calls, "results": results}
+    if args.quality:
+        line["quality"] = quality(args.epochs)
+    print(json.dumps(line))
+
+
+if __name__ == "__main__":
+    main()

@@ -526,78 +526,152 @@ Plan plan_grad(int64_t rows, int64_t cols) {
 
 bool softmax_dim_ok(int dim) { return dim == 64 || dim == 128 || dim == 192 || dim == 256; }
 
+// The workspace of one call, in carve order: the bf16 pairs of the session rows and of the columns (the table, or
+// the gathered pool), the partials (the forward's [3][ranges][B] or a split gradient pass's [ranges][rows][D],
+// whichever is larger), then the pool loss's own buffers, which are 0 for the full loss.
 struct Layout {
-  size_t s_pair, e_pair, fwd_part, grad_part, total;
+  size_t s_pair, c_pair, part, d_pool, bias, hits, coef, scatter;
+  size_t total() const { return 2 * s_pair + 2 * c_pair + part + d_pool + bias + hits + coef + scatter + 256; }
 };
-Layout layout(int64_t batch, int64_t items, int dim) {
-  Layout l;
+Layout layout(int64_t batch, int64_t cols, int dim) {
+  Layout l = {};
   l.s_pair = align_up((size_t)batch * dim * 2);
-  l.e_pair = align_up((size_t)items * dim * 2);
-  const Plan pf = plan_fwd(batch, items), ps = plan_grad(batch, items), pe = plan_grad(items, batch);
-  l.fwd_part = align_up((size_t)3 * pf.ranges * batch * sizeof(float));
+  l.c_pair = align_up((size_t)cols * dim * 2);
+  const Plan pf = plan_fwd(batch, cols), ps = plan_grad(batch, cols), pe = plan_grad(cols, batch);
+  const size_t fp = (size_t)3 * pf.ranges * batch * sizeof(float);
   const size_t gs = ps.ranges > 1 ? (size_t)ps.ranges * batch * dim * sizeof(float) : 0;
-  const size_t ge = pe.ranges > 1 ? (size_t)pe.ranges * items * dim * sizeof(float) : 0;
-  l.grad_part = align_up(gs > ge ? gs : ge);
-  l.total = 2 * l.s_pair + 2 * l.e_pair + (l.fwd_part > l.grad_part ? l.fwd_part : l.grad_part) + 256;
+  const size_t ge = pe.ranges > 1 ? (size_t)pe.ranges * cols * dim * sizeof(float) : 0;
+  const size_t g = gs > ge ? gs : ge;
+  l.part = align_up(fp > g ? fp : g);
   return l;
 }
 
+// the tensor maps of the session and column pairs and the buffers carved for them; the pool's stay null for the
+// full loss
 struct Operands {
-  CUtensorMap s_hi, s_lo, e_hi, e_lo;
-  float* part;
+  CUtensorMap s_hi, s_lo, c_hi, c_lo;
+  float* part = nullptr;
+  float *d_pool = nullptr, *bias = nullptr, *coef = nullptr;
+  int2* hits = nullptr;
+  void* scatter_ws = nullptr;
+  size_t scatter_bytes = 0;
 };
 
-// splits sess and table into their bf16 pairs inside the workspace and encodes the four tensor maps
-int prepare(const float* sess, const float* table, int64_t batch, int64_t items, int dim, void* ws, size_t ws_bytes,
-            cudaStream_t stream, Operands* o) {
-  const Layout l = layout(batch, items, dim);
-  if (ws == nullptr || ws_bytes < l.total) {
-    set_error("full_softmax: workspace too small (%zu < %zu bytes)", ws_bytes, l.total);
+// the checks of both losses, in this order: dim, the loss's own size ranges (`ranges()` sets the message and returns
+// ETPGT_EINVAL when one fails), null arguments, temperature and padding_idx
+template <class Ranges>
+int check_args(const char* name, int dim, Ranges ranges, bool args_set, float temperature, int64_t padding_idx,
+               int64_t items) {
+  ETPGT_REQUIRE(softmax_dim_ok(dim), "%s: dim %d is not supported (dim must be one of 64, 128, 192, 256)", name, dim);
+  const int rc = ranges();
+  if (rc != ETPGT_OK) return rc;
+  ETPGT_REQUIRE(args_set, "%s: null argument", name);
+  ETPGT_REQUIRE(temperature > 0.f, "%s: temperature must be positive", name);
+  ETPGT_REQUIRE(padding_idx >= -1 && padding_idx < items, "%s: padding_idx must be -1 or an item id", name);
+  return ETPGT_OK;
+}
+
+// Checks the workspace, carves the two bf16 pairs and the partials, splits sess, lets `columns(w, c_hi, c_lo)` fill
+// the column pair (and carve what else the loss needs from w), then encodes the four tensor maps.
+template <class Columns>
+int prepare(const char* name, const Layout& l, const float* sess, int64_t batch, int64_t cols, int dim, void* ws,
+            size_t ws_bytes, cudaStream_t stream, Operands* o, Columns columns) {
+  if (ws == nullptr || ws_bytes < l.total()) {
+    set_error("%s: workspace too small (%zu < %zu bytes)", name, ws_bytes, l.total());
     return ETPGT_EWORKSPACE;
   }
   Workspace w(ws, ws_bytes);
   void* s_hi = w.take<char>(l.s_pair);
   void* s_lo = w.take<char>(l.s_pair);
-  void* e_hi = w.take<char>(l.e_pair);
-  void* e_lo = w.take<char>(l.e_pair);
-  o->part = w.take<float>((l.fwd_part > l.grad_part ? l.fwd_part : l.grad_part) / sizeof(float));
+  auto* c_hi = w.take<__nv_bfloat16>(l.c_pair / 2);
+  auto* c_lo = w.take<__nv_bfloat16>(l.c_pair / 2);
+  o->part = w.take<float>(l.part / sizeof(float));
   int rc = etpgt_split_bf16(sess, batch, dim, dim, s_hi, s_lo, dim, nullptr, nullptr, 0, nullptr, nullptr, 0, stream);
   if (rc != ETPGT_OK) return rc;
-  rc = etpgt_split_bf16(table, items, dim, dim, e_hi, e_lo, dim, nullptr, nullptr, 0, nullptr, nullptr, 0, stream);
+  rc = columns(w, c_hi, c_lo);
   if (rc != ETPGT_OK) return rc;
   if (!(make_map_bf16(&o->s_hi, s_hi, batch, dim, dim, TILE) && make_map_bf16(&o->s_lo, s_lo, batch, dim, dim, TILE) &&
-        make_map_bf16(&o->e_hi, e_hi, items, dim, dim, TILE) && make_map_bf16(&o->e_lo, e_lo, items, dim, dim, TILE))) {
-    set_error("full_softmax: cuTensorMapEncodeTiled failed");
+        make_map_bf16(&o->c_hi, c_hi, cols, dim, dim, TILE) && make_map_bf16(&o->c_lo, c_lo, cols, dim, dim, TILE))) {
+    set_error("%s: cuTensorMapEncodeTiled failed", name);
     return ETPGT_ECUDA;
   }
   return ETPGT_OK;
 }
 
-int check_args(const float* sess, const float* table, const int64_t* targets, int64_t batch, int64_t items, int dim,
-               float temperature, int64_t padding_idx) {
-  ETPGT_REQUIRE(softmax_dim_ok(dim), "full_softmax: dim %d is not supported (dim must be one of 64, 128, 192, 256)",
-                dim);
-  ETPGT_REQUIRE(batch >= 1 && items >= 2 && batch < (int64_t(1) << 31) && items < (int64_t(1) << 31),
-                "full_softmax: need batch >= 1 and num_items >= 2 (got %lld, %lld)", (long long)batch,
-                (long long)items);
-  ETPGT_REQUIRE(sess != nullptr && table != nullptr && targets != nullptr, "full_softmax: null argument");
-  ETPGT_REQUIRE(temperature > 0.f, "full_softmax: temperature must be positive");
-  ETPGT_REQUIRE(padding_idx >= -1 && padding_idx < items, "full_softmax: padding_idx must be -1 or an item id");
-  return ETPGT_OK;
+// the loss is the mean over total_sessions, or over the batch when that is not positive
+double mean_over(double total_sessions, int64_t batch) { return total_sessions > 0 ? total_sessions : (double)batch; }
+
+// the Params every pass of one call shares; each pass sets rows, cols, its column ranges and out
+Params call_params(int dim, float temperature, double total, int64_t padding_idx, const Operands& o,
+                   const int64_t* targets, const float* lse = nullptr, const float* d_loss = nullptr) {
+  Params p = {};
+  p.dim = dim;
+  p.inv_t = 1.f / temperature;
+  p.gscale = (float)(1.0 / ((double)temperature * total));
+  p.targets = targets;
+  p.lse = lse;
+  p.d_loss = d_loss;
+  p.padding_idx = padding_idx;
+  p.part = o.part;
+  p.bias = o.bias;
+  p.hits = o.hits;
+  return p;
 }
 
 template <int MODE, bool POOL = false>
 int launch(const CUtensorMap& r_hi, const CUtensorMap& r_lo, const CUtensorMap& c_hi, const CUtensorMap& c_lo,
-           const Params& p, int grid, cudaStream_t stream) {
+           const Params& p, int grid, const char* name, cudaStream_t stream) {
   const size_t smem = Cfg<MODE>::smem + sizeof(Bars);
   cudaFuncSetAttribute(full_softmax_tc_kernel<MODE, POOL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   full_softmax_tc_kernel<MODE, POOL><<<grid, kThreads, smem, stream>>>(r_hi, r_lo, c_hi, c_lo, p);
-  if (POOL) {
-    ETPGT_CHECK_LAUNCH(MODE == FWD ? "pool_softmax_fwd" : MODE == DS ? "pool_softmax_bwd_sess" : "pool_softmax_bwd_pool");
-  } else {
-    ETPGT_CHECK_LAUNCH(MODE == FWD ? "full_softmax_fwd" : MODE == DS ? "full_softmax_bwd_sess" : "full_softmax_bwd_table");
+  ETPGT_CHECK_LAUNCH(name);
+  return ETPGT_OK;
+}
+
+// One gradient pass (DS or DE) over rows x cols into out [rows, D].  Split into column ranges, its partials are
+// summed into out in range order (added to out when `accumulate`, row skip_row left alone).
+template <int MODE, bool POOL = false>
+int grad_pass(const CUtensorMap& r_hi, const CUtensorMap& r_lo, const CUtensorMap& c_hi, const CUtensorMap& c_lo,
+              Params p, int64_t rows, int64_t cols, float* out, int accumulate, int64_t skip_row, const char* name,
+              const char* combine_name, cudaStream_t stream) {
+  const Plan pl = plan_grad(rows, cols);
+  p.rows = rows;
+  p.cols = cols;
+  p.tiles_per_range = pl.tiles_per_range;
+  p.ranges = pl.ranges;
+  p.out = out;
+  const int rc = launch<MODE, POOL>(r_hi, r_lo, c_hi, c_lo, p, pl.grid, name, stream);
+  if (rc != ETPGT_OK) return rc;
+  if (pl.ranges > 1) {
+    grad_combine_kernel<<<grid_for(rows * p.dim / 4, 256, 8), 256, 0, stream>>>(p.part, pl.ranges, rows, p.dim,
+                                                                                accumulate, skip_row, out);
+    ETPGT_CHECK_LAUNCH(combine_name);
   }
   return ETPGT_OK;
+}
+
+// ---------------------------------------------------------------------------- full-catalogue softmax: host
+
+int full_check_args(const float* sess, const float* table, const int64_t* targets, int64_t batch, int64_t items,
+                    int dim, float temperature, int64_t padding_idx) {
+  const auto ranges = [&] {
+    ETPGT_REQUIRE(batch >= 1 && items >= 2 && batch < (int64_t(1) << 31) && items < (int64_t(1) << 31),
+                  "full_softmax: need batch >= 1 and num_items >= 2 (got %lld, %lld)", (long long)batch,
+                  (long long)items);
+    return ETPGT_OK;
+  };
+  return check_args("full_softmax", dim, ranges, sess != nullptr && table != nullptr && targets != nullptr,
+                    temperature, padding_idx, items);
+}
+
+// the columns are the table, split into its bf16 pair
+int full_prepare(const float* sess, const float* table, int64_t batch, int64_t items, int dim, void* ws,
+                 size_t ws_bytes, cudaStream_t stream, Operands* o) {
+  return prepare("full_softmax", layout(batch, items, dim), sess, batch, items, dim, ws, ws_bytes, stream, o,
+                 [&](Workspace&, __nv_bfloat16* c_hi, __nv_bfloat16* c_lo) {
+                   return etpgt_split_bf16(table, items, dim, dim, c_hi, c_lo, dim, nullptr, nullptr, 0, nullptr,
+                                           nullptr, 0, stream);
+                 });
 }
 
 // ---------------------------------------------------------------------------- shared-pool softmax: small kernels
@@ -704,88 +778,58 @@ pool_positive_bwd_kernel(const float* __restrict__ table, const int64_t* __restr
   }
 }
 
-struct PoolLayout {
-  size_t s_pair, c_pair, part, d_pool, bias, hits, coef, scatter, total;
-};
-PoolLayout pool_layout(int64_t batch, int64_t m, int dim) {
-  PoolLayout l;
-  l.s_pair = align_up((size_t)batch * dim * 2);
-  l.c_pair = align_up((size_t)m * dim * 2);
-  const Plan pf = plan_fwd(batch, m), ps = plan_grad(batch, m), pe = plan_grad(m, batch);
-  const size_t fp = (size_t)3 * pf.ranges * batch * sizeof(float);
-  const size_t gs = ps.ranges > 1 ? (size_t)ps.ranges * batch * dim * sizeof(float) : 0;
-  const size_t ge = pe.ranges > 1 ? (size_t)pe.ranges * m * dim * sizeof(float) : 0;
-  l.part = align_up(fp > gs ? (fp > ge ? fp : ge) : (gs > ge ? gs : ge));
+// ---------------------------------------------------------------------------- shared-pool softmax: host
+
+// the full loss's layout over the M pool rows, plus d_pool, the pool's bias, the sessions' hit ranges and positive
+// coefficients, and the workspace of the two row scatters
+Layout pool_layout(int64_t batch, int64_t m, int dim) {
+  Layout l = layout(batch, m, dim);
   l.d_pool = align_up((size_t)m * dim * sizeof(float));
   l.bias = align_up((size_t)m * sizeof(float));
   l.hits = align_up((size_t)batch * sizeof(int2));
   l.coef = align_up((size_t)batch * sizeof(float));
   l.scatter = align_up(etpgt_scatter_rows_workspace_bytes(batch > m ? batch : m));
-  l.total = 2 * l.s_pair + 2 * l.c_pair + l.part + l.d_pool + l.bias + l.hits + l.coef + l.scatter + 256;
   return l;
 }
-
-struct PoolOperands {
-  CUtensorMap s_hi, s_lo, c_hi, c_lo;
-  float *part, *d_pool, *bias, *coef;
-  int2* hits;
-  void* scatter_ws;
-  size_t scatter_bytes;
-};
 
 int pool_check_args(const float* sess, const float* table, const int64_t* targets, const int64_t* pool_ids,
                     const float* log_q, int64_t batch, int64_t items, int64_t m, int dim, float temperature,
                     int64_t padding_idx) {
-  ETPGT_REQUIRE(softmax_dim_ok(dim), "pool_softmax: dim %d is not supported (dim must be one of 64, 128, 192, 256)",
-                dim);
-  ETPGT_REQUIRE(batch >= 1 && batch < (int64_t(1) << 31), "pool_softmax: batch must be in [1, 2^31) (got %lld)",
-                (long long)batch);
-  ETPGT_REQUIRE(m >= 1 && m < (int64_t(1) << 31), "pool_softmax: num_sampled must be in [1, 2^31) (got %lld)",
-                (long long)m);
-  ETPGT_REQUIRE(items >= 1 && items < (int64_t(1) << 31), "pool_softmax: num_items must be in [1, 2^31) (got %lld)",
-                (long long)items);
-  ETPGT_REQUIRE(sess != nullptr && table != nullptr && targets != nullptr && pool_ids != nullptr && log_q != nullptr,
-                "pool_softmax: null argument");
-  ETPGT_REQUIRE(temperature > 0.f, "pool_softmax: temperature must be positive");
-  ETPGT_REQUIRE(padding_idx >= -1 && padding_idx < items, "pool_softmax: padding_idx must be -1 or an item id");
-  return ETPGT_OK;
+  const auto ranges = [&] {
+    ETPGT_REQUIRE(batch >= 1 && batch < (int64_t(1) << 31), "pool_softmax: batch must be in [1, 2^31) (got %lld)",
+                  (long long)batch);
+    ETPGT_REQUIRE(m >= 1 && m < (int64_t(1) << 31), "pool_softmax: num_sampled must be in [1, 2^31) (got %lld)",
+                  (long long)m);
+    ETPGT_REQUIRE(items >= 1 && items < (int64_t(1) << 31), "pool_softmax: num_items must be in [1, 2^31) (got %lld)",
+                  (long long)items);
+    return ETPGT_OK;
+  };
+  return check_args("pool_softmax", dim, ranges,
+                    sess != nullptr && table != nullptr && targets != nullptr && pool_ids != nullptr && log_q != nullptr,
+                    temperature, padding_idx, items);
 }
 
-// splits sess, gathers and splits the pool rows, finds the hit ranges (and z_pos when given) and encodes the maps
+// the columns are the pool rows, gathered and split; also finds the hit ranges (and z_pos when given)
 int pool_prepare(const float* sess, const float* table, const int64_t* targets, const int64_t* pool_ids,
                  const float* log_q, int64_t batch, int64_t m, int dim, float inv_t, int64_t padding_idx,
-                 float* z_pos, void* ws, size_t ws_bytes, cudaStream_t stream, PoolOperands* o) {
-  const PoolLayout l = pool_layout(batch, m, dim);
-  if (ws == nullptr || ws_bytes < l.total) {
-    set_error("pool_softmax: workspace too small (%zu < %zu bytes)", ws_bytes, l.total);
-    return ETPGT_EWORKSPACE;
-  }
-  Workspace w(ws, ws_bytes);
-  void* s_hi = w.take<char>(l.s_pair);
-  void* s_lo = w.take<char>(l.s_pair);
-  auto* c_hi = w.take<__nv_bfloat16>(l.c_pair / 2);
-  auto* c_lo = w.take<__nv_bfloat16>(l.c_pair / 2);
-  o->part = w.take<float>(l.part / sizeof(float));
-  o->d_pool = w.take<float>(l.d_pool / sizeof(float));
-  o->bias = w.take<float>(l.bias / sizeof(float));
-  o->hits = w.take<int2>(l.hits / sizeof(int2));
-  o->coef = w.take<float>(l.coef / sizeof(float));
-  o->scatter_bytes = l.scatter;
-  o->scatter_ws = w.take<char>(l.scatter);
-  int rc = etpgt_split_bf16(sess, batch, dim, dim, s_hi, s_lo, dim, nullptr, nullptr, 0, nullptr, nullptr, 0, stream);
-  if (rc != ETPGT_OK) return rc;
-  pool_gather_split_kernel<<<grid_for(m * dim / 4, 256, 8), 256, 0, stream>>>(pool_ids, log_q, table, m, dim,
-                                                                             padding_idx, c_hi, c_lo, o->bias);
-  ETPGT_CHECK_LAUNCH("pool_softmax_gather");
-  pool_rows_kernel<<<grid_for(batch, 8, 8), 256, 0, stream>>>(sess, table, targets, pool_ids, batch, m, dim, inv_t,
-                                                              o->hits, z_pos);
-  ETPGT_CHECK_LAUNCH("pool_softmax_rows");
-  if (!(make_map_bf16(&o->s_hi, s_hi, batch, dim, dim, TILE) && make_map_bf16(&o->s_lo, s_lo, batch, dim, dim, TILE) &&
-        make_map_bf16(&o->c_hi, c_hi, m, dim, dim, TILE) && make_map_bf16(&o->c_lo, c_lo, m, dim, dim, TILE))) {
-    set_error("pool_softmax: cuTensorMapEncodeTiled failed");
-    return ETPGT_ECUDA;
-  }
-  return ETPGT_OK;
+                 float* z_pos, void* ws, size_t ws_bytes, cudaStream_t stream, Operands* o) {
+  const Layout l = pool_layout(batch, m, dim);
+  return prepare("pool_softmax", l, sess, batch, m, dim, ws, ws_bytes, stream, o,
+                 [&](Workspace& w, __nv_bfloat16* c_hi, __nv_bfloat16* c_lo) {
+                   o->d_pool = w.take<float>(l.d_pool / sizeof(float));
+                   o->bias = w.take<float>(l.bias / sizeof(float));
+                   o->hits = w.take<int2>(l.hits / sizeof(int2));
+                   o->coef = w.take<float>(l.coef / sizeof(float));
+                   o->scatter_bytes = l.scatter;
+                   o->scatter_ws = w.take<char>(l.scatter);
+                   pool_gather_split_kernel<<<grid_for(m * dim / 4, 256, 8), 256, 0, stream>>>(
+                       pool_ids, log_q, table, m, dim, padding_idx, c_hi, c_lo, o->bias);
+                   ETPGT_CHECK_LAUNCH("pool_softmax_gather");
+                   pool_rows_kernel<<<grid_for(batch, 8, 8), 256, 0, stream>>>(sess, table, targets, pool_ids, batch,
+                                                                               m, dim, inv_t, o->hits, z_pos);
+                   ETPGT_CHECK_LAUNCH("pool_softmax_rows");
+                   return ETPGT_OK;
+                 });
 }
 
 }  // namespace
@@ -795,7 +839,7 @@ using namespace etpgt;
 
 extern "C" size_t etpgt_full_softmax_workspace_bytes(int64_t batch, int64_t num_items, int dim) {
   if (batch < 1 || num_items < 1 || dim < 1) return 256;
-  return layout(batch, num_items, dim).total;
+  return layout(batch, num_items, dim).total();
 }
 
 extern "C" int etpgt_full_softmax_fwd(const float* sess, const float* table, const int64_t* targets, int64_t batch,
@@ -803,26 +847,21 @@ extern "C" int etpgt_full_softmax_fwd(const float* sess, const float* table, con
                                       int64_t padding_idx, float* lse, float* loss, void* ws, size_t ws_bytes,
                                       etpgt_stream_t stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  int rc = check_args(sess, table, targets, batch, num_items, dim, temperature, padding_idx);
+  int rc = full_check_args(sess, table, targets, batch, num_items, dim, temperature, padding_idx);
   if (rc != ETPGT_OK) return rc;
   ETPGT_REQUIRE(lse != nullptr && loss != nullptr, "full_softmax_fwd: lse and loss are required");
   Operands o;
-  rc = prepare(sess, table, batch, num_items, dim, ws, ws_bytes, stream, &o);
+  rc = full_prepare(sess, table, batch, num_items, dim, ws, ws_bytes, stream, &o);
   if (rc != ETPGT_OK) return rc;
+  const double total = mean_over(total_sessions, batch);
   const Plan pl = plan_fwd(batch, num_items);
-  Params p = {};
+  Params p = call_params(dim, temperature, total, padding_idx, o, targets);
   p.rows = batch;
   p.cols = num_items;
-  p.dim = dim;
   p.tiles_per_range = pl.tiles_per_range;
   p.ranges = pl.ranges;
-  p.inv_t = 1.f / temperature;
-  p.targets = targets;
-  p.padding_idx = padding_idx;
-  p.part = o.part;
-  rc = launch<FWD>(o.s_hi, o.s_lo, o.e_hi, o.e_lo, p, pl.grid, stream);
+  rc = launch<FWD>(o.s_hi, o.s_lo, o.c_hi, o.c_lo, p, pl.grid, "full_softmax_fwd", stream);
   if (rc != ETPGT_OK) return rc;
-  const double total = total_sessions > 0 ? total_sessions : (double)batch;
   fwd_combine_kernel<<<1, kCombineThreads, 0, stream>>>(o.part, pl.ranges, pl.tiles_per_range, batch, num_items,
                                                         targets, total, lse, loss);
   ETPGT_CHECK_LAUNCH("full_softmax_fwd_combine");
@@ -834,59 +873,31 @@ extern "C" int etpgt_full_softmax_bwd(const float* sess, const float* table, con
                                       double total_sessions, int64_t padding_idx, float* d_sess,
                                       float* d_table_accumulate, void* ws, size_t ws_bytes, etpgt_stream_t stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  int rc = check_args(sess, table, targets, batch, num_items, dim, temperature, padding_idx);
+  int rc = full_check_args(sess, table, targets, batch, num_items, dim, temperature, padding_idx);
   if (rc != ETPGT_OK) return rc;
   ETPGT_REQUIRE(lse != nullptr && d_loss != nullptr, "full_softmax_bwd: lse and d_loss are required");
   if (d_sess == nullptr && d_table_accumulate == nullptr) return ETPGT_OK;
   Operands o;
-  rc = prepare(sess, table, batch, num_items, dim, ws, ws_bytes, stream, &o);
+  rc = full_prepare(sess, table, batch, num_items, dim, ws, ws_bytes, stream, &o);
   if (rc != ETPGT_OK) return rc;
-  const double total = total_sessions > 0 ? total_sessions : (double)batch;
-  Params p = {};
-  p.dim = dim;
-  p.inv_t = 1.f / temperature;
-  p.gscale = (float)(1.0 / ((double)temperature * total));
-  p.targets = targets;
-  p.lse = lse;
-  p.d_loss = d_loss;
-  p.padding_idx = padding_idx;
-  p.part = o.part;
+  const Params p =
+      call_params(dim, temperature, mean_over(total_sessions, batch), padding_idx, o, targets, lse, d_loss);
   if (d_sess != nullptr) {
-    const Plan pl = plan_grad(batch, num_items);
-    p.rows = batch;
-    p.cols = num_items;
-    p.tiles_per_range = pl.tiles_per_range;
-    p.ranges = pl.ranges;
-    p.out = d_sess;
-    rc = launch<DS>(o.s_hi, o.s_lo, o.e_hi, o.e_lo, p, pl.grid, stream);
+    rc = grad_pass<DS>(o.s_hi, o.s_lo, o.c_hi, o.c_lo, p, batch, num_items, d_sess, 0, -1, "full_softmax_bwd_sess",
+                       "full_softmax_bwd_sess_combine", stream);
     if (rc != ETPGT_OK) return rc;
-    if (pl.ranges > 1) {
-      grad_combine_kernel<<<grid_for(batch * dim / 4, 256, 8), 256, 0, stream>>>(o.part, pl.ranges, batch, dim, 0, -1,
-                                                                                 d_sess);
-      ETPGT_CHECK_LAUNCH("full_softmax_bwd_sess_combine");
-    }
   }
   if (d_table_accumulate != nullptr) {
-    const Plan pl = plan_grad(num_items, batch);
-    p.rows = num_items;
-    p.cols = batch;
-    p.tiles_per_range = pl.tiles_per_range;
-    p.ranges = pl.ranges;
-    p.out = d_table_accumulate;
-    rc = launch<DE>(o.e_hi, o.e_lo, o.s_hi, o.s_lo, p, pl.grid, stream);
+    rc = grad_pass<DE>(o.c_hi, o.c_lo, o.s_hi, o.s_lo, p, num_items, batch, d_table_accumulate, 1, padding_idx,
+                       "full_softmax_bwd_table", "full_softmax_bwd_table_combine", stream);
     if (rc != ETPGT_OK) return rc;
-    if (pl.ranges > 1) {
-      grad_combine_kernel<<<grid_for(num_items * dim / 4, 256, 8), 256, 0, stream>>>(
-          o.part, pl.ranges, num_items, dim, 1, padding_idx, d_table_accumulate);
-      ETPGT_CHECK_LAUNCH("full_softmax_bwd_table_combine");
-    }
   }
   return ETPGT_OK;
 }
 
 extern "C" size_t etpgt_pool_softmax_workspace_bytes(int64_t batch, int64_t num_sampled, int dim) {
   if (batch < 1 || num_sampled < 1 || dim < 1) return 256;
-  return pool_layout(batch, num_sampled, dim).total;
+  return pool_layout(batch, num_sampled, dim).total();
 }
 
 extern "C" int etpgt_pool_softmax_fwd(const float* sess, const float* table, const int64_t* targets,
@@ -900,25 +911,19 @@ extern "C" int etpgt_pool_softmax_fwd(const float* sess, const float* table, con
   if (rc != ETPGT_OK) return rc;
   ETPGT_REQUIRE(lse != nullptr && z_pos != nullptr && loss != nullptr,
                 "pool_softmax_fwd: lse, z_pos and loss are required");
-  PoolOperands o;
+  Operands o;
   rc = pool_prepare(sess, table, targets, pool_ids, log_q, batch, num_sampled, dim, 1.f / temperature, padding_idx,
                     z_pos, ws, ws_bytes, stream, &o);
   if (rc != ETPGT_OK) return rc;
+  const double total = mean_over(total_sessions, batch);
   const Plan pl = plan_fwd(batch, num_sampled);
-  Params p = {};
+  Params p = call_params(dim, temperature, total, -1, o, nullptr);
   p.rows = batch;
   p.cols = num_sampled;
-  p.dim = dim;
   p.tiles_per_range = pl.tiles_per_range;
   p.ranges = pl.ranges;
-  p.inv_t = 1.f / temperature;
-  p.padding_idx = -1;
-  p.part = o.part;
-  p.bias = o.bias;
-  p.hits = o.hits;
-  rc = launch<FWD, true>(o.s_hi, o.s_lo, o.c_hi, o.c_lo, p, pl.grid, stream);
+  rc = launch<FWD, true>(o.s_hi, o.s_lo, o.c_hi, o.c_lo, p, pl.grid, "pool_softmax_fwd", stream);
   if (rc != ETPGT_OK) return rc;
-  const double total = total_sessions > 0 ? total_sessions : (double)batch;
   pool_combine_kernel<<<1, kCombineThreads, 0, stream>>>(o.part, pl.ranges, batch, z_pos, total, lse, loss);
   ETPGT_CHECK_LAUNCH("pool_softmax_fwd_combine");
   return ETPGT_OK;
@@ -937,53 +942,23 @@ extern "C" int etpgt_pool_softmax_bwd(const float* sess, const float* table, con
   ETPGT_REQUIRE(lse != nullptr && z_pos != nullptr && d_loss != nullptr,
                 "pool_softmax_bwd: lse, z_pos and d_loss are required");
   if (d_sess == nullptr && d_table_accumulate == nullptr) return ETPGT_OK;
-  PoolOperands o;
+  Operands o;
   rc = pool_prepare(sess, table, targets, pool_ids, log_q, batch, num_sampled, dim, 1.f / temperature, padding_idx,
                     nullptr, ws, ws_bytes, stream, &o);
   if (rc != ETPGT_OK) return rc;
-  const double total = total_sessions > 0 ? total_sessions : (double)batch;
-  Params p = {};
-  p.dim = dim;
-  p.inv_t = 1.f / temperature;
-  p.gscale = (float)(1.0 / ((double)temperature * total));
-  p.lse = lse;
-  p.d_loss = d_loss;
-  p.padding_idx = -1;
-  p.part = o.part;
-  p.bias = o.bias;
-  p.hits = o.hits;
+  const Params p = call_params(dim, temperature, mean_over(total_sessions, batch), -1, o, nullptr, lse, d_loss);
   if (d_sess != nullptr) {
-    const Plan pl = plan_grad(batch, num_sampled);
-    p.rows = batch;
-    p.cols = num_sampled;
-    p.tiles_per_range = pl.tiles_per_range;
-    p.ranges = pl.ranges;
-    p.out = d_sess;
-    rc = launch<DS, true>(o.s_hi, o.s_lo, o.c_hi, o.c_lo, p, pl.grid, stream);
+    rc = grad_pass<DS, true>(o.s_hi, o.s_lo, o.c_hi, o.c_lo, p, batch, num_sampled, d_sess, 0, -1,
+                             "pool_softmax_bwd_sess", "pool_softmax_bwd_sess_combine", stream);
     if (rc != ETPGT_OK) return rc;
-    if (pl.ranges > 1) {
-      grad_combine_kernel<<<grid_for(batch * dim / 4, 256, 8), 256, 0, stream>>>(o.part, pl.ranges, batch, dim, 0, -1,
-                                                                                 d_sess);
-      ETPGT_CHECK_LAUNCH("pool_softmax_bwd_sess_combine");
-    }
   }
   pool_positive_bwd_kernel<<<grid_for(batch, 8, 8), 256, 0, stream>>>(table, targets, z_pos, lse, d_loss, batch, dim,
                                                                       p.gscale, o.coef, d_sess);
   ETPGT_CHECK_LAUNCH("pool_softmax_bwd_positive");
   if (d_table_accumulate != nullptr) {
-    const Plan pl = plan_grad(num_sampled, batch);
-    p.rows = num_sampled;
-    p.cols = batch;
-    p.tiles_per_range = pl.tiles_per_range;
-    p.ranges = pl.ranges;
-    p.out = o.d_pool;
-    rc = launch<DE, true>(o.c_hi, o.c_lo, o.s_hi, o.s_lo, p, pl.grid, stream);
+    rc = grad_pass<DE, true>(o.c_hi, o.c_lo, o.s_hi, o.s_lo, p, num_sampled, batch, o.d_pool, 0, -1,
+                             "pool_softmax_bwd_pool", "pool_softmax_bwd_pool_combine", stream);
     if (rc != ETPGT_OK) return rc;
-    if (pl.ranges > 1) {
-      grad_combine_kernel<<<grid_for(num_sampled * dim / 4, 256, 8), 256, 0, stream>>>(
-          o.part, pl.ranges, num_sampled, dim, 0, -1, o.d_pool);
-      ETPGT_CHECK_LAUNCH("pool_softmax_bwd_pool_combine");
-    }
     // d_table[p_j] += d_pool[j], then d_table[t_b] += coef[b] s_b: each in ascending position, padding skipped
     rc = etpgt_scatter_rows(pool_ids, nullptr, o.d_pool, num_sampled, 1, dim, num_items, padding_idx,
                             d_table_accumulate, o.scatter_ws, o.scatter_bytes, stream);

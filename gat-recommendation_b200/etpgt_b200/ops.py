@@ -38,6 +38,20 @@ def _grad_sink(table: torch.Tensor):
     return grad_sink_for(table) if table.dtype == torch.float32 and table.is_contiguous() else None
 
 
+def _table_grad(ctx, shape, device):
+    """(buffer the library ADDS the table gradient into, what backward returns for the table, input 1): the optim
+    gradient sink and None when one is registered, else a dense fp32 zero tensor twice; (None, None) if not needed."""
+    if not ctx.needs_input_grad[1]:
+        return None, None
+    sink = _grad_sink(ctx.table_ref)
+    d_table = sink if sink is not None else torch.zeros(shape, dtype=torch.float32, device=device)
+    return d_table, (None if sink is not None else d_table)
+
+
+def _weight_and_padding(item_embeddings):
+    return getattr(item_embeddings, "weight", item_embeddings), getattr(item_embeddings, "padding_idx", None)
+
+
 def _i64(t: torch.Tensor) -> torch.Tensor:
     return t.contiguous() if t.dtype == torch.int64 else t.long().contiguous()
 
@@ -405,10 +419,7 @@ class EmbedPE(torch.autograd.Function):
         d_out = _f32(d_out)
         dev = d_out.device
         n = ids.numel()
-        d_table = sink = None
-        if ctx.needs_input_grad[1]:
-            sink = _grad_sink(ctx.table_ref)   # persistent buffer owned by etpgt_b200.optim: rows are ADDED
-            d_table = sink if sink is not None else torch.zeros(num_items, dim, dtype=torch.float32, device=dev)
+        d_table, table_grad = _table_grad(ctx, (num_items, dim), dev)
         d_w = d_b = None
         if pe is not None:
             d_w = torch.empty(dim, k_pe, dtype=torch.float32, device=dev)
@@ -418,7 +429,7 @@ class EmbedPE(torch.autograd.Function):
         call("etpgt_embed_pe_bwd_planned", ptr(ids), n, ptr(d_out), num_items, ptr(pe), per_node, k_pe, dim,
              padding_idx, ptr(plan.sorted_key) if plan else None, ptr(plan.perm) if plan else None,
              ptr(d_table), ptr(d_w), ptr(d_b), ptr(ws), ws.numel(), stream())
-        return None, (None if sink is not None else d_table), None, None, d_w, d_b, None, None
+        return None, table_grad, None, None, d_w, d_b, None, None
 
 
 # ------------------------------------------------------------------------------ TransformerConv
@@ -1352,29 +1363,39 @@ class SampledLoss(torch.autograd.Function):
         dev = sess.device
         d_loss = _f32(d_losses)[0:1].contiguous()
         d_sess = torch.empty_like(sess)
-        d_table = sink = None
-        if ctx.needs_input_grad[1]:
-            sink = _grad_sink(ctx.table_ref)
-            d_table = sink if sink is not None else torch.zeros_like(table)
+        d_table, table_grad = _table_grad(ctx, table.shape, dev)
         ws = workspace(size("etpgt_sampled_loss_workspace_bytes", b, num_neg, dim), dev)
         plan = ctx.plan if d_table is not None and ctx.plan is not None and ctx.plan.m == b * (num_neg + 1) else None
         call("etpgt_sampled_loss_bwd_planned", ptr(sess), ptr(table), ptr(targets), ptr(negatives), b, num_neg, dim,
              mode, alpha, temperature, total, ptr(scores), ptr(d_loss), table.size(0), padding_idx,
              ptr(plan.sorted_key) if plan else None, ptr(plan.perm) if plan else None, ptr(d_sess),
              ptr(d_table), ptr(ws), ws.numel(), stream())
-        return d_sess, (None if sink is not None else d_table), None, None, None, None, None, None, None
+        return d_sess, table_grad, None, None, None, None, None, None, None
 
 
 def sampled_loss(sess, item_embeddings, targets, negatives, kind: str, alpha=0.7, temperature=1.0,
                  total_sessions=None) -> torch.Tensor:
     """`item_embeddings` is the nn.Embedding the reference passes around (trainer.py:103)."""
-    weight = item_embeddings.weight if hasattr(item_embeddings, "weight") else item_embeddings
-    padding_idx = getattr(item_embeddings, "padding_idx", None)
+    weight, padding_idx = _weight_and_padding(item_embeddings)
     return SampledLoss.apply(sess, weight, targets, negatives, LOSS_MODES[kind], alpha, temperature,
                              total_sessions, padding_idx)
 
 
 # ------------------------------------------------------------------------------ full-catalogue softmax
+
+
+def _softmax_inputs(name, sess, table, targets, *more_cuda):
+    """Contiguous fp32 sess [B, D] and table [I, D] and int64 targets [B], checked as both softmax losses check them
+    (`name` in the messages); the (tensor, what) pairs of `more_cuda` must be on the GPU too."""
+    for t, what in ((sess, "session embeddings"), (table, "item embeddings"), (targets, "targets"), *more_cuda):
+        _require_cuda(t, what)
+    sess_c, table_c, targets = _f32(sess), _f32(table), _i64(targets)
+    if sess_c.dim() != 2 or table_c.dim() != 2 or sess_c.size(1) != table_c.size(1):
+        raise RuntimeError(f"{name}: sess [B, D] and table [I, D] expected; got "
+                           f"{tuple(sess_c.shape)} and {tuple(table_c.shape)}")
+    if targets.dim() != 1 or targets.size(0) != sess_c.size(0):
+        raise RuntimeError(f"target_items must be [batch={sess_c.size(0)}]; got {tuple(targets.shape)}")
+    return sess_c, table_c, targets
 
 
 class FullSoftmaxLoss(torch.autograd.Function):
@@ -1384,16 +1405,8 @@ class FullSoftmaxLoss(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, sess, table, targets, temperature, total_sessions, padding_idx):
-        _require_cuda(sess, "session embeddings")
-        _require_cuda(table, "item embeddings")
-        _require_cuda(targets, "targets")
-        sess_c, table_c, targets = _f32(sess), _f32(table), _i64(targets)
-        if sess_c.dim() != 2 or table_c.dim() != 2 or sess_c.size(1) != table_c.size(1):
-            raise RuntimeError(f"full_softmax_loss: sess [B, D] and table [I, D] expected; got "
-                               f"{tuple(sess_c.shape)} and {tuple(table_c.shape)}")
+        sess_c, table_c, targets = _softmax_inputs("full_softmax_loss", sess, table, targets)
         b, dim = sess_c.shape
-        if targets.dim() != 1 or targets.size(0) != b:
-            raise RuntimeError(f"target_items must be [batch={b}]; got {tuple(targets.shape)}")
         dev = sess_c.device
         total = float(total_sessions if total_sessions else b)
         pad = -1 if padding_idx is None else int(padding_idx)
@@ -1416,22 +1429,18 @@ class FullSoftmaxLoss(torch.autograd.Function):
         dev = sess.device
         d_loss = _f32(d_loss).reshape(1).contiguous()
         d_sess = torch.empty_like(sess) if ctx.needs_input_grad[0] else None
-        d_table = sink = None
-        if ctx.needs_input_grad[1]:
-            sink = _grad_sink(ctx.table_ref)
-            d_table = sink if sink is not None else torch.zeros_like(table)
+        d_table, table_grad = _table_grad(ctx, table.shape, dev)
         ws = workspace(size("etpgt_full_softmax_workspace_bytes", b, table.size(0), dim), dev)
         call("etpgt_full_softmax_bwd", ptr(sess), ptr(table), ptr(targets), ptr(lse), ptr(d_loss), b, table.size(0),
              dim, temperature, total, pad, ptr(d_sess), ptr(d_table), ptr(ws), ws.numel(), stream())
-        return d_sess, (None if sink is not None else d_table), None, None, None, None
+        return d_sess, table_grad, None, None, None, None
 
 
 def full_softmax_loss(sess, item_embeddings, targets, temperature=1.0, total_sessions=None) -> torch.Tensor:
     """Softmax cross-entropy of `targets` over the whole catalogue.  `item_embeddings` is the nn.Embedding (its
     padding_idx column is left out of the softmax and its row gets no gradient) or a bare weight tensor.  The table
     gradient goes into the etpgt_b200.optim gradient sink when one is registered, else it is returned densely."""
-    weight = item_embeddings.weight if hasattr(item_embeddings, "weight") else item_embeddings
-    padding_idx = getattr(item_embeddings, "padding_idx", None)
+    weight, padding_idx = _weight_and_padding(item_embeddings)
     return FullSoftmaxLoss.apply(sess, weight, targets, temperature, total_sessions, padding_idx)[0]
 
 
@@ -1502,17 +1511,11 @@ class PoolSoftmaxLoss(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, sess, table, targets, pool_ids, log_q, temperature, total_sessions, padding_idx, validate):
-        for t, what in ((sess, "session embeddings"), (table, "item embeddings"), (targets, "targets"),
-                        (pool_ids, "pool_ids"), (log_q, "log_q")):
-            _require_cuda(t, what)
-        sess_c, table_c, targets, pool, lq = _f32(sess), _f32(table), _i64(targets), _i64(pool_ids), _f32(log_q)
-        if sess_c.dim() != 2 or table_c.dim() != 2 or sess_c.size(1) != table_c.size(1):
-            raise RuntimeError(f"pool_softmax_loss: sess [B, D] and table [I, D] expected; got "
-                               f"{tuple(sess_c.shape)} and {tuple(table_c.shape)}")
+        sess_c, table_c, targets = _softmax_inputs("pool_softmax_loss", sess, table, targets, (pool_ids, "pool_ids"),
+                                                   (log_q, "log_q"))
+        pool, lq = _i64(pool_ids), _f32(log_q)
         b, dim = sess_c.shape
         items = table_c.size(0)
-        if targets.dim() != 1 or targets.size(0) != b:
-            raise RuntimeError(f"target_items must be [batch={b}]; got {tuple(targets.shape)}")
         if pool.dim() != 1 or pool.numel() == 0:
             raise RuntimeError(f"pool_softmax_loss: pool_ids must be a non-empty [M]; got {tuple(pool.shape)}")
         if lq.shape != pool.shape:
@@ -1549,15 +1552,12 @@ class PoolSoftmaxLoss(torch.autograd.Function):
         dev = sess.device
         d_loss = _f32(d_loss).reshape(1).contiguous()
         d_sess = torch.empty_like(sess) if ctx.needs_input_grad[0] else None
-        d_table = sink = None
-        if ctx.needs_input_grad[1]:
-            sink = _grad_sink(ctx.table_ref)
-            d_table = sink if sink is not None else torch.zeros_like(table)
+        d_table, table_grad = _table_grad(ctx, table.shape, dev)
         ws = workspace(size("etpgt_pool_softmax_workspace_bytes", b, m, dim), dev)
         call("etpgt_pool_softmax_bwd", ptr(sess), ptr(table), ptr(targets), ptr(pool), ptr(lq), ptr(lse), ptr(z_pos),
              ptr(d_loss), b, table.size(0), m, dim, temperature, total, pad, ptr(d_sess), ptr(d_table), ptr(ws),
              ws.numel(), stream())
-        return d_sess, (None if sink is not None else d_table), None, None, None, None, None, None, None
+        return d_sess, table_grad, None, None, None, None, None, None, None
 
 
 def pool_softmax_loss(sess, item_embeddings, targets, pool_ids, log_q, temperature=1.0,
@@ -1568,8 +1568,7 @@ def pool_softmax_loss(sess, item_embeddings, targets, pool_ids, log_q, temperatu
     nn.Embedding (its padding_idx never counts as a negative and its row gets no gradient) or a bare weight tensor.
     The table gradient goes into the etpgt_b200.optim gradient sink when one is registered, else it is returned
     densely (non-zero on the pool and target rows only)."""
-    weight = item_embeddings.weight if hasattr(item_embeddings, "weight") else item_embeddings
-    padding_idx = getattr(item_embeddings, "padding_idx", None)
+    weight, padding_idx = _weight_and_padding(item_embeddings)
     return PoolSoftmaxLoss.apply(sess, weight, targets, pool_ids, log_q, temperature, total_sessions, padding_idx,
                                  True)[0]
 

@@ -81,8 +81,7 @@ class SharedPoolSoftmaxLoss(nn.Module):
         self._cum = None
 
     def forward(self, session_embeddings, target_items, negative_items, item_embeddings) -> torch.Tensor:
-        weight = item_embeddings.weight if hasattr(item_embeddings, "weight") else item_embeddings
-        padding_idx = getattr(item_embeddings, "padding_idx", None)
+        weight, padding_idx = ops._weight_and_padding(item_embeddings)
         items = weight.size(0)
         if self._cum is None or self._cum.device != weight.device or self._cum.numel() != items + 1:
             self._cum = ops.item_sampling_table(self.item_counts, self.sampling_power,

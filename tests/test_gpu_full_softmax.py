@@ -7,6 +7,8 @@ import numpy as np
 import pytest
 import torch
 
+from softmax_loss_util import err, grads, model_and_batch
+
 TOL = 1e-4
 
 
@@ -112,11 +114,6 @@ def _reference(sess, table, targets, temperature=1.0, total=None, padding_idx=0,
     return loss * d_loss / total, lse, d_sess, d_table
 
 
-def _err(got, want):
-    got, want = torch.as_tensor(got).double(), torch.as_tensor(want).double().to(torch.as_tensor(got).device)
-    return float((got - want).abs().max() / want.abs().max().clamp_min(1e-300))
-
-
 def _inputs(b, items, dim, seed, scale=0.3):
     g = torch.Generator(device="cuda").manual_seed(seed)
     sess = torch.randn(b, dim, device="cuda", generator=g) * scale
@@ -128,7 +125,7 @@ def _inputs(b, items, dim, seed, scale=0.3):
 def _check(sess, table, targets, temperature=1.0, total=None, padding_idx=0, tol=TOL):
     got = _run(sess, table, targets, temperature, total, padding_idx)
     want = _reference(sess, table, targets, temperature, total, padding_idx)
-    errs = {name: _err(g, w) for name, g, w in zip(("loss", "lse", "d_sess", "d_table"), got, want)}
+    errs = {name: err(g, w) for name, g, w in zip(("loss", "lse", "d_sess", "d_table"), got, want)}
     assert all(v <= tol for v in errs.values()), errs
     return got
 
@@ -178,7 +175,7 @@ def test_all_equal_logits():
     targets = torch.randint(1, items, (b,), device="cuda")
     loss, lse, d_sess, d_table = _run(sess, table, targets)
     w_loss, w_lse, _, w_dt = _reference(sess, table, targets)
-    assert _err(loss, w_loss) <= TOL and _err(lse, w_lse) <= TOL and _err(d_table, w_dt) <= TOL
+    assert err(loss, w_loss) <= TOL and err(lse, w_lse) <= TOL and err(d_table, w_dt) <= TOL
     want = np.log(items - 1) + 0.0                     # every logit equal: lse - z_t = log(I - 1)
     assert abs(float(loss) - want) <= 1e-5 * want
     # dS = mean_j E_j - E_t = 0 exactly when every row of E is the same: there is no scale to be relative to, so
@@ -217,7 +214,7 @@ def test_d_table_accumulates_onto_existing_values():
     base[0] = 7.0
     _, _, _, d_table = _run(sess, table, targets, d_table=base.clone())
     want = _reference(sess, table, targets)[3] + base.double()
-    assert _err(d_table - base, want - base.double()) <= TOL
+    assert err(d_table - base, want - base.double()) <= TOL
     assert torch.all(d_table[0] == 7.0)                 # the padding row is left untouched
 
 
@@ -226,7 +223,7 @@ def test_upstream_gradient_scales_the_backward():
     sess, table, targets = _inputs(200, 3000, 64, seed=6)
     got = _run(sess, table, targets, d_loss=-2.5)
     want = _reference(sess, table, targets, d_loss=-2.5)
-    assert _err(got[2], want[2]) <= TOL and _err(got[3], want[3]) <= TOL
+    assert err(got[2], want[2]) <= TOL and err(got[3], want[3]) <= TOL
 
 
 @pytest.mark.gpu
@@ -247,11 +244,11 @@ def test_full_size():
     loss, lse, d_sess, d_table = _run(sess, table, targets)
     rows = torch.randperm(b, device="cuda", generator=torch.Generator(device="cuda").manual_seed(1))[:512]
     w_loss, w_lse, w_ds, w_dt = _reference(sess, table, targets, rows_only=rows)
-    assert _err(loss, torch.tensor(w_loss)) <= TOL
-    assert _err(lse, w_lse) <= TOL
-    assert _err(d_sess[rows], w_ds[rows]) <= TOL
+    assert err(loss, torch.tensor(w_loss)) <= TOL
+    assert err(lse, w_lse) <= TOL
+    assert err(d_sess[rows], w_ds[rows]) <= TOL
     item_rows = torch.randperm(items, device="cuda")[:2048]
-    assert _err(d_table[item_rows], w_dt[item_rows]) <= TOL
+    assert err(d_table[item_rows], w_dt[item_rows]) <= TOL
 
 
 @pytest.mark.gpu
@@ -276,24 +273,6 @@ def test_bad_targets_shape_is_rejected():
 # ------------------------------------------------------------------------------ GPU: autograd and model level
 
 
-def _model_and_batch(dim=64, sessions=256):
-    from etpgt_b200 import data, synth
-    from etpgt_b200.model import create_graph_transformer_optimized
-
-    d = synth.generate(num_sessions=1200, graph_sessions=900, num_items=400, clusters=16, seed=5)
-    graph = data.ItemGraph(d.item_i, d.item_j, d.num_items)
-    store = data.SessionStore(d.sess_ptr, d.sess_items)
-    torch.manual_seed(1)
-    model = create_graph_transformer_optimized(d.num_items, dim, dim, num_layers=2, num_heads=2, dropout=0.0,
-                                               use_laplacian_pe=False).cuda()
-    batch = data.build_batch(graph, store, np.arange(sessions), 50, False, False)
-    return model, batch, (d, graph, store)
-
-
-def _grads(model):
-    return {n: p.grad.detach().clone() for n, p in model.named_parameters() if p.grad is not None}
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("opt_kind", ["torch", "etpgt"])
 def test_model_gradients_match_fp64_cross_entropy(opt_kind):
@@ -302,7 +281,7 @@ def test_model_gradients_match_fp64_cross_entropy(opt_kind):
     from etpgt_b200 import ops, optim
 
     temperature = 0.5
-    model, batch, _ = _model_and_batch()
+    model, batch, _ = model_and_batch()
     model.train()
     table = model.item_embedding.weight
     if opt_kind == "torch":
@@ -315,7 +294,7 @@ def test_model_gradients_match_fp64_cross_entropy(opt_kind):
     loss.backward()
     if opt_kind == "etpgt":
         assert optim.grad_sink_for(table) is table.grad        # the table gradient went into the sink
-    got = _grads(model)
+    got = grads(model)
     got_loss = float(loss.detach())
     # the same forward, then the fp64 torch loss over the table without its padding column
     for p in model.parameters():
@@ -324,7 +303,7 @@ def test_model_gradients_match_fp64_cross_entropy(opt_kind):
     logits = sess.double() @ table.double()[1:].T / temperature
     want_loss = F.cross_entropy(logits, batch.target_item - 1)
     want_loss.backward()
-    want = _grads(model)
+    want = grads(model)
     want_loss = float(want_loss.detach())
     assert abs(got_loss - want_loss) <= TOL * abs(want_loss)
     assert set(got) == set(want)
@@ -335,7 +314,7 @@ def test_model_gradients_match_fp64_cross_entropy(opt_kind):
         if float(want[name].abs().max()) <= 1e-6 * scale:
             assert float((got[name] - want[name]).abs().max()) <= 1e-6 * scale, name
             continue
-        assert _err(got[name], want[name]) <= TOL, (name, _err(got[name], want[name]))
+        assert err(got[name], want[name]) <= TOL, (name, err(got[name], want[name]))
     # one optimizer step runs on either gradient path
     opt.step()
 
@@ -346,7 +325,7 @@ def test_trainer_takes_the_per_operator_path_and_learns(tmp_path):
     from etpgt_b200.train.losses import create_loss_function
     from etpgt_b200.train.trainer import Trainer
 
-    model, _, (d, graph, store) = _model_and_batch()
+    model, _, (d, graph, store) = model_and_batch()
 
     def batches(lo, hi, step0):
         out = []

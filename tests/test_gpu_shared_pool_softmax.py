@@ -9,13 +9,9 @@ import pytest
 import torch
 
 from shared_pool_ref import pool_softmax_fp64, sample_item_pool
+from softmax_loss_util import err, grads, model_and_batch
 
 TOL = 1e-4
-
-
-def _err(got, want):
-    got, want = torch.as_tensor(got).double(), torch.as_tensor(want).double().to(torch.as_tensor(got).device)
-    return float((got - want).abs().max() / want.abs().max().clamp_min(1e-300))
 
 
 def _zipf_counts(num_items, a=1.5, seed=0):
@@ -117,7 +113,7 @@ def test_pool_of_every_item_reduces_to_the_full_loss(dim, temperature):
               temperature, 0.0, 0, ptr(d_sess), ptr(d_table), ptr(ws), ws.numel(), _lib.stream())
     torch.cuda.synchronize()
     for name, g, w in zip(("loss", "lse", "d_sess", "d_table"), got, (loss[0], lse, d_sess, d_table)):
-        assert _err(g, w) <= 1e-5, (name, _err(g, w))
+        assert err(g, w) <= 1e-5, (name, err(g, w))
 
 
 @pytest.mark.gpu
@@ -129,7 +125,7 @@ def test_matches_fp64_on_the_grid(batch, m, dim):
     sess, table, targets, pool, log_q = _inputs(batch, items, dim, m, seed=batch + m + dim)
     got = _run(sess, table, targets, pool, log_q, temperature=0.5)
     want = pool_softmax_fp64(sess, table, targets, pool, log_q, temperature=0.5)
-    errs = {name: _err(g, w) for name, g, w in zip(("loss", "lse", "d_sess", "d_table"), got, want)}
+    errs = {name: err(g, w) for name, g, w in zip(("loss", "lse", "d_sess", "d_table"), got, want)}
     assert all(v <= TOL for v in errs.values()), errs
     # row 0's target is pool[0]; with M = 1 its whole pool is its target: P = 1 exactly and its gradient is zero
     if m == 1:
@@ -147,7 +143,7 @@ def test_pool_entirely_the_target_gives_zero_gradient_for_that_row():
     want = pool_softmax_fp64(sess, table, targets, pool, log_q)
     assert float(got[2][0].abs().max()) == 0.0
     for name, g, w in zip(("loss", "lse", "d_sess", "d_table"), got, want):
-        assert _err(g, w) <= TOL, name
+        assert err(g, w) <= TOL, name
 
 
 @pytest.mark.gpu
@@ -160,8 +156,8 @@ def test_accumulates_and_keeps_padding_and_untouched_rows():
     base = torch.randn(items, dim, device="cuda")
     got = _run(sess, table, targets, pool, log_q, d_table=base.clone())
     want = pool_softmax_fp64(sess, table, targets, pool, log_q)
-    assert _err(got[0], want[0]) <= TOL and _err(got[2], want[2]) <= TOL
-    assert _err(got[3] - base, want[3]) <= TOL
+    assert err(got[0], want[0]) <= TOL and err(got[2], want[2]) <= TOL
+    assert err(got[3] - base, want[3]) <= TOL
     touched = torch.zeros(items, dtype=torch.bool, device="cuda")
     touched[pool] = True
     touched[targets] = True
@@ -205,10 +201,10 @@ def test_bit_reproducible_and_data_parallel_halves():
     h = b // 2
     lo = _run(sess[:h].contiguous(), table, targets[:h].contiguous(), pool, log_q, total=b)
     hi = _run(sess[h:].contiguous(), table, targets[h:].contiguous(), pool, log_q, total=b)
-    assert _err(lo[0] + hi[0], a[0]) <= 1e-5
-    assert _err(torch.cat([lo[1], hi[1]]), a[1]) <= 1e-5
-    assert _err(torch.cat([lo[2], hi[2]]), a[2]) <= 1e-5
-    assert _err(lo[3] + hi[3], a[3]) <= 1e-5
+    assert err(lo[0] + hi[0], a[0]) <= 1e-5
+    assert err(torch.cat([lo[1], hi[1]]), a[1]) <= 1e-5
+    assert err(torch.cat([lo[2], hi[2]]), a[2]) <= 1e-5
+    assert err(lo[3] + hi[3], a[3]) <= 1e-5
 
 
 # ------------------------------------------------------------------------------ host errors
@@ -255,30 +251,12 @@ def test_unsorted_pool_is_sorted_with_its_log_q():
 # ------------------------------------------------------------------------------ model and Trainer
 
 
-def _model_and_batch(dim=64, sessions=256):
-    from etpgt_b200 import data, synth
-    from etpgt_b200.model import create_graph_transformer_optimized
-
-    d = synth.generate(num_sessions=1200, graph_sessions=900, num_items=400, clusters=16, seed=5)
-    graph = data.ItemGraph(d.item_i, d.item_j, d.num_items)
-    store = data.SessionStore(d.sess_ptr, d.sess_items)
-    torch.manual_seed(1)
-    model = create_graph_transformer_optimized(d.num_items, dim, dim, num_layers=2, num_heads=2, dropout=0.0,
-                                               use_laplacian_pe=False).cuda()
-    batch = data.build_batch(graph, store, np.arange(sessions), 50, False, False)
-    return model, batch, (d, graph, store)
-
-
-def _grads(model):
-    return {n: p.grad.detach().clone() for n, p in model.named_parameters() if p.grad is not None}
-
-
 @pytest.mark.gpu
 def test_model_gradients_match_fp64_objective():
     from etpgt_b200 import ops
 
     temperature = 0.5
-    model, batch, (d, _, _) = _model_and_batch()
+    model, batch, (d, _, _) = model_and_batch()
     model.train()
     cum = ops.item_sampling_table(num_items=d.num_items, device="cuda")
     pool, log_q = ops.sample_item_pool(cum, 300, seed=1, step=0)
@@ -287,7 +265,7 @@ def test_model_gradients_match_fp64_objective():
     loss = ops.pool_softmax_loss(model(batch), model.item_embedding, batch.target_item, pool, log_q,
                                  temperature=temperature)
     loss.backward()
-    got, got_loss = _grads(model), float(loss.detach())
+    got, got_loss = grads(model), float(loss.detach())
     for p in model.parameters():
         p.grad = None
     sess = model(batch).double()
@@ -298,7 +276,7 @@ def test_model_gradients_match_fp64_objective():
     z = z.masked_fill((pool[None, :] == t[:, None]) | (pool == 0)[None, :], -float("inf"))
     want_loss = (torch.logsumexp(torch.cat([z_pos[:, None], z], 1), 1) - z_pos).mean()
     want_loss.backward()
-    want, want_loss = _grads(model), float(want_loss.detach())
+    want, want_loss = grads(model), float(want_loss.detach())
     assert abs(got_loss - want_loss) <= TOL * abs(want_loss)
     assert set(got) == set(want)
     scale = max(float(g.abs().max()) for g in want.values())
@@ -306,7 +284,7 @@ def test_model_gradients_match_fp64_objective():
         if float(want[name].abs().max()) <= 1e-6 * scale:
             assert float((got[name] - want[name]).abs().max()) <= 1e-6 * scale, name
             continue
-        assert _err(got[name], want[name]) <= TOL, (name, _err(got[name], want[name]))
+        assert err(got[name], want[name]) <= TOL, (name, err(got[name], want[name]))
 
 
 @pytest.mark.gpu
@@ -316,7 +294,7 @@ def test_trainer_learns_with_the_shared_pool(opt_kind, tmp_path):
     from etpgt_b200.train.losses import create_loss_function
     from etpgt_b200.train.trainer import Trainer
 
-    model, _, (d, graph, store) = _model_and_batch()
+    model, _, (d, graph, store) = model_and_batch()
 
     def batches(lo, hi, step0):
         out = []

@@ -16,7 +16,6 @@ from __future__ import annotations
 
 import argparse
 import json
-import subprocess
 import sys
 import tempfile
 from pathlib import Path
@@ -27,35 +26,9 @@ import torch
 ROOT = Path(__file__).resolve().parents[1]
 sys.path.insert(0, str(ROOT / "gat-recommendation_b200"))
 
+from bench_full_softmax import gpu_info, timed  # noqa: E402
+
 DIM = 256
-
-
-def gpu_info() -> dict:
-    info = {"gpu": torch.cuda.get_device_name(0)}
-    try:
-        out = subprocess.run(["nvidia-smi", "--id=0", "--query-gpu=power.limit,clocks.max.sm",
-                              "--format=csv,noheader,nounits"], capture_output=True, text=True, timeout=30).stdout
-        power, clock = [v.strip() for v in out.strip().split(",")]
-        info.update(power_limit_w=float(power), max_sm_clock_mhz=float(clock))
-    except Exception as e:   # the numbers still stand, without the card's limits
-        info["power_limit_w"] = f"unavailable ({type(e).__name__})"
-    return info
-
-
-def timed(fn, reps: int, calls: int) -> float:
-    """Median ms per call over `reps` windows of `calls` calls, after one warm-up call."""
-    fn()
-    torch.cuda.synchronize()
-    times = []
-    for _ in range(reps):
-        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        a.record()
-        for _ in range(calls):
-            fn()
-        b.record()
-        b.synchronize()
-        times.append(a.elapsed_time(b) / calls)
-    return sorted(times)[len(times) // 2]
 
 
 def bench_shape(b: int, m: int, items: int, reps: int, calls: int) -> dict:

@@ -20,6 +20,9 @@
 // The backward recomputes the forward's logits bit for bit (same MMA sequence, operands swapped in DE) and keeps
 // them, lse and the running maxima in natural units (exp(x) = 2^(x log2 e) on the MUFU unit): where the softmax
 // is exact — one eligible column, P = 1 — the gradient is exactly zero, not rounding noise.
+// With PREC = ETPGT_SOFTMAX_BF16 (opt-in, a different numerical contract) S, the columns and G are rounded once to
+// bf16 and every product is one MMA per k-step; the CTA's 128 rows x D then stay resident in shared memory (<= 64 KB)
+// and the column tiles stream through a ring of single boxes.  Everything else is the same code.
 //
 // The same kernel, instantiated with POOL, computes the sampled softmax over one pool of M negatives shared by the
 // batch, with the log-Q correction (Bengio & Senecal 2008; Jean et al. 2015; Yi et al. 2019).  For pool ids p [M]
@@ -68,18 +71,30 @@ __device__ __forceinline__ int chunk_pos(int64_t id, int64_t base) {
   const int64_t d = id - base;
   return d >= 0 && d < 32 ? (int)d : -1;
 }
-template <int MODE> struct Cfg {
-  static constexpr int stages = MODE == FWD ? 3 : 2;
-  static constexpr uint32_t tmem_cols = MODE == FWD ? 256 : 512;
-  static constexpr size_t smem = 1024 + (size_t)stages * STAGE_BYTES + (MODE == FWD ? 0 : G_BYTES) + 256;
-};
-
-struct __align__(8) Bars {
-  uint64_t full[3], empty[3];
+// one set of barriers for up to S ring stages; rfull (bf16 only) follows tmem_base so that the split-bf16 kernels keep
+// their offsets
+template <int S> struct __align__(8) Bars {
+  uint64_t full[S], empty[S];
   uint64_t lfull[2], lempty[2];   // logits buffers
   uint64_t gfull, gempty;         // G tile in shared memory
   uint64_t accfull, accempty;    // gradient accumulator: one phase per drain group
   uint32_t tmem_base;
+  uint64_t rfull;                 // bf16: the resident row tile
+};
+
+// Shared memory, in order: the resident row tile (bf16 only), the TMA ring, the G tile (DS, DE) and the barriers.
+// split-bf16: ring stages of row hi, row lo, column hi, column lo (64 KB), G as hi and lo (64 KB).
+// bf16: the CTA's 128 rows x D stay resident (<= 64 KB), the column tiles stream through a ring of single 16 KB boxes,
+// and G is one bf16 copy (32 KB): 192 KB + 32 KB in DS / DE, one CTA per SM.
+template <int MODE, int PREC = ETPGT_SOFTMAX_BF16X3> struct Cfg {
+  static constexpr bool bf16 = PREC == ETPGT_SOFTMAX_BF16;
+  static constexpr int stages = bf16 ? 8 : MODE == FWD ? 3 : 2;
+  static constexpr uint32_t stage_bytes = bf16 ? KB_BYTES : STAGE_BYTES;
+  static constexpr uint32_t rows_bytes = bf16 ? 4 * KB_BYTES : 0;
+  static constexpr uint32_t g_bytes = MODE == FWD ? 0 : bf16 ? 2 * KB_BYTES : G_BYTES;
+  static constexpr uint32_t tmem_cols = MODE == FWD ? 256 : 512;
+  using Barriers = Bars<bf16 ? stages : 3>;
+  static constexpr size_t smem = 1024 + rows_bytes + (size_t)stages * stage_bytes + g_bytes + 256;
 };
 
 struct Params {
@@ -98,16 +113,19 @@ struct Params {
   const int2* hits;             // POOL: per session, the pool positions [x, y) equal to its target
 };
 
-template <int MODE, bool POOL = false>
+template <int MODE, bool POOL = false, int PREC = ETPGT_SOFTMAX_BF16X3>
 __global__ void __launch_bounds__(kThreads, 1)
 full_softmax_tc_kernel(const __grid_constant__ CUtensorMap map_r_hi, const __grid_constant__ CUtensorMap map_r_lo,
                        const __grid_constant__ CUtensorMap map_c_hi, const __grid_constant__ CUtensorMap map_c_lo,
                        const Params p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-  constexpr int kStages = Cfg<MODE>::stages;
-  uint8_t* smem_g = smem + kStages * STAGE_BYTES;
-  Bars* bars = reinterpret_cast<Bars*>(smem_g + (MODE == FWD ? 0 : G_BYTES));
+  using C = Cfg<MODE, PREC>;
+  constexpr bool kBf16 = C::bf16;
+  constexpr int kStages = C::stages;
+  uint8_t* ring = smem + C::rows_bytes;  // bf16: the resident row tile comes first
+  uint8_t* smem_g = ring + kStages * C::stage_bytes;
+  auto* bars = reinterpret_cast<typename C::Barriers*>(smem_g + C::g_bytes);
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -127,20 +145,42 @@ full_softmax_tc_kernel(const __grid_constant__ CUtensorMap map_r_hi, const __gri
     mbar_init(&bars->gempty, 1);
     mbar_init(&bars->accfull, 1);
     mbar_init(&bars->accempty, 4);
+    if constexpr (kBf16) mbar_init(&bars->rfull, 1);
     fence_barrier_init();
     tma_prefetch_desc(&map_r_hi);
-    tma_prefetch_desc(&map_r_lo);
+    if constexpr (!kBf16) tma_prefetch_desc(&map_r_lo);
     tma_prefetch_desc(&map_c_hi);
-    tma_prefetch_desc(&map_c_lo);
+    if constexpr (!kBf16) tma_prefetch_desc(&map_c_lo);
   }
-  if (warp == 1) tmem_alloc(&bars->tmem_base, Cfg<MODE>::tmem_cols);
+  if (warp == 1) tmem_alloc(&bars->tmem_base, C::tmem_cols);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = bars->tmem_base;
 
   if (warp == 0) {
-    if (lane == 0) {
+    if (kBf16 && lane == 0) {
+      int stage = 0;
+      uint32_t phase = 0;
+      // the CTA's rows once, then the k-blocks of the column tiles one box per stage, in the order the MMA warp
+      // consumes them: logits of tile j, then the gradient product of tile j - 1
+      mbar_expect_tx(&bars->rfull, (uint32_t)nkb * KB_BYTES);
+      for (int kb = 0; kb < nkb; ++kb)
+        tma_load_2d(&map_r_hi, &bars->rfull, smem + kb * KB_BYTES, kb * BLOCK_K, rt * TILE);
+      auto load = [&](int ct) {
+        for (int kb = 0; kb < nkb; ++kb) {
+          mbar_wait(&bars->empty[stage], phase ^ 1);
+          mbar_expect_tx(&bars->full[stage], KB_BYTES);
+          tma_load_2d(&map_c_hi, &bars->full[stage], ring + stage * KB_BYTES, kb * BLOCK_K, ct * TILE);
+          if (++stage == kStages) { stage = 0; phase ^= 1; }
+        }
+      };
+      for (int j = 0; j < n; ++j) {
+        load(ct0 + j);
+        if (MODE != FWD && j > 0) load(ct0 + j - 1);
+      }
+      if (MODE != FWD) load(ct1 - 1);
+    } else if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
       // the k-blocks of column tile ct, with the row tile's (logits) or alone (second pass of the gradients)
@@ -166,7 +206,64 @@ full_softmax_tc_kernel(const __grid_constant__ CUtensorMap map_r_hi, const __gri
       if (MODE != FWD) load(ct1 - 1, false);
     }
   } else if (warp == 1) {
-    if (lane == 0) {
+    if (kBf16 && lane == 0) {
+      int stage = 0;
+      uint32_t phase = 0;
+      constexpr uint32_t idesc_l = instr_desc_bf16(TILE, TILE);
+      constexpr uint32_t idesc_g = instr_desc_bf16_major(TILE, BLOCK_K, false, true);
+      const uint32_t rows = smem_u32(smem), g = smem_u32(smem_g);
+      // the same gradient product as below with one bf16 G and one bf16 column tile: one MMA per k-step
+      auto grad = [&](int j) {
+        const int group = j / kDrainTiles;
+        const bool group_start = j % kDrainTiles == 0, group_end = (j + 1) % kDrainTiles == 0 || j == n - 1;
+        if (group_start && group > 0) mbar_wait(&bars->accempty, (uint32_t)(group - 1) & 1);  // drained
+        mbar_wait(&bars->gfull, (uint32_t)j & 1);
+        tc_fence_after();
+        for (int kb = 0; kb < nkb; ++kb) {
+          mbar_wait(&bars->full[stage], phase);
+          tc_fence_after();
+          const uint32_t c = smem_u32(ring + stage * KB_BYTES);
+          const uint32_t tmem_d = tmem_base + ACC_COL + (uint32_t)(kb * BLOCK_K);
+#pragma unroll
+          for (int kk = 0; kk < TILE / UMMA_K; ++kk) {
+            const uint32_t off_a = (uint32_t)(kk >> 2) * KB_BYTES + (uint32_t)(kk & 3) * UMMA_K * 2;
+            const uint32_t off_b = (uint32_t)kk * UMMA_K * 128;
+            umma_bf16(tmem_d, make_desc_sw128(g + off_a), make_desc_mn_sw128(c + off_b, KB_BYTES), idesc_g,
+                      (group_start && kk == 0) ? 0u : 1u);
+          }
+          umma_commit(&bars->empty[stage]);
+          if (++stage == kStages) { stage = 0; phase ^= 1; }
+        }
+        umma_commit(&bars->gempty);
+        if (group_end) umma_commit(&bars->accfull);
+      };
+      mbar_wait(&bars->rfull, 0);
+      tc_fence_after();
+      for (int j = 0; j < n; ++j) {
+        const int b = j & 1;
+        mbar_wait(&bars->lempty[b], ((uint32_t)(j >> 1) & 1) ^ 1);
+        tc_fence_after();
+        const uint32_t tmem_d = tmem_base + (uint32_t)(b * TILE);
+        for (int kb = 0; kb < nkb; ++kb) {
+          mbar_wait(&bars->full[stage], phase);
+          tc_fence_after();
+          const uint32_t r = rows + (uint32_t)kb * KB_BYTES, c = smem_u32(ring + stage * KB_BYTES);
+          // one product per k-step in the same k order in every pass (DE has the operands swapped), so the
+          // recomputed logits are the forward's bit for bit
+#pragma unroll
+          for (int kk = 0; kk < BLOCK_K / UMMA_K; ++kk) {
+            const uint32_t off = (uint32_t)kk * UMMA_K * 2;
+            umma_bf16(tmem_d, make_desc_sw128(r + off), make_desc_sw128(c + off), idesc_l,
+                      (kb == 0 && kk == 0) ? 0u : 1u);
+          }
+          umma_commit(&bars->empty[stage]);
+          if (++stage == kStages) { stage = 0; phase ^= 1; }
+        }
+        umma_commit(&bars->lfull[b]);
+        if (MODE != FWD && j > 0) grad(j - 1);
+      }
+      if (MODE != FWD) grad(n - 1);
+    } else if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
       constexpr uint32_t idesc_l = instr_desc_bf16(TILE, TILE);
@@ -413,7 +510,8 @@ full_softmax_tc_kernel(const __grid_constant__ CUtensorMap map_r_hi, const __gri
             }
             g[e] = pr * gscale;
           }
-          // split into the bf16 pair; 128-byte swizzle of the K-major A operand (16-byte unit ^ row % 8)
+          // split into the bf16 pair (bf16: only hi is stored, G rounded once); 128-byte swizzle of the K-major A
+          // operand (16-byte unit ^ row % 8)
           uint8_t* g_kb = g_row + (c >> 6) * KB_BYTES;
 #pragma unroll
           for (int u = 0; u < 4; ++u) {
@@ -429,7 +527,8 @@ full_softmax_tc_kernel(const __grid_constant__ CUtensorMap map_r_hi, const __gri
             }
             const uint32_t off = (uint32_t)(((((c & 63) >> 3) + u) ^ (lane & 7)) << 4);
             *reinterpret_cast<uint4*>(g_kb + off) = make_uint4(h[0], h[1], h[2], h[3]);
-            *reinterpret_cast<uint4*>(g_kb + 2 * KB_BYTES + off) = make_uint4(l[0], l[1], l[2], l[3]);
+            if constexpr (!kBf16)
+              *reinterpret_cast<uint4*>(g_kb + 2 * KB_BYTES + off) = make_uint4(l[0], l[1], l[2], l[3]);
           }
         }
         fence_proxy_async_smem();  // generic-proxy writes -> visible to the tensor cores
@@ -443,7 +542,7 @@ full_softmax_tc_kernel(const __grid_constant__ CUtensorMap map_r_hi, const __gri
   __syncthreads();
   if (warp == 1) {
     tc_fence_after();
-    tmem_dealloc(tmem_base, Cfg<MODE>::tmem_cols);
+    tmem_dealloc(tmem_base, C::tmem_cols);
   }
 }
 
@@ -550,6 +649,7 @@ Layout layout(int64_t batch, int64_t cols, int dim) {
 // full loss
 struct Operands {
   CUtensorMap s_hi, s_lo, c_hi, c_lo;
+  void* s_slots = nullptr;      // the session pair's 2 * s_pair bytes
   float* part = nullptr;
   float *d_pool = nullptr, *bias = nullptr, *coef = nullptr;
   int2* hits = nullptr;
@@ -572,10 +672,12 @@ int check_args(const char* name, int dim, Ranges ranges, bool args_set, float te
 }
 
 // Checks the workspace, carves the two bf16 pairs and the partials, splits sess, lets `columns(w, c_hi, c_lo)` fill
-// the column pair (and carve what else the loss needs from w), then encodes the four tensor maps.
+// the column pair (and carve what else the loss needs from w), then encodes the four tensor maps.  bf16: the same
+// carve, but sess and the columns are rounded once into the hi slots (c_lo is null for `columns`), the lo slots stay
+// unused and the lo maps are the hi maps.
 template <class Columns>
-int prepare(const char* name, const Layout& l, const float* sess, int64_t batch, int64_t cols, int dim, void* ws,
-            size_t ws_bytes, cudaStream_t stream, Operands* o, Columns columns) {
+int prepare(const char* name, const Layout& l, const float* sess, int64_t batch, int64_t cols, int dim, bool bf16,
+            void* ws, size_t ws_bytes, cudaStream_t stream, Operands* o, Columns columns) {
   if (ws == nullptr || ws_bytes < l.total()) {
     set_error("%s: workspace too small (%zu < %zu bytes)", name, ws_bytes, l.total());
     return ETPGT_EWORKSPACE;
@@ -586,15 +688,31 @@ int prepare(const char* name, const Layout& l, const float* sess, int64_t batch,
   auto* c_hi = w.take<__nv_bfloat16>(l.c_pair / 2);
   auto* c_lo = w.take<__nv_bfloat16>(l.c_pair / 2);
   o->part = w.take<float>(l.part / sizeof(float));
-  int rc = etpgt_split_bf16(sess, batch, dim, dim, s_hi, s_lo, dim, nullptr, nullptr, 0, nullptr, nullptr, 0, stream);
+  o->s_slots = s_hi;
+  int rc = bf16 ? etpgt_f32_to_bf16(sess, s_hi, batch * dim, stream)
+                : etpgt_split_bf16(sess, batch, dim, dim, s_hi, s_lo, dim, nullptr, nullptr, 0, nullptr, nullptr, 0,
+                                   stream);
   if (rc != ETPGT_OK) return rc;
-  rc = columns(w, c_hi, c_lo);
+  rc = columns(w, c_hi, bf16 ? nullptr : c_lo);
   if (rc != ETPGT_OK) return rc;
-  if (!(make_map_bf16(&o->s_hi, s_hi, batch, dim, dim, TILE) && make_map_bf16(&o->s_lo, s_lo, batch, dim, dim, TILE) &&
-        make_map_bf16(&o->c_hi, c_hi, cols, dim, dim, TILE) && make_map_bf16(&o->c_lo, c_lo, cols, dim, dim, TILE))) {
+  if (!(make_map_bf16(&o->s_hi, s_hi, batch, dim, dim, TILE) && make_map_bf16(&o->c_hi, c_hi, cols, dim, dim, TILE) &&
+        (bf16 || (make_map_bf16(&o->s_lo, s_lo, batch, dim, dim, TILE) &&
+                  make_map_bf16(&o->c_lo, c_lo, cols, dim, dim, TILE))))) {
     set_error("%s: cuTensorMapEncodeTiled failed", name);
     return ETPGT_ECUDA;
   }
+  if (bf16) {
+    o->s_lo = o->s_hi;
+    o->c_lo = o->c_hi;
+  }
+  return ETPGT_OK;
+}
+
+// precision is one of the two ETPGT_SOFTMAX_* values
+int check_precision(const char* name, int precision) {
+  ETPGT_REQUIRE(precision == ETPGT_SOFTMAX_BF16X3 || precision == ETPGT_SOFTMAX_BF16,
+                "%s: precision %d is not supported (ETPGT_SOFTMAX_BF16X3 = 0 or ETPGT_SOFTMAX_BF16 = 1)", name,
+                precision);
   return ETPGT_OK;
 }
 
@@ -618,14 +736,24 @@ Params call_params(int dim, float temperature, double total, int64_t padding_idx
   return p;
 }
 
-template <int MODE, bool POOL = false>
-int launch(const CUtensorMap& r_hi, const CUtensorMap& r_lo, const CUtensorMap& c_hi, const CUtensorMap& c_lo,
-           const Params& p, int grid, const char* name, cudaStream_t stream) {
-  const size_t smem = Cfg<MODE>::smem + sizeof(Bars);
-  cudaFuncSetAttribute(full_softmax_tc_kernel<MODE, POOL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  full_softmax_tc_kernel<MODE, POOL><<<grid, kThreads, smem, stream>>>(r_hi, r_lo, c_hi, c_lo, p);
+template <int MODE, bool POOL, int PREC>
+int launch_prec(const CUtensorMap& r_hi, const CUtensorMap& r_lo, const CUtensorMap& c_hi, const CUtensorMap& c_lo,
+                const Params& p, int grid, const char* name, cudaStream_t stream) {
+  using C = Cfg<MODE, PREC>;
+  const size_t smem = C::smem + sizeof(typename C::Barriers);
+  cudaFuncSetAttribute(full_softmax_tc_kernel<MODE, POOL, PREC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                       (int)smem);
+  full_softmax_tc_kernel<MODE, POOL, PREC><<<grid, kThreads, smem, stream>>>(r_hi, r_lo, c_hi, c_lo, p);
   ETPGT_CHECK_LAUNCH(name);
   return ETPGT_OK;
+}
+// the kernel of `precision`; a bf16 call's lo maps are its hi maps and are not read
+template <int MODE, bool POOL = false>
+int launch(const CUtensorMap& r_hi, const CUtensorMap& r_lo, const CUtensorMap& c_hi, const CUtensorMap& c_lo,
+           const Params& p, int grid, const char* name, int precision, cudaStream_t stream) {
+  return precision == ETPGT_SOFTMAX_BF16
+             ? launch_prec<MODE, POOL, ETPGT_SOFTMAX_BF16>(r_hi, r_lo, c_hi, c_lo, p, grid, name, stream)
+             : launch_prec<MODE, POOL, ETPGT_SOFTMAX_BF16X3>(r_hi, r_lo, c_hi, c_lo, p, grid, name, stream);
 }
 
 // One gradient pass (DS or DE) over rows x cols into out [rows, D].  Split into column ranges, its partials are
@@ -633,14 +761,14 @@ int launch(const CUtensorMap& r_hi, const CUtensorMap& r_lo, const CUtensorMap& 
 template <int MODE, bool POOL = false>
 int grad_pass(const CUtensorMap& r_hi, const CUtensorMap& r_lo, const CUtensorMap& c_hi, const CUtensorMap& c_lo,
               Params p, int64_t rows, int64_t cols, float* out, int accumulate, int64_t skip_row, const char* name,
-              const char* combine_name, cudaStream_t stream) {
+              const char* combine_name, int precision, cudaStream_t stream) {
   const Plan pl = plan_grad(rows, cols);
   p.rows = rows;
   p.cols = cols;
   p.tiles_per_range = pl.tiles_per_range;
   p.ranges = pl.ranges;
   p.out = out;
-  const int rc = launch<MODE, POOL>(r_hi, r_lo, c_hi, c_lo, p, pl.grid, name, stream);
+  const int rc = launch<MODE, POOL>(r_hi, r_lo, c_hi, c_lo, p, pl.grid, name, precision, stream);
   if (rc != ETPGT_OK) return rc;
   if (pl.ranges > 1) {
     grad_combine_kernel<<<grid_for(rows * p.dim / 4, 256, 8), 256, 0, stream>>>(p.part, pl.ranges, rows, p.dim,
@@ -664,11 +792,12 @@ int full_check_args(const float* sess, const float* table, const int64_t* target
                     temperature, padding_idx, items);
 }
 
-// the columns are the table, split into its bf16 pair
-int full_prepare(const float* sess, const float* table, int64_t batch, int64_t items, int dim, void* ws,
+// the columns are the table, split into its bf16 pair (bf16: rounded once)
+int full_prepare(const float* sess, const float* table, int64_t batch, int64_t items, int dim, bool bf16, void* ws,
                  size_t ws_bytes, cudaStream_t stream, Operands* o) {
-  return prepare("full_softmax", layout(batch, items, dim), sess, batch, items, dim, ws, ws_bytes, stream, o,
+  return prepare("full_softmax", layout(batch, items, dim), sess, batch, items, dim, bf16, ws, ws_bytes, stream, o,
                  [&](Workspace&, __nv_bfloat16* c_hi, __nv_bfloat16* c_lo) {
+                   if (c_lo == nullptr) return etpgt_f32_to_bf16(table, c_hi, items * dim, stream);
                    return etpgt_split_bf16(table, items, dim, dim, c_hi, c_lo, dim, nullptr, nullptr, 0, nullptr,
                                            nullptr, 0, stream);
                  });
@@ -677,7 +806,8 @@ int full_prepare(const float* sess, const float* table, int64_t batch, int64_t i
 // ---------------------------------------------------------------------------- shared-pool softmax: small kernels
 
 // pool rows gathered from the table and split into the bf16 pair (hi = bf16(x), lo = bf16(x - hi), as
-// etpgt_split_bf16), and bias[j] = log_q[j], or +inf for a padding entry (its logit is then -inf in every pass)
+// etpgt_split_bf16; hi only when lo is null), and bias[j] = log_q[j], or +inf for a padding entry (its logit is then
+// -inf in every pass)
 __global__ void __launch_bounds__(256)
 pool_gather_split_kernel(const int64_t* __restrict__ pool, const float* __restrict__ log_q,
                          const float* __restrict__ table, int64_t m, int dim, int64_t padding_idx,
@@ -694,13 +824,22 @@ pool_gather_split_kernel(const int64_t* __restrict__ pool, const float* __restri
     for (int t = 0; t < 4; ++t) {
       const __nv_bfloat16 h = __float2bfloat16_rn(xs[t]);
       hi[j * dim + k + t] = h;
-      lo[j * dim + k + t] = __float2bfloat16_rn(xs[t] - __bfloat162float(h));
+      if (lo != nullptr) lo[j * dim + k + t] = __float2bfloat16_rn(xs[t] - __bfloat162float(h));
     }
   }
 }
 
+// x, or x rounded to bf16 (round to nearest even) and back: the operands of the bf16 loss
+template <bool BF16>
+__device__ __forceinline__ float operand(float x) {
+  if constexpr (BF16) return __bfloat162float(__float2bfloat16_rn(x));
+  return x;
+}
+
 // one warp per session: its hit range [lower_bound, upper_bound) of the target in the sorted pool and, with
-// z_pos != NULL, z_pos = (s_b . e_{t_b}) / T in fp32 (lane-strided products, then a fixed butterfly)
+// z_pos != NULL, z_pos = (s_b . e_{t_b}) / T in fp32 (lane-strided products, then a fixed butterfly; BF16: of the
+// rounded operands, whose products are exact)
+template <bool BF16 = false>
 __global__ void __launch_bounds__(256)
 pool_rows_kernel(const float* __restrict__ sess, const float* __restrict__ table, const int64_t* __restrict__ targets,
                  const int64_t* __restrict__ pool, int64_t batch, int64_t m, int dim, float inv_t,
@@ -724,7 +863,8 @@ pool_rows_kernel(const float* __restrict__ sess, const float* __restrict__ table
     }
     if (z_pos == nullptr) continue;
     float acc = 0.f;
-    for (int k = lane; k < dim; k += 32) acc = fmaf(sess[b * dim + k], table[t * dim + k], acc);
+    for (int k = lane; k < dim; k += 32)
+      acc = fmaf(operand<BF16>(sess[b * dim + k]), operand<BF16>(table[t * dim + k]), acc);
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
     if (lane == 0) z_pos[b] = acc * inv_t;
@@ -761,7 +901,9 @@ pool_combine_kernel(const float* __restrict__ part, int ranges, int64_t rows, co
 }
 
 // the positive's gradient: coef[b] = d_loss (exp(z_pos - lse) - 1) / (T B_total) and, with d_sess != NULL,
-// d_sess[b] += coef[b] e_{t_b}; one warp per session
+// d_sess[b] += coef[b] e_{t_b}; one warp per session.  BF16: coef[b] is the positive's entry of G, computed as the
+// loss kernel computes G and rounded to bf16 like it, and d_sess[b] += coef[b] bf16(e_{t_b}) (an exact product)
+template <bool BF16 = false>
 __global__ void __launch_bounds__(256)
 pool_positive_bwd_kernel(const float* __restrict__ table, const int64_t* __restrict__ targets,
                          const float* __restrict__ z_pos, const float* __restrict__ lse, const float* __restrict__ d_loss,
@@ -770,12 +912,20 @@ pool_positive_bwd_kernel(const float* __restrict__ table, const int64_t* __restr
   const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
   const float dl = __ldg(d_loss) * gscale;
   for (int64_t b = blockIdx.x * (int64_t)(blockDim.x >> 5) + (threadIdx.x >> 5); b < batch; b += nwarps) {
-    const float c = dl * (expf(z_pos[b] - lse[b]) - 1.f);
+    const float c = BF16 ? operand<true>((fast_exp2((z_pos[b] - lse[b]) * kLog2e) - 1.f) * dl)
+                         : dl * (expf(z_pos[b] - lse[b]) - 1.f);
     if (lane == 0) coef[b] = c;
     if (d_sess == nullptr) continue;
     const float* e = table + targets[b] * dim;
-    for (int k = lane; k < dim; k += 32) d_sess[b * dim + k] = fmaf(c, e[k], d_sess[b * dim + k]);
+    for (int k = lane; k < dim; k += 32) d_sess[b * dim + k] = fmaf(c, operand<BF16>(e[k]), d_sess[b * dim + k]);
   }
+}
+
+// dst = bf16(src) as fp32: the rounded sessions whose rows the bf16 loss's positive adds to the table
+__global__ void __launch_bounds__(256) round_bf16_kernel(const float* __restrict__ src, float* __restrict__ dst,
+                                                         int64_t n) {
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
+    dst[i] = operand<true>(src[i]);
 }
 
 // ---------------------------------------------------------------------------- shared-pool softmax: host
@@ -809,12 +959,13 @@ int pool_check_args(const float* sess, const float* table, const int64_t* target
                     temperature, padding_idx, items);
 }
 
-// the columns are the pool rows, gathered and split; also finds the hit ranges (and z_pos when given)
+// the columns are the pool rows, gathered and split (bf16: rounded once); also finds the hit ranges (and z_pos when
+// given)
 int pool_prepare(const float* sess, const float* table, const int64_t* targets, const int64_t* pool_ids,
-                 const float* log_q, int64_t batch, int64_t m, int dim, float inv_t, int64_t padding_idx,
+                 const float* log_q, int64_t batch, int64_t m, int dim, float inv_t, int64_t padding_idx, bool bf16,
                  float* z_pos, void* ws, size_t ws_bytes, cudaStream_t stream, Operands* o) {
   const Layout l = pool_layout(batch, m, dim);
-  return prepare("pool_softmax", l, sess, batch, m, dim, ws, ws_bytes, stream, o,
+  return prepare("pool_softmax", l, sess, batch, m, dim, bf16, ws, ws_bytes, stream, o,
                  [&](Workspace& w, __nv_bfloat16* c_hi, __nv_bfloat16* c_lo) {
                    o->d_pool = w.take<float>(l.d_pool / sizeof(float));
                    o->bias = w.take<float>(l.bias / sizeof(float));
@@ -825,8 +976,12 @@ int pool_prepare(const float* sess, const float* table, const int64_t* targets, 
                    pool_gather_split_kernel<<<grid_for(m * dim / 4, 256, 8), 256, 0, stream>>>(
                        pool_ids, log_q, table, m, dim, padding_idx, c_hi, c_lo, o->bias);
                    ETPGT_CHECK_LAUNCH("pool_softmax_gather");
-                   pool_rows_kernel<<<grid_for(batch, 8, 8), 256, 0, stream>>>(sess, table, targets, pool_ids, batch,
-                                                                               m, dim, inv_t, o->hits, z_pos);
+                   if (bf16)
+                     pool_rows_kernel<true><<<grid_for(batch, 8, 8), 256, 0, stream>>>(
+                         sess, table, targets, pool_ids, batch, m, dim, inv_t, o->hits, z_pos);
+                   else
+                     pool_rows_kernel<<<grid_for(batch, 8, 8), 256, 0, stream>>>(sess, table, targets, pool_ids, batch,
+                                                                                 m, dim, inv_t, o->hits, z_pos);
                    ETPGT_CHECK_LAUNCH("pool_softmax_rows");
                    return ETPGT_OK;
                  });
@@ -842,16 +997,18 @@ extern "C" size_t etpgt_full_softmax_workspace_bytes(int64_t batch, int64_t num_
   return layout(batch, num_items, dim).total();
 }
 
-extern "C" int etpgt_full_softmax_fwd(const float* sess, const float* table, const int64_t* targets, int64_t batch,
-                                      int64_t num_items, int dim, float temperature, double total_sessions,
-                                      int64_t padding_idx, float* lse, float* loss, void* ws, size_t ws_bytes,
-                                      etpgt_stream_t stream_) {
+extern "C" int etpgt_full_softmax_fwd_ex(const float* sess, const float* table, const int64_t* targets, int64_t batch,
+                                         int64_t num_items, int dim, float temperature, double total_sessions,
+                                         int64_t padding_idx, float* lse, float* loss, void* ws, size_t ws_bytes,
+                                         etpgt_stream_t stream_, int precision) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  int rc = full_check_args(sess, table, targets, batch, num_items, dim, temperature, padding_idx);
+  int rc = check_precision("full_softmax_fwd", precision);
+  if (rc != ETPGT_OK) return rc;
+  rc = full_check_args(sess, table, targets, batch, num_items, dim, temperature, padding_idx);
   if (rc != ETPGT_OK) return rc;
   ETPGT_REQUIRE(lse != nullptr && loss != nullptr, "full_softmax_fwd: lse and loss are required");
   Operands o;
-  rc = full_prepare(sess, table, batch, num_items, dim, ws, ws_bytes, stream, &o);
+  rc = full_prepare(sess, table, batch, num_items, dim, precision == ETPGT_SOFTMAX_BF16, ws, ws_bytes, stream, &o);
   if (rc != ETPGT_OK) return rc;
   const double total = mean_over(total_sessions, batch);
   const Plan pl = plan_fwd(batch, num_items);
@@ -860,7 +1017,7 @@ extern "C" int etpgt_full_softmax_fwd(const float* sess, const float* table, con
   p.cols = num_items;
   p.tiles_per_range = pl.tiles_per_range;
   p.ranges = pl.ranges;
-  rc = launch<FWD>(o.s_hi, o.s_lo, o.c_hi, o.c_lo, p, pl.grid, "full_softmax_fwd", stream);
+  rc = launch<FWD>(o.s_hi, o.s_lo, o.c_hi, o.c_lo, p, pl.grid, "full_softmax_fwd", precision, stream);
   if (rc != ETPGT_OK) return rc;
   fwd_combine_kernel<<<1, kCombineThreads, 0, stream>>>(o.part, pl.ranges, pl.tiles_per_range, batch, num_items,
                                                         targets, total, lse, loss);
@@ -868,31 +1025,51 @@ extern "C" int etpgt_full_softmax_fwd(const float* sess, const float* table, con
   return ETPGT_OK;
 }
 
-extern "C" int etpgt_full_softmax_bwd(const float* sess, const float* table, const int64_t* targets, const float* lse,
-                                      const float* d_loss, int64_t batch, int64_t num_items, int dim, float temperature,
-                                      double total_sessions, int64_t padding_idx, float* d_sess,
-                                      float* d_table_accumulate, void* ws, size_t ws_bytes, etpgt_stream_t stream_) {
+extern "C" int etpgt_full_softmax_fwd(const float* sess, const float* table, const int64_t* targets, int64_t batch,
+                                      int64_t num_items, int dim, float temperature, double total_sessions,
+                                      int64_t padding_idx, float* lse, float* loss, void* ws, size_t ws_bytes,
+                                      etpgt_stream_t stream) {
+  return etpgt_full_softmax_fwd_ex(sess, table, targets, batch, num_items, dim, temperature, total_sessions,
+                                   padding_idx, lse, loss, ws, ws_bytes, stream, ETPGT_SOFTMAX_BF16X3);
+}
+
+extern "C" int etpgt_full_softmax_bwd_ex(const float* sess, const float* table, const int64_t* targets,
+                                         const float* lse, const float* d_loss, int64_t batch, int64_t num_items,
+                                         int dim, float temperature, double total_sessions, int64_t padding_idx,
+                                         float* d_sess, float* d_table_accumulate, void* ws, size_t ws_bytes,
+                                         etpgt_stream_t stream_, int precision) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  int rc = full_check_args(sess, table, targets, batch, num_items, dim, temperature, padding_idx);
+  int rc = check_precision("full_softmax_bwd", precision);
+  if (rc != ETPGT_OK) return rc;
+  rc = full_check_args(sess, table, targets, batch, num_items, dim, temperature, padding_idx);
   if (rc != ETPGT_OK) return rc;
   ETPGT_REQUIRE(lse != nullptr && d_loss != nullptr, "full_softmax_bwd: lse and d_loss are required");
   if (d_sess == nullptr && d_table_accumulate == nullptr) return ETPGT_OK;
   Operands o;
-  rc = full_prepare(sess, table, batch, num_items, dim, ws, ws_bytes, stream, &o);
+  rc = full_prepare(sess, table, batch, num_items, dim, precision == ETPGT_SOFTMAX_BF16, ws, ws_bytes, stream, &o);
   if (rc != ETPGT_OK) return rc;
   const Params p =
       call_params(dim, temperature, mean_over(total_sessions, batch), padding_idx, o, targets, lse, d_loss);
   if (d_sess != nullptr) {
     rc = grad_pass<DS>(o.s_hi, o.s_lo, o.c_hi, o.c_lo, p, batch, num_items, d_sess, 0, -1, "full_softmax_bwd_sess",
-                       "full_softmax_bwd_sess_combine", stream);
+                       "full_softmax_bwd_sess_combine", precision, stream);
     if (rc != ETPGT_OK) return rc;
   }
   if (d_table_accumulate != nullptr) {
     rc = grad_pass<DE>(o.c_hi, o.c_lo, o.s_hi, o.s_lo, p, num_items, batch, d_table_accumulate, 1, padding_idx,
-                       "full_softmax_bwd_table", "full_softmax_bwd_table_combine", stream);
+                       "full_softmax_bwd_table", "full_softmax_bwd_table_combine", precision, stream);
     if (rc != ETPGT_OK) return rc;
   }
   return ETPGT_OK;
+}
+
+extern "C" int etpgt_full_softmax_bwd(const float* sess, const float* table, const int64_t* targets, const float* lse,
+                                      const float* d_loss, int64_t batch, int64_t num_items, int dim, float temperature,
+                                      double total_sessions, int64_t padding_idx, float* d_sess,
+                                      float* d_table_accumulate, void* ws, size_t ws_bytes, etpgt_stream_t stream) {
+  return etpgt_full_softmax_bwd_ex(sess, table, targets, lse, d_loss, batch, num_items, dim, temperature,
+                                   total_sessions, padding_idx, d_sess, d_table_accumulate, ws, ws_bytes, stream,
+                                   ETPGT_SOFTMAX_BF16X3);
 }
 
 extern "C" size_t etpgt_pool_softmax_workspace_bytes(int64_t batch, int64_t num_sampled, int dim) {
@@ -900,20 +1077,23 @@ extern "C" size_t etpgt_pool_softmax_workspace_bytes(int64_t batch, int64_t num_
   return pool_layout(batch, num_sampled, dim).total();
 }
 
-extern "C" int etpgt_pool_softmax_fwd(const float* sess, const float* table, const int64_t* targets,
-                                      const int64_t* pool_ids, const float* log_q, int64_t batch, int64_t num_items,
-                                      int64_t num_sampled, int dim, float temperature, double total_sessions,
-                                      int64_t padding_idx, float* lse, float* z_pos, float* loss, void* ws,
-                                      size_t ws_bytes, etpgt_stream_t stream_) {
+extern "C" int etpgt_pool_softmax_fwd_ex(const float* sess, const float* table, const int64_t* targets,
+                                         const int64_t* pool_ids, const float* log_q, int64_t batch,
+                                         int64_t num_items, int64_t num_sampled, int dim, float temperature,
+                                         double total_sessions, int64_t padding_idx, float* lse, float* z_pos,
+                                         float* loss, void* ws, size_t ws_bytes, etpgt_stream_t stream_,
+                                         int precision) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  int rc = pool_check_args(sess, table, targets, pool_ids, log_q, batch, num_items, num_sampled, dim, temperature,
-                           padding_idx);
+  int rc = check_precision("pool_softmax_fwd", precision);
+  if (rc != ETPGT_OK) return rc;
+  rc = pool_check_args(sess, table, targets, pool_ids, log_q, batch, num_items, num_sampled, dim, temperature,
+                       padding_idx);
   if (rc != ETPGT_OK) return rc;
   ETPGT_REQUIRE(lse != nullptr && z_pos != nullptr && loss != nullptr,
                 "pool_softmax_fwd: lse, z_pos and loss are required");
   Operands o;
   rc = pool_prepare(sess, table, targets, pool_ids, log_q, batch, num_sampled, dim, 1.f / temperature, padding_idx,
-                    z_pos, ws, ws_bytes, stream, &o);
+                    precision == ETPGT_SOFTMAX_BF16, z_pos, ws, ws_bytes, stream, &o);
   if (rc != ETPGT_OK) return rc;
   const double total = mean_over(total_sessions, batch);
   const Plan pl = plan_fwd(batch, num_sampled);
@@ -922,10 +1102,77 @@ extern "C" int etpgt_pool_softmax_fwd(const float* sess, const float* table, con
   p.cols = num_sampled;
   p.tiles_per_range = pl.tiles_per_range;
   p.ranges = pl.ranges;
-  rc = launch<FWD, true>(o.s_hi, o.s_lo, o.c_hi, o.c_lo, p, pl.grid, "pool_softmax_fwd", stream);
+  rc = launch<FWD, true>(o.s_hi, o.s_lo, o.c_hi, o.c_lo, p, pl.grid, "pool_softmax_fwd", precision, stream);
   if (rc != ETPGT_OK) return rc;
   pool_combine_kernel<<<1, kCombineThreads, 0, stream>>>(o.part, pl.ranges, batch, z_pos, total, lse, loss);
   ETPGT_CHECK_LAUNCH("pool_softmax_fwd_combine");
+  return ETPGT_OK;
+}
+
+extern "C" int etpgt_pool_softmax_fwd(const float* sess, const float* table, const int64_t* targets,
+                                      const int64_t* pool_ids, const float* log_q, int64_t batch, int64_t num_items,
+                                      int64_t num_sampled, int dim, float temperature, double total_sessions,
+                                      int64_t padding_idx, float* lse, float* z_pos, float* loss, void* ws,
+                                      size_t ws_bytes, etpgt_stream_t stream) {
+  return etpgt_pool_softmax_fwd_ex(sess, table, targets, pool_ids, log_q, batch, num_items, num_sampled, dim,
+                                   temperature, total_sessions, padding_idx, lse, z_pos, loss, ws, ws_bytes, stream,
+                                   ETPGT_SOFTMAX_BF16X3);
+}
+
+extern "C" int etpgt_pool_softmax_bwd_ex(const float* sess, const float* table, const int64_t* targets,
+                                         const int64_t* pool_ids, const float* log_q, const float* lse,
+                                         const float* z_pos, const float* d_loss, int64_t batch, int64_t num_items,
+                                         int64_t num_sampled, int dim, float temperature, double total_sessions,
+                                         int64_t padding_idx, float* d_sess, float* d_table_accumulate, void* ws,
+                                         size_t ws_bytes, etpgt_stream_t stream_, int precision) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  int rc = check_precision("pool_softmax_bwd", precision);
+  if (rc != ETPGT_OK) return rc;
+  rc = pool_check_args(sess, table, targets, pool_ids, log_q, batch, num_items, num_sampled, dim, temperature,
+                       padding_idx);
+  if (rc != ETPGT_OK) return rc;
+  ETPGT_REQUIRE(lse != nullptr && z_pos != nullptr && d_loss != nullptr,
+                "pool_softmax_bwd: lse, z_pos and d_loss are required");
+  if (d_sess == nullptr && d_table_accumulate == nullptr) return ETPGT_OK;
+  const bool bf16 = precision == ETPGT_SOFTMAX_BF16;
+  Operands o;
+  rc = pool_prepare(sess, table, targets, pool_ids, log_q, batch, num_sampled, dim, 1.f / temperature, padding_idx,
+                    bf16, nullptr, ws, ws_bytes, stream, &o);
+  if (rc != ETPGT_OK) return rc;
+  const Params p = call_params(dim, temperature, mean_over(total_sessions, batch), -1, o, nullptr, lse, d_loss);
+  if (d_sess != nullptr) {
+    rc = grad_pass<DS, true>(o.s_hi, o.s_lo, o.c_hi, o.c_lo, p, batch, num_sampled, d_sess, 0, -1,
+                             "pool_softmax_bwd_sess", "pool_softmax_bwd_sess_combine", precision, stream);
+    if (rc != ETPGT_OK) return rc;
+  }
+  if (bf16)
+    pool_positive_bwd_kernel<true><<<grid_for(batch, 8, 8), 256, 0, stream>>>(table, targets, z_pos, lse, d_loss,
+                                                                              batch, dim, p.gscale, o.coef, d_sess);
+  else
+    pool_positive_bwd_kernel<<<grid_for(batch, 8, 8), 256, 0, stream>>>(table, targets, z_pos, lse, d_loss, batch,
+                                                                        dim, p.gscale, o.coef, d_sess);
+  ETPGT_CHECK_LAUNCH("pool_softmax_bwd_positive");
+  if (d_table_accumulate != nullptr) {
+    rc = grad_pass<DE, true>(o.c_hi, o.c_lo, o.s_hi, o.s_lo, p, num_sampled, batch, o.d_pool, 0, -1,
+                             "pool_softmax_bwd_pool", "pool_softmax_bwd_pool_combine", precision, stream);
+    if (rc != ETPGT_OK) return rc;
+    // d_table[p_j] += d_pool[j], then d_table[t_b] += coef[b] s_b: each in ascending position, padding skipped
+    rc = etpgt_scatter_rows(pool_ids, nullptr, o.d_pool, num_sampled, 1, dim, num_items, padding_idx,
+                            d_table_accumulate, o.scatter_ws, o.scatter_bytes, stream);
+    if (rc != ETPGT_OK) return rc;
+    const float* s_rows = sess;
+    if (bf16) {
+      // bf16(s_b) as fp32 rows, in the session pair's slots (2 * s_pair >= batch * dim * 4 bytes): the passes that
+      // read the bf16 sessions from there are done
+      float* rounded = static_cast<float*>(o.s_slots);
+      round_bf16_kernel<<<grid_for(batch * dim, 256, 8), 256, 0, stream>>>(sess, rounded, batch * dim);
+      ETPGT_CHECK_LAUNCH("pool_softmax_bwd_round");
+      s_rows = rounded;
+    }
+    rc = etpgt_scatter_rows(targets, o.coef, s_rows, batch, 1, dim, num_items, padding_idx, d_table_accumulate,
+                            o.scatter_ws, o.scatter_bytes, stream);
+    if (rc != ETPGT_OK) return rc;
+  }
   return ETPGT_OK;
 }
 
@@ -934,38 +1181,8 @@ extern "C" int etpgt_pool_softmax_bwd(const float* sess, const float* table, con
                                       const float* z_pos, const float* d_loss, int64_t batch, int64_t num_items,
                                       int64_t num_sampled, int dim, float temperature, double total_sessions,
                                       int64_t padding_idx, float* d_sess, float* d_table_accumulate, void* ws,
-                                      size_t ws_bytes, etpgt_stream_t stream_) {
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  int rc = pool_check_args(sess, table, targets, pool_ids, log_q, batch, num_items, num_sampled, dim, temperature,
-                           padding_idx);
-  if (rc != ETPGT_OK) return rc;
-  ETPGT_REQUIRE(lse != nullptr && z_pos != nullptr && d_loss != nullptr,
-                "pool_softmax_bwd: lse, z_pos and d_loss are required");
-  if (d_sess == nullptr && d_table_accumulate == nullptr) return ETPGT_OK;
-  Operands o;
-  rc = pool_prepare(sess, table, targets, pool_ids, log_q, batch, num_sampled, dim, 1.f / temperature, padding_idx,
-                    nullptr, ws, ws_bytes, stream, &o);
-  if (rc != ETPGT_OK) return rc;
-  const Params p = call_params(dim, temperature, mean_over(total_sessions, batch), -1, o, nullptr, lse, d_loss);
-  if (d_sess != nullptr) {
-    rc = grad_pass<DS, true>(o.s_hi, o.s_lo, o.c_hi, o.c_lo, p, batch, num_sampled, d_sess, 0, -1,
-                             "pool_softmax_bwd_sess", "pool_softmax_bwd_sess_combine", stream);
-    if (rc != ETPGT_OK) return rc;
-  }
-  pool_positive_bwd_kernel<<<grid_for(batch, 8, 8), 256, 0, stream>>>(table, targets, z_pos, lse, d_loss, batch, dim,
-                                                                      p.gscale, o.coef, d_sess);
-  ETPGT_CHECK_LAUNCH("pool_softmax_bwd_positive");
-  if (d_table_accumulate != nullptr) {
-    rc = grad_pass<DE, true>(o.c_hi, o.c_lo, o.s_hi, o.s_lo, p, num_sampled, batch, o.d_pool, 0, -1,
-                             "pool_softmax_bwd_pool", "pool_softmax_bwd_pool_combine", stream);
-    if (rc != ETPGT_OK) return rc;
-    // d_table[p_j] += d_pool[j], then d_table[t_b] += coef[b] s_b: each in ascending position, padding skipped
-    rc = etpgt_scatter_rows(pool_ids, nullptr, o.d_pool, num_sampled, 1, dim, num_items, padding_idx,
-                            d_table_accumulate, o.scatter_ws, o.scatter_bytes, stream);
-    if (rc != ETPGT_OK) return rc;
-    rc = etpgt_scatter_rows(targets, o.coef, sess, batch, 1, dim, num_items, padding_idx, d_table_accumulate,
-                            o.scatter_ws, o.scatter_bytes, stream);
-    if (rc != ETPGT_OK) return rc;
-  }
-  return ETPGT_OK;
+                                      size_t ws_bytes, etpgt_stream_t stream) {
+  return etpgt_pool_softmax_bwd_ex(sess, table, targets, pool_ids, log_q, lse, z_pos, d_loss, batch, num_items,
+                                   num_sampled, dim, temperature, total_sessions, padding_idx, d_sess,
+                                   d_table_accumulate, ws, ws_bytes, stream, ETPGT_SOFTMAX_BF16X3);
 }

@@ -98,6 +98,10 @@ _PROTOTYPES = {
     "etpgt_pool_softmax_workspace_bytes": (Z, [L, L, I]),
     "etpgt_pool_softmax_fwd": (I, [P, P, P, P, P, L, L, L, I, F, D, L, P, P, P, P, Z, P]),
     "etpgt_pool_softmax_bwd": (I, [P, P, P, P, P, P, P, P, L, L, L, I, F, D, L, P, P, P, Z, P]),
+    "etpgt_full_softmax_fwd_ex": (I, [P, P, P, L, L, I, F, D, L, P, P, P, Z, P, I]),
+    "etpgt_full_softmax_bwd_ex": (I, [P, P, P, P, P, L, L, I, F, D, L, P, P, P, Z, P, I]),
+    "etpgt_pool_softmax_fwd_ex": (I, [P, P, P, P, P, L, L, L, I, F, D, L, P, P, P, P, Z, P, I]),
+    "etpgt_pool_softmax_bwd_ex": (I, [P, P, P, P, P, P, P, P, L, L, L, I, F, D, L, P, P, P, Z, P, I]),
     "etpgt_score_topk_workspace_bytes": (Z, [L, L, I, I]),
     "etpgt_score_topk_f32": (I, [P, P, L, L, I, I, L, P, P, P, Z, P]),
     "etpgt_f32_to_bf16": (I, [P, P, L, P]),

@@ -1398,13 +1398,26 @@ def _softmax_inputs(name, sess, table, targets, *more_cuda):
     return sess_c, table_c, targets
 
 
+SOFTMAX_PRECISIONS = {"bf16x3": 0, "bf16": 1}     # ETPGT_SOFTMAX_BF16X3, ETPGT_SOFTMAX_BF16
+
+
+def _softmax_precision(precision) -> int:
+    """The ABI value of a softmax loss precision: "bf16x3" (split-bf16 products, ~1e-5 relative to fp64, the default)
+    or "bf16" (S, E and G rounded once to bf16, one bf16 MMA per product, for training)."""
+    if not isinstance(precision, str) or precision not in SOFTMAX_PRECISIONS:
+        raise ValueError(f"softmax loss precision must be \"bf16x3\" or \"bf16\"; got {precision!r}")
+    return SOFTMAX_PRECISIONS[precision]
+
+
 class FullSoftmaxLoss(torch.autograd.Function):
-    """Cross-entropy over every item of the table (the padding row left out), etpgt_full_softmax_fwd / _bwd:
-    tcgen05 split-bf16 GEMMs with the softmax in the epilogue, so the [B, I] logits never exist.  Returns the
-    scalar mean over `total_sessions` (default: the batch)."""
+    """Cross-entropy over every item of the table (the padding row left out), etpgt_full_softmax_fwd_ex / _bwd_ex:
+    tcgen05 GEMMs with the softmax in the epilogue, so the [B, I] logits never exist.  `precision` "bf16x3" (default)
+    makes every product split-bf16, "bf16" rounds S, E and G once to bf16.  Returns the scalar mean over
+    `total_sessions` (default: the batch)."""
 
     @staticmethod
-    def forward(ctx, sess, table, targets, temperature, total_sessions, padding_idx):
+    def forward(ctx, sess, table, targets, temperature, total_sessions, padding_idx, precision="bf16x3"):
+        prec = _softmax_precision(precision)
         sess_c, table_c, targets = _softmax_inputs("full_softmax_loss", sess, table, targets)
         b, dim = sess_c.shape
         dev = sess_c.device
@@ -1413,35 +1426,40 @@ class FullSoftmaxLoss(torch.autograd.Function):
         lse = torch.empty(b, dtype=torch.float32, device=dev)
         loss = torch.empty(1, dtype=torch.float32, device=dev)
         ws = workspace(size("etpgt_full_softmax_workspace_bytes", b, table_c.size(0), dim), dev)
-        call("etpgt_full_softmax_fwd", ptr(sess_c), ptr(table_c), ptr(targets), b, table_c.size(0), dim,
-             float(temperature), total, pad, ptr(lse), ptr(loss), ptr(ws), ws.numel(), stream())
+        call("etpgt_full_softmax_fwd_ex", ptr(sess_c), ptr(table_c), ptr(targets), b, table_c.size(0), dim,
+             float(temperature), total, pad, ptr(lse), ptr(loss), ptr(ws), ws.numel(), stream(), prec)
         ctx.save_for_backward(sess_c, table_c, targets, lse)
         ctx.table_ref = table
-        ctx.meta = (float(temperature), total, pad)
+        ctx.meta = (float(temperature), total, pad, prec)
         ctx.mark_non_differentiable(lse)
         return loss[0], lse
 
     @staticmethod
     def backward(ctx, d_loss, _d_lse):
         sess, table, targets, lse = ctx.saved_tensors
-        temperature, total, pad = ctx.meta
+        temperature, total, pad, prec = ctx.meta
         b, dim = sess.shape
         dev = sess.device
         d_loss = _f32(d_loss).reshape(1).contiguous()
         d_sess = torch.empty_like(sess) if ctx.needs_input_grad[0] else None
         d_table, table_grad = _table_grad(ctx, table.shape, dev)
         ws = workspace(size("etpgt_full_softmax_workspace_bytes", b, table.size(0), dim), dev)
-        call("etpgt_full_softmax_bwd", ptr(sess), ptr(table), ptr(targets), ptr(lse), ptr(d_loss), b, table.size(0),
-             dim, temperature, total, pad, ptr(d_sess), ptr(d_table), ptr(ws), ws.numel(), stream())
-        return d_sess, table_grad, None, None, None, None
+        call("etpgt_full_softmax_bwd_ex", ptr(sess), ptr(table), ptr(targets), ptr(lse), ptr(d_loss), b,
+             table.size(0), dim, temperature, total, pad, ptr(d_sess), ptr(d_table), ptr(ws), ws.numel(), stream(),
+             prec)
+        return d_sess, table_grad, None, None, None, None, None
 
 
-def full_softmax_loss(sess, item_embeddings, targets, temperature=1.0, total_sessions=None) -> torch.Tensor:
+def full_softmax_loss(sess, item_embeddings, targets, temperature=1.0, total_sessions=None,
+                      precision="bf16x3") -> torch.Tensor:
     """Softmax cross-entropy of `targets` over the whole catalogue.  `item_embeddings` is the nn.Embedding (its
     padding_idx column is left out of the softmax and its row gets no gradient) or a bare weight tensor.  The table
-    gradient goes into the etpgt_b200.optim gradient sink when one is registered, else it is returned densely."""
+    gradient goes into the etpgt_b200.optim gradient sink when one is registered, else it is returned densely.
+    precision "bf16x3" (default): split-bf16 products, ~1e-5 relative to fp64.  "bf16": the sessions, the table and
+    the softmax gradient are rounded once to bf16 and every product is one bf16 MMA (fp32 accumulation); lse and the
+    softmax stay fp32.  A different numerical contract for training, not the same result faster."""
     weight, padding_idx = _weight_and_padding(item_embeddings)
-    return FullSoftmaxLoss.apply(sess, weight, targets, temperature, total_sessions, padding_idx)[0]
+    return FullSoftmaxLoss.apply(sess, weight, targets, temperature, total_sessions, padding_idx, precision)[0]
 
 
 # ------------------------------------------------------------------------------ shared-pool sampled softmax
@@ -1507,10 +1525,13 @@ class PoolSoftmaxLoss(torch.autograd.Function):
         z_pos[b] = s_b . e_{t_b} / T,   z[b, j] = s_b . e_{p_j} / T - log_q[j]  (-inf where p_j is t_b or padding)
         loss = sum_b (logsumexp(z_pos[b], z[b, :]) - z_pos[b]) / total_sessions
     `validate` checks the pool ids against the table and sorts an unsorted pool (one device-to-host copy); pools from
-    `sample_item_pool` are sorted and in range already.  Returns (loss, lse)."""
+    `sample_item_pool` are sorted and in range already.  `precision` as FullSoftmaxLoss ("bf16": the positive is the
+    fp32 dot of the rounded operands).  Returns (loss, lse)."""
 
     @staticmethod
-    def forward(ctx, sess, table, targets, pool_ids, log_q, temperature, total_sessions, padding_idx, validate):
+    def forward(ctx, sess, table, targets, pool_ids, log_q, temperature, total_sessions, padding_idx, validate,
+                precision="bf16x3"):
+        prec = _softmax_precision(precision)
         sess_c, table_c, targets = _softmax_inputs("pool_softmax_loss", sess, table, targets, (pool_ids, "pool_ids"),
                                                    (log_q, "log_q"))
         pool, lq = _i64(pool_ids), _f32(log_q)
@@ -1535,18 +1556,18 @@ class PoolSoftmaxLoss(torch.autograd.Function):
         z_pos = torch.empty(b, dtype=torch.float32, device=dev)
         loss = torch.empty(1, dtype=torch.float32, device=dev)
         ws = workspace(size("etpgt_pool_softmax_workspace_bytes", b, m, dim), dev)
-        call("etpgt_pool_softmax_fwd", ptr(sess_c), ptr(table_c), ptr(targets), ptr(pool), ptr(lq), b, items, m, dim,
-             float(temperature), total, pad, ptr(lse), ptr(z_pos), ptr(loss), ptr(ws), ws.numel(), stream())
+        call("etpgt_pool_softmax_fwd_ex", ptr(sess_c), ptr(table_c), ptr(targets), ptr(pool), ptr(lq), b, items, m,
+             dim, float(temperature), total, pad, ptr(lse), ptr(z_pos), ptr(loss), ptr(ws), ws.numel(), stream(), prec)
         ctx.save_for_backward(sess_c, table_c, targets, pool, lq, lse, z_pos)
         ctx.table_ref = table
-        ctx.meta = (float(temperature), total, pad)
+        ctx.meta = (float(temperature), total, pad, prec)
         ctx.mark_non_differentiable(lse)
         return loss[0], lse
 
     @staticmethod
     def backward(ctx, d_loss, _d_lse):
         sess, table, targets, pool, lq, lse, z_pos = ctx.saved_tensors
-        temperature, total, pad = ctx.meta
+        temperature, total, pad, prec = ctx.meta
         b, dim = sess.shape
         m = pool.numel()
         dev = sess.device
@@ -1554,23 +1575,24 @@ class PoolSoftmaxLoss(torch.autograd.Function):
         d_sess = torch.empty_like(sess) if ctx.needs_input_grad[0] else None
         d_table, table_grad = _table_grad(ctx, table.shape, dev)
         ws = workspace(size("etpgt_pool_softmax_workspace_bytes", b, m, dim), dev)
-        call("etpgt_pool_softmax_bwd", ptr(sess), ptr(table), ptr(targets), ptr(pool), ptr(lq), ptr(lse), ptr(z_pos),
-             ptr(d_loss), b, table.size(0), m, dim, temperature, total, pad, ptr(d_sess), ptr(d_table), ptr(ws),
-             ws.numel(), stream())
-        return d_sess, table_grad, None, None, None, None, None, None, None
+        call("etpgt_pool_softmax_bwd_ex", ptr(sess), ptr(table), ptr(targets), ptr(pool), ptr(lq), ptr(lse),
+             ptr(z_pos), ptr(d_loss), b, table.size(0), m, dim, temperature, total, pad, ptr(d_sess), ptr(d_table),
+             ptr(ws), ws.numel(), stream(), prec)
+        return d_sess, table_grad, None, None, None, None, None, None, None, None
 
 
 def pool_softmax_loss(sess, item_embeddings, targets, pool_ids, log_q, temperature=1.0,
-                      total_sessions=None) -> torch.Tensor:
+                      total_sessions=None, precision="bf16x3") -> torch.Tensor:
     """Sampled softmax cross-entropy of `targets` against the shared negative pool `pool_ids` [M] with its log-Q
     correction `log_q` [M] = log(M q(pool_ids)) (see PoolSoftmaxLoss; `sample_item_pool` draws both).  The pool is
     sorted (with its log_q) when it is not sorted already; ids outside the table raise.  `item_embeddings` is the
     nn.Embedding (its padding_idx never counts as a negative and its row gets no gradient) or a bare weight tensor.
     The table gradient goes into the etpgt_b200.optim gradient sink when one is registered, else it is returned
-    densely (non-zero on the pool and target rows only)."""
+    densely (non-zero on the pool and target rows only).  `precision` "bf16x3" (default) or "bf16", as in
+    full_softmax_loss."""
     weight, padding_idx = _weight_and_padding(item_embeddings)
     return PoolSoftmaxLoss.apply(sess, weight, targets, pool_ids, log_q, temperature, total_sessions, padding_idx,
-                                 True)[0]
+                                 True, precision)[0]
 
 
 # ------------------------------------------------------------------------------ scoring / top-k

@@ -485,6 +485,40 @@ int etpgt_pool_softmax_bwd(const float* sess, const float* table, const int64_t*
                            int64_t batch, int64_t num_items, int64_t num_sampled, int dim, float temperature,
                            double total_sessions, int64_t padding_idx, float* d_sess, float* d_table_accumulate,
                            void* ws, size_t ws_bytes, etpgt_stream_t stream);
+/* Precision of both softmax losses.  The four calls above are the _ex calls with ETPGT_SOFTMAX_BF16X3.
+ * ETPGT_SOFTMAX_BF16X3: every product is split-bf16 (x = hi + lo, hi.hi + hi.lo + lo.hi, fp32 accumulation), ~1e-5
+ *   relative to the fp64 objective.
+ * ETPGT_SOFTMAX_BF16: a different numerical contract, for training.  S (sess), E (the table rows, or the gathered pool
+ *   rows) and G = (P - onehot) / (T B_total) are each rounded once to bf16 (round to nearest even) and every product
+ *   is one bf16 MMA with fp32 accumulation.  Everything else is as above: lse, the online max and sum and the target
+ *   logit in fp32; the pool's log_q, padding entries and hits; the pool's positive is the fp32 gather-dot of the
+ *   rounded operands, z_pos = bf16(s_b) . bf16(e_t) / T, with gradient terms c_b bf16(e_t) into d_sess and
+ *   c_b bf16(s_b) into the table, where c_b = (exp(z_pos - lse) - 1) d_loss / (T B_total) is the positive's entry of G
+ *   and rounded to bf16 like the rest of G (products of two bf16 values are exact in fp32), so a pool of every
+ *   non-padding item with log_q = 0 is still the bf16 full loss.  Deterministic, no atomics.  lse and the loss are
+ *   within ~1e-4 of the fp64 objective of the rounded S and E.
+ * The _ex calls take the workspace of etpgt_full_softmax_workspace_bytes / etpgt_pool_softmax_workspace_bytes in both
+ * precisions: a bf16 call needs no more (it uses less).  Any other precision returns ETPGT_EINVAL. */
+#define ETPGT_SOFTMAX_BF16X3 0
+#define ETPGT_SOFTMAX_BF16 1
+int etpgt_full_softmax_fwd_ex(const float* sess, const float* table, const int64_t* targets, int64_t batch,
+                              int64_t num_items, int dim, float temperature, double total_sessions,
+                              int64_t padding_idx, float* lse, float* loss, void* ws, size_t ws_bytes,
+                              etpgt_stream_t stream, int precision);
+int etpgt_full_softmax_bwd_ex(const float* sess, const float* table, const int64_t* targets, const float* lse,
+                              const float* d_loss, int64_t batch, int64_t num_items, int dim, float temperature,
+                              double total_sessions, int64_t padding_idx, float* d_sess,
+                              float* d_table_accumulate, void* ws, size_t ws_bytes, etpgt_stream_t stream,
+                              int precision);
+int etpgt_pool_softmax_fwd_ex(const float* sess, const float* table, const int64_t* targets, const int64_t* pool_ids,
+                              const float* log_q, int64_t batch, int64_t num_items, int64_t num_sampled, int dim,
+                              float temperature, double total_sessions, int64_t padding_idx, float* lse, float* z_pos,
+                              float* loss, void* ws, size_t ws_bytes, etpgt_stream_t stream, int precision);
+int etpgt_pool_softmax_bwd_ex(const float* sess, const float* table, const int64_t* targets, const int64_t* pool_ids,
+                              const float* log_q, const float* lse, const float* z_pos, const float* d_loss,
+                              int64_t batch, int64_t num_items, int64_t num_sampled, int dim, float temperature,
+                              double total_sessions, int64_t padding_idx, float* d_sess, float* d_table_accumulate,
+                              void* ws, size_t ws_bytes, etpgt_stream_t stream, int precision);
 
 /* ---- a9/a10: full-catalogue scoring with fused top-k and metrics ------------------------
  * etpgt/model/base.py:59-78, etpgt/utils/metrics.py:6-66.  Scores are never materialised.

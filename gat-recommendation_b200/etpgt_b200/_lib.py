@@ -33,6 +33,8 @@ _PROTOTYPES = {
     "etpgt_sample_negatives": (I, [ctypes.c_uint64, ctypes.c_uint32, L, P, P, P, L, I, L, I, P, P]),
     "etpgt_sample_item_pool_workspace_bytes": (Z, [L]),
     "etpgt_sample_item_pool": (I, [P, L, L, ctypes.c_uint64, ctypes.c_uint32, P, P, P, Z, P]),
+    "etpgt_in_batch_columns_workspace_bytes": (Z, [L, L]),
+    "etpgt_in_batch_columns": (I, [P, L, P, P, L, P, P, L, L, L, D, P, P, P, Z, P]),
     "etpgt_embed_pe_fwd": (I, [P, L, P, L, P, I, P, P, I, I, P, P]),
     "etpgt_embed_pe_fwd_split": (I, [P, L, P, L, P, I, P, P, I, I, P, P, P, P]),
     "etpgt_embed_pe_bwd_workspace_bytes": (Z, [L, I, I]),

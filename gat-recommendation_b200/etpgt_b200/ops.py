@@ -1595,6 +1595,50 @@ def pool_softmax_loss(sess, item_embeddings, targets, pool_ids, log_q, temperatu
                                  True, precision)[0]
 
 
+def in_batch_columns(targets, freq, last, step, decay, padding_idx, pool_ids=None, pool_log_q=None):
+    """The in-batch negatives of `targets` [B] as columns of PoolSoftmaxLoss (etpgt_in_batch_columns): (columns
+    int64 [M + B] ascending, log_q fp32 [M + B]), the optional sorted pool `pool_ids` / `pool_log_q` [M]
+    (sample_item_pool) merged in, pool entries first among equal ids, then the in-batch entries in session order.
+    Updates the streaming estimate of each item's share of the targets in place first: for each distinct target i
+    (in [0, I), not `padding_idx`) with n copies,
+        freq[i] = freq[i] (1 - decay)^(step - last[i]) + decay n / B,   last[i] = step
+    with freq fp64 [I] and last int64 [I] on the device; steps must increase from call to call.  An in-batch column
+    gets log_q = log(B freq[t_b]) after the update; the padding id and ids outside the table get +inf (never a
+    negative) and leave freq / last alone.  No host read, no synchronisation."""
+    for t, what in ((targets, "targets"), (freq, "freq"), (last, "last")):
+        _require_cuda(t, what)
+    if freq.dtype != torch.float64 or last.dtype != torch.int64 or freq.dim() != 1 or last.shape != freq.shape \
+            or not freq.is_contiguous() or not last.is_contiguous():
+        raise ValueError("in_batch_columns: freq must be a contiguous fp64 [num_items] and last a contiguous int64 of "
+                         f"the same shape; got {freq.dtype} {tuple(freq.shape)} and {last.dtype} {tuple(last.shape)}")
+    targets = _i64(targets)
+    if targets.dim() != 1 or targets.numel() == 0:
+        raise ValueError(f"in_batch_columns: targets must be a non-empty [B]; got {tuple(targets.shape)}")
+    if not 0.0 < float(decay) <= 1.0:
+        raise ValueError(f"in_batch_columns: decay must be in (0, 1]; got {decay}")
+    if int(step) < 0:
+        raise ValueError(f"in_batch_columns: step must be >= 0; got {step}")
+    if (pool_ids is None) != (pool_log_q is None):
+        raise ValueError("in_batch_columns: pool_ids and pool_log_q go together")
+    m = 0
+    if pool_ids is not None:
+        _require_cuda(pool_ids, "pool_ids")
+        _require_cuda(pool_log_q, "pool_log_q")
+        pool_ids, pool_log_q = _i64(pool_ids), _f32(pool_log_q)
+        if pool_ids.dim() != 1 or pool_log_q.shape != pool_ids.shape:
+            raise ValueError(f"in_batch_columns: pool_ids {tuple(pool_ids.shape)} and pool_log_q "
+                             f"{tuple(pool_log_q.shape)} must be the same [M]")
+        m = pool_ids.numel()
+    b = targets.numel()
+    columns = torch.empty(m + b, dtype=torch.int64, device=targets.device)
+    log_q = torch.empty(m + b, dtype=torch.float32, device=targets.device)
+    ws = workspace(size("etpgt_in_batch_columns_workspace_bytes", b, m), targets.device)
+    call("etpgt_in_batch_columns", ptr(targets), b, ptr(pool_ids) if m else None, ptr(pool_log_q) if m else None, m,
+         ptr(freq), ptr(last), freq.numel(), -1 if padding_idx is None else int(padding_idx), int(step), float(decay),
+         ptr(columns), ptr(log_q), ptr(ws), ws.numel(), stream())
+    return columns, log_q
+
+
 # ------------------------------------------------------------------------------ scoring / top-k
 
 

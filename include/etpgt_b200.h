@@ -109,6 +109,22 @@ int etpgt_sample_negatives(uint64_t seed, uint32_t step, int64_t session_base,
 size_t etpgt_sample_item_pool_workspace_bytes(int64_t num_sampled);
 int etpgt_sample_item_pool(const int64_t* cum, int64_t num_items, int64_t num_sampled, uint64_t seed, uint32_t step,
                            int64_t* pool_ids, float* log_q, void* ws, size_t ws_bytes, etpgt_stream_t stream);
+/* In-batch negatives for etpgt_pool_softmax_*: the column list of the batch's targets [batch] (one column per
+ * session) merged with the optional sorted pool pool_ids / pool_log_q [num_pool] of etpgt_sample_item_pool
+ * (num_pool = 0: no pool, both may be NULL).  columns [num_pool + batch] is written ascending; among equal ids the pool
+ * entries come first, then the in-batch entries in session order.  A pool entry keeps its log_q.  First the streaming
+ * estimate of each item's share of the targets is updated: for each distinct target i in [0, num_items), i !=
+ * padding_idx, with n copies among the batch,
+ *   freq[i] = freq[i] * (1 - decay)^(step - last[i]) + decay * n / batch,   last[i] = step
+ * (freq fp64 [num_items], last int64 [num_items]; steps increase from call to call).  The in-batch column of session
+ * b then gets log_q = (float) log(batch * freq[t_b]) in fp64, read after the update.  A target outside
+ * [0, num_items) never touches freq / last; its column, and that of a padding target, gets log_q = +inf (never a
+ * negative).  decay in (0, 1], step >= 0.  Deterministic, no allocation, no synchronisation, graph-capturable. */
+size_t etpgt_in_batch_columns_workspace_bytes(int64_t batch, int64_t num_pool);
+int etpgt_in_batch_columns(const int64_t* targets, int64_t batch, const int64_t* pool_ids, const float* pool_log_q,
+                           int64_t num_pool, double* freq, int64_t* last, int64_t num_items, int64_t padding_idx,
+                           int64_t step, double decay, int64_t* columns, float* log_q, void* ws, size_t ws_bytes,
+                           etpgt_stream_t stream);
 
 /* ---- a4: item embedding + Laplacian-PE projection -------------------------------------
  * out[n] = table[ids[n]] (+ pe[pe_row(n)] @ w_pe^T + b_pe);  pe_row(n) = n when

@@ -12,12 +12,24 @@
 //   etpgt_split_bf16      fp32 [R,C] -> hi/lo bf16 row-major and/or transposed (K-major operands
 //                         for both the forward and the weight-gradient GEMM) + column sums
 //   etpgt_gemm_bf16x3     C[M,N] = A[M,K] B[N,K]^T (+ bias[N]); persistent warp-specialised
-//                         kernel: TMA ring (A and B k-blocks, SWIZZLE_128B) -> tcgen05.mma
-//                         128x128x16 or 128x256x16 -> multi-stage TMEM -> epilogue warps -> swizzled smem
-//                         staging -> TMA tile stores (coalesced 128-byte rows, edges clipped);
+//                         kernel on CTA pairs: TMA ring (A and B k-blocks, SWIZZLE_128B) -> tcgen05.mma
+//                         256x128x16 or 256x256x16 (cta_group::2) -> multi-stage TMEM -> epilogue warps ->
+//                         swizzled smem staging -> TMA tile stores (coalesced 128-byte rows, edges clipped);
 //                         optional split-K with a fixed-order reduction (deterministic).
+//
+// Why CTA pairs: the GEMMs of a layer are bound by L2 -> shared-memory traffic (~1.6 GB in ~145 us each with one
+// CTA per 128 x 128 tile = 11 TB/s at 50 % tensor-pipe activity), and a CTA working alone pulls its own copy of the
+// B tile (in the forward projection all 148 CTAs reload the same 256 x 1024 weight matrix per k-block).  Here two CTAs
+// on the two SMs of a TPC execute ONE tcgen05.mma of M = 256: each loads its own 128 rows of A and only HALF of the B
+// tile, and the tensor cores of both SMs read both halves, so the B traffic per SM halves and a stage shrinks from 96
+// to 64 KB (three stages instead of two at BN = 256).  Measured on the three GEMMs of one layer (M = 99,132, K or
+// N = 256 / 1,024, split-bf16): forward / dX / dW 0.142 / 0.140 / 0.148 ms with one CTA per tile, 0.128 / 0.133 /
+// 0.130 ms on pairs.
+// Roles: warp 0 of BOTH CTAs is a TMA producer (its A rows, its B half; completion bytes are counted on the LEADER's
+// full barrier, which expects two producer arrivals), warp 1 of the leader issues the MMAs and commits to the
+// stage-empty / accumulator-full barriers of both CTAs (multicast commit), warps 2-5 of both CTAs drain their own 128
+// accumulator rows from their own TMEM and release the accumulator stage on the leader's barrier (8 arrivals).
 #include <math.h>
-#include <stdlib.h>
 
 #include "tc_common.cuh"
 
@@ -27,18 +39,12 @@ namespace {
 using namespace tc;
 
 constexpr int BLOCK_M = 128;
-// Output tiles are 128 x BN with BN = 128 or 256 (template parameter, chosen per call by gemm_plan).  The
-// GEMMs of a layer are bound by L2 -> shared-memory bandwidth (~1.6 GB in ~145 us each with 128 x 128
-// tiles = 11 TB/s at 50 % tensor-pipe activity); BN = 256 raises the flops per operand byte by a third and
-// pays off for the forward projection (short K) and the split-K weight gradient; the long-K dX GEMM keeps
-// BN = 128 (three 64 KB stages pipeline better than two 96 KB ones, and its tile count fills the SMs evenly).
+// Output tiles are 256 x BN per pair (128 x BN per CTA) with BN = 256 when N > 128, else 128 (template parameter,
+// chosen per call by gemm_plan): the wider tile raises the flops per operand byte by a third.
 constexpr int kTmemCols = 512;  // all of TMEM: 512 / BN accumulator stages
 constexpr int kThreads = 192;  // warp 0 TMA, warp 1 MMA, warps 2-5 epilogue
 constexpr uint32_t TILE_BYTES = BLOCK_M * BLOCK_K * 2;    // A: 16 KB per operand part per k-block
 constexpr uint32_t MN_BOX_BYTES = 64 * BLOCK_K * 2;       // one 64(k) x 64(mn) box of an MN-major operand
-template <int PARTS, int BN> struct StageCount {          // ring depth that fits 227 KB next to the store boxes
-  static constexpr int value = PARTS == 2 ? (BN == 256 ? 2 : 3) : 4;
-};
 constexpr int kEpiWarps = 4;
 constexpr uint32_t CD_BOX_BYTES = 32 * 32 * 4;  // one 32-row x 32-column fp32 store box
 constexpr uint32_t CD_BYTES = kEpiWarps * 2 * CD_BOX_BYTES;  // double-buffered per epilogue warp
@@ -97,209 +103,7 @@ __device__ __forceinline__ void act_store8(const ActEpilogue& act, float4 a, flo
 }
 
 // PARTS = 1: plain bf16 (A_hi, B_hi).  PARTS = 2: split operands, three products.
-template <int PARTS, int BLOCK_N>
-__global__ void __launch_bounds__(kThreads, 1)
-gemm_bf16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constant__ CUtensorMap map_a_lo,
-                   const __grid_constant__ CUtensorMap map_b_hi, const __grid_constant__ CUtensorMap map_b_lo,
-                   const __grid_constant__ CUtensorMap map_c /* C, or the [split_k][M][N] partials */,
-                   int64_t M, int64_t N, int64_t K, int m_tiles, int n_tiles, int split_k, int kb_per_split,
-                   const float* __restrict__ bias, int a_mn, int b_mn, int accumulate, const ActEpilogue act) {
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-  constexpr int kStages = StageCount<PARTS, BLOCK_N>::value;
-  constexpr int kAccStages = kTmemCols / BLOCK_N;
-  constexpr uint32_t B_TILE_BYTES = BLOCK_N * BLOCK_K * 2;  // B: 16 / 32 KB per operand part per k-block
-  constexpr uint32_t kInstrDesc = instr_desc_bf16(BLOCK_M, BLOCK_N);
-  constexpr uint32_t STAGE_BYTES = PARTS * (TILE_BYTES + B_TILE_BYTES);  // A parts then B parts
-  uint8_t* smem_cd = smem + kStages * STAGE_BYTES;  // 1024-byte aligned (stage sizes are multiples of 16 KB)
-  GemmBarriers* bars = reinterpret_cast<GemmBarriers*>(smem_cd + CD_BYTES);
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const int total_kb = (int)((K + BLOCK_K - 1) / BLOCK_K);
-  const int64_t total_units = (int64_t)m_tiles * n_tiles * split_k;
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < 4; ++s) { mbar_init(&bars->full[s], 1); mbar_init(&bars->empty[s], 1); }
-    for (int s = 0; s < 4; ++s) { mbar_init(&bars->acc_full[s], 1); mbar_init(&bars->acc_empty[s], 4); }
-    fence_barrier_init();
-    tma_prefetch_desc(&map_a_hi);
-    tma_prefetch_desc(&map_b_hi);
-    tma_prefetch_desc(&map_c);
-    if (PARTS == 2) { tma_prefetch_desc(&map_a_lo); tma_prefetch_desc(&map_b_lo); }
-  }
-  if (warp == 1) tmem_alloc(&bars->tmem_base, kTmemCols);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = bars->tmem_base;
-
-  // unit -> (split, m_tile, n_tile); n fastest so that co-resident CTAs share the A tile in L2
-  auto decode = [&](int64_t u, int& ks, int& mt, int& nt) {
-    nt = (int)(u % n_tiles);
-    mt = (int)((u / n_tiles) % m_tiles);
-    ks = (int)(u / ((int64_t)n_tiles * m_tiles));
-  };
-
-  if (warp == 0) {
-    if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int64_t u = blockIdx.x; u < total_units; u += gridDim.x) {
-        int ks, mt, nt;
-        decode(u, ks, mt, nt);
-        const int kb0 = ks * kb_per_split;
-        const int kb1 = kb0 + kb_per_split < total_kb ? kb0 + kb_per_split : total_kb;
-        for (int kb = kb0; kb < kb1; ++kb) {
-          mbar_wait(&bars->empty[stage], phase ^ 1);
-          mbar_expect_tx(&bars->full[stage], STAGE_BYTES);
-          uint8_t* st = smem + stage * STAGE_BYTES;
-          // K-major operand: one box of `rows` rows x 64 k.  MN-major operand (global [K, MN] row-major):
-          // rows / 64 stacked boxes of 64 k-rows x 64 mn columns.
-          auto load = [&](const CUtensorMap* map, uint8_t* dst, int mn0, int mn_major, int rows) {
-            if (mn_major) {
-              for (int b = 0; b < rows / 64; ++b)
-                tma_load_2d(map, &bars->full[stage], dst + b * MN_BOX_BYTES, mn0 + 64 * b, kb * BLOCK_K);
-            } else {
-              tma_load_2d(map, &bars->full[stage], dst, kb * BLOCK_K, mn0);
-            }
-          };
-          load(&map_a_hi, st, mt * BLOCK_M, a_mn, BLOCK_M);
-          if (PARTS == 2) load(&map_a_lo, st + TILE_BYTES, mt * BLOCK_M, a_mn, BLOCK_M);
-          load(&map_b_hi, st + PARTS * TILE_BYTES, nt * BLOCK_N, b_mn, BLOCK_N);
-          if (PARTS == 2) load(&map_b_lo, st + PARTS * TILE_BYTES + B_TILE_BYTES, nt * BLOCK_N, b_mn, BLOCK_N);
-          if (++stage == kStages) { stage = 0; phase ^= 1; }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
-      int t = 0;
-      const uint32_t idesc = kInstrDesc | (a_mn ? 1u << 15 : 0u) | (b_mn ? 1u << 16 : 0u);
-      for (int64_t u = blockIdx.x; u < total_units; u += gridDim.x, ++t) {
-        int ks, mt, nt;
-        decode(u, ks, mt, nt);
-        const int kb0 = ks * kb_per_split;
-        const int kb1 = kb0 + kb_per_split < total_kb ? kb0 + kb_per_split : total_kb;
-        const int acc = t % kAccStages;
-        mbar_wait(&bars->acc_empty[acc], ((uint32_t)(t / kAccStages) & 1) ^ 1);
-        tc_fence_after();
-        const uint32_t tmem_d = tmem_base + (uint32_t)(acc * BLOCK_N);
-        for (int kb = kb0; kb < kb1; ++kb) {
-          mbar_wait(&bars->full[stage], phase);
-          tc_fence_after();
-          const uint32_t a_hi = smem_u32(smem + stage * STAGE_BYTES);
-          const uint32_t a_lo = a_hi + TILE_BYTES;
-          const uint32_t b_hi = a_hi + PARTS * TILE_BYTES;
-          const uint32_t b_lo = b_hi + B_TILE_BYTES;
-#pragma unroll
-          for (int kk = 0; kk < BLOCK_K / UMMA_K; ++kk) {
-            // one UMMA_K = 16 step: 32 bytes along a K-major swizzle row, 16 rows (2 KB) of an MN-major tile
-            const uint32_t off_a = a_mn ? kk * UMMA_K * 128 : kk * UMMA_K * 2;
-            const uint32_t off_b = b_mn ? kk * UMMA_K * 128 : kk * UMMA_K * 2;
-            const uint32_t first = (kb == kb0 && kk == 0) ? 0u : 1u;
-            const uint64_t da_hi = a_mn ? make_desc_mn_sw128(a_hi + off_a, MN_BOX_BYTES) : make_desc_sw128(a_hi + off_a);
-            const uint64_t db_hi = b_mn ? make_desc_mn_sw128(b_hi + off_b, MN_BOX_BYTES) : make_desc_sw128(b_hi + off_b);
-            umma_bf16(tmem_d, da_hi, db_hi, idesc, first);
-            if (PARTS == 2) {
-              const uint64_t da_lo = a_mn ? make_desc_mn_sw128(a_lo + off_a, MN_BOX_BYTES) : make_desc_sw128(a_lo + off_a);
-              const uint64_t db_lo = b_mn ? make_desc_mn_sw128(b_lo + off_b, MN_BOX_BYTES) : make_desc_sw128(b_lo + off_b);
-              umma_bf16(tmem_d, da_hi, db_lo, idesc, 1u);
-              umma_bf16(tmem_d, da_lo, db_hi, idesc, 1u);
-            }
-          }
-          umma_commit(&bars->empty[stage]);
-          if (++stage == kStages) { stage = 0; phase ^= 1; }
-        }
-        umma_commit(&bars->acc_full[acc]);
-      }
-    }
-  } else {
-    // TMEM lane quarter = warp % 4.  Each warp drains its 32 rows x 128 columns in four 32-column
-    // chunks: tcgen05.ld -> (+bias) -> 128B-swizzled staging box -> one TMA store per chunk, so
-    // global memory sees whole 128-byte row segments instead of 32 scattered 16-byte pieces.
-    const int quarter = warp & 3;
-    uint8_t* my_cd = smem_cd + (warp - 2) * 2 * CD_BOX_BYTES;
-    const bool add_bias = bias != nullptr && split_k == 1;
-    int buf = 0;
-    int t = 0;
-    for (int64_t u = blockIdx.x; u < total_units; u += gridDim.x, ++t) {
-      int ks, mt, nt;
-      decode(u, ks, mt, nt);
-      const int acc = t % kAccStages;
-      mbar_wait(&bars->acc_full[acc], (uint32_t)(t / kAccStages) & 1);
-      tc_fence_after();
-      const int row0 = mt * BLOCK_M + quarter * 32;
-      const int col0 = nt * BLOCK_N;
-      const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(acc * BLOCK_N);
-#pragma unroll 1
-      for (int c0 = 0; c0 < BLOCK_N; c0 += 32) {
-        // the chunk's 32 bias values are requested BEFORE the TMEM load so that both latencies overlap
-        float4 bv[8];
-        const bool bias_on = add_bias && (int64_t)col0 + c0 + 32 <= N;
-        if (bias_on) {
-#pragma unroll
-          for (int j = 0; j < 8; ++j) bv[j] = ldg4(bias + col0 + c0 + 4 * j);
-        }
-        uint32_t v[32];
-        tmem_ld_32x32(taddr + (uint32_t)c0, v);
-        if (c0 + 32 == BLOCK_N) {  // accumulator fully read: hand the TMEM stage back before storing
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&bars->acc_empty[acc]);
-        }
-        if ((int64_t)col0 + c0 >= N) continue;  // whole chunk past the last column (warp-uniform)
-        // the store issued two chunks ago (same staging box) must have finished reading it
-        if (lane == 0) tma_store_wait_read<1>();
-        __syncwarp();
-        uint8_t* box = my_cd + buf * CD_BOX_BYTES + lane * 128;
-        float4 prev = zero4();
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          float4 o = make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]),
-                                 __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3]));
-          const int64_t col = (int64_t)col0 + c0 + 4 * j;
-          if (bias_on) o = add4(o, bv[j]);
-          else if (add_bias && col + 3 < N) o = add4(o, ldg4(bias + col));   // ragged last chunk
-          *reinterpret_cast<float4*>(box + ((j ^ (lane & 7)) << 4)) = o;
-          if (act.hi != nullptr) {   // warp-uniform
-            if (j & 1) { if (row0 + lane < M && col + 3 < N) act_store8(act, prev, o, row0 + lane, col - 4, N); }
-            else prev = o;
-          }
-        }
-        fence_proxy_async_smem();
-        __syncwarp();
-        if (lane == 0) {
-          if (accumulate && split_k == 1) tma_reduce_add_3d(&map_c, my_cd + buf * CD_BOX_BYTES, col0 + c0, row0, 0);
-          else tma_store_3d(&map_c, my_cd + buf * CD_BOX_BYTES, col0 + c0, row0, split_k > 1 ? ks : 0);
-          tma_store_commit();
-        }
-        buf ^= 1;
-      }
-    }
-    if (lane == 0) tma_store_wait_all();
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, kTmemCols);
-  }
-}
-
-// ---- the same GEMM on CTA pairs (cta_group::2) ---------------------------------------------------------------
-// The single-CTA kernel above is bound by L2 -> shared-memory traffic: every CTA pulls its own copy of the B tile
-// (the weights in the forward projection: all 148 CTAs reload the same 256 x 1024 matrix per k-block).  Here two
-// CTAs on the two SMs of a TPC execute ONE tcgen05.mma of M = 256: each loads its own 128 rows of A and only HALF
-// of the B tile, the tensor cores of both SMs read both halves — B traffic per SM halves, a stage shrinks from 96 to
-// 64 KB (three stages instead of two at BLOCK_N = 256).  Roles: warp 0 of BOTH CTAs is a TMA producer (its A rows,
-// its B half; completion bytes are counted on the LEADER's full barrier, which expects two producer arrivals),
-// warp 1 of the leader issues the MMAs and commits to the stage-empty / accumulator-full barriers of both CTAs
-// (multicast commit), warps 2-5 of both CTAs drain their own 128 accumulator rows from their own TMEM and release
-// the accumulator stage on the leader's barrier (8 arrivals).
-template <int PARTS, int BN> struct StageCount2 {
+template <int PARTS, int BN> struct StageCount2 {          // ring depth that fits 227 KB next to the store boxes
   static constexpr int value = PARTS == 2 ? (BN == 256 ? 3 : 4) : 4;
 };
 
@@ -616,39 +420,20 @@ colsum_reduce_kernel(const float* __restrict__ partial, int64_t parts, int64_t c
 }
 
 struct GemmPlan {
-  int m_tiles, n_tiles, split_k, kb_per_split, grid, block_n;
-  bool pairs;    // CTA pairs (cta_group::2): m_tiles then counts 256-row tiles, grid = 2 x pairs
+  int m_tiles, n_tiles, split_k, kb_per_split, grid, block_n;   // m_tiles counts 256-row pair tiles; grid = 2 x pairs
 };
-
-bool use_cta_pairs() {
-  static int mode = -1;
-  if (mode < 0) {
-    const char* env = getenv("ETPGT_GEMM_2CTA");      // default on; 0 selects the single-CTA kernel (comparison)
-    mode = env != nullptr ? (atoi(env) != 0) : 1;
-  }
-  return mode == 1;
-}
 
 GemmPlan gemm_plan(int64_t M, int64_t N, int64_t K, int want_split) {
   GemmPlan p;
-  // 128 x 256 tiles for the short-K forward projection and for split-K problems (the weight gradient);
-  // 128 x 128 otherwise (see the note at the top); ETPGT_GEMM_BN=128|256 overrides for tuning
-  p.pairs = use_cta_pairs();
-  // (CTA pairs: a stage is 64 KB at 256 columns, three fit, so the long-K dX GEMM takes the wide tile as well)
-  p.block_n = (N > 128 && (p.pairs || K <= 512 || want_split != 1)) ? 256 : 128;
-  if (const char* forced = getenv("ETPGT_GEMM_BN")) {
-    const int f = atoi(forced);
-    if (f == 128 || f == 256) p.block_n = f;
-  }
-  const int tile_m = p.pairs ? 2 * BLOCK_M : BLOCK_M;
-  p.m_tiles = (int)((M + tile_m - 1) / tile_m);
+  p.block_n = N > 128 ? 256 : 128;   // see the note at the top
+  p.m_tiles = (int)((M + 2 * BLOCK_M - 1) / (2 * BLOCK_M));
   p.n_tiles = (int)((N + p.block_n - 1) / p.block_n);
   const int total_kb = (int)((K + BLOCK_K - 1) / BLOCK_K);
+  const int workers = kNumSMs / 2;   // SM pairs
   int split = 1;
   if (want_split != 1) {
     // few output tiles and a long K: split K until about two waves of units exist
     const int64_t tiles = (int64_t)p.m_tiles * p.n_tiles;
-    const int workers = p.pairs ? kNumSMs / 2 : kNumSMs;
     if (tiles < workers && total_kb >= 16) {
       split = (int)((2 * workers + tiles - 1) / tiles);
       if (split > total_kb / 8) split = total_kb / 8;
@@ -659,13 +444,8 @@ GemmPlan gemm_plan(int64_t M, int64_t N, int64_t K, int want_split) {
   p.kb_per_split = (total_kb + split - 1) / split;
   p.split_k = (total_kb + p.kb_per_split - 1) / p.kb_per_split;
   const int64_t units = (int64_t)p.m_tiles * p.n_tiles * p.split_k;
-  if (p.pairs) {
-    p.grid = 2 * (int)(units < kNumSMs / 2 ? units : kNumSMs / 2);
-    if (p.grid < 2) p.grid = 2;
-    return p;
-  }
-  p.grid = (int)(units < kNumSMs ? units : kNumSMs);
-  if (p.grid < 1) p.grid = 1;
+  p.grid = 2 * (int)(units < workers ? units : workers);
+  if (p.grid < 2) p.grid = 2;
   return p;
 }
 
@@ -734,13 +514,13 @@ static int gemm_run(const void* a_hi, const void* a_lo, const void* b_hi, const 
     return ETPGT_EWORKSPACE;
   }
   CUtensorMap ma_hi, ma_lo, mb_hi, mb_lo;
-  // K-major operand [MN, K]: boxes of 128 (A) / BN (B) rows x 64 k.  MN-major operand [K, MN]: boxes of 64 k-rows x 64 mn.
+  // K-major operand [MN, K]: boxes of 128 (A) / BN / 2 (B: this CTA's half) rows x 64 k.  MN-major operand [K, MN]: boxes of 64 k-rows x 64 mn.
   auto map_a = [&](CUtensorMap* m, const void* ptr_) {
     return a_mn_major ? make_map_bf16(m, ptr_, K, M, lda, 64) : make_map_bf16(m, ptr_, M, K, lda, BLOCK_M);
   };
   auto map_b = [&](CUtensorMap* m, const void* ptr_) {
     return b_mn_major ? make_map_bf16(m, ptr_, K, N, ldb, 64)
-                      : make_map_bf16(m, ptr_, N, K, ldb, p.pairs ? p.block_n / 2 : p.block_n);
+                      : make_map_bf16(m, ptr_, N, K, ldb, p.block_n / 2);
   };
   bool ok = map_a(&ma_hi, a_hi) && map_b(&mb_hi, b_hi);
   if (a_lo != nullptr) ok = ok && map_a(&ma_lo, a_lo) && map_b(&mb_lo, b_lo);
@@ -758,16 +538,6 @@ static int gemm_run(const void* a_hi, const void* a_lo, const void* b_hi, const 
   }
   const int parts = a_lo != nullptr ? 2 : 1;
 #define LAUNCH(PARTS_, BN_)                                                                                       \
-  {                                                                                                               \
-    const size_t smem = 1024 + (size_t)StageCount<PARTS_, BN_>::value * PARTS_ * (TILE_BYTES + BN_ * BLOCK_K * 2) + \
-                        CD_BYTES + sizeof(GemmBarriers) + 64;                                                     \
-    cudaFuncSetAttribute(gemm_bf16x3_kernel<PARTS_, BN_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-    gemm_bf16x3_kernel<PARTS_, BN_><<<p.grid, kThreads, smem, stream>>>(ma_hi, ma_lo, mb_hi, mb_lo, mc, M, N, K,   \
-                                                                       p.m_tiles, p.n_tiles, p.split_k,           \
-                                                                       p.kb_per_split, bias, a_mn_major != 0,     \
-                                                                       b_mn_major != 0, accumulate != 0, act);    \
-  }
-#define LAUNCH2(PARTS_, BN_)                                                                                      \
   {                                                                                                               \
     const size_t smem = 1024 + (size_t)StageCount2<PARTS_, BN_>::value * PARTS_ * (TILE_BYTES + BN_ / 2 * BLOCK_K * 2) + \
                         CD_BYTES + sizeof(GemmBarriers) + 64;                                                     \
@@ -788,16 +558,10 @@ static int gemm_run(const void* a_hi, const void* a_lo, const void* b_hi, const 
                        p.m_tiles, p.n_tiles, p.split_k, p.kb_per_split, bias, (int)(a_mn_major != 0),             \
                        (int)(b_mn_major != 0), (int)(accumulate != 0), act);                                      \
   }
-  if (p.pairs) {
-    if (parts == 2 && p.block_n == 256) LAUNCH2(2, 256)
-    else if (parts == 2) LAUNCH2(2, 128)
-    else if (p.block_n == 256) LAUNCH2(1, 256)
-    else LAUNCH2(1, 128)
-  } else if (parts == 2 && p.block_n == 256) LAUNCH(2, 256)
+  if (parts == 2 && p.block_n == 256) LAUNCH(2, 256)
   else if (parts == 2) LAUNCH(2, 128)
   else if (p.block_n == 256) LAUNCH(1, 256)
   else LAUNCH(1, 128)
-#undef LAUNCH2
 #undef LAUNCH
   ETPGT_CHECK_LAUNCH("gemm_bf16x3");
   if (p.split_k > 1) {

@@ -15,8 +15,6 @@
 //
 // HBM-bound: 4 reads + 3 (4 with zero_grad) writes of 4 bytes per element; float4 accesses, chunked
 // multi-tensor launch (one CTA = one 4,096-element chunk of one tensor).
-#include <stdlib.h>
-
 #include "peer.cuh"
 
 namespace etpgt {
@@ -425,15 +423,10 @@ extern "C" int etpgt_dp_adam_table(const etpgt_comm_t* comm, size_t param_offset
   a.exp_avg_sq = exp_avg_sq;
   a.begin4 = row_begin * (dim / 4);
   a.end4 = row_end * (dim / 4);
-  // one CTA per SM: see the kernel's comment (ETPGT_DP_TABLE_CTAS: tuning knob for the grid)
-  int cap = kNumSMs;
-  if (const char* forced = getenv("ETPGT_DP_TABLE_CTAS")) {
-    const int f = atoi(forced);
-    if (f >= 1 && f <= 8 * kNumSMs) cap = f;
-  }
+  // one CTA per SM: see the kernel's comment
   auto grid_of = [&](int un) {
     const int64_t tiles = (a.end4 - a.begin4 + (int64_t)kThreads * un - 1) / ((int64_t)kThreads * un);
-    return (int)(tiles < cap ? tiles : cap);
+    return (int)(tiles < kNumSMs ? tiles : kNumSMs);
   };
   if (c.world <= 2) {
     dp_adam_table_kernel<8, 2><<<grid_of(8), kThreads, 0, stream>>>(c, a, s);

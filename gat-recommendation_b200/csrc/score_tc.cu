@@ -3,11 +3,12 @@
 // etpgt/model/base.py:59-78 (`torch.matmul(S, E.t())` + `torch.topk`).  The [B, I] score matrix is
 // never written.
 //
-// GEMM kernel (one CTA = 128 sessions x a contiguous range of 256-item tiles; CTA pairs: 256 sessions):
+// GEMM kernel (one CTA pair = 256 sessions x a contiguous range of 256-item tiles; each CTA holds 128 sessions):
 //   warp 0      TMA producer: session tile once (DIM/64 k-blocks of 128x64 bf16, SWIZZLE_128B), then
-//               a ring of item k-blocks (256x64 bf16; a pair: 128x64 per CTA) with mbarrier full/empty hand-shakes
-//   warp 1      TMEM allocator + single-thread tcgen05.mma issuer (UMMA 128x256x16, a pair: 256x256x16 issued by
-//               the leader; kind::f16), accumulators double-buffered in the 512 TMEM columns
+//               a ring of item k-blocks (128x64 bf16 per CTA: half of a 256-item block) with mbarrier full/empty
+//               hand-shakes
+//   warp 1      TMEM allocator + single-thread tcgen05.mma issuer (UMMA 256x256x16 issued by the leader;
+//               kind::f16), accumulators double-buffered in the 512 TMEM columns
 //   warps 2-9   epilogue: two warps per TMEM lane quarter (lane = session row), one per column half of a tile
 //
 // Epilogue = "piece dump".  Measured on B200: with an epilogue that only loads TMEM and takes
@@ -31,9 +32,11 @@
 // threshold — '>=' there, because that warp's pieces may have higher ids).  About 200-250 pieces
 // (14 KB) per row are dumped.  (A variant with the lists kept by separate merge warps in shared
 // memory was measured and dropped: whenever the merge fell behind, the thresholds went stale, more
-// pieces qualified and the merge fell further behind — 630-1,700 pieces per row.)
+// pieces qualified and the merge fell further behind — 630-1,700 pieces per row.  Four warps per
+// quarter, each over 64 columns of a tile, were measured slower as well: four lists over a quarter of
+// the pieces each dumped 350 instead of 215 pieces per row, 0.93 instead of 0.75 ms.)
 //
-// CTA pairs (default): two CTAs on the two SMs of a TPC execute ONE tcgen05.mma of M = 256 (cta_group::2).  Each
+// CTA pairs: two CTAs on the two SMs of a TPC execute ONE tcgen05.mma of M = 256 (cta_group::2).  Each
 // keeps its own 128 session rows resident and loads only HALF of every item k-block (128 of the 256 item rows);
 // the tensor cores of both SMs read both halves, so the L2 -> shared-memory traffic per SM — 62 B/clk at the full
 // MMA rate against ~43 B/clk per SM that the L2 sustains chip-wide — halves, and a stage shrinks to 16 KB (six
@@ -76,21 +79,23 @@ constexpr int BLOCK_M = 128;   // sessions per CTA (TMEM lanes)
 constexpr int BLOCK_N = 256;   // items per accumulator tile (TMEM columns)
 constexpr int CHUNK = 32;      // columns per tcgen05.ld
 constexpr int DUMPW = 16;      // columns per dumped piece (64 bytes)
-constexpr int kMaxStages = 6;  // ring of item k-blocks (3 of 32 KB per CTA, 6 of 16 KB per CTA of a pair)
+constexpr int LOAD_N = BLOCK_N / 2;  // item rows each CTA of a pair loads per k-block
+constexpr int kStages = 6;     // ring of item k-blocks, 16 KB each
 constexpr int kAccStages = 2;  // TMEM accumulator double buffer
 constexpr int kTmemCols = 512;
-constexpr int kMaxColParts = 4;     // epilogue warps per TMEM lane quarter (each takes 256 / parts columns of a tile)
-constexpr int threads_for(int col_parts) { return 32 * (2 + 4 * col_parts); }
+constexpr int kColParts = 2;   // epilogue warps per TMEM lane quarter (each takes 128 columns of a tile)
+constexpr int kThreads = 32 * (2 + 4 * kColParts);
 constexpr int kMaxKTc = 32;
 constexpr int kPendingMerge = 16;  // capacity: maxima a row may have waiting (merge threshold - 1 + pieces per tile half)
-constexpr int kDefaultPendingMerge = 8;
+constexpr int kDefaultPendingMerge = 8;   // merge threshold
+static_assert(kDefaultPendingMerge - 1 + BLOCK_N / kColParts / DUMPW <= kPendingMerge, "pending buffer too small");
 constexpr uint32_t A_KBLOCK_BYTES = BLOCK_M * BLOCK_K * 2;  // 16 KB
-constexpr uint32_t B_STAGE_BYTES = BLOCK_N * BLOCK_K * 2;   // 32 KB (a pair: 16 KB in each CTA)
+constexpr uint32_t B_STAGE_BYTES = LOAD_N * BLOCK_K * 2;    // 16 KB
 
 struct __align__(8) Barriers {
   uint64_t a_full;
-  uint64_t b_full[kMaxStages];
-  uint64_t b_empty[kMaxStages];
+  uint64_t b_full[kStages];
+  uint64_t b_empty[kStages];
   uint64_t acc_full[kAccStages];
   uint64_t acc_empty[kAccStages];
   uint32_t tmem_base;
@@ -98,8 +103,8 @@ struct __align__(8) Barriers {
 
 // Shared-memory scratch of the epilogue warps.
 struct RowShared {
-  float pending[4 * kMaxColParts][kPendingMerge][32];  // piece maxima waiting for the warp's lockstep merge
-  float thr[kMaxColParts][BLOCK_M];                    // [column part][row]: that warp's current threshold
+  float pending[4 * kColParts][kPendingMerge][32];  // piece maxima waiting for the warp's lockstep merge
+  float thr[kColParts][BLOCK_M];                    // [column part][row]: that warp's current threshold
 };
 
 // Dump buffers, per (row, range): `cap` slots of 32 scores + the chunk's first column (relative to the
@@ -108,12 +113,10 @@ struct DumpBuffers {
   float* scores;      // [rows*splits][cap][DUMPW]
   int2* meta;         // [rows*splits][cap]: (first column of the piece relative to the range, bits of the piece's
                       // maximum) — the select kernel reads these first
-  int32_t* count;     // [col_parts][rows*splits]: pieces dumped by each column part
-  float* threshold;   // [col_parts][rows*splits]: final threshold of each column part
+  int32_t* count;     // [kColParts][rows*splits]: pieces dumped by each column part
+  float* threshold;   // [kColParts][rows*splits]: final threshold of each column part
   int64_t units;      // rows*splits
-  int cap;            // slots per (row, range) = (col_parts / 2) sub-buffers of cap_sub slots; two column parts share a
-  int cap_sub;        // sub-buffer and fill it from both ends (no shared counter)
-  int col_parts;
+  int cap;            // slots per (row, range); the two column parts fill them from both ends (no shared counter)
 };
 
 // Work units.  One CTA per SM and one long range per row is the cheapest (every range pays a warm-up
@@ -125,7 +128,7 @@ struct Schedule {
   int tail_splits;      // item ranges per remaining row tile
   int tiles_per_split;  // 256-item tiles per tail range
   int total_tiles;
-  int unit_rows;        // rows of a row tile: 128 (one CTA) or 256 (a CTA pair)
+  int unit_rows;        // rows of a row tile: 256 (a CTA pair)
   __host__ __device__ int64_t full_rows() const { return (int64_t)m_full * unit_rows; }
   __host__ __device__ int parts_of_row(int64_t row) const { return row < full_rows() ? 1 : tail_splits; }
   // index of (row, part) in the count / threshold arrays; x cap in the slot arrays
@@ -264,27 +267,25 @@ __device__ __forceinline__ void merge_pending(RowState<KCAP>& st, uint32_t my_pe
   st_shared_f32(thr_own_addr, st.thr);
 }
 
-// NUM_KB = DIM / 64; KCAP = piece maxima tracked per row and column part (>= k); PAIR = CTA pairs; CP = column parts;
-// EXCL = the rows' exclusion lists are applied (`excl` is ignored otherwise)
-template <int NUM_KB, int KCAP, bool PAIR, int CP, bool EXCL>
-__global__ void __launch_bounds__(threads_for(CP), 1)
+// NUM_KB = DIM / 64; KCAP = piece maxima tracked per row and column part (>= k); EXCL = the rows' exclusion lists
+// are applied (`excl` is ignored otherwise)
+template <int NUM_KB, int KCAP, bool EXCL>
+__global__ void __launch_bounds__(kThreads, 1)
 score_dump_tc_kernel(const __grid_constant__ CUtensorMap map_sess, const __grid_constant__ CUtensorMap map_items,
                      int64_t batch, int64_t num_items, int stages, Schedule sch, DumpBuffers dump,
                      int pending_merge /* <= kPendingMerge */, Exclusion excl) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-  constexpr int LOAD_N = PAIR ? BLOCK_N / 2 : BLOCK_N;          // item rows this CTA loads per k-block
-  constexpr uint32_t STAGE_BYTES = LOAD_N * BLOCK_K * 2;
-  constexpr uint32_t kInstrDesc = instr_desc_bf16(PAIR ? 2 * BLOCK_M : BLOCK_M, BLOCK_N);
+  constexpr uint32_t kInstrDesc = instr_desc_bf16(2 * BLOCK_M, BLOCK_N);
   uint8_t* smem_a = smem;                                   // NUM_KB x 16 KB
-  uint8_t* smem_b = smem_a + NUM_KB * A_KBLOCK_BYTES;       // stages x STAGE_BYTES
-  RowShared* rs = reinterpret_cast<RowShared*>(smem_b + stages * STAGE_BYTES);
+  uint8_t* smem_b = smem_a + NUM_KB * A_KBLOCK_BYTES;       // stages x B_STAGE_BYTES
+  RowShared* rs = reinterpret_cast<RowShared*>(smem_b + stages * B_STAGE_BYTES);
   Barriers* bars = reinterpret_cast<Barriers*>(rs + 1);
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-  const uint32_t rank = PAIR ? cluster_ctarank() : 0;       // 0 = the pair's leader
-  const int unit = PAIR ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;
+  const uint32_t rank = cluster_ctarank();                  // 0 = the pair's leader
+  const int unit = (int)(blockIdx.x >> 1);
   int m_unit, part;
   int64_t tile_begin, tile_end;
   if (unit < sch.m_full) {
@@ -296,65 +297,51 @@ score_dump_tc_kernel(const __grid_constant__ CUtensorMap map_sess, const __grid_
     tile_begin = (int64_t)part * sch.tiles_per_split;
     tile_end = tile_begin + sch.tiles_per_split < sch.total_tiles ? tile_begin + sch.tiles_per_split : sch.total_tiles;
   }
-  const int m_tile = PAIR ? 2 * m_unit + (int)rank : m_unit;   // this CTA's 128 session rows
+  const int m_tile = 2 * m_unit + (int)rank;   // this CTA's 128 session rows
   const int num_tiles = tile_end > tile_begin ? (int)(tile_end - tile_begin) : 0;
 
   if (threadIdx.x == 0) {
     // barriers that gate the MMAs count the producers of BOTH CTAs and live in the leader
-    mbar_init(&bars->a_full, PAIR ? 2 : 1);
-    for (int s = 0; s < kMaxStages; ++s) { mbar_init(&bars->b_full[s], PAIR ? 2 : 1); mbar_init(&bars->b_empty[s], 1); }
+    mbar_init(&bars->a_full, 2);
+    for (int s = 0; s < kStages; ++s) { mbar_init(&bars->b_full[s], 2); mbar_init(&bars->b_empty[s], 1); }
     for (int s = 0; s < kAccStages; ++s) {
       mbar_init(&bars->acc_full[s], 1);
-      mbar_init(&bars->acc_empty[s], PAIR ? 2 * 4 * CP : 4 * CP);
+      mbar_init(&bars->acc_empty[s], 2 * 4 * kColParts);
     }
     fence_barrier_init();
     tma_prefetch_desc(&map_sess);
     tma_prefetch_desc(&map_items);
   }
-  for (int i = threadIdx.x; i < kMaxColParts * BLOCK_M; i += threads_for(CP)) (&rs->thr[0][0])[i] = -INFINITY;
-  if (warp == 1) {
-    if (PAIR) tmem_alloc_2sm(&bars->tmem_base, kTmemCols);
-    else tmem_alloc(&bars->tmem_base, kTmemCols);
-  }
+  for (int i = threadIdx.x; i < kColParts * BLOCK_M; i += kThreads) (&rs->thr[0][0])[i] = -INFINITY;
+  if (warp == 1) tmem_alloc_2sm(&bars->tmem_base, kTmemCols);
   tc_fence_before();
   __syncthreads();
-  if (PAIR) cluster_sync_all();   // both CTAs' barriers are initialised before anything crosses the pair
+  cluster_sync_all();   // both CTAs' barriers are initialised before anything crosses the pair
   tc_fence_after();
   const uint32_t tmem_base = bars->tmem_base;
 
   if (warp == 0) {
-    // ===================== TMA producer (one elected lane; in a pair: of each CTA) =====================
+    // ===================== TMA producer (one elected lane of each CTA) =====================
     if (lane == 0 && num_tiles > 0) {
-      if (PAIR) {
-        const uint32_t a_full = mapa_shared(smem_u32(&bars->a_full), 0);
-        mbar_arrive_expect_tx_cluster(a_full, NUM_KB * A_KBLOCK_BYTES);
-        for (int kb = 0; kb < NUM_KB; ++kb)
-          tma_load_2d_2sm(&map_sess, a_full, smem_a + kb * A_KBLOCK_BYTES, kb * BLOCK_K, m_tile * BLOCK_M);
-      } else {
-        mbar_expect_tx(&bars->a_full, NUM_KB * A_KBLOCK_BYTES);
-        for (int kb = 0; kb < NUM_KB; ++kb)
-          tma_load_2d(&map_sess, &bars->a_full, smem_a + kb * A_KBLOCK_BYTES, kb * BLOCK_K, m_tile * BLOCK_M);
-      }
+      const uint32_t a_full = mapa_shared(smem_u32(&bars->a_full), 0);
+      mbar_arrive_expect_tx_cluster(a_full, NUM_KB * A_KBLOCK_BYTES);
+      for (int kb = 0; kb < NUM_KB; ++kb)
+        tma_load_2d_2sm(&map_sess, a_full, smem_a + kb * A_KBLOCK_BYTES, kb * BLOCK_K, m_tile * BLOCK_M);
       int stage = 0;
       uint32_t phase = 0;
       for (int t = 0; t < num_tiles; ++t) {
-        const int row0 = (int)((tile_begin + t) * BLOCK_N) + (int)rank * LOAD_N;   // a pair: this CTA's half
+        const int row0 = (int)((tile_begin + t) * BLOCK_N) + (int)rank * LOAD_N;   // this CTA's half
         for (int kb = 0; kb < NUM_KB; ++kb) {
           mbar_wait(&bars->b_empty[stage], phase ^ 1);
-          if (PAIR) {
-            const uint32_t full = mapa_shared(smem_u32(&bars->b_full[stage]), 0);
-            mbar_arrive_expect_tx_cluster(full, STAGE_BYTES);
-            tma_load_2d_2sm(&map_items, full, smem_b + stage * STAGE_BYTES, kb * BLOCK_K, row0);
-          } else {
-            mbar_expect_tx(&bars->b_full[stage], STAGE_BYTES);
-            tma_load_2d(&map_items, &bars->b_full[stage], smem_b + stage * STAGE_BYTES, kb * BLOCK_K, row0);
-          }
+          const uint32_t full = mapa_shared(smem_u32(&bars->b_full[stage]), 0);
+          mbar_arrive_expect_tx_cluster(full, B_STAGE_BYTES);
+          tma_load_2d_2sm(&map_items, full, smem_b + stage * B_STAGE_BYTES, kb * BLOCK_K, row0);
           if (++stage == stages) { stage = 0; phase ^= 1; }
         }
       }
     }
   } else if (warp == 1) {
-    // ===================== MMA issuer (one elected lane; in a pair: of the leader) =====================
+    // ===================== MMA issuer (one elected lane of the leader) =====================
     if (lane == 0 && rank == 0 && num_tiles > 0) {
       mbar_wait(&bars->a_full, 0);
       tc_fence_after();
@@ -370,33 +357,30 @@ score_dump_tc_kernel(const __grid_constant__ CUtensorMap map_sess, const __grid_
           mbar_wait(&bars->b_full[stage], phase);
           tc_fence_after();
           const uint32_t a_addr = smem_u32(smem_a + kb * A_KBLOCK_BYTES);
-          const uint32_t b_addr = smem_u32(smem_b + stage * STAGE_BYTES);
+          const uint32_t b_addr = smem_u32(smem_b + stage * B_STAGE_BYTES);
 #pragma unroll
           for (int kk = 0; kk < BLOCK_K / UMMA_K; ++kk) {
             const uint64_t da = make_desc_sw128(a_addr + kk * UMMA_K * 2);
             const uint64_t db = make_desc_sw128(b_addr + kk * UMMA_K * 2);
-            if (PAIR) umma_bf16_2sm(tmem_d, da, db, kInstrDesc, (kb | kk) != 0 ? 1u : 0u);
-            else umma_bf16(tmem_d, da, db, kInstrDesc, (kb | kk) != 0 ? 1u : 0u);
+            umma_bf16_2sm(tmem_d, da, db, kInstrDesc, (kb | kk) != 0 ? 1u : 0u);
           }
           // frees the smem stage (in both CTAs) once these MMAs have read it
-          if (PAIR) umma_commit_2sm(&bars->b_empty[stage]);
-          else umma_commit(&bars->b_empty[stage]);
+          umma_commit_2sm(&bars->b_empty[stage]);
           if (++stage == stages) { stage = 0; phase ^= 1; }
         }
         // accumulator tile complete (each CTA's epilogue reads its own 128 rows from its own TMEM)
-        if (PAIR) umma_commit_2sm(&bars->acc_full[acc]);
-        else umma_commit(&bars->acc_full[acc]);
+        umma_commit_2sm(&bars->acc_full[acc]);
       }
     }
   } else {
-    // ========== epilogue: 4 * CP warps; TMEM lane quarter = warp % 4, column part = (warp - 2) / 4 ==========
+    // ========== epilogue: 8 warps; TMEM lane quarter = warp % 4, column part = (warp - 2) / 4 ==========
     const int quarter = warp & 3;
     const int cpart = (warp - 2) >> 2;
     const int row = quarter * 32 + lane;       // session row inside the tile == TMEM lane
     const int64_t grow = (int64_t)m_tile * BLOCK_M + row;
     const bool live = grow < batch;
     const int64_t pidx = live ? sch.part_index(grow, part) : 0;
-    const int64_t slot0 = pidx * (int64_t)dump.cap + (cpart >> 1) * dump.cap_sub;   // this pair of parts' sub-buffer
+    const int64_t slot0 = pidx * (int64_t)dump.cap;
     float* my_scores = dump.scores + slot0 * DUMPW;
     int2* my_meta = dump.meta + slot0;
     RowState<KCAP> st;
@@ -408,12 +392,12 @@ score_dump_tc_kernel(const __grid_constant__ CUtensorMap map_sess, const __grid_
     const uint32_t my_pending = smem_u32(&rs->pending[warp - 2][0][lane]);
     const uint32_t thr_row_addr = smem_u32(&rs->thr[0][row]);
     const uint32_t thr_own_addr = thr_row_addr + (uint32_t)(cpart * BLOCK_M * sizeof(float));
-    const uint32_t acc_empty0 = PAIR ? mapa_shared(smem_u32(&bars->acc_empty[0]), 0) : smem_u32(&bars->acc_empty[0]);
-    constexpr int PART_N = BLOCK_N / CP;
+    const uint32_t acc_empty0 = mapa_shared(smem_u32(&bars->acc_empty[0]), 0);
+    constexpr int PART_N = BLOCK_N / kColParts;
     // loop constants pinned in registers (as kernel parameters they were re-read from the constant bank on the
     // divergent path: ~2 % of the epilogue's stall samples)
-    int cap = dump.cap_sub, merge_at = pending_merge;
-    int slot_first = (cpart & 1) ? dump.cap_sub - 1 : 0, slot_step = (cpart & 1) ? -1 : 1;
+    int cap = dump.cap, merge_at = pending_merge;
+    int slot_first = (cpart & 1) ? dump.cap - 1 : 0, slot_step = (cpart & 1) ? -1 : 1;
     asm volatile("" : "+r"(cap), "+r"(merge_at), "+r"(slot_first), "+r"(slot_step));
     // exclusion cursor: starts at the lower bound of the range's first id in the row's list
     ExclCursor* ex = reinterpret_cast<ExclCursor*>(bars + 1) + (threadIdx.x - 64);
@@ -443,35 +427,27 @@ score_dump_tc_kernel(const __grid_constant__ CUtensorMap map_sess, const __grid_
       // This warp's columns of the tile go to registers as early as the register file allows (all chunks but one,
       // the last into the first one's registers once that is worked off) and the accumulator
       // is handed back before the rest is processed and before any merge: the MMA issuer (which needs every epilogue
-      // warp — of both CTAs of a pair — to let go) no longer waits for a warp that is busy in a lockstep merge.
-      constexpr int NCH = PART_N / CHUNK;             // 4 or 2
-      constexpr int NBUF = NCH - 1;                   // 3 or 1 (96 registers per thread with 18 warps)
+      // warp of both CTAs to let go) no longer waits for a warp that is busy in a lockstep merge.
+      constexpr int NCH = PART_N / CHUNK;             // 4
+      constexpr int NBUF = NCH - 1;                   // 3 (96 registers per thread)
       uint32_t raw[NBUF][CHUNK];
 #pragma unroll
       for (int c = 0; c < NBUF; ++c) tmem_ld_32x32_issue(taddr + (uint32_t)(c * CHUNK), raw[c]);
-      // the other column parts' thresholds: a little stale at worst, still valid bounds
-      float thr_other = -INFINITY;
-#pragma unroll
-      for (int o = 1; o < CP; ++o)
-        thr_other = fmaxf(thr_other, ld_shared_f32(thr_row_addr + (uint32_t)(((cpart + o) % CP) * BLOCK_M * sizeof(float))));
+      // the other column part's threshold: a little stale at worst, still a valid bound
+      const float thr_other = ld_shared_f32(thr_row_addr + (uint32_t)((cpart ^ 1) * BLOCK_M * sizeof(float)));
 #pragma unroll
       for (int c = 0; c < NBUF; ++c) tmem_ld_wait(raw[c]);
-      if (NCH > NBUF) {
-        chunk_hits<KCAP, EXCL>(raw[0], st, col0, limit, my_scores, my_meta, cap, slot_first, slot_step, my_pending,
-                               thr_other, ex_col, ex);
-        tmem_ld_32x32(taddr + (uint32_t)(NBUF * CHUNK), raw[0]);
-      }
+      chunk_hits<KCAP, EXCL>(raw[0], st, col0, limit, my_scores, my_meta, cap, slot_first, slot_step, my_pending,
+                             thr_other, ex_col, ex);
+      tmem_ld_32x32(taddr + (uint32_t)(NBUF * CHUNK), raw[0]);
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) {
-        if (PAIR) mbar_arrive_cluster(acc_empty0 + (uint32_t)(acc * sizeof(uint64_t)));
-        else mbar_arrive(&bars->acc_empty[acc]);
-      }
+      if (lane == 0) mbar_arrive_cluster(acc_empty0 + (uint32_t)(acc * sizeof(uint64_t)));
       // the lockstep merge (long: up to 15 passes of the sorting network) comes AFTER the hand-back, so that it never
       // sits between an accumulator becoming ready and this warp letting go of it
       merge_pending<KCAP>(st, my_pending, thr_own_addr, merge_at);
 #pragma unroll
-      for (int c = NCH > NBUF ? 1 : 0; c < NCH; ++c)
+      for (int c = 1; c < NCH; ++c)
         chunk_hits<KCAP, EXCL>(raw[c % NBUF], st, col0 + c * CHUNK, limit - c * CHUNK, my_scores, my_meta, cap,
                                slot_first, slot_step, my_pending, thr_other, ex_col, ex);
     }
@@ -483,11 +459,10 @@ score_dump_tc_kernel(const __grid_constant__ CUtensorMap map_sess, const __grid_
   }
   tc_fence_before();
   __syncthreads();
-  if (PAIR) cluster_sync_all();   // neither CTA's shared memory / TMEM goes away while the other still uses it
+  cluster_sync_all();   // neither CTA's shared memory / TMEM goes away while the other still uses it
   if (warp == 1) {
     tc_fence_after();
-    if (PAIR) tmem_dealloc_2sm(tmem_base, kTmemCols);
-    else tmem_dealloc(tmem_base, kTmemCols);
+    tmem_dealloc_2sm(tmem_base, kTmemCols);
   }
 }
 
@@ -530,22 +505,19 @@ score_select_kernel(DumpBuffers dump, int64_t batch, Schedule sch, int k, int64_
   float tau = -INFINITY;
   bool overflow = false;
   const int splits = sch.parts_of_row(row);
-  const int cparts = dump.col_parts;
   for (int s = 0; s < splits; ++s) {
     const int64_t pi = sch.part_index(row, s);
-    for (int c = 0; c < cparts; c += 2) {
-      tau = fmaxf(tau, fmaxf(dump.threshold[c * dump.units + pi], dump.threshold[(c + 1) * dump.units + pi]));
-      overflow = overflow || dump.count[c * dump.units + pi] + dump.count[(c + 1) * dump.units + pi] > dump.cap_sub;
-    }
+    tau = fmaxf(tau, fmaxf(dump.threshold[pi], dump.threshold[dump.units + pi]));
+    overflow = overflow || dump.count[pi] + dump.count[dump.units + pi] > dump.cap;
   }
   __syncwarp();
   if (!overflow) {
-    for (int seg = 0; seg < cparts * splits; ++seg) {
-      // a (row, range) slot buffer is col_parts / 2 sub-buffers, each filled from both ends by two column parts
-      const int s = seg / cparts, c = seg % cparts;
+    for (int seg = 0; seg < kColParts * splits; ++seg) {
+      // a (row, range) slot buffer is filled from both ends by the two column parts
+      const int s = seg / kColParts, c = seg % kColParts;
       const int64_t pi = sch.part_index(row, s);
       const int n = dump.count[c * dump.units + pi];
-      const int64_t slot0 = pi * (int64_t)dump.cap + (c >> 1) * dump.cap_sub + ((c & 1) ? dump.cap_sub - n : 0);
+      const int64_t slot0 = pi * (int64_t)dump.cap + (c ? dump.cap - n : 0);
       const int range_col0 = sch.first_tile(row, s) * BLOCK_N;
       // the piece maxima first (one coalesced 8-byte load per piece): the pieces that reach tau — a few dozen of the
       // ~200 dumped per row — are collected as (slot, first column) pairs ...
@@ -794,43 +766,20 @@ __global__ void f32_to_bf16_kernel(const float* __restrict__ src, __nv_bfloat16*
 
 struct TcPlan {
   Schedule sch;
-  int grid;
-  int cap, cap_sub;
-  int col_parts;   // epilogue warps per TMEM lane quarter: 2 (default) or 4
-  bool pairs;   // CTA pairs (cta_group::2): a row tile is 256 rows, grid = 2 x units, workers = 74 SM pairs
+  int grid;   // 2 x units: one CTA pair per unit
+  int cap;
 };
-
-bool use_cta_pairs() {
-  static const bool on = [] {
-    const char* e = getenv("ETPGT_SCORE_2CTA");   // comparison knob: 0 = one CTA per unit (round 1's kernel shape)
-    return e == nullptr || atoi(e) != 0;
-  }();
-  return on;
-}
-
-int epilogue_col_parts() {
-  static const int parts = [] {
-    // two epilogue warps per lane quarter; 4 (comparison knob) was measured slower: 350 instead of 215 dumped pieces
-    // per row (four lists over a quarter of the pieces each) and 0.93 instead of 0.75 ms
-    const char* e = getenv("ETPGT_SCORE_EPI");
-    return e != nullptr && atoi(e) == 4 ? 4 : 2;
-  }();
-  return parts;
-}
 
 TcPlan tc_plan(int64_t batch, int64_t num_items, int k) {
   TcPlan p;
-  p.pairs = use_cta_pairs();
-  p.col_parts = epilogue_col_parts();
-  const int unit_rows = p.pairs ? 2 * BLOCK_M : BLOCK_M;
-  const int workers = p.pairs ? kNumSMs / 2 : kNumSMs;
+  const int unit_rows = 2 * BLOCK_M;
+  const int workers = kNumSMs / 2;   // SM pairs
   const int m_tiles = (int)((batch + unit_rows - 1) / unit_rows);
   const int total_tiles = (int)((num_items + BLOCK_N - 1) / BLOCK_N);
   // tail ranges stay >= 64 tiles (512 chunks) so that every range's own threshold is tight enough for
   // the select kernel's survivor buffer
   int max_splits = total_tiles / 64 > 1 ? total_tiles / 64 : 1;
   if (max_splits > 32) max_splits = 32;
-  const int max_forced = total_tiles / 32 > 1 ? (total_tiles / 32 > 32 ? 32 : total_tiles / 32) : 1;   // tuning knob only
   const int m_full = (m_tiles / workers) * workers;   // whole waves: one full-catalogue unit per row tile
   const int tail = m_tiles - m_full;
   int splits = 1;
@@ -844,39 +793,32 @@ TcPlan tc_plan(int64_t batch, int64_t num_items, int k) {
       const double cost = (double)waves * ((double)per / (double)total_tiles + 0.5);
       if (cost < best_cost - 1e-9) { best_cost = cost; splits = s; }
     }
-    if (const char* forced = getenv("ETPGT_SCORE_SPLITS")) {  // tuning knob
-      const int f = atoi(forced);
-      if (f >= 1 && f <= max_forced) splits = f;
-    }
   }
   p.sch.unit_rows = unit_rows;
   p.sch.m_full = m_full;
   p.sch.total_tiles = total_tiles;
   p.sch.tiles_per_split = (total_tiles + splits - 1) / splits;
   p.sch.tail_splits = (total_tiles + p.sch.tiles_per_split - 1) / p.sch.tiles_per_split;
-  p.grid = (m_full + tail * p.sch.tail_splits) * (p.pairs ? 2 : 1);
+  p.grid = (m_full + tail * p.sch.tail_splits) * 2;
   // slots per (row, range): every column part keeps its own list over its share of the pieces, so
   // ~ P*K*(1 + ln(pieces/(P*K))) pieces are expected (+ ~25 % from the lockstep merges); 1.6x head-room (sized
   // for the longest range), overflow is handled exactly by the fallback kernel
   const double chunks = (double)(m_full > 0 ? total_tiles : p.sch.tiles_per_split) * (BLOCK_N / DUMPW);
   const int kc = k <= 10 ? 10 : k <= 20 ? 20 : 32;
-  const double lists = (double)p.col_parts * kc;
+  const double lists = (double)kColParts * kc;
   double expect = lists * (1.0 + (chunks > lists ? log(chunks / lists) : 0.0));
-  int cap = (int)(1.6 * expect) + 16;
-  if (cap > (int)chunks) cap = (int)chunks;
+  p.cap = (int)(1.6 * expect) + 16;
+  if (p.cap > (int)chunks) p.cap = (int)chunks;
   if (const char* forced = getenv("ETPGT_SCORE_CAP")) {  // test hook: force slot-buffer overflow
     const int f = atoi(forced);
-    if (f >= 1) cap = f;
+    if (f >= 1) p.cap = f;
   }
-  const int subs = p.col_parts / 2;
-  p.cap_sub = (cap + subs - 1) / subs < 1 ? 1 : (cap + subs - 1) / subs;
-  p.cap = p.cap_sub * subs;
   return p;
 }
 
-size_t tc_smem_bytes(int num_kb, int stages, bool pairs) {
-  return 1024 + (size_t)num_kb * A_KBLOCK_BYTES + (size_t)stages * (pairs ? B_STAGE_BYTES / 2 : B_STAGE_BYTES) +
-         sizeof(RowShared) + sizeof(Barriers) + 64;
+size_t tc_smem_bytes(int num_kb) {
+  return 1024 + (size_t)num_kb * A_KBLOCK_BYTES + (size_t)kStages * B_STAGE_BYTES + sizeof(RowShared) +
+         sizeof(Barriers) + 64;
 }
 
 }  // namespace
@@ -898,7 +840,7 @@ extern "C" size_t etpgt_score_topk_bf16_workspace_bytes(int64_t batch, int64_t n
   const TcPlan p = tc_plan(batch, num_items, k);
   const size_t units = (size_t)p.sch.num_parts(batch);
   return align_up(units * p.cap * DUMPW * sizeof(float)) + align_up(units * p.cap * sizeof(int2)) +
-         2 * align_up(kMaxColParts * units * sizeof(float)) + 2 * align_up((size_t)batch * sizeof(int32_t)) + 256;
+         2 * align_up(kColParts * units * sizeof(float)) + 2 * align_up((size_t)batch * sizeof(int32_t)) + 256;
 }
 
 namespace {
@@ -929,66 +871,49 @@ int score_topk_bf16_run(const void* sess_bf16, const void* table_bf16, int64_t b
   }
   if (batch == 0) return ETPGT_OK;
   const TcPlan p = tc_plan(batch, num_items, k);
-  // the exclusion variant exists for the default kernel shape only (CTA pairs, two column parts)
-  ETPGT_REQUIRE(!use_excl || (p.pairs && p.col_parts == 2),
-                "score_topk_bf16_exclude: exclusion needs the default scorer configuration (unset ETPGT_SCORE_2CTA and "
-                "ETPGT_SCORE_EPI)");
   Workspace w(ws, ws_bytes);
   const size_t units = (size_t)p.sch.num_parts(batch);
   DumpBuffers dump;
   dump.scores = w.take<float>(units * p.cap * DUMPW);
   dump.meta = w.take<int2>(units * p.cap);
-  dump.count = w.take<int32_t>(kMaxColParts * units);
-  dump.threshold = w.take<float>(kMaxColParts * units);
+  dump.count = w.take<int32_t>(kColParts * units);
+  dump.threshold = w.take<float>(kColParts * units);
   dump.units = (int64_t)units;
   dump.cap = p.cap;
-  dump.cap_sub = p.cap_sub;
-  dump.col_parts = p.col_parts;
   int32_t* redo = w.take<int32_t>(batch);
   CUtensorMap map_sess, map_items;
   if (!make_map_bf16(&map_sess, sess_bf16, batch, dim, dim, BLOCK_M) ||
-      !make_map_bf16(&map_items, table_bf16, num_items, dim, dim, p.pairs ? BLOCK_N / 2 : BLOCK_N)) {
+      !make_map_bf16(&map_items, table_bf16, num_items, dim, dim, LOAD_N)) {
     set_error("score_topk_bf16: cuTensorMapEncodeTiled failed");
     return ETPGT_ECUDA;
   }
   const int num_kb = dim / BLOCK_K;
-  const int stages = p.pairs ? kMaxStages : kMaxStages / 2;
-  int pending_merge = kDefaultPendingMerge;
-  if (const char* forced = getenv("ETPGT_SCORE_PENDING")) {  // tuning knob
-    const int f = atoi(forced);
-    if (f >= 1 && f <= kPendingMerge + 1 - BLOCK_N / 2 / DUMPW) pending_merge = f;
-  }
   // the exclusion variant keeps its epilogue threads' cursors behind the barriers
-  const size_t smem = tc_smem_bytes(num_kb, stages, p.pairs) + (use_excl ? 4 * 2 * 32 * sizeof(ExclCursor) : 0);
+  const size_t smem = tc_smem_bytes(num_kb) + (use_excl ? 4 * kColParts * 32 * sizeof(ExclCursor) : 0);
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(p.grid);
-  cfg.blockDim = dim3(threads_for(p.col_parts));
+  cfg.blockDim = dim3(kThreads);
   cfg.dynamicSmemBytes = smem;
   cfg.stream = stream;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = p.pairs ? 2 : 1;
+  attr[0].val.clusterDim.x = 2;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-#define LAUNCH4(NKB, KC, PR, CP_, EX)                                                                              \
-  {                                                                                                                \
-    cudaFuncSetAttribute(score_dump_tc_kernel<NKB, KC, PR, CP_, EX>, cudaFuncAttributeMaxDynamicSharedMemorySize,  \
-                         (int)smem);                                                                               \
-    cudaLaunchKernelEx(&cfg, score_dump_tc_kernel<NKB, KC, PR, CP_, EX>, map_sess, map_items, batch, num_items,    \
-                       stages, p.sch, dump, pending_merge, excl);                                                  \
+  // the ring depth and the merge threshold are passed at run time, as in the kernel that was measured (the epilogue
+  // pins the merge threshold in a register)
+#define LAUNCH3(NKB, KC, EX)                                                                                         \
+  {                                                                                                                  \
+    cudaFuncSetAttribute(score_dump_tc_kernel<NKB, KC, EX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+    cudaLaunchKernelEx(&cfg, score_dump_tc_kernel<NKB, KC, EX>, map_sess, map_items, batch, num_items, kStages,      \
+                       p.sch, dump, kDefaultPendingMerge, excl);                                                     \
   }
-#define LAUNCH3(NKB, KC, PR)                           \
-  {                                                    \
-    if (p.col_parts == 4) LAUNCH4(NKB, KC, PR, 4, false) \
-    else LAUNCH4(NKB, KC, PR, 2, false)                \
-  }
-#define LAUNCH2(NKB, KC)                            \
-  {                                                 \
-    if (use_excl) LAUNCH4(NKB, KC, true, 2, true)   \
-    else if (p.pairs) LAUNCH3(NKB, KC, true)        \
-    else LAUNCH3(NKB, KC, false)                    \
+#define LAUNCH2(NKB, KC)                   \
+  {                                        \
+    if (use_excl) LAUNCH3(NKB, KC, true)   \
+    else LAUNCH3(NKB, KC, false)           \
   }
 #define LAUNCH(NKB)                    \
   {                                    \
@@ -1011,7 +936,6 @@ int score_topk_bf16_run(const void* sess_bf16, const void* table_bf16, int64_t b
 #undef LAUNCH
 #undef LAUNCH2
 #undef LAUNCH3
-#undef LAUNCH4
   ETPGT_CHECK_LAUNCH("score_dump_tc");
   if (stats) cudaEventRecord(ev[1], stream);
   score_select_kernel<<<(unsigned)((batch + kSelectWarps - 1) / kSelectWarps), kSelectWarps * 32, 0, stream>>>(
@@ -1037,7 +961,7 @@ int score_topk_bf16_run(const void* sess_bf16, const void* table_bf16, int64_t b
   }
   ETPGT_CHECK_LAUNCH("score_redo");
   if (stats) {   // dump volume, fallback rows, kernel times
-    std::vector<int32_t> h_redo(batch), h_count(kMaxColParts * units);
+    std::vector<int32_t> h_redo(batch), h_count(kColParts * units);
     cudaStreamSynchronize(stream);
     float ms_dump = 0.f, ms_select = 0.f;
     cudaEventElapsedTime(&ms_dump, ev[0], ev[1]);
@@ -1045,12 +969,12 @@ int score_topk_bf16_run(const void* sess_bf16, const void* table_bf16, int64_t b
     for (auto& e : ev) cudaEventDestroy(e);
     fprintf(stderr, "score_topk_bf16: dump %.3f ms, select %.3f ms\n", ms_dump, ms_select);
     cudaMemcpy(h_redo.data(), redo, batch * sizeof(int32_t), cudaMemcpyDeviceToHost);
-    cudaMemcpy(h_count.data(), dump.count, kMaxColParts * units * sizeof(int32_t), cudaMemcpyDeviceToHost);
+    cudaMemcpy(h_count.data(), dump.count, kColParts * units * sizeof(int32_t), cudaMemcpyDeviceToHost);
     int64_t redo_rows = 0, pieces = 0, worst = 0;
     for (int64_t i = 0; i < batch; ++i) redo_rows += h_redo[i];
     for (size_t i = 0; i < units; ++i) {
       int64_t c = 0;
-      for (int cp = 0; cp < p.col_parts; ++cp) c += h_count[(size_t)cp * units + i];
+      for (int cp = 0; cp < kColParts; ++cp) c += h_count[(size_t)cp * units + i];
       pieces += c;
       worst = c > worst ? c : worst;
     }

@@ -22,7 +22,6 @@ Configurations the driver does not cover (FFN, attention readout, per-node PE, e
 from __future__ import annotations
 
 import ctypes
-import os
 import weakref
 from ctypes import c_double, c_float, c_int32, c_int64, c_size_t, c_uint64, c_void_p
 
@@ -357,7 +356,7 @@ class FusedTrainStep:
             # one host call; under peer-memory data parallelism the driver exchanges the BatchNorm sums itself
             if self.graph is True or (self.graph == "auto" and n <= self.GRAPH_MAX_NODES):
                 self._run_graph(phases)
-            elif peer is not None and backward and not os.environ.get("ETPGT_DP_NO_OVERLAP"):
+            elif peer is not None and backward:
                 # the table gradient is complete one phase before the end (the driver orders the backward tail that
                 # way): mark that point, so that the optimizer can run the table's reduce-scatter + AdamW + all-gather
                 # on its exchange stream UNDERNEATH the last phase (weight gradient of layer 0, PE projection gradient)

@@ -1,7 +1,6 @@
 """Timing of the three GEMMs of one TransformerConv layer at the bench batch (N = 99,132 nodes, D = 256): forward
-projection [N,256]x[1024,256]^T, dX [N,1024]x[1024,256] (+ TMA reduce-add), dW [1024,N]x[N,256] (split-K), with the
-single-CTA kernel or with CTA pairs (ETPGT_GEMM_2CTA=1).  Prints ms per GEMM and the worst error vs fp64."""
-import os
+projection [N,256]x[1024,256]^T, dX [N,1024]x[1024,256] (+ TMA reduce-add), dW [1024,N]x[N,256] (split-K).
+Prints ms per GEMM and the worst error vs fp64."""
 import sys
 from pathlib import Path
 
@@ -43,7 +42,6 @@ fwd = lambda: ops._gemm_x3(x_hi, x_lo, w_hi, w_lo, n, w4, d, d, d, b)           
 res = torch.zeros(n, d, device=dev)
 dx = lambda: ops._gemm_x3(g_hi, g_lo, w_hi, w_lo, n, d, w4, w4, d, None, b_mn=True, accumulate_into=res)   # noqa: E731
 dw = lambda: ops._gemm_x3(g_hi, g_lo, x_hi, x_lo, w4, d, n, w4, d, None, split_k=0, a_mn=True, b_mn=True)  # noqa: E731
-mode = os.environ.get("ETPGT_GEMM_2CTA", "0")
 y = fwd()
 err_f = ((y.double() - (x.double() @ w.double().t() + b.double())).abs().max() / y.double().abs().max()).item()
 res.zero_()
@@ -52,5 +50,5 @@ err_x = ((gx.double() - dy.double() @ w.double()).abs().max() / gx.double().abs(
 gw = dw()
 ref_w = dy.double().t() @ x.double()
 err_w = ((gw.double() - ref_w).abs().max() / ref_w.abs().max()).item()
-print(f"2cta={mode}: errors fwd {err_f:.2e} dX {err_x:.2e} dW {err_w:.2e}")
-print(f"2cta={mode}: fwd {timed(fwd):.4f} ms, dX {timed(dx):.4f} ms, dW {timed(dw):.4f} ms")
+print(f"errors fwd {err_f:.2e} dX {err_x:.2e} dW {err_w:.2e}")
+print(f"fwd {timed(fwd):.4f} ms, dX {timed(dx):.4f} ms, dW {timed(dw):.4f} ms")

@@ -15,7 +15,7 @@ namespace {
 
 constexpr int kThreads = 256;
 constexpr int kRowsPerGroup = 4;  // register blocking: one item row is reused for 4 sessions
-constexpr int kMaxK = 64;
+constexpr int kMaxK = 64;   // the fp32 scorer; the merges take k <= ETPGT_SCORE_MAX_K
 constexpr int64_t kNoId = INT64_MAX;
 
 struct Cand { float val; int32_t idx; };
@@ -227,6 +227,123 @@ topk_merge_parts_kernel(const char* __restrict__ parts, int num_parts, size_t pa
   if (lane == 0 && hit_pos != nullptr) hit_pos[row] = found;
 }
 
+// k > 64: one CTA per row.  Candidates that beat the bar are appended to a shared buffer of kWideBuf (score, id)
+// pairs; whenever the next block of 256 could overflow it, the buffer is bitonic-sorted by (score desc, id asc), exact
+// duplicates are dropped (as the selection passes above drop them) and it is cut to the best k, whose last pair
+// becomes the bar.  A row costs a few sorts instead of k passes over its parts * k candidates.
+constexpr int kWideBuf = 2048;
+
+__device__ void wide_sort_pairs(float* sv, int64_t* si, int n) {
+  int p = 1;
+  while (p < n) p <<= 1;
+  for (int i = n + (int)threadIdx.x; i < p; i += kThreads) { sv[i] = -INFINITY; si[i] = kNoId; }
+  __syncthreads();
+  for (int size = 2; size <= p; size <<= 1) {
+    for (int stride = size >> 1; stride > 0; stride >>= 1) {
+      for (int t = threadIdx.x; t < p / 2; t += kThreads) {
+        const int lo = (t / stride) * 2 * stride + (t % stride), hi = lo + stride;
+        const bool desc = (lo & size) == 0;
+        const float av = sv[lo], bv = sv[hi];
+        const int64_t ai = si[lo], bi = si[hi];
+        if (better(bv, bi, av, ai) == desc) { sv[lo] = bv; si[lo] = bi; sv[hi] = av; si[hi] = ai; }
+      }
+      __syncthreads();
+    }
+  }
+}
+
+// Whole CTA: sorts, de-duplicates and cuts the buffer to k once it could overflow (force: always); returns the
+// number of pairs kept and sets the bar once k are known.
+__device__ int wide_cut(float* sv, int64_t* si, int* s_n, int k, bool force, bool& have_bar, float& bar_v,
+                        int64_t& bar_i) {
+  __syncthreads();
+  int n = *s_n;
+  __syncthreads();
+  if (!force && n <= kWideBuf - kThreads) return n;
+  wide_sort_pairs(sv, si, n);
+  if (threadIdx.x < 32) {   // compaction by warp 0: writes never pass the chunk being read
+    const int lane = threadIdx.x;
+    int kept = 0;
+    float cv = 0.f;
+    int64_t ci = 0;
+    for (int c0 = 0; c0 < n && kept < k; c0 += 32) {
+      const int c = c0 + lane;
+      const float v = c < n ? sv[c] : 0.f;
+      const int64_t i = c < n ? si[c] : 0;
+      float pv = __shfl_up_sync(0xffffffffu, v, 1);
+      int64_t pi = __shfl_up_sync(0xffffffffu, i, 1);
+      if (lane == 0) { pv = cv; pi = ci; }
+      const bool keep = c < n && (c == 0 || !(pv == v && pi == i));
+      cv = __shfl_sync(0xffffffffu, v, 31);
+      ci = __shfl_sync(0xffffffffu, i, 31);
+      const unsigned m = __ballot_sync(0xffffffffu, keep);
+      const int pos = kept + __popc(m & ((1u << lane) - 1));
+      __syncwarp();
+      if (keep && pos < k) { sv[pos] = v; si[pos] = i; }
+      kept += __popc(m);
+      __syncwarp();
+    }
+    if (lane == 0) *s_n = kept < k ? kept : k;
+  }
+  __syncthreads();
+  n = *s_n;
+  if (n == k) { have_bar = true; bar_v = sv[k - 1]; bar_i = si[k - 1]; }
+  __syncthreads();
+  return n;
+}
+
+// PARTS: the rank-major layout of topk_merge_parts_kernel; otherwise [batch, m] candidate arrays.
+template <bool PARTS>
+__global__ void __launch_bounds__(kThreads)
+topk_merge_wide_kernel(const float* __restrict__ cand_val, const int64_t* __restrict__ cand_idx, int64_t m,
+                       const char* __restrict__ parts, int num_parts, size_t part_stride, size_t idx_offset,
+                       int64_t row_begin, int k, float* __restrict__ top_val, int64_t* __restrict__ top_idx,
+                       const int64_t* __restrict__ targets, int32_t* __restrict__ hit_pos) {
+  __shared__ float sv[kWideBuf];
+  __shared__ int64_t si[kWideBuf];
+  __shared__ int s_n, s_found;
+  const int64_t row = blockIdx.x;
+  const int64_t total = PARTS ? (int64_t)num_parts * k : m;
+  const int64_t src = (row_begin + row) * k;
+  if (threadIdx.x == 0) { s_n = 0; s_found = INT_MAX; }
+  __syncthreads();
+  bool have_bar = false;
+  float bar_v = -INFINITY;
+  int64_t bar_i = kNoId;
+  for (int64_t c0 = 0; c0 < total; c0 += kThreads) {
+    const int64_t c = c0 + threadIdx.x;
+    if (c < total) {
+      float v;
+      int64_t i;
+      if (PARTS) {
+        const char* part = parts + (size_t)(c / k) * part_stride;
+        v = reinterpret_cast<const float*>(part)[src + c % k];
+        i = reinterpret_cast<const int64_t*>(part + idx_offset)[src + c % k];
+      } else {
+        v = cand_val[row * m + c];
+        i = cand_idx[row * m + c];
+      }
+      if (!have_bar || better(v, i, bar_v, bar_i)) {
+        const int pos = atomicAdd(&s_n, 1);
+        sv[pos] = v;
+        si[pos] = i;
+      }
+    }
+    wide_cut(sv, si, &s_n, k, false, have_bar, bar_v, bar_i);
+  }
+  const int n = wide_cut(sv, si, &s_n, k, true, have_bar, bar_v, bar_i);
+  const int64_t target = targets != nullptr ? targets[row] : kNoId;
+  for (int t = threadIdx.x; t < k; t += kThreads) {
+    const float v = t < n ? sv[t] : -INFINITY;
+    const int64_t i = t < n ? si[t] : kNoId;
+    top_val[row * k + t] = v;
+    top_idx[row * k + t] = i;
+    if (targets != nullptr && i == target) atomicMin(&s_found, t);
+  }
+  __syncthreads();
+  if (threadIdx.x == 0 && hit_pos != nullptr) hit_pos[row] = s_found == INT_MAX ? -1 : s_found;
+}
+
 // hit_pos[b] = position of the target in the top-k (-1: missed) -> acc[0] += #hits within k, acc[1] += sum of
 // 1/log2(pos + 2) over them (etpgt/utils/metrics.py:6-66); one CTA, fixed order: deterministic.
 __global__ void __launch_bounds__(1024)
@@ -297,8 +414,15 @@ extern "C" size_t etpgt_score_topk_workspace_bytes(int64_t batch, int64_t num_it
 
 extern "C" int etpgt_topk_merge(const float* cand_val, const int64_t* cand_idx, int64_t batch, int parts, int k,
                                 float* top_val, int64_t* top_idx, etpgt_stream_t stream) {
-  ETPGT_REQUIRE(batch >= 0 && parts >= 1 && k >= 1 && k <= kMaxK, "topk_merge: bad sizes (k <= %d)", kMaxK);
+  ETPGT_REQUIRE(batch >= 0 && parts >= 1 && k >= 1 && k <= ETPGT_SCORE_MAX_K, "topk_merge: bad sizes (k <= %d)",
+                ETPGT_SCORE_MAX_K);
   if (batch == 0) return ETPGT_OK;
+  if (k > kMaxK) {
+    topk_merge_wide_kernel<false><<<(unsigned)batch, kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+        cand_val, cand_idx, (int64_t)parts * k, nullptr, 0, 0, 0, 0, k, top_val, top_idx, nullptr, nullptr);
+    ETPGT_CHECK_LAUNCH("topk_merge_wide");
+    return ETPGT_OK;
+  }
   const int64_t warps_per_cta = kThreads / 32;
   topk_merge_kernel<<<(unsigned)((batch + warps_per_cta - 1) / warps_per_cta), kThreads, 0,
                       static_cast<cudaStream_t>(stream)>>>(cand_val, cand_idx, batch, (int64_t)parts * k, k, top_val,
@@ -318,10 +442,13 @@ int score_topk_f32_run(const float* sess, const float* table, int64_t batch, int
   ETPGT_REQUIRE(supported_dim(dim), "score_topk: unsupported dim %d", dim);
   ETPGT_REQUIRE(batch >= 0 && num_items >= 1, "score_topk: bad sizes");
   if (k_any) {
-    ETPGT_REQUIRE(k >= 1 && k <= kMaxK, "score_topk: k=%d must be in [1, %d]", k, kMaxK);
+    ETPGT_REQUIRE(k >= 1 && k <= kMaxK,
+                  "score_topk: k=%d must be in [1, %d] for the fp32 scorer (the bf16 scorer takes k <= %d)", k, kMaxK,
+                  ETPGT_SCORE_MAX_K);
   } else {
-    ETPGT_REQUIRE(k >= 1 && k <= kMaxK && k <= num_items, "score_topk: k=%d must be in [1, min(%d, num_items)]", k,
-                  kMaxK);
+    ETPGT_REQUIRE(k >= 1 && k <= kMaxK && k <= num_items,
+                  "score_topk: k=%d must be in [1, min(%d, num_items)] for the fp32 scorer (the bf16 scorer takes k <= "
+                  "%d)", k, kMaxK, ETPGT_SCORE_MAX_K);
   }
   if (ws_bytes < etpgt_score_topk_workspace_bytes(batch, num_items, dim, k)) {
     set_error("score_topk: workspace too small");
@@ -384,7 +511,8 @@ extern "C" int etpgt_topk_merge_parts(const void* parts, int num_parts, size_t p
                                       int64_t rows_total, int k, int64_t row_begin, int64_t rows, float* top_val,
                                       int64_t* top_idx, const int64_t* targets, int32_t* hit_pos,
                                       etpgt_stream_t stream) {
-  ETPGT_REQUIRE(num_parts >= 1 && num_parts <= 64 && k >= 1 && k <= kMaxK, "topk_merge_parts: bad sizes (k <= %d)", kMaxK);
+  ETPGT_REQUIRE(num_parts >= 1 && num_parts <= 64 && k >= 1 && k <= ETPGT_SCORE_MAX_K,
+                "topk_merge_parts: bad sizes (k <= %d)", ETPGT_SCORE_MAX_K);
   ETPGT_REQUIRE(rows >= 0 && row_begin >= 0 && row_begin + rows <= rows_total, "topk_merge_parts: bad row range");
   ETPGT_REQUIRE(idx_offset % 8 == 0 && part_stride % 8 == 0 && idx_offset >= (size_t)rows_total * k * sizeof(float) &&
                     part_stride >= idx_offset + (size_t)rows_total * k * sizeof(int64_t),
@@ -392,6 +520,13 @@ extern "C" int etpgt_topk_merge_parts(const void* parts, int num_parts, size_t p
   ETPGT_REQUIRE(rows == 0 || (parts && top_val && top_idx), "topk_merge_parts: null pointer");
   ETPGT_REQUIRE((targets == nullptr) == (hit_pos == nullptr), "topk_merge_parts: targets and hit_pos come together");
   if (rows == 0) return ETPGT_OK;
+  if (k > kMaxK) {
+    topk_merge_wide_kernel<true><<<(unsigned)rows, kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+        nullptr, nullptr, 0, static_cast<const char*>(parts), num_parts, part_stride, idx_offset, row_begin, k, top_val,
+        top_idx, targets, hit_pos);
+    ETPGT_CHECK_LAUNCH("topk_merge_parts_wide");
+    return ETPGT_OK;
+  }
   const int64_t warps_per_cta = kThreads / 32;
   topk_merge_parts_kernel<<<(unsigned)((rows + warps_per_cta - 1) / warps_per_cta), kThreads, 0,
                             static_cast<cudaStream_t>(stream)>>>(static_cast<const char*>(parts), num_parts,

@@ -54,6 +54,21 @@
 // id asc) with a bitonic sort of 64-bit keys in registers.  Rows whose slot buffer overflowed (adversarial score
 // orders) are recomputed exactly by a CUDA-core fallback kernel, so the result is always exact.
 //
+// k > 32 (up to ETPGT_SCORE_MAX_K = 256): the list keeps 32 entries, and the value tracked for a dumped piece is its
+// M-th largest score instead of its maximum, M = ceil(k / 32) in {2, 4, 8} (M = 1 below 33: the same code as before).
+// Proof that thr stays a lower bound of the row's k-th best score: 32 distinct pieces each hold M items >= thr, so at
+// least 32 * M >= k items are >= thr.  The dump test still decides on the piece maximum (a piece holding a top-k item
+// has maximum >= the k-th best score >= thr), and the tie argument above carries over unchanged: the items that set
+// thr were seen earlier, in ascending id order, and the other part's threshold is compared with '>='.  A piece that is
+// not dumped has M-th value <= maximum <= thr, so merging only the dumped pieces' values loses nothing.  The M-th
+// value is computed on the divergent hit path only (a 16 x M insertion network), so the hot loop is unchanged.  The
+// bound is weak when the scores are not clustered by id: 32 pieces need M items each above thr, and on normal scores
+// the threshold stops far below the k-th best (DESIGN.md §4), so for k > 32 the slot buffer has a slot for every piece
+// and never overflows.  The select for k > 32 (one CTA per row) keeps its own bar: a shared buffer of candidate keys
+// that is sorted and cut to the best k whenever it could overflow; the bar is the k-th key, and pieces whose maximum
+// is below its score are not read.  The fallback for k > 32 scores a flagged row on the CUDA cores into the same
+// buffer.
+//
 // Exclusion (etpgt_score_topk_bf16_exclude, the EXCL variant): every row may name item ids it must not receive (the
 // session's own items, the padding id).  The epilogue sets those columns to -inf BEFORE the piece maxima are taken:
 // an excluded item holding one of the K best piece maxima would otherwise raise the threshold above the K-th best
@@ -85,7 +100,7 @@ constexpr int kAccStages = 2;  // TMEM accumulator double buffer
 constexpr int kTmemCols = 512;
 constexpr int kColParts = 2;   // epilogue warps per TMEM lane quarter (each takes 128 columns of a tile)
 constexpr int kThreads = 32 * (2 + 4 * kColParts);
-constexpr int kMaxKTc = 32;
+constexpr int kMaxKNarrow = 32;   // k classes up to here: one piece maximum per list entry, the warp-per-row select
 constexpr int kPendingMerge = 16;  // capacity: maxima a row may have waiting (merge threshold - 1 + pieces per tile half)
 constexpr int kDefaultPendingMerge = 8;   // merge threshold
 static_assert(kDefaultPendingMerge - 1 + BLOCK_N / kColParts / DUMPW <= kPendingMerge, "pending buffer too small");
@@ -168,17 +183,38 @@ __device__ __forceinline__ int excl_col(int64_t id, int64_t base) {
 // Per-row state of the piece-dump epilogue (one thread = one session row = one TMEM lane, one column half).
 template <int KCAP>
 struct RowState {
-  float best[KCAP];   // the KCAP largest piece maxima of this row (this half) so far, descending
-  float thr;          // = best[KCAP - 1] as of the last merge: a lower bound of the row's K-th best score
+  float best[KCAP];   // the KCAP largest tracked piece values of this row (this half) so far, descending
+  float thr;          // = best[KCAP - 1] as of the last merge: a lower bound of the row's (KCAP * M)-th best score
   int count, pending;
 };
 
+// The M-th largest of the DUMPW scores v[j0, j0 + DUMPW): a branch-free insertion network (j0 is a compile-time
+// offset in the unrolled callers, so v stays in registers).
+template <int M>
+__device__ __forceinline__ float piece_mth(const float (&v)[CHUNK], int j0) {
+  float top[M];
+#pragma unroll
+  for (int s = 0; s < M; ++s) top[s] = -INFINITY;
+#pragma unroll
+  for (int j = 0; j < DUMPW; ++j) {
+    float x = v[j0 + j];
+#pragma unroll
+    for (int s = 0; s < M; ++s) {
+      const float hi = fmaxf(top[s], x);
+      x = fminf(top[s], x);
+      top[s] = hi;
+    }
+  }
+  return top[M - 1];
+}
+
 // One 32-column chunk of a row: piece maxima, dump of the pieces that beat the thresholds; their maxima wait in the
-// warp's pending buffer for the merge at the end of the tile.
+// warp's pending buffer for the merge at the end of the tile.  The tracked value of a dumped piece is its M-th largest
+// score (M = 1: its maximum); the dump test itself always uses the maximum.
 //   slot_first / slot_step: this warp fills the slot buffer upwards from 0 or downwards from cap - 1
 // (The hot loop has to stay inside the instruction cache: with four inlined copies of chunk + merge ncu showed 1.8
 // "no instruction" stall cycles per issued instruction; the merge exists once per kernel now.)
-template <int KCAP, bool EXCL>
+template <int KCAP, int M, bool EXCL>
 __device__ __forceinline__ void chunk_hits(const uint32_t (&raw)[CHUNK], RowState<KCAP>& st, int col,
                                            int limit_rel /* real columns left from this chunk on */,
                                            float* my_scores, int2* my_meta, int cap, int slot_first, int slot_step,
@@ -226,7 +262,8 @@ __device__ __forceinline__ void chunk_hits(const uint32_t (&raw)[CHUNK], RowStat
   for (int h = 0; h < CHUNK / DUMPW; ++h) {
     if (hit[h]) {
       const int n = st.count++;
-      st_shared_f32(my_pending + st.pending * 32 * sizeof(float), mx[h]);  // waits for the lockstep merge
+      const float tracked = M == 1 ? mx[h] : piece_mth<M>(v, h * DUMPW);
+      st_shared_f32(my_pending + st.pending * 32 * sizeof(float), tracked);  // waits for the lockstep merge
       ++st.pending;
       if (n < cap) {
         const int slot = slot_first + slot_step * n;
@@ -267,9 +304,9 @@ __device__ __forceinline__ void merge_pending(RowState<KCAP>& st, uint32_t my_pe
   st_shared_f32(thr_own_addr, st.thr);
 }
 
-// NUM_KB = DIM / 64; KCAP = piece maxima tracked per row and column part (>= k); EXCL = the rows' exclusion lists
-// are applied (`excl` is ignored otherwise)
-template <int NUM_KB, int KCAP, bool EXCL>
+// NUM_KB = DIM / 64; KCAP = piece values tracked per row and column part; M = which largest score of a piece is
+// tracked (KCAP * M >= k); EXCL = the rows' exclusion lists are applied (`excl` is ignored otherwise)
+template <int NUM_KB, int KCAP, int M, bool EXCL>
 __global__ void __launch_bounds__(kThreads, 1)
 score_dump_tc_kernel(const __grid_constant__ CUtensorMap map_sess, const __grid_constant__ CUtensorMap map_items,
                      int64_t batch, int64_t num_items, int stages, Schedule sch, DumpBuffers dump,
@@ -437,7 +474,7 @@ score_dump_tc_kernel(const __grid_constant__ CUtensorMap map_sess, const __grid_
       const float thr_other = ld_shared_f32(thr_row_addr + (uint32_t)((cpart ^ 1) * BLOCK_M * sizeof(float)));
 #pragma unroll
       for (int c = 0; c < NBUF; ++c) tmem_ld_wait(raw[c]);
-      chunk_hits<KCAP, EXCL>(raw[0], st, col0, limit, my_scores, my_meta, cap, slot_first, slot_step, my_pending,
+      chunk_hits<KCAP, M, EXCL>(raw[0], st, col0, limit, my_scores, my_meta, cap, slot_first, slot_step, my_pending,
                              thr_other, ex_col, ex);
       tmem_ld_32x32(taddr + (uint32_t)(NBUF * CHUNK), raw[0]);
       tc_fence_before();
@@ -448,7 +485,7 @@ score_dump_tc_kernel(const __grid_constant__ CUtensorMap map_sess, const __grid_
       merge_pending<KCAP>(st, my_pending, thr_own_addr, merge_at);
 #pragma unroll
       for (int c = 1; c < NCH; ++c)
-        chunk_hits<KCAP, EXCL>(raw[c % NBUF], st, col0 + c * CHUNK, limit - c * CHUNK, my_scores, my_meta, cap,
+        chunk_hits<KCAP, M, EXCL>(raw[c % NBUF], st, col0 + c * CHUNK, limit - c * CHUNK, my_scores, my_meta, cap,
                                slot_first, slot_step, my_pending, thr_other, ex_col, ex);
     }
     merge_pending<KCAP>(st, my_pending, thr_own_addr, 1);   // what is still waiting: the final threshold
@@ -648,6 +685,131 @@ score_select_kernel(DumpBuffers dump, int64_t batch, Schedule sch, int k, int64_
   }
 }
 
+// k > 32: one CTA per row.  The candidates are gathered as packed keys into a shared buffer of kWideBuf; whenever
+// it could overflow with the next block of 256, it is sorted (bitonic network in shared memory) and cut to the best
+// k, whose last key becomes the bar a later candidate must beat.  Keys are unique (they carry the column), so "beats
+// the k-th key" is exact and the order of arrival does not matter.  Pieces are kept when their maximum reaches the
+// current bar's score (>=: an item of the same score with a lower id would still beat it).
+constexpr int kWideThreads = 256;
+constexpr int kWideBuf = 2048;
+
+// Sorts keys[0, n) descending (every thread of the CTA takes part; n <= kWideBuf).
+__device__ void wide_sort(uint64_t* keys, int n) {
+  int p = 1;
+  while (p < n) p <<= 1;
+  for (int i = n + (int)threadIdx.x; i < p; i += kWideThreads) keys[i] = 0;
+  __syncthreads();
+  for (int size = 2; size <= p; size <<= 1) {
+    for (int stride = size >> 1; stride > 0; stride >>= 1) {
+      for (int i = threadIdx.x; i < p / 2; i += kWideThreads) {
+        const int lo = (i / stride) * 2 * stride + (i % stride), hi = lo + stride;
+        const bool desc = (lo & size) == 0;
+        const uint64_t a = keys[lo], b = keys[hi];
+        if ((a < b) == desc) { keys[lo] = b; keys[hi] = a; }
+      }
+      __syncthreads();
+    }
+  }
+}
+
+// Called by the whole CTA between blocks of appends: cuts the buffer to the best k once it could overflow (force:
+// always).  Returns the number of keys kept; bar = the k-th key once k are known (0 before).
+__device__ int wide_compact(uint64_t* keys, int* s_n, int k, bool force, uint64_t& bar) {
+  __syncthreads();
+  int n = *s_n;
+  __syncthreads();   // every thread has read the count before the next appends
+  if (force || n > kWideBuf - kWideThreads) {
+    wide_sort(keys, n);
+    n = n < k ? n : k;
+    if (n == k) bar = keys[k - 1];
+    __syncthreads();
+    if (threadIdx.x == 0) *s_n = n;
+    __syncthreads();
+  }
+  return n;
+}
+
+// Writes the row's sorted keys[0, n) as k results (sentinels past n) and the target's position.
+__device__ void wide_emit(const uint64_t* keys, int n, int k, int64_t row, int64_t id_base, float* top_val,
+                          int64_t* top_idx, const int64_t* targets, int32_t* hit_pos, int* s_found) {
+  if (threadIdx.x == 0) *s_found = INT_MAX;
+  __syncthreads();
+  const int64_t target = targets != nullptr ? targets[row] : -1;
+  for (int t = threadIdx.x; t < k; t += kWideThreads) {
+    const uint64_t key = t < n ? keys[t] : 0;
+    float v;
+    int64_t col;
+    decode_key(key, v, col);
+    const int64_t id = key == 0 ? INT64_MAX : id_base + col;
+    top_val[row * k + t] = v;
+    top_idx[row * k + t] = id;
+    if (targets != nullptr && id == target) atomicMin(s_found, t);
+  }
+  __syncthreads();
+  if (threadIdx.x == 0 && targets != nullptr) hit_pos[row] = *s_found == INT_MAX ? -1 : *s_found;
+}
+
+__global__ void __launch_bounds__(kWideThreads)
+score_select_wide_kernel(DumpBuffers dump, int64_t batch, Schedule sch, int k, int64_t id_base,
+                         float* __restrict__ top_val, int64_t* __restrict__ top_idx, int32_t* __restrict__ redo,
+                         const int64_t* __restrict__ targets, int32_t* __restrict__ hit_pos) {
+  __shared__ uint64_t s_key[kWideBuf];
+  __shared__ int2 s_flag[kWideThreads];   // qualifying pieces of one block of records: (slot, first column)
+  __shared__ int s_n, s_nf, s_found;
+  const int64_t row = blockIdx.x;
+  const int splits = sch.parts_of_row(row);
+  float tau = -INFINITY;
+  bool overflow = false;
+  for (int s = 0; s < splits; ++s) {
+    const int64_t pi = sch.part_index(row, s);
+    tau = fmaxf(tau, fmaxf(dump.threshold[pi], dump.threshold[dump.units + pi]));
+    overflow = overflow || dump.count[pi] + dump.count[dump.units + pi] > dump.cap;
+  }
+  if (overflow) {   // CTA-uniform
+    if (threadIdx.x == 0) redo[row] = 1;
+    return;
+  }
+  if (threadIdx.x == 0) { redo[row] = 0; s_n = 0; }
+  uint64_t bar = 0;
+  float bar_v = tau;                        // pieces below this cannot hold a candidate
+  const int sub = threadIdx.x >> 4, e = threadIdx.x & 15;
+  for (int seg = 0; seg < kColParts * splits; ++seg) {
+    const int s = seg / kColParts, c = seg % kColParts;
+    const int64_t pi = sch.part_index(row, s);
+    const int n = dump.count[c * dump.units + pi];
+    const int64_t slot0 = pi * (int64_t)dump.cap + (c ? dump.cap - n : 0);
+    const int range_col0 = sch.first_tile(row, s) * BLOCK_N;
+    for (int c0 = 0; c0 < n; c0 += kWideThreads) {
+      __syncthreads();
+      if (threadIdx.x == 0) s_nf = 0;
+      __syncthreads();
+      if (c0 + (int)threadIdx.x < n) {
+        const int2 m = __ldcs(dump.meta + slot0 + c0 + threadIdx.x);
+        const float pm = __int_as_float(m.y);
+        if (pm >= bar_v && pm > -INFINITY)
+          s_flag[atomicAdd(&s_nf, 1)] = make_int2(c0 + (int)threadIdx.x, range_col0 + m.x);
+      }
+      __syncthreads();
+      const int nf = s_nf;
+      for (int f0 = 0; f0 < nf; f0 += kWideThreads / DUMPW) {   // 16 pieces at a time, one score per thread
+        if (f0 + sub < nf) {
+          const int2 fl = s_flag[f0 + sub];
+          const float v = __ldcs(dump.scores + (slot0 + fl.x) * DUMPW + e);
+          const uint64_t key = candidate_key(v, fl.y + e);
+          if (v >= tau && v > -INFINITY && key > bar) s_key[atomicAdd(&s_n, 1)] = key;
+        }
+        wide_compact(s_key, &s_n, k, false, bar);
+        if (bar != 0) {
+          int64_t col_unused;
+          decode_key(bar, bar_v, col_unused);
+        }
+      }
+    }
+  }
+  const int n = wide_compact(s_key, &s_n, k, true, bar);
+  wide_emit(s_key, n, k, row, id_base, top_val, top_idx, targets, hit_pos, &s_found);
+}
+
 // Exact CUDA-core recomputation of the rows flagged in `redo` (slot-buffer or tie overflow): one CTA
 // per row, every thread scores a strided share of the items (fp32 accumulation of the same bf16
 // operands) and keeps a private sorted k-list; lists are merged through shared memory.
@@ -753,6 +915,49 @@ score_redo_kernel(const __nv_bfloat16* __restrict__ sess, const __nv_bfloat16* _
   }
 }
 
+// k > 32: exact CUDA-core recomputation of a flagged row, one CTA per row: each block of 256 items is scored (one
+// item per thread, the same fp32 arithmetic as score_redo_kernel) into the shared key buffer of the wide select.
+// EXCL: a candidate that beats the bar is looked up in the row's list, staged in shared memory.
+template <bool EXCL>
+__global__ void __launch_bounds__(kWideThreads)
+score_redo_wide_kernel(const __nv_bfloat16* __restrict__ sess, const __nv_bfloat16* __restrict__ table, int64_t batch,
+                       int64_t num_items, int dim, int k, int64_t id_base, const int32_t* __restrict__ redo,
+                       float* __restrict__ top_val, int64_t* __restrict__ top_idx,
+                       const int64_t* __restrict__ targets, int32_t* __restrict__ hit_pos, Exclusion excl) {
+  extern __shared__ int64_t wide_smem[];     // the row's exclusion list (EXCL), then the session row [dim] as fp32
+  __shared__ uint64_t s_key[kWideBuf];
+  __shared__ int s_n, s_found;
+  int64_t* s_excl = wide_smem;
+  float* s_row = reinterpret_cast<float*>(wide_smem + (EXCL ? excl.width : 0));
+  for (int64_t row = blockIdx.x; row < batch; row += gridDim.x) {
+    if (redo[row] == 0) continue;           // CTA-uniform
+    __syncthreads();                        // the previous row's buffers are no longer read
+    for (int d = threadIdx.x; d < dim; d += kWideThreads) s_row[d] = __bfloat162float(sess[row * dim + d]);
+    if (EXCL)
+      for (int64_t i = threadIdx.x; i < excl.width; i += kWideThreads) s_excl[i] = excl.ids[row * excl.width + i];
+    if (threadIdx.x == 0) s_n = 0;
+    __syncthreads();
+    uint64_t bar = 0;
+    for (int64_t item0 = 0; item0 < num_items; item0 += kWideThreads) {
+      const int64_t item = item0 + threadIdx.x;
+      if (item < num_items) {
+        const __nv_bfloat16* e = table + item * dim;
+        float acc = 0.f;
+        for (int d = 0; d < dim; d += 2) {
+          const float2 p = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(e + d));
+          acc = fmaf(s_row[d], p.x, acc);
+          acc = fmaf(s_row[d + 1], p.y, acc);
+        }
+        const uint64_t key = candidate_key(acc, (int32_t)item);
+        if (key > bar && !(EXCL && listed(s_excl, (int)excl.width, id_base + item))) s_key[atomicAdd(&s_n, 1)] = key;
+      }
+      wide_compact(s_key, &s_n, k, false, bar);
+    }
+    const int n = wide_compact(s_key, &s_n, k, true, bar);
+    wide_emit(s_key, n, k, row, id_base, top_val, top_idx, targets, hit_pos, &s_found);
+  }
+}
+
 __global__ void f32_to_bf16_kernel(const float* __restrict__ src, __nv_bfloat16* __restrict__ dst, int64_t n4) {
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
     const float4 v = ldg4(src + 4 * i);
@@ -804,11 +1009,17 @@ TcPlan tc_plan(int64_t batch, int64_t num_items, int k) {
   // ~ P*K*(1 + ln(pieces/(P*K))) pieces are expected (+ ~25 % from the lockstep merges); 1.6x head-room (sized
   // for the longest range), overflow is handled exactly by the fallback kernel
   const double chunks = (double)(m_full > 0 ? total_tiles : p.sch.tiles_per_split) * (BLOCK_N / DUMPW);
-  const int kc = k <= 10 ? 10 : k <= 20 ? 20 : 32;
-  const double lists = (double)kColParts * kc;
-  double expect = lists * (1.0 + (chunks > lists ? log(chunks / lists) : 0.0));
-  p.cap = (int)(1.6 * expect) + 16;
-  if (p.cap > (int)chunks) p.cap = (int)chunks;
+  if (k <= kMaxKNarrow) {
+    const int kc = k <= 10 ? 10 : k <= 20 ? 20 : 32;
+    const double lists = (double)kColParts * kc;
+    double expect = lists * (1.0 + (chunks > lists ? log(chunks / lists) : 0.0));
+    p.cap = (int)(1.6 * expect) + 16;
+    if (p.cap > (int)chunks) p.cap = (int)chunks;
+  } else {
+    // k > 32 tracks the M-th largest score of a piece, a much weaker bound on random score orders (DESIGN.md §4):
+    // a slot for every piece of the range, so the slot buffer never overflows
+    p.cap = (int)chunks;
+  }
   if (const char* forced = getenv("ETPGT_SCORE_CAP")) {  // test hook: force slot-buffer overflow
     const int f = atoi(forced);
     if (f >= 1) p.cap = f;
@@ -858,10 +1069,10 @@ int score_topk_bf16_run(const void* sess_bf16, const void* table_bf16, int64_t b
                 "score_topk_bf16: dim %d must be a multiple of 64 up to 256", dim);
   ETPGT_REQUIRE(batch >= 0 && num_items >= 1 && num_items < (int64_t(1) << 31), "score_topk_bf16: bad sizes");
   if (k_any) {
-    ETPGT_REQUIRE(k >= 1 && k <= kMaxKTc, "score_topk_bf16: k=%d must be in [1, %d]", k, kMaxKTc);
+    ETPGT_REQUIRE(k >= 1 && k <= ETPGT_SCORE_MAX_K, "score_topk_bf16: k=%d must be in [1, %d]", k, ETPGT_SCORE_MAX_K);
   } else {
-    ETPGT_REQUIRE(k >= 1 && k <= kMaxKTc && k <= num_items, "score_topk_bf16: k=%d must be in [1, min(%d, num_items)]",
-                  k, kMaxKTc);
+    ETPGT_REQUIRE(k >= 1 && k <= ETPGT_SCORE_MAX_K && k <= num_items,
+                  "score_topk_bf16: k=%d must be in [1, min(%d, num_items)]", k, ETPGT_SCORE_MAX_K);
   }
   ETPGT_REQUIRE(((uintptr_t)sess_bf16 & 15) == 0 && ((uintptr_t)table_bf16 & 15) == 0,
                 "score_topk_bf16: operands must be 16-byte aligned");
@@ -904,25 +1115,29 @@ int score_topk_bf16_run(const void* sess_bf16, const void* table_bf16, int64_t b
   cfg.numAttrs = 1;
   // the ring depth and the merge threshold are passed at run time, as in the kernel that was measured (the epilogue
   // pins the merge threshold in a register)
-#define LAUNCH3(NKB, KC, EX)                                                                                         \
-  {                                                                                                                  \
-    cudaFuncSetAttribute(score_dump_tc_kernel<NKB, KC, EX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-    cudaLaunchKernelEx(&cfg, score_dump_tc_kernel<NKB, KC, EX>, map_sess, map_items, batch, num_items, kStages,      \
-                       p.sch, dump, kDefaultPendingMerge, excl);                                                     \
+#define LAUNCH3(NKB, KC, M, EX)                                                                             \
+  {                                                                                                         \
+    cudaFuncSetAttribute(score_dump_tc_kernel<NKB, KC, M, EX>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+                         (int)smem);                                                                        \
+    cudaLaunchKernelEx(&cfg, score_dump_tc_kernel<NKB, KC, M, EX>, map_sess, map_items, batch, num_items,   \
+                       kStages, p.sch, dump, kDefaultPendingMerge, excl);                                   \
   }
-#define LAUNCH2(NKB, KC)                   \
+#define LAUNCH2(NKB, KC, M)                  \
+  {                                          \
+    if (use_excl) LAUNCH3(NKB, KC, M, true)  \
+    else LAUNCH3(NKB, KC, M, false)          \
+  }
+#define LAUNCH(NKB)                        \
   {                                        \
-    if (use_excl) LAUNCH3(NKB, KC, true)   \
-    else LAUNCH3(NKB, KC, false)           \
-  }
-#define LAUNCH(NKB)                    \
-  {                                    \
-    if (k <= 10) LAUNCH2(NKB, 10)      \
-    else if (k <= 20) LAUNCH2(NKB, 20) \
-    else LAUNCH2(NKB, 32)              \
+    if (k <= 10) LAUNCH2(NKB, 10, 1)       \
+    else if (k <= 20) LAUNCH2(NKB, 20, 1)  \
+    else if (k <= 32) LAUNCH2(NKB, 32, 1)  \
+    else if (k <= 64) LAUNCH2(NKB, 32, 2)  \
+    else if (k <= 128) LAUNCH2(NKB, 32, 4) \
+    else LAUNCH2(NKB, 32, 8)               \
   }
   const bool stats = getenv("ETPGT_SCORE_STATS") != nullptr;   // tuning aid (synchronises)
-  cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
+  cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
   if (stats) {
     for (auto& e : ev) cudaEventCreate(&e);
     cudaEventRecord(ev[0], stream);
@@ -938,36 +1153,60 @@ int score_topk_bf16_run(const void* sess_bf16, const void* table_bf16, int64_t b
 #undef LAUNCH3
   ETPGT_CHECK_LAUNCH("score_dump_tc");
   if (stats) cudaEventRecord(ev[1], stream);
-  score_select_kernel<<<(unsigned)((batch + kSelectWarps - 1) / kSelectWarps), kSelectWarps * 32, 0, stream>>>(
-      dump, batch, p.sch, k, id_base, top_val, top_idx, redo, targets, hit_pos);
+  if (k <= kMaxKNarrow) {
+    score_select_kernel<<<(unsigned)((batch + kSelectWarps - 1) / kSelectWarps), kSelectWarps * 32, 0, stream>>>(
+        dump, batch, p.sch, k, id_base, top_val, top_idx, redo, targets, hit_pos);
+  } else {
+    score_select_wide_kernel<<<(unsigned)batch, kWideThreads, 0, stream>>>(dump, batch, p.sch, k, id_base, top_val,
+                                                                            top_idx, redo, targets, hit_pos);
+  }
   ETPGT_CHECK_LAUNCH("score_select");
   if (stats) cudaEventRecord(ev[2], stream);
-  const size_t redo_smem = ((size_t)dim + (size_t)kRedoThreads * k * 2) * sizeof(float) +
-                           (use_excl ? (size_t)excl.width * sizeof(int64_t) : 0);
-  const int64_t redo_blocks = (batch + kRedoThreads - 1) / kRedoThreads;
-  const unsigned redo_grid = (unsigned)(redo_blocks < 2 * kNumSMs ? redo_blocks : 2 * kNumSMs);
-  if (use_excl) {
-    if (redo_smem > 48 * 1024)
-      cudaFuncSetAttribute(score_redo_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)redo_smem);
-    score_redo_kernel<true><<<redo_grid, kRedoThreads, redo_smem, stream>>>(
-        static_cast<const __nv_bfloat16*>(sess_bf16), static_cast<const __nv_bfloat16*>(table_bf16), batch,
-        num_items, dim, k, id_base, redo, top_val, top_idx, targets, hit_pos, excl);
+  if (k > kMaxKNarrow) {
+    const size_t wide_smem = (use_excl ? (size_t)excl.width * sizeof(int64_t) : 0) + (size_t)dim * sizeof(float);
+    const unsigned wide_grid = (unsigned)(batch < 4 * kNumSMs ? batch : 4 * kNumSMs);
+    if (use_excl) {
+      if (wide_smem > 16 * 1024)
+        cudaFuncSetAttribute(score_redo_wide_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wide_smem);
+      score_redo_wide_kernel<true><<<wide_grid, kWideThreads, wide_smem, stream>>>(
+          static_cast<const __nv_bfloat16*>(sess_bf16), static_cast<const __nv_bfloat16*>(table_bf16), batch,
+          num_items, dim, k, id_base, redo, top_val, top_idx, targets, hit_pos, excl);
+    } else {
+      score_redo_wide_kernel<false><<<wide_grid, kWideThreads, wide_smem, stream>>>(
+          static_cast<const __nv_bfloat16*>(sess_bf16), static_cast<const __nv_bfloat16*>(table_bf16), batch,
+          num_items, dim, k, id_base, redo, top_val, top_idx, targets, hit_pos, excl);
+    }
+    ETPGT_CHECK_LAUNCH("score_redo_wide");
   } else {
-    if (redo_smem > 48 * 1024)
-      cudaFuncSetAttribute(score_redo_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)redo_smem);
-    score_redo_kernel<false><<<redo_grid, kRedoThreads, redo_smem, stream>>>(
-        static_cast<const __nv_bfloat16*>(sess_bf16), static_cast<const __nv_bfloat16*>(table_bf16), batch,
-        num_items, dim, k, id_base, redo, top_val, top_idx, targets, hit_pos, excl);
+    const size_t redo_smem = ((size_t)dim + (size_t)kRedoThreads * k * 2) * sizeof(float) +
+                             (use_excl ? (size_t)excl.width * sizeof(int64_t) : 0);
+    const int64_t redo_blocks = (batch + kRedoThreads - 1) / kRedoThreads;
+    const unsigned redo_grid = (unsigned)(redo_blocks < 2 * kNumSMs ? redo_blocks : 2 * kNumSMs);
+    if (use_excl) {
+      if (redo_smem > 48 * 1024)
+        cudaFuncSetAttribute(score_redo_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)redo_smem);
+      score_redo_kernel<true><<<redo_grid, kRedoThreads, redo_smem, stream>>>(
+          static_cast<const __nv_bfloat16*>(sess_bf16), static_cast<const __nv_bfloat16*>(table_bf16), batch,
+          num_items, dim, k, id_base, redo, top_val, top_idx, targets, hit_pos, excl);
+    } else {
+      if (redo_smem > 48 * 1024)
+        cudaFuncSetAttribute(score_redo_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)redo_smem);
+      score_redo_kernel<false><<<redo_grid, kRedoThreads, redo_smem, stream>>>(
+          static_cast<const __nv_bfloat16*>(sess_bf16), static_cast<const __nv_bfloat16*>(table_bf16), batch,
+          num_items, dim, k, id_base, redo, top_val, top_idx, targets, hit_pos, excl);
+    }
+    ETPGT_CHECK_LAUNCH("score_redo");
   }
-  ETPGT_CHECK_LAUNCH("score_redo");
+  if (stats) cudaEventRecord(ev[3], stream);
   if (stats) {   // dump volume, fallback rows, kernel times
     std::vector<int32_t> h_redo(batch), h_count(kColParts * units);
     cudaStreamSynchronize(stream);
-    float ms_dump = 0.f, ms_select = 0.f;
+    float ms_dump = 0.f, ms_select = 0.f, ms_redo = 0.f;
     cudaEventElapsedTime(&ms_dump, ev[0], ev[1]);
     cudaEventElapsedTime(&ms_select, ev[1], ev[2]);
+    cudaEventElapsedTime(&ms_redo, ev[2], ev[3]);
     for (auto& e : ev) cudaEventDestroy(e);
-    fprintf(stderr, "score_topk_bf16: dump %.3f ms, select %.3f ms\n", ms_dump, ms_select);
+    fprintf(stderr, "score_topk_bf16: dump %.3f ms, select %.3f ms, fallback %.3f ms\n", ms_dump, ms_select, ms_redo);
     cudaMemcpy(h_redo.data(), redo, batch * sizeof(int32_t), cudaMemcpyDeviceToHost);
     cudaMemcpy(h_count.data(), dump.count, kColParts * units * sizeof(int32_t), cudaMemcpyDeviceToHost);
     int64_t redo_rows = 0, pieces = 0, worst = 0;

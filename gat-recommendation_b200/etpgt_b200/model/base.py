@@ -41,10 +41,9 @@ class BaseRecommendationModel(nn.Module, ABC):
         reference's offline predict (base.py:73-76).  exclude_sorted: rows already ascending (skips a sort)."""
         precision = self.score_precision
         if precision == "auto":
-            # small batches: fp32 CUDA-core scorer (the reference's arithmetic); evaluation-sized batches:
+            # small batches: fp32 CUDA-core scorer (the reference's arithmetic); evaluation-sized batches and k > 64:
             # tcgen05 bf16 scorer (BASELINE.json: bf16 GEMM within 1e-2, ties to the lower id)
-            big = session_embeddings.size(0) >= 64
-            precision = "bf16" if big and ops.tensor_core_scoring_supported(session_embeddings.size(1), k) else "fp32"
+            precision = ops.auto_score_precision(session_embeddings.size(0), session_embeddings.size(1), k)
         _, top = ops.score_topk(session_embeddings, self.get_item_embeddings(), k, precision=precision,
                                 exclude=exclude_items, exclude_sorted=exclude_sorted)
         return top

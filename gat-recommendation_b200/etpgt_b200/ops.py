@@ -1652,8 +1652,41 @@ def to_bf16(t: torch.Tensor) -> torch.Tensor:
     return dst
 
 
+SCORE_MAX_K = 256        # ETPGT_SCORE_MAX_K: the tensor-core scorer and the merges
+SCORE_F32_MAX_K = 64     # the fp32 CUDA-core scorer
+_SCORE_WS_BUDGET = 4 << 30   # bf16 workspace per call for k > 32: larger batches are scored in row chunks
+
+
+def score_row_chunks(batch: int, items: int, k: int, budget: int = _SCORE_WS_BUDGET) -> tuple[int, int]:
+    """(rows per call, workspace bytes) of the bf16 scorer.  For k > 32 the workspace holds a slot for every 16-item
+    piece of a row, so the batch is halved until one call's workspace fits `budget` (a single row may still exceed
+    it).  The workspace is the larger of the full chunks' and the last chunk's need: the library's sizing is not
+    monotone in the row count (the split plan depends on it).  k <= 32: one call for the whole batch."""
+    def need(n):
+        return size("etpgt_score_topk_bf16_workspace_bytes", n, items, k)
+
+    rows = batch
+    if k > 32:
+        while rows > 1 and need(rows) > budget:
+            rows = (rows + 1) // 2
+    ws = need(max(rows, 0))
+    last = batch - (batch - 1) // rows * rows if batch > rows else rows
+    if last != rows:
+        ws = max(ws, need(last))
+    return rows, ws
+
+
 def tensor_core_scoring_supported(dim: int, k: int) -> bool:
-    return dim in (64, 128, 192, 256) and 1 <= k <= 32
+    return dim in (64, 128, 192, 256) and 1 <= k <= SCORE_MAX_K
+
+
+def auto_score_precision(batch: int, dim: int, k: int) -> str:
+    """The scorer `precision="auto"` picks (predict, sharded_predict): for k <= 32, the tensor-core scorer from 64 rows
+    on and the fp32 CUDA-core scorer (the reference's arithmetic) below; for 33 <= k <= 64 the fp32 scorer; above 64
+    the tensor-core scorer at every batch size, the only one there."""
+    if k > SCORE_F32_MAX_K and tensor_core_scoring_supported(dim, k):
+        return "bf16"
+    return "bf16" if batch >= 64 and k <= 32 and tensor_core_scoring_supported(dim, k) else "fp32"
 
 
 def _exclusion_rows(exclude: torch.Tensor, b: int, dev, rows_sorted: bool) -> torch.Tensor:
@@ -1702,21 +1735,31 @@ def score_topk(sess: torch.Tensor, table: torch.Tensor, k: int, id_base: int = 0
         top_idx = torch.empty(b, k, dtype=torch.int64, device=dev)
     if precision == "bf16":
         sess_h, table_h = to_bf16(sess), to_bf16(table)
-        ws = workspace(size("etpgt_score_topk_bf16_workspace_bytes", b, items, k), dev)
+        rows, ws_bytes = score_row_chunks(b, items, k)
+        ws = workspace(ws_bytes, dev)
         hit_pos = None
         if targets is not None:
             targets = _i64(targets)
             hit_pos = torch.empty(b, dtype=torch.int32, device=dev)
-        if exclude is None:
-            call("etpgt_score_topk_bf16_eval", ptr(sess_h), ptr(table_h), b, items, dim, k, id_base, ptr(top_val),
-                 ptr(top_idx), ptr(targets), ptr(hit_pos), ptr(ws), ws.numel(), stream())
-        else:
-            call("etpgt_score_topk_bf16_exclude", ptr(sess_h), ptr(table_h), b, items, dim, k, id_base, ptr(top_val),
-                 ptr(top_idx), ptr(targets), ptr(hit_pos), ptr(exclude), exclude.size(1), ptr(ws), ws.numel(),
-                 stream())
+        for r0 in range(0, b, rows) if b > 0 else [0]:   # rows == b == 0: one call that checks the arguments
+            n = min(rows, b - r0)
+            s_h = sess_h[r0:r0 + n]
+            tv, ti = top_val[r0:r0 + n], top_idx[r0:r0 + n]
+            tg = targets[r0:r0 + n] if targets is not None else None
+            hp = hit_pos[r0:r0 + n] if hit_pos is not None else None
+            if exclude is None:
+                call("etpgt_score_topk_bf16_eval", ptr(s_h), ptr(table_h), n, items, dim, k, id_base, ptr(tv),
+                     ptr(ti), ptr(tg), ptr(hp), ptr(ws), ws.numel(), stream())
+            else:
+                call("etpgt_score_topk_bf16_exclude", ptr(s_h), ptr(table_h), n, items, dim, k, id_base, ptr(tv),
+                     ptr(ti), ptr(tg), ptr(hp), ptr(exclude[r0:r0 + n]), exclude.size(1), ptr(ws), ws.numel(),
+                     stream())
         return (top_val, top_idx) if targets is None else (top_val, top_idx, hit_pos)
     if precision != "fp32":
         raise ValueError(f"Unknown scoring precision: {precision}")
+    if k > SCORE_F32_MAX_K:
+        raise RuntimeError(f"score_topk: k={k} exceeds the fp32 scorer's bound of {SCORE_F32_MAX_K}; "
+                         f'precision="bf16" takes k <= {SCORE_MAX_K}')
     sess_c, table_c = _f32(sess.detach()), _f32(table.detach())
     ws = workspace(size("etpgt_score_topk_workspace_bytes", b, items, dim, k), dev)
     if exclude is None:

@@ -125,7 +125,7 @@ def sharded_predict(model, session_embeddings: torch.Tensor, k: int = 20, group=
         precision = getattr(model, "score_precision", "auto")
     if size == 1:
         if precision == "auto":
-            precision = "bf16" if b_local >= 64 and ops.tensor_core_scoring_supported(width, k) else "fp32"
+            precision = ops.auto_score_precision(b_local, width, k)
         if targets is None:
             return ops.score_topk(session_embeddings, table, k, precision=precision, exclude=exclude,
                                   exclude_sorted=exclude_sorted)[1]
@@ -160,7 +160,7 @@ def sharded_predict(model, session_embeddings: torch.Tensor, k: int = 20, group=
         if not exclude_sorted:   # sorted once here rather than by every scoring call below
             everyone_ex = torch.sort(everyone_ex, dim=1).values
     if precision == "auto":
-        precision = "bf16" if total >= 64 and ops.tensor_core_scoring_supported(width, k) else "fp32"
+        precision = ops.auto_score_precision(total, width, k)
     # this rank's candidates for ALL sessions, packed as one block: val [total, k] f32 | idx [total, k] i64
     lo, hi = item_shard(table.size(0), rank, size)
     kk = min(k, hi - lo)

@@ -149,7 +149,11 @@ class Trainer:
     @torch.no_grad()
     def evaluate(self) -> dict:
         self.model.eval()
-        k_max = max(self.k_values)
+        # k <= 64 and k > 64 are ranked by separate calls: "auto" may pick another scorer for k > 64 (the fp32 CUDA-core
+        # scorer stops at 64), and a deep k must not change recall@20, the early-stopping metric, on any batch
+        shallow = [k for k in self.k_values if k <= ops.SCORE_F32_MAX_K]
+        deep = [k for k in self.k_values if k > ops.SCORE_F32_MAX_K]
+        depths = [max(group) for group in (shallow, deep) if group]
         # [hits, ndcg] per k, then the session count: ONE tensor, so that data parallelism sums it in one collective
         acc = torch.zeros(2 * len(self.k_values) + 1, dtype=torch.float64, device=self.device)
         sessions = 0
@@ -166,19 +170,20 @@ class Trainer:
                 counts = getattr(batch, "rank_sessions", None)
                 if exclude is not None and width is None:
                     counts = None              # the ranks' list widths differ: exchanged with the counts
-                _, hit = parallel.sharded_predict(self.model, sess, k=k_max, group=self._group, counts=counts,
-                                                  targets=batch.target_item, exclude=exclude, exclude_sorted=True)
+                hits = [parallel.sharded_predict(self.model, sess, k=d, group=self._group, counts=counts,
+                                                 targets=batch.target_item, exclude=exclude, exclude_sorted=True)[1]
+                        for d in depths]
                 if getattr(batch, "replicated", False) and self._rank != 0:
                     continue                   # every rank holds the same sessions: counted once
                 for j, k in enumerate(self.k_values):
-                    ops.hit_metrics(hit, k, acc[2 * j:2 * j + 2])
+                    ops.hit_metrics(hits[0 if k <= depths[0] else -1], k, acc[2 * j:2 * j + 2])
             else:
                 # fused scoring + top-k; the target's position comes out of the scorer's select epilogue
                 # (group=False: this Trainer is not data parallel, even if the process has a group initialised)
-                _, hit = parallel.sharded_predict(self.model, sess, k=k_max, group=False, targets=batch.target_item,
-                                                  exclude=exclude, exclude_sorted=True)
+                hits = [parallel.sharded_predict(self.model, sess, k=d, group=False, targets=batch.target_item,
+                                                 exclude=exclude, exclude_sorted=True)[1] for d in depths]
                 for j, k in enumerate(self.k_values):
-                    ops.hit_metrics(hit, k, acc[2 * j:2 * j + 2])
+                    ops.hit_metrics(hits[0 if k <= depths[0] else -1], k, acc[2 * j:2 * j + 2])
             sessions += int(batch.target_item.shape[0])
         acc[-1] = sessions
         if self._world > 1:

@@ -538,14 +538,19 @@ int etpgt_pool_softmax_bwd_ex(const float* sess, const float* table, const int64
 
 /* ---- a9/a10: full-catalogue scoring with fused top-k and metrics ------------------------
  * etpgt/model/base.py:59-78, etpgt/utils/metrics.py:6-66.  Scores are never materialised.
- * Ties go to the lower item id.  id_base offsets the ids of an item-table shard. */
+ * Ties go to the lower item id.  id_base offsets the ids of an item-table shard.
+ * k bounds: the tensor-core scorer and both merges take 1 <= k <= ETPGT_SCORE_MAX_K; the fp32 CUDA-core scorer takes
+ * 1 <= k <= 64.  A larger k returns ETPGT_EINVAL. */
+#define ETPGT_SCORE_MAX_K 256
 size_t etpgt_score_topk_workspace_bytes(int64_t batch, int64_t num_items, int dim, int k);
 /* fp32 CUDA-core path (exact reference arithmetic, small batches). */
 int etpgt_score_topk_f32(const float* sess, const float* table, int64_t batch, int64_t num_items,
                          int dim, int k, int64_t id_base, float* top_val, int64_t* top_idx,
                          void* ws, size_t ws_bytes, etpgt_stream_t stream);
 /* Tensor-core path: bf16 operands (row-major [rows, dim], 16-byte aligned, dim in {64,128,192,256}),
- * fp32 accumulation in TMEM, tcgen05.mma fed by TMA, top-k (k <= 32) fused into the TMEM epilogue.
+ * fp32 accumulation in TMEM, tcgen05.mma fed by TMA, top-k (k <= ETPGT_SCORE_MAX_K) fused into the TMEM epilogue.
+ * The workspace grows with k: for k > 32 it holds a slot for every 16-item piece of the catalogue per session row
+ * (72 bytes per 16 items), so callers score large batches in row chunks (etpgt_b200.ops.score_topk does).
  * Oracle: fp64 scores of the bf16-rounded operands (oracle/model_ref.predict(bf16_inputs=True)). */
 int etpgt_f32_to_bf16(const float* src, void* dst_bf16, int64_t n, etpgt_stream_t stream);
 size_t etpgt_score_topk_bf16_workspace_bytes(int64_t batch, int64_t num_items, int k);

@@ -27,6 +27,21 @@
 namespace etpgt {
 namespace {
 
+// Edges per unroll group of the session-batch (sparse) variants
+template <int DIM>
+constexpr int kSparseUnroll = RowGeom<DIM>::V > 1 ? 1 : 2;
+
+// [begin, begin + deg) = the edge range of `node` in ptr (rowptr or colptr); deg = 0 past the last node
+__device__ __forceinline__ void node_range(const int32_t* __restrict__ ptr, int64_t node, int64_t num_nodes, int& begin,
+                                           int& deg) {
+  begin = 0;
+  deg = 0;
+  if (node < num_nodes) {
+    begin = ptr[node];
+    deg = ptr[node + 1] - begin;
+  }
+}
+
 // ------------------------------------------------------------------------------- forward
 // (measured on the 32,768-session batch, dim 256: four resident CTAs per SM — 64 registers — run the sparse variant
 // 12 % faster than three; the backward kernels lose more to spills than they gain from a fourth CTA)
@@ -48,12 +63,14 @@ tconv_fwd_kernel(const float* __restrict__ qkvs, int64_t num_nodes, const int32_
 
   const int64_t nrow = valid ? node : 0;
   const float* self = qkvs + nrow * 4 * DIM;
-  float4 q[V];
+  int begin, deg;
+  node_range(rowptr, node, num_nodes, begin, deg);
+  float4 q[V], xr[V];
   load_row<DIM>(self, lig, q);
-  const int begin = valid ? rowptr[nrow] : 0;
-  int deg = valid ? rowptr[nrow + 1] - begin : 0;
+  load_row<DIM>(self + 3 * DIM, lig, xr);
   const bool hub = deg > hub_threshold;   // cut into chunks by the hub kernels (tconv_hub.cu), skipped here
   if (hub) deg = 0;
+  const EdgeMeta meta = load_edge_meta(col, alpha_mask != nullptr ? eperm : nullptr, begin, deg, 0, lig);
   int deg_max = deg;
 #pragma unroll
   for (int off = 16; off > 0; off >>= 1) deg_max = max(deg_max, __shfl_xor_sync(0xffffffffu, deg_max, off));
@@ -62,8 +79,8 @@ tconv_fwd_kernel(const float* __restrict__ qkvs, int64_t num_nodes, const int32_
   float4 acc[V];
 #pragma unroll
   for (int v = 0; v < V; ++v) { m[v] = -INFINITY; l[v] = 0.f; acc[v] = zero4(); }
-  fwd_edges<DIM, HEAD_DIM, UNROLL>(qkvs, q, col, eperm, alpha_mask, begin, deg, deg_max, nrow, lig, m, l, acc);
-  fwd_epilogue<DIM, HEAD_DIM>(self, valid && !hub, nrow, lig, m, l, acc, w_beta, out, agg_out, beta_out, m_out,
+  fwd_edges<DIM, HEAD_DIM, UNROLL>(qkvs, q, col, eperm, alpha_mask, begin, deg, deg_max, nrow, lig, meta, m, l, acc);
+  fwd_epilogue<DIM, HEAD_DIM>(xr, valid && !hub, nrow, lig, m, l, acc, w_beta, out, agg_out, beta_out, m_out,
                               invl_out);
 }
 
@@ -91,7 +108,17 @@ tconv_fwd_stats_kernel(const float* __restrict__ qkvs, int64_t num_nodes, const 
   for (int v = 0; v < V; ++v)
 #pragma unroll
     for (int c = 0; c < 4; ++c) { stat_mine[4 * (v * LPN + lig) + c] = 0.0; stat_mine[DIM + 4 * (v * LPN + lig) + c] = 0.0; }
-  for (int64_t base = blockIdx.x * nodes_per_cta; base < num_nodes; base += (int64_t)gridDim.x * nodes_per_cta) {
+  // Each warp walks its nodes one ahead: the next node's edge range is loaded at the top of an iteration and the
+  // first chunk of its edge metadata after this node's edges, so neither waits on the other's loads.
+  const int64_t stride = (int64_t)gridDim.x * nodes_per_cta;
+  const int32_t* ep = alpha_mask != nullptr ? eperm : nullptr;
+  // deg = -1: a hub row (cut into chunks by the hub kernels, tconv_hub.cu, skipped here); the edge walk takes it as a
+  // row without edges
+  int begin, deg;
+  node_range(rowptr, blockIdx.x * nodes_per_cta + warp_in_cta * G::GROUPS + lane / LPN, num_nodes, begin, deg);
+  if (deg > hub_threshold) deg = -1;
+  EdgeMeta meta = load_edge_meta(col, ep, begin, deg, 0, lig);
+  for (int64_t base = blockIdx.x * nodes_per_cta; base < num_nodes; base += stride) {
     const int64_t warp_base = base + warp_in_cta * G::GROUPS;
     if (warp_base >= num_nodes) continue;  // warp-uniform
     const int64_t node = warp_base + lane / LPN;
@@ -100,10 +127,9 @@ tconv_fwd_stats_kernel(const float* __restrict__ qkvs, int64_t num_nodes, const 
     const float* self = qkvs + nrow * 4 * DIM;
     float4 q[V];
     load_row<DIM>(self, lig, q);
-    const int begin = valid ? rowptr[nrow] : 0;
-    int deg = valid ? rowptr[nrow + 1] - begin : 0;
-    const bool hub = deg > hub_threshold;
-    if (hub) deg = 0;
+    int next_begin, next_deg;
+    node_range(rowptr, node + stride, num_nodes, next_begin, next_deg);
+    if (next_deg > hub_threshold) next_deg = -1;
     int deg_max = deg;
 #pragma unroll
     for (int off = 16; off > 0; off >>= 1) deg_max = max(deg_max, __shfl_xor_sync(0xffffffffu, deg_max, off));
@@ -111,9 +137,14 @@ tconv_fwd_stats_kernel(const float* __restrict__ qkvs, int64_t num_nodes, const 
     float4 acc[V];
 #pragma unroll
     for (int v = 0; v < V; ++v) { m[v] = -INFINITY; l[v] = 0.f; acc[v] = zero4(); }
-    fwd_edges<DIM, HEAD_DIM, UNROLL>(qkvs, q, col, eperm, alpha_mask, begin, deg, deg_max, nrow, lig, m, l, acc);
-    fwd_epilogue<DIM, HEAD_DIM>(self, valid && !hub, nrow, lig, m, l, acc, w_beta, out, agg_out, beta_out, m_out,
+    fwd_edges<DIM, HEAD_DIM, UNROLL>(qkvs, q, col, eperm, alpha_mask, begin, deg, deg_max, nrow, lig, meta, m, l, acc);
+    meta = load_edge_meta(col, ep, next_begin, next_deg, 0, lig);
+    float4 xr[V];
+    load_row<DIM>(self + 3 * DIM, lig, xr);
+    fwd_epilogue<DIM, HEAD_DIM>(xr, valid && deg >= 0, nrow, lig, m, l, acc, w_beta, out, agg_out, beta_out, m_out,
                                 invl_out, stat_mine);
+    begin = next_begin;
+    deg = next_deg;
   }
   stats_flush<DIM>(stat_s, stat_partial + (size_t)blockIdx.x * 2 * DIM);
 }
@@ -131,12 +162,14 @@ __global__ void stats_reduce_kernel(const double* __restrict__ partial, int part
 }
 
 // ------------------------------------------------------------ backward, destination pass
+// LANES (session batches): edge metadata in lanes, nodes walked one ahead; else (dense graphs) the serial walk over
+// 4-edge groups, each node's edge range loaded in its own iteration (the lane walk measured slower there).
 // Per destination i: gate backward (d_agg, d_skip, w_beta partials), delta_h = <d_agg, agg>_h,
 // then over in-edges: alpha (recomputed from saved m, 1/l), d_alpha = <d_agg, v_j>_h,
 // d_logit = alpha (d_alpha*mask - delta), d_query += scale*d_logit*k_j.  Emits per-edge
 // (alpha*mask, scale*d_logit) for the source pass.
-template <int DIM, int HEAD_DIM, int UNROLL, bool COLSUM>
-__global__ void __launch_bounds__(kThreads, UNROLL <= 2 ? 3 : 2)
+template <int DIM, int HEAD_DIM, bool LANES, bool COLSUM>
+__global__ void __launch_bounds__(kThreads, LANES ? 3 : 2)
 tconv_bwd_dst_kernel(const float* __restrict__ qkvs, const float* __restrict__ d_out, int64_t num_nodes,
                      const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
                      const int32_t* __restrict__ eperm, const float* __restrict__ w_beta,
@@ -169,7 +202,19 @@ tconv_bwd_dst_kernel(const float* __restrict__ qkvs, const float* __restrict__ d
     if (COLSUM) { st4(mine + wb * DIM + 4 * f, zero4()); st4(mine + (wb + 1) * DIM + 4 * f, zero4()); }
   }
 
-  for (int64_t base = blockIdx.x * nodes_per_cta; base < num_nodes; base += (int64_t)gridDim.x * nodes_per_cta) {
+  constexpr int UNROLL = LANES ? kSparseUnroll<DIM> : kEdgeUnroll;
+  const int64_t stride = (int64_t)gridDim.x * nodes_per_cta;
+  const int32_t* ep = alpha_mask != nullptr ? eperm : nullptr;
+  // deg = -1: a hub row (edges, d_query and its column sums: the hub kernels, tconv_hub.cu); the edge walks take it
+  // as a row without edges
+  int begin = 0, deg = 0;
+  EdgeMeta meta{0, 0};
+  if constexpr (LANES) {
+    node_range(rowptr, blockIdx.x * nodes_per_cta + warp_in_cta * G::GROUPS + lane / LPN, num_nodes, begin, deg);
+    if (deg > hub_threshold) deg = -1;
+    meta = load_edge_meta(col, ep, begin, deg, 0, lig);
+  }
+  for (int64_t base = blockIdx.x * nodes_per_cta; base < num_nodes; base += stride) {
     const int64_t warp_base = base + warp_in_cta * G::GROUPS;
     if (warp_base >= num_nodes) continue;  // warp-uniform
     const int64_t node = warp_base + lane / LPN;
@@ -182,6 +227,14 @@ tconv_bwd_dst_kernel(const float* __restrict__ qkvs, const float* __restrict__ d
     load_row<DIM>(self + 3 * DIM, lig, xr);
     load_row<DIM>(agg + nrow * DIM, lig, ag);
     load_row<DIM>(self, lig, q);
+    int next_begin = 0, next_deg = 0;
+    if constexpr (LANES) {
+      node_range(rowptr, node + stride, num_nodes, next_begin, next_deg);
+    } else {
+      node_range(rowptr, node, num_nodes, begin, deg);
+      if (deg > hub_threshold) deg = -1;
+    }
+    if (next_deg > hub_threshold) next_deg = -1;
     if (w_beta != nullptr) {
       const float b = beta[nrow];
       float part = 0.f;
@@ -225,19 +278,21 @@ tconv_bwd_dst_kernel(const float* __restrict__ qkvs, const float* __restrict__ d
     }
     head_reduce<DIM, HEAD_DIM>(delta);
 
-    const int begin = valid ? rowptr[nrow] : 0;
-    int deg = valid ? rowptr[nrow + 1] - begin : 0;
-    const bool hub = deg > hub_threshold;   // edges, d_query and its column sums: the hub kernels (tconv_hub.cu)
-    if (hub) deg = 0;
     int deg_max = deg;
 #pragma unroll
     for (int off = 16; off > 0; off >>= 1) deg_max = max(deg_max, __shfl_xor_sync(0xffffffffu, deg_max, off));
     float4 dq[V];
 #pragma unroll
     for (int v = 0; v < V; ++v) dq[v] = zero4();
-    bwd_dst_edges<DIM, HEAD_DIM, UNROLL>(qkvs, q, dag, delta, mh, il, col, eperm, alpha_mask, begin, deg, deg_max, nrow,
-                                         lig, ecoef, dq);
-    if (valid && !hub) {
+    if constexpr (!LANES) {
+      bwd_dst_edges_serial<DIM, HEAD_DIM, UNROLL>(qkvs, q, dag, delta, mh, il, col, eperm, alpha_mask, begin, deg, deg_max,
+                                                  nrow, lig, ecoef, dq);
+    } else {
+      bwd_dst_edges<DIM, HEAD_DIM, UNROLL>(qkvs, q, dag, delta, mh, il, col, eperm, alpha_mask, begin, deg, deg_max, nrow,
+                                           lig, meta, ecoef, dq);
+      meta = load_edge_meta(col, ep, next_begin, next_deg, 0, lig);
+    }
+    if (valid && deg >= 0) {
 #pragma unroll
       for (int v = 0; v < V; ++v) {
         store_grad4(d_qkvs, d_hi, d_lo, nrow * 4 * DIM + 4 * (v * LPN + lig), dq[v]);
@@ -246,6 +301,10 @@ tconv_bwd_dst_kernel(const float* __restrict__ qkvs, const float* __restrict__ d
           st4(slot, add4(ld4(slot), dq[v]));
         }
       }
+    }
+    if constexpr (LANES) {
+      begin = next_begin;
+      deg = next_deg;
     }
   }
 
@@ -307,7 +366,9 @@ reduce_partials_kernel(const float* __restrict__ partial, int parts, int width, 
 // ------------------------------------------------------------------ backward, source pass
 // Per source j over its out-edges (CSC): d_key_j += scale*d_logit_e * q_i, d_value_j +=
 // alpha_e*mask_e * d_agg_i.  One owner group per row, ascending CSC order: deterministic.
-template <int DIM, int HEAD_DIM, bool COLSUM>
+// LANES (session batches): edge metadata in lanes, nodes walked one ahead; else (dense graphs) each lane group walks
+// its own edges with the serial source walk, loading its node's edge range in the node's own iteration.
+template <int DIM, int HEAD_DIM, bool LANES, bool COLSUM>
 __global__ void __launch_bounds__(kThreads, COLSUM ? 3 : 4)
 tconv_bwd_src_kernel(const float* __restrict__ qkvs, int64_t num_nodes, const int32_t* __restrict__ colptr,
                      const int32_t* __restrict__ row, const int32_t* __restrict__ cpos,
@@ -322,22 +383,57 @@ tconv_bwd_src_kernel(const float* __restrict__ qkvs, int64_t num_nodes, const in
   float4 ck[V], cv[V];   // column sums of d_key / d_value over this CTA's rows (bias gradients)
 #pragma unroll
   for (int v = 0; v < V; ++v) { ck[v] = zero4(); cv[v] = zero4(); }
-  // grid-stride over node groups: with the column sums wanted the grid is capped (a few CTAs per SM), so
-  // that only a few hundred per-CTA partials have to be reduced afterwards
-  for (int64_t base = blockIdx.x * nodes_per_cta; base < num_nodes; base += (int64_t)gridDim.x * nodes_per_cta) {
-    const int64_t node = base + (threadIdx.x >> 5) * G::GROUPS + lane / LPN;
-    if (node >= num_nodes) continue;
-    const int begin = colptr[node], end = colptr[node + 1];
-    if (end - begin > hub_threshold) continue;   // a hub source: tconv_hub.cu
-    float4 dk[V], dv[V];
-#pragma unroll
-    for (int v = 0; v < V; ++v) { dk[v] = zero4(); dv[v] = zero4(); }
-    bwd_src_edges<DIM, HEAD_DIM>(qkvs, d_agg, ecoef, row, cpos, begin, end, lig, dk, dv);
+  // the gradient rows of a non-hub source, and their column sums
+  auto finish = [&](int64_t node, const float4 (&dk)[V], const float4 (&dv)[V]) {
 #pragma unroll
     for (int v = 0; v < V; ++v) {
       store_grad4(d_qkvs, d_hi, d_lo, node * 4 * DIM + DIM + 4 * (v * LPN + lig), dk[v]);
       store_grad4(d_qkvs, d_hi, d_lo, node * 4 * DIM + 2 * DIM + 4 * (v * LPN + lig), dv[v]);
       if (COLSUM) { ck[v] = add4(ck[v], dk[v]); cv[v] = add4(cv[v], dv[v]); }
+    }
+  };
+  // grid-stride over node groups: with the column sums wanted the grid is capped (a few CTAs per SM), so
+  // that only a few hundred per-CTA partials have to be reduced afterwards
+  const int64_t stride = (int64_t)gridDim.x * nodes_per_cta;
+  if constexpr (!LANES) {
+    for (int64_t base = blockIdx.x * nodes_per_cta; base < num_nodes; base += stride) {
+      const int64_t node = base + (threadIdx.x >> 5) * G::GROUPS + lane / LPN;
+      if (node >= num_nodes) continue;
+      const int begin = colptr[node], end = colptr[node + 1];
+      if (end - begin > hub_threshold) continue;   // a hub source: tconv_hub.cu
+      float4 dk[V], dv[V];
+#pragma unroll
+      for (int v = 0; v < V; ++v) { dk[v] = zero4(); dv[v] = zero4(); }
+      bwd_src_edges_serial<DIM, HEAD_DIM>(qkvs, d_agg, ecoef, row, cpos, begin, end, lig, dk, dv);
+      finish(node, dk, dv);
+    }
+  } else {
+    int begin, deg;
+    node_range(colptr, blockIdx.x * nodes_per_cta + (threadIdx.x >> 5) * G::GROUPS + lane / LPN, num_nodes, begin, deg);
+    bool hub = deg > hub_threshold;   // a hub source: tconv_hub.cu
+    if (hub) deg = 0;
+    EdgeMeta meta = load_edge_meta(row, cpos, begin, deg, 0, lig);
+    for (int64_t base = blockIdx.x * nodes_per_cta; base < num_nodes; base += stride) {
+      const int64_t warp_base = base + (threadIdx.x >> 5) * G::GROUPS;
+      if (warp_base >= num_nodes) continue;  // warp-uniform
+      const int64_t node = warp_base + lane / LPN;
+      int next_begin, next_deg;
+      node_range(colptr, node + stride, num_nodes, next_begin, next_deg);
+      const bool next_hub = next_deg > hub_threshold;
+      if (next_hub) next_deg = 0;
+      int deg_max = deg;
+#pragma unroll
+      for (int off = 16; off > 0; off >>= 1) deg_max = max(deg_max, __shfl_xor_sync(0xffffffffu, deg_max, off));
+      float4 dk[V], dv[V];
+#pragma unroll
+      for (int v = 0; v < V; ++v) { dk[v] = zero4(); dv[v] = zero4(); }
+      bwd_src_edges<DIM, HEAD_DIM, kSparseUnroll<DIM>>(qkvs, d_agg, ecoef, row, cpos, begin, deg, deg_max, lig, meta, dk,
+                                                       dv);
+      meta = load_edge_meta(row, cpos, next_begin, next_deg, 0, lig);
+      if (node < num_nodes && !hub) finish(node, dk, dv);
+      begin = next_begin;
+      deg = next_deg;
+      hub = next_hub;
     }
   }
   if (COLSUM) {
@@ -415,13 +511,13 @@ static int tconv_fwd_impl(const float* qkvs, int64_t num_nodes, int dim, int hea
       parts = grid_for(num_nodes, (int)npc, sparse ? kStatCtasPerSm : 2);                        \
       const size_t smem = (size_t)npc * 2 * D * sizeof(double);                                  \
       if (sparse)                                                                                \
-        tconv_fwd_stats_kernel<D, C, 2><<<parts, kThreads, smem, stream>>>(qkvs, num_nodes, rowptr, col, eperm, w_beta, \
+        tconv_fwd_stats_kernel<D, C, kSparseUnroll<D>><<<parts, kThreads, smem, stream>>>(qkvs, num_nodes, rowptr, col, eperm, w_beta, \
                                             alpha_mask, out, agg, beta, m, inv_l, hub_threshold, stat_partial); \
       else                                                                                       \
         tconv_fwd_stats_kernel<D, C, 4><<<parts, kThreads, smem, stream>>>(qkvs, num_nodes, rowptr, col, eperm, w_beta, \
                                             alpha_mask, out, agg, beta, m, inv_l, hub_threshold, stat_partial); \
     } else if (sparse)                                                                           \
-      tconv_fwd_kernel<D, C, 2><<<(unsigned)grid, kThreads, 0, stream>>>(qkvs, num_nodes, rowptr, col, eperm,   \
+      tconv_fwd_kernel<D, C, kSparseUnroll<D>><<<(unsigned)grid, kThreads, 0, stream>>>(qkvs, num_nodes, rowptr, col, eperm,   \
                                                           w_beta, alpha_mask, out, agg, beta, m, inv_l, hub_threshold); \
     else                                                                                         \
       tconv_fwd_kernel<D, C, 4><<<(unsigned)grid, kThreads, 0, stream>>>(qkvs, num_nodes, rowptr, col, eperm,   \
@@ -520,8 +616,8 @@ extern "C" int etpgt_tconv_bwd_split_hub(const float* qkvs, const float* d_out, 
     const int npc = (kThreads / 32) * RowGeom<D>::GROUPS;                                            \
     grid_a = dst_pass_grid(num_nodes, npc, sparse);                                                        \
     const size_t smem = (size_t)npc * width * sizeof(float);                                         \
-    auto kern = sparse ? (want_colsum ? tconv_bwd_dst_kernel<D, C, 2, true> : tconv_bwd_dst_kernel<D, C, 2, false>) \
-                       : (want_colsum ? tconv_bwd_dst_kernel<D, C, 4, true> : tconv_bwd_dst_kernel<D, C, 4, false>); \
+    auto kern = sparse ? (want_colsum ? tconv_bwd_dst_kernel<D, C, true, true> : tconv_bwd_dst_kernel<D, C, true, false>) \
+                       : (want_colsum ? tconv_bwd_dst_kernel<D, C, false, true> : tconv_bwd_dst_kernel<D, C, false, false>); \
     kern<<<grid_a, kThreads, smem, stream>>>(qkvs, d_out, num_nodes, rowptr, col, eperm, w_beta, alpha_mask, agg,    \
                                              beta, m, inv_l, d_qkvs, d_hi, d_lo, d_agg, ecoef, partial, hub_threshold); \
   }
@@ -550,7 +646,8 @@ extern "C" int etpgt_tconv_bwd_split_hub(const float* qkvs, const float* d_out, 
     grid_src = (num_nodes + npc - 1) / npc;                                                         \
     if (want_colsum && grid_src > 8 * kNumSMs) grid_src = 8 * kNumSMs;                              \
     const size_t smem = want_colsum ? (size_t)npc * 2 * D * sizeof(float) : 0;                      \
-    auto kern = want_colsum ? tconv_bwd_src_kernel<D, C, true> : tconv_bwd_src_kernel<D, C, false>; \
+    auto kern = sparse ? (want_colsum ? tconv_bwd_src_kernel<D, C, true, true> : tconv_bwd_src_kernel<D, C, true, false>) \
+                       : (want_colsum ? tconv_bwd_src_kernel<D, C, false, true> : tconv_bwd_src_kernel<D, C, false, false>); \
     kern<<<(unsigned)grid_src, kThreads, smem, stream>>>(qkvs, num_nodes, colptr, row, cpos, d_agg, ecoef, d_qkvs, \
                                                          d_hi, d_lo, src_partial, hub_threshold);   \
   }

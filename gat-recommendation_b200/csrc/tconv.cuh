@@ -45,28 +45,58 @@ __device__ __forceinline__ void store_grad4(float* __restrict__ d_f32, __nv_bflo
 
 // ---- the edge walks and the node epilogue, shared by the row kernels (tconv.cu) and the hub kernels (tconv_hub.cu)
 
+// Edge metadata of one chunk of LPN edges of a lane group's row: lane `lig` of the group holds edge c0 + lig (`a` =
+// col / row, `b` = eperm / cpos; `b` stays 0 when its array is NULL), loaded in one coalesced step.  The walks take an
+// edge's indices from the lane that holds them (__shfl_sync), so the gathers of an unroll group wait on no index load;
+// a row of more than LPN edges loads its further chunks as the walk reaches them.  The persistent kernels load chunk 0
+// of a node's row while the previous node computes.
+struct EdgeMeta { int32_t a, b; };
+__device__ __forceinline__ EdgeMeta load_edge_meta(const int32_t* __restrict__ a, const int32_t* __restrict__ b,
+                                                   int begin, int count, int c0, int lig) {
+  EdgeMeta e{0, 0};
+  if (c0 + lig < count) {
+    e.a = a[begin + c0 + lig];
+    if (b != nullptr) e.b = b[begin + c0 + lig];
+  }
+  return e;
+}
+// lane of this lane group that holds edge k of the current chunk
+template <int DIM>
+__device__ __forceinline__ int meta_lane(int k) { return ((threadIdx.x & 31) & ~(RowGeom<DIM>::LPN - 1)) + k; }
+
 // Forward: one-pass online softmax over `count` in-edges starting at CSR position `begin` (count_max = the
 // warp-uniform loop bound: the head reductions are warp shuffles).  m / l / acc are carried in and out.
+// meta: chunk 0 of the row, load_edge_meta(col, alpha_mask ? eperm : NULL, begin, count, 0, lig).  The attention-mask
+// value of an edge is loaded through its eperm together with the edge's key / value rows.
 template <int DIM, int HEAD_DIM, int UNROLL>
 __device__ __forceinline__ void fwd_edges(const float* __restrict__ qkvs, const float4 (&q)[RowGeom<DIM>::V],
                                           const int32_t* __restrict__ col, const int32_t* __restrict__ eperm,
                                           const float* __restrict__ alpha_mask, int begin, int count, int count_max,
-                                          int64_t idle_row, int lig, float (&m)[RowGeom<DIM>::V],
+                                          int64_t idle_row, int lig, EdgeMeta meta, float (&m)[RowGeom<DIM>::V],
                                           float (&l)[RowGeom<DIM>::V], float4 (&acc)[RowGeom<DIM>::V]) {
-  constexpr int V = RowGeom<DIM>::V;
+  constexpr int V = RowGeom<DIM>::V, LPN = RowGeom<DIM>::LPN;
   constexpr int HEADS = DIM / HEAD_DIM;
+  static_assert(LPN % UNROLL == 0, "an unroll group must not straddle two metadata chunks");
   const float scale = rsqrtf((float)HEAD_DIM);
   for (int e0 = 0; e0 < count_max; e0 += UNROLL) {
+    const int c0 = e0 & ~(LPN - 1);
+    if (e0 == c0 && c0 > 0) meta = load_edge_meta(col, alpha_mask != nullptr ? eperm : nullptr, begin, count, c0, lig);
     float4 kr[UNROLL][V], vr[UNROLL][V];
-    int pos[UNROLL];
+    float mk[UNROLL][V];
+    bool on[UNROLL];
 #pragma unroll
     for (int u = 0; u < UNROLL; ++u) {
-      const bool on = e0 + u < count;
-      pos[u] = on ? begin + e0 + u : -1;
-      const int64_t j = on ? col[pos[u]] : idle_row;
+      on[u] = e0 + u < count;
+      const int j32 = __shfl_sync(0xffffffffu, meta.a, meta_lane<DIM>(e0 - c0 + u));
+      const int64_t j = on[u] ? j32 : idle_row;
       const float* other = qkvs + j * 4 * DIM;
       load_row<DIM>(other + DIM, lig, kr[u]);
       load_row<DIM>(other + 2 * DIM, lig, vr[u]);
+      if (alpha_mask != nullptr) {
+        const int64_t ep = __shfl_sync(0xffffffffu, meta.b, meta_lane<DIM>(e0 - c0 + u));
+#pragma unroll
+        for (int v = 0; v < V; ++v) mk[u][v] = on[u] ? alpha_mask[ep * HEADS + head_of<DIM, HEAD_DIM>(v, lig)] : 0.f;
+      }
     }
 #pragma unroll
     for (int u = 0; u < UNROLL; ++u) {
@@ -74,7 +104,7 @@ __device__ __forceinline__ void fwd_edges(const float* __restrict__ qkvs, const 
 #pragma unroll
       for (int v = 0; v < V; ++v) a[v] = dot4(q[v], kr[u][v]);
       head_reduce<DIM, HEAD_DIM>(a);
-      if (pos[u] >= 0) {
+      if (on[u]) {
 #pragma unroll
         for (int v = 0; v < V; ++v) {
           const float logit = a[v] * scale;
@@ -82,8 +112,7 @@ __device__ __forceinline__ void fwd_edges(const float* __restrict__ qkvs, const 
           const float corr = expf(m[v] - m_new);
           float p = expf(logit - m_new);
           l[v] = l[v] * corr + p;
-          if (alpha_mask != nullptr)
-            p *= alpha_mask[(int64_t)eperm[pos[u]] * HEADS + head_of<DIM, HEAD_DIM>(v, lig)];
+          if (alpha_mask != nullptr) p *= mk[u][v];
           acc[v] = fma4(p, vr[u][v], scale4(corr, acc[v]));
           m[v] = m_new;
         }
@@ -92,13 +121,13 @@ __device__ __forceinline__ void fwd_edges(const float* __restrict__ qkvs, const 
   }
 }
 
-// Forward node epilogue: agg = acc / (l + eps), gate beta = sigmoid(w . [agg, x_r, agg - x_r]), out = beta x_r +
-// (1 - beta) agg; saves agg, beta, m, 1/l.  Every lane of the warp must call it (group_sum shuffles); `store`
+// Forward node epilogue, given the node's skip row xr: agg = acc / (l + eps), gate beta = sigmoid(w . [agg, x_r,
+// agg - x_r]), out = beta x_r + (1 - beta) agg; saves agg, beta, m, 1/l.  Every lane of the warp must call it (group_sum shuffles); `store`
 // says whether this lane group owns a row.
 // `stats` (or NULL): this lane group's running column sums in shared memory, [sum o | sum o^2] as 2*DIM doubles (each
 // lane owns its own slots): the BatchNorm statistics of the layer output, taken while the row is still in registers.
 template <int DIM, int HEAD_DIM>
-__device__ __forceinline__ void fwd_epilogue(const float* __restrict__ self, bool store, int64_t nrow, int lig,
+__device__ __forceinline__ void fwd_epilogue(const float4 (&xr)[RowGeom<DIM>::V], bool store, int64_t nrow, int lig,
                                              const float (&m)[RowGeom<DIM>::V], const float (&l)[RowGeom<DIM>::V],
                                              const float4 (&acc)[RowGeom<DIM>::V], const float* __restrict__ w_beta,
                                              float* __restrict__ out, float* __restrict__ agg_out,
@@ -108,8 +137,7 @@ __device__ __forceinline__ void fwd_epilogue(const float* __restrict__ self, boo
   constexpr int V = G::V, LPN = G::LPN;
   constexpr int HEADS = DIM / HEAD_DIM;
   constexpr int HEAD_F4 = HEAD_DIM / 4;
-  float4 xr[V], ag[V];
-  load_row<DIM>(self + 3 * DIM, lig, xr);
+  float4 ag[V];
   float zpart = 0.f;
 #pragma unroll
   for (int v = 0; v < V; ++v) {
@@ -162,11 +190,12 @@ __device__ __forceinline__ void stats_flush(const double* __restrict__ smem_stat
   }
 }
 
-// Backward, destination side: over `count` in-edges of destination i starting at CSR position `begin`:
+// Backward, destination side, one lane group per destination loading its edge indices as it goes: the dense-graph
+// destination pass and the hub chunks, where the metadata-in-lanes walk below measured slower.  Over `count` in-edges of destination i starting at CSR position `begin`:
 // alpha (recomputed from the saved m, 1/l), d_alpha = <d_agg_i, v_j>_h, d_logit = alpha (d_alpha mask - delta),
 // dq += scale d_logit k_j; emits per-edge (alpha mask, scale d_logit) for the source pass.
 template <int DIM, int HEAD_DIM, int UNROLL>
-__device__ __forceinline__ void bwd_dst_edges(const float* __restrict__ qkvs, const float4 (&q)[RowGeom<DIM>::V],
+__device__ __forceinline__ void bwd_dst_edges_serial(const float* __restrict__ qkvs, const float4 (&q)[RowGeom<DIM>::V],
                                               const float4 (&dag)[RowGeom<DIM>::V],
                                               const float (&delta)[RowGeom<DIM>::V], const float (&mh)[RowGeom<DIM>::V],
                                               const float (&il)[RowGeom<DIM>::V], const int32_t* __restrict__ col,
@@ -212,13 +241,77 @@ __device__ __forceinline__ void bwd_dst_edges(const float* __restrict__ qkvs, co
   }
 }
 
-// Backward, source side: over CSC positions [p0, p1) of source j: dk += scale d_logit_e q_i, dv += alpha_e mask_e
-// d_agg_i (coefficients written by the destination pass in CSR order, found through cpos).
+// Backward, destination side, session batches: over `count` in-edges of destination i starting at CSR position `begin`:
+// alpha (recomputed from the saved m, 1/l), d_alpha = <d_agg_i, v_j>_h, d_logit = alpha (d_alpha mask - delta),
+// dq += scale d_logit k_j; emits per-edge (alpha mask, scale d_logit) for the source pass.
+// meta: chunk 0 of the row, as for fwd_edges.
+template <int DIM, int HEAD_DIM, int UNROLL>
+__device__ __forceinline__ void bwd_dst_edges(const float* __restrict__ qkvs, const float4 (&q)[RowGeom<DIM>::V],
+                                              const float4 (&dag)[RowGeom<DIM>::V],
+                                              const float (&delta)[RowGeom<DIM>::V], const float (&mh)[RowGeom<DIM>::V],
+                                              const float (&il)[RowGeom<DIM>::V], const int32_t* __restrict__ col,
+                                              const int32_t* __restrict__ eperm, const float* __restrict__ alpha_mask,
+                                              int begin, int count, int count_max, int64_t idle_row, int lig,
+                                              EdgeMeta meta, float2* __restrict__ ecoef, float4 (&dq)[RowGeom<DIM>::V]) {
+  constexpr int V = RowGeom<DIM>::V, LPN = RowGeom<DIM>::LPN;
+  constexpr int HEADS = DIM / HEAD_DIM;
+  constexpr int HEAD_F4 = HEAD_DIM / 4;
+  static_assert(LPN % UNROLL == 0, "an unroll group must not straddle two metadata chunks");
+  const float scale = rsqrtf((float)HEAD_DIM);
+  for (int c0 = 0; c0 < count_max; c0 += LPN) {
+    if (c0 > 0) meta = load_edge_meta(col, alpha_mask != nullptr ? eperm : nullptr, begin, count, c0, lig);
+    const int c_end = min(c0 + LPN, count_max);
+    for (int e0 = c0; e0 < c_end; e0 += UNROLL) {
+      float4 kr[UNROLL][V], vr[UNROLL][V];
+      float mk[UNROLL][V];
+      bool on[UNROLL];
+#pragma unroll
+      for (int u = 0; u < UNROLL; ++u) {
+        on[u] = e0 + u < count;
+        const int j32 = __shfl_sync(0xffffffffu, meta.a, meta_lane<DIM>(e0 - c0 + u));
+        const int64_t j = on[u] ? j32 : idle_row;
+        const float* other = qkvs + j * 4 * DIM;
+        load_row<DIM>(other + DIM, lig, kr[u]);
+        load_row<DIM>(other + 2 * DIM, lig, vr[u]);
+        if (alpha_mask != nullptr) {
+          const int64_t ep = __shfl_sync(0xffffffffu, meta.b, meta_lane<DIM>(e0 - c0 + u));
+#pragma unroll
+          for (int v = 0; v < V; ++v) mk[u][v] = on[u] ? alpha_mask[ep * HEADS + head_of<DIM, HEAD_DIM>(v, lig)] : 0.f;
+        }
+      }
+#pragma unroll
+      for (int u = 0; u < UNROLL; ++u) {
+        float a[V], da[V];
+#pragma unroll
+        for (int v = 0; v < V; ++v) { a[v] = dot4(q[v], kr[u][v]); da[v] = dot4(dag[v], vr[u][v]); }
+        head_reduce<DIM, HEAD_DIM>(a);
+        head_reduce<DIM, HEAD_DIM>(da);
+        if (on[u]) {
+#pragma unroll
+          for (int v = 0; v < V; ++v) {
+            const float alpha = expf(a[v] * scale - mh[v]) * il[v];
+            const float mask = alpha_mask != nullptr ? mk[u][v] : 1.f;
+            const int h = head_of<DIM, HEAD_DIM>(v, lig);
+            const float dlogit = alpha * (da[v] * mask - delta[v]) * scale;
+            dq[v] = fma4(dlogit, kr[u][v], dq[v]);
+            if ((v * LPN + lig) % HEAD_F4 == 0)
+              ecoef[(int64_t)(begin + e0 + u) * HEADS + h] = make_float2(alpha * mask, dlogit);
+          }
+        }
+      }
+    }
+  }
+}
+
+// Backward, source side, one lane group per source walking its own edges (no shuffles, no warp-uniform bound): the
+// dense-graph source pass and the hub chunks, where the metadata-in-lanes walk below measured slower (on dense rows
+// its registers cost a resident CTA).  Over CSC positions [p0, p1) of source j: dk += scale d_logit_e q_i,
+// dv += alpha_e mask_e d_agg_i (coefficients written by the destination pass in CSR order, found through cpos).
 template <int DIM, int HEAD_DIM>
-__device__ __forceinline__ void bwd_src_edges(const float* __restrict__ qkvs, const float* __restrict__ d_agg,
-                                              const float2* __restrict__ ecoef, const int32_t* __restrict__ row,
-                                              const int32_t* __restrict__ cpos, int p_begin, int p_end, int lig,
-                                              float4 (&dk)[RowGeom<DIM>::V], float4 (&dv)[RowGeom<DIM>::V]) {
+__device__ __forceinline__ void bwd_src_edges_serial(const float* __restrict__ qkvs, const float* __restrict__ d_agg,
+                                                     const float2* __restrict__ ecoef, const int32_t* __restrict__ row,
+                                                     const int32_t* __restrict__ cpos, int p_begin, int p_end, int lig,
+                                                     float4 (&dk)[RowGeom<DIM>::V], float4 (&dv)[RowGeom<DIM>::V]) {
   constexpr int V = RowGeom<DIM>::V;
   constexpr int HEADS = DIM / HEAD_DIM;
   for (int p0 = p_begin; p0 < p_end; p0 += kEdgeUnroll) {
@@ -244,6 +337,53 @@ __device__ __forceinline__ void bwd_src_edges(const float* __restrict__ qkvs, co
       for (int v = 0; v < V; ++v) {
         dk[v] = fma4(c[u][v].y, qr[u][v], dk[v]);
         dv[v] = fma4(c[u][v].x, gr[u][v], dv[v]);
+      }
+    }
+  }
+}
+
+// Backward, source side, session batches: over the `count` CSC positions from p_begin of source j (count_max = the warp-uniform loop
+// bound): dk += scale d_logit_e q_i, dv += alpha_e mask_e d_agg_i (coefficients written by the destination pass in
+// CSR order, found through cpos).  meta: chunk 0, load_edge_meta(row, cpos, p_begin, count, 0, lig); an edge's
+// coefficients are loaded with its q and d_agg rows.
+template <int DIM, int HEAD_DIM, int UNROLL>
+__device__ __forceinline__ void bwd_src_edges(const float* __restrict__ qkvs, const float* __restrict__ d_agg,
+                                              const float2* __restrict__ ecoef, const int32_t* __restrict__ row,
+                                              const int32_t* __restrict__ cpos, int p_begin, int count, int count_max,
+                                              int lig, EdgeMeta meta, float4 (&dk)[RowGeom<DIM>::V],
+                                              float4 (&dv)[RowGeom<DIM>::V]) {
+  constexpr int V = RowGeom<DIM>::V, LPN = RowGeom<DIM>::LPN;
+  constexpr int HEADS = DIM / HEAD_DIM;
+  static_assert(LPN % UNROLL == 0, "an unroll group must not straddle two metadata chunks");
+  for (int c0 = 0; c0 < count_max; c0 += LPN) {
+    if (c0 > 0) meta = load_edge_meta(row, cpos, p_begin, count, c0, lig);
+    const int c_end = min(c0 + LPN, count_max);
+    for (int e0 = c0; e0 < c_end; e0 += UNROLL) {
+      float4 qr[UNROLL][V], gr[UNROLL][V];
+      float2 c[UNROLL][V];
+      bool on[UNROLL];
+#pragma unroll
+      for (int u = 0; u < UNROLL; ++u) {
+        // an edge past the row's end reads row 0 and edge 0 (a lane past its node's edges holds zeros) and adds
+        // nothing: its coefficients are zero
+        on[u] = e0 + u < count;
+        const int64_t i = __shfl_sync(0xffffffffu, meta.a, meta_lane<DIM>(e0 - c0 + u));
+        const int64_t e = __shfl_sync(0xffffffffu, meta.b, meta_lane<DIM>(e0 - c0 + u));
+        load_row<DIM>(qkvs + i * 4 * DIM, lig, qr[u]);
+        load_row<DIM>(d_agg + i * DIM, lig, gr[u]);
+#pragma unroll
+        for (int v = 0; v < V; ++v) {
+          c[u][v] = ecoef[e * HEADS + head_of<DIM, HEAD_DIM>(v, lig)];
+          if (!on[u]) c[u][v] = make_float2(0.f, 0.f);
+        }
+      }
+#pragma unroll
+      for (int u = 0; u < UNROLL; ++u) {
+#pragma unroll
+        for (int v = 0; v < V; ++v) {
+          dk[v] = fma4(c[u][v].y, qr[u][v], dk[v]);
+          dv[v] = fma4(c[u][v].x, gr[u][v], dv[v]);
+        }
       }
     }
   }

@@ -95,8 +95,9 @@ tconv_fwd_hub_chunk_kernel(const float* __restrict__ qkvs, const int32_t* __rest
     float4 acc[V];
 #pragma unroll
     for (int v = 0; v < V; ++v) { m[v] = -INFINITY; l[v] = 0.f; acc[v] = zero4(); }
+    const EdgeMeta meta = load_edge_meta(col, alpha_mask != nullptr ? eperm : nullptr, ch.edge_begin + b, cnt, 0, lig);
     fwd_edges<DIM, HEAD_DIM, kEdgeUnroll>(qkvs, q, col, eperm, alpha_mask, ch.edge_begin + b, cnt, cnt_max, ch.node, lig,
-                                          m, l, acc);
+                                          meta, m, l, acc);
     float* mine = part_s + group * STRIDE;
 #pragma unroll
     for (int v = 0; v < V; ++v) {
@@ -187,7 +188,9 @@ tconv_fwd_hub_combine_kernel(const float* __restrict__ qkvs, const int32_t* __re
       }
     }
     const int64_t nrow = r.node;
-    fwd_epilogue<DIM, HEAD_DIM>(qkvs + nrow * 4 * DIM, valid, nrow, lig, m, l, acc, w_beta, out, agg_out, beta_out, m_out,
+    float4 xr[V];
+    load_row<DIM>(qkvs + nrow * 4 * DIM + 3 * DIM, lig, xr);
+    fwd_epilogue<DIM, HEAD_DIM>(xr, valid, nrow, lig, m, l, acc, w_beta, out, agg_out, beta_out, m_out,
                                 invl_out, stat_mine);
   }
   if (stat_rows != nullptr) stats_flush<DIM>(stat_s, stat_rows + (size_t)blockIdx.x * 2 * DIM);
@@ -243,8 +246,8 @@ tconv_bwd_dst_hub_chunk_kernel(const float* __restrict__ qkvs, const int32_t* __
     float4 dq[V];
 #pragma unroll
     for (int v = 0; v < V; ++v) dq[v] = zero4();
-    bwd_dst_edges<DIM, HEAD_DIM, kEdgeUnroll>(qkvs, q, dag, delta, mh, il, col, eperm, alpha_mask, ch.edge_begin + b, cnt,
-                                              cnt_max, nrow, lig, ecoef, dq);
+    bwd_dst_edges_serial<DIM, HEAD_DIM, kEdgeUnroll>(qkvs, q, dag, delta, mh, il, col, eperm, alpha_mask, ch.edge_begin + b,
+                                                     cnt, cnt_max, nrow, lig, ecoef, dq);
 #pragma unroll
     for (int v = 0; v < V; ++v) st4(part_s + group * DIM + 4 * (v * LPN + lig), dq[v]);
     __syncthreads();
@@ -353,7 +356,8 @@ tconv_bwd_src_hub_chunk_kernel(const float* __restrict__ qkvs, const int32_t* __
     float4 dk[V], dv[V];
 #pragma unroll
     for (int v = 0; v < V; ++v) { dk[v] = zero4(); dv[v] = zero4(); }
-    bwd_src_edges<DIM, HEAD_DIM>(qkvs, d_agg, ecoef, row, cpos, ch.edge_begin + b, ch.edge_begin + b + cnt, lig, dk, dv);
+    bwd_src_edges_serial<DIM, HEAD_DIM>(qkvs, d_agg, ecoef, row, cpos, ch.edge_begin + b, ch.edge_begin + b + cnt, lig,
+                                        dk, dv);
 #pragma unroll
     for (int v = 0; v < V; ++v) {
       st4(part_s + group * 2 * DIM + 4 * (v * LPN + lig), dk[v]);
